@@ -1,8 +1,13 @@
 #!/usr/bin/env python
-"""bench.py -- the driver's benchmark contract for the WHVI hot path on B200.
+"""bench.py -- the benchmark of the WHVI hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
     (N > 1: python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...)
+
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy (float32): `loss` (summed over
+the ranks), `grad.<parameter>` (the all-reduced gradient the optimiser consumed) and `param.<parameter>` (the
+parameters after its Adam update).  Inputs, parameters and noise are seeded, so two builds run with the same
+arguments can be compared output for output.
 
 Workload (BASELINE.json configs[3], the largest one that fits a single GPU): a wide WHVI
 MLP of three WHVILinear(4096, 4096) layers with ReLU between them, minibatch B = 8192,
@@ -23,7 +28,7 @@ the batched-FWHT GB/s sweep over all ranks (`fwht`), the MC predictive-evaluatio
 BASELINE config 5 over all ranks (`eval`), and -- N = 1 only -- the CPU baseline.
 
 `--impl reference`: the reference's OWN layer code (oracle/_ref/refpy, byte-compiled unmodified from
-/root/reference/src by oracle/build.py) on the host cores: each step = one MC sample of one
+the reference sources by oracle/build.py) on the host cores: each step = one MC sample of one
 WHVILinear(4096, 4096) over all 8192 rows, forward + backward.
 """
 from __future__ import annotations
@@ -230,6 +235,27 @@ def run_reference_arm(args):
     return 0
 
 
+def dump_outputs(out_dir, model, flat, loss, grad, world, rank):
+    """--dump-outputs: the last timed step's loss, its all-reduced gradient and the parameters after its update, as
+    float32 .npy files named after the parameters.  Every rank takes part in the loss all-reduce; rank 0 writes."""
+    import numpy as np
+    import torch.distributed as dist
+    loss = loss.detach().clone()
+    if world > 1:
+        dist.all_reduce(loss)
+    if rank != 0:
+        return
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "loss.npy", loss.cpu().numpy())
+    names = {id(p): name for name, p in model.named_parameters()}
+    grad, param = grad.cpu().numpy(), flat.param.cpu().numpy()
+    for p, off in zip(flat.params, flat.offsets):
+        n = p.numel()
+        np.save(out / f"grad.{names[id(p)]}.npy", grad[off:off + n].reshape(p.shape))
+        np.save(out / f"param.{names[id(p)]}.npy", param[off:off + n].reshape(p.shape))
+
+
 # --------------------------------------------------------------------------- our arm
 def run_ours(args):
     import torch
@@ -286,9 +312,11 @@ def run_ours(args):
             total = loss.detach() if total is None else total + loss.detach()
         return total
 
-    def step(x, y):
+    def step(x, y, grad_out=None):
         total = fwd_bwd(x, y)
         flat.all_reduce()  # one NCCL all-reduce on the flat gradient buffer (no-op at N = 1)
+        if grad_out is not None:  # --dump-outputs: keep the gradient that zero_grad() is about to clear
+            grad_out.copy_(flat.grad)
         opt.step()
         opt.zero_grad()
         return total
@@ -344,9 +372,18 @@ def run_ours(args):
     WF.LAUNCH_COUNTS.clear()
     timed_calls = ("whvi_layer_bwd_fused_f32", "whvi_layer_bwd_scaled_f32", "whvi_layer_fwd_fused_f32", "whvi_layer_loss_f32")
     WF.EVENT_SINK = {k: [] for k in timed_calls}
+    last_grad = torch.empty_like(flat.grad) if args.dump_outputs else None
+    losses = []
+
+    def timed_step():
+        final = len(losses) == args.steps - 1
+        losses.append(step(x_dev, y_dev, last_grad if final else None))
+
     with ClockSampler(local_rank) as clk:
-        ms_total = timed(lambda: step(x_dev, y_dev), args.steps)
+        ms_total = timed(timed_step, args.steps)
     sink, WF.EVENT_SINK = WF.EVENT_SINK, None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, model, flat, losses[-1], last_grad, world, rank)
     launches = sum(WF.LAUNCH_COUNTS.values())
     ms_step = ms_total / args.steps
     rows_per_step = S_TOTAL * B * N_LAYERS
@@ -506,7 +543,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eval", action="store_true")
     ap.add_argument("--eval-inputs", type=int, default=0, help="inputs of the config-5 evaluation leg (0: a bounded default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the last timed step's loss, gradient and updated parameters to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the timed steps of --impl ours")
     if args.impl == "reference":
         return run_reference_arm(args)
     if int(os.environ.get("WORLD_SIZE", "1")) == 1:
