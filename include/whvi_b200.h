@@ -179,6 +179,28 @@ WHVI_API int whvi_layer_loss_f32(const float* x, int64_t x_sample_stride, const 
                                  whvi_stream_t stream);
 
 /*
+ * Training with bf16 activations in HBM (x, dy, dx bf16; parameters, their gradients, the target, the workspace and all
+ * arithmetic fp32).  Each call is its fp32 counterpart on the widened inputs with the same plan, so
+ *   dx = bf16( dx of the fp32 call on float(x), float(dy) ), rounded once at the store, and
+ *   dg, ds1, ds2, dbias (and sq_partials) are bit-identical to the fp32 call's for float(x), float(dy).
+ * The workspace is the fp32 call's: whvi_layer_bwd_workspace_bytes / whvi_layer_loss_sizes.
+ * whvi_layer_bwd_bf16 is whvi_layer_bwd_scaled_f32 (dy_scale: device scalar, NULL = 1; flags: WHVI_LAYER_RELU_IN;
+ * D = 4 ... 8192); the saved-output + target mode of whvi_layer_bwd_fused_f32 is fp32 only.
+ * whvi_layer_loss_bf16 is whvi_layer_loss_f32 (128 <= D <= 4096; target fp32).
+ * Alignment: fp32 pointers 16 bytes; x and dy 16 bytes (they are fetched by bulk async copies), dx 8 bytes.  The bulk copies
+ * also need B * D % 8 == 0 (whole 16-byte units per sample); the only shape that breaks it, D = 4 with an odd B, is
+ * rejected with WHVI_E_SHAPE -- a caller can pad B with a zero row of x and dy, which adds zero to every gradient.
+ */
+WHVI_API int whvi_layer_bwd_bf16(const void* x, int64_t x_sample_stride, const void* dy, const float* dy_scale, const float* g,
+                                 const float* s1, const float* s2, void* dx, float* dg, float* ds1, float* ds2, float* dbias,
+                                 void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int flags,
+                                 whvi_stream_t stream);
+WHVI_API int whvi_layer_loss_bf16(const void* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2,
+                                  const float* bias, const float* target, void* dx, float* dg, float* ds1, float* ds2, float* dbias,
+                                  float* sq_partials, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D,
+                                  int flags, whvi_stream_t stream);
+
+/*
  * Reparameterisation (src/weights.py:43-50, :82-83, :92-93), one eps row per MC sample:
  *   mode 0:  g[s,:] = mu + softplus(rho) * eps[s,:]              (diagonal; the reference)
  *   mode 1:  reserved -- the dense form g[s,:] = mu + L eps[s,:] is whvi_reparam_dense_f32 below (it needs a workspace).

@@ -75,6 +75,11 @@ SIGNATURES = {
     "whvi_fwht_bf16": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p]),
     "whvi_layer_fwd_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64,
                                     c_int, c_void_p]),
+    "whvi_layer_bwd_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                    c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_int, c_void_p]),
+    "whvi_layer_loss_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_int,
+                                     c_void_p]),
     "whvi_fwht_f64": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p]),
     "whvi_mc_moments_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p]),
     "whvi_mc_moments_strided_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64,

@@ -184,6 +184,44 @@ int whvi_layer_bwd_scaled_f32(const float* x, int64_t x_sample_stride, const flo
                             flags, nullptr, nullptr, dy_scale, stream);
 }
 
+// bf16 activations (x, dy, dx): the fp32 kernels' plan on widened tiles, dx rounded once at the store.  x and dy arrive by
+// bulk async copies, which need 16-byte-aligned addresses and sizes: with 2-byte elements a sample (B * D elements) and the
+// tail tile of a sample are whole 16-byte units only when B * D % 8 == 0 (it fails only at D = 4 with an odd B).
+static int check_bf16_io(const char* who, const void* x, const void* dy, const void* dx, int64_t B, int64_t D)
+{
+    if ((B * D) % 8 != 0)
+        return fail(WHVI_E_SHAPE, "%s: B * D = %lld must be a multiple of 8 for bf16 activations (pad B)", who, (long long)(B * D));
+    if (!aligned16(x) || !aligned16(dy) || (reinterpret_cast<uintptr_t>(dx) & 7u))
+        return fail(WHVI_E_ALIGN, "%s: x and dy must be 16-byte aligned, dx 8-byte aligned", who);
+    return WHVI_OK;
+}
+
+int whvi_layer_bwd_bf16(const void* x, int64_t x_sample_stride, const void* dy, const float* dy_scale, const float* g,
+                        const float* s1, const float* s2, void* dx, float* dg, float* ds1, float* ds2, float* dbias,
+                        void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int flags, whvi_stream_t stream)
+{
+    if (int rc = check_layer_shape("layer_bwd_bf16", S, B, D, x_sample_stride)) return rc;
+    if (flags & ~WHVI_LAYER_RELU_IN) return fail(WHVI_E_MODE, "layer_bwd_bf16: unknown flags %d", flags);
+    if (!dg || !ds1 || !ds2) return fail(WHVI_E_NULL, "layer_bwd_bf16: null output pointer");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (S == 0 || B == 0) {  // empty sums
+        if (S > 0) cudaMemsetAsync(dg, 0, sizeof(float) * size_t(S) * D, st);
+        cudaMemsetAsync(ds1, 0, sizeof(float) * D, st);
+        cudaMemsetAsync(ds2, 0, sizeof(float) * D, st);
+        if (dbias) cudaMemsetAsync(dbias, 0, sizeof(float) * D, st);
+        return check_launch("layer_bwd_bf16(empty)");
+    }
+    if (!x || !dy || !g || !s1 || !s2) return fail(WHVI_E_NULL, "layer_bwd_bf16: null pointer");
+    if (!aligned16(g) || !aligned16(s1) || !aligned16(s2) || !aligned16(workspace))
+        return fail(WHVI_E_ALIGN, "layer_bwd_bf16: fp32 pointers must be 16-byte aligned");
+    if (int rc = check_bf16_io("layer_bwd_bf16", x, dy, dx, B, D)) return rc;
+    LayerBwdCall c{static_cast<const float*>(x), static_cast<const float*>(dy), g, s1, s2, nullptr, nullptr, dy_scale,
+                   static_cast<float*>(dx), dg, ds1, ds2, dbias, static_cast<float*>(workspace), workspace_bytes, x_sample_stride, S, B,
+                   flags & WHVI_LAYER_RELU_IN, nullptr};
+    c.bf16 = 1;
+    return launch_layer_bwd(c, D, st);
+}
+
 int whvi_layer_loss_sizes(int64_t S, int64_t B, int64_t D, size_t* workspace_bytes, int64_t* sq_count)
 {
     if (!workspace_bytes || !sq_count) return fail(WHVI_E_NULL, "layer_loss_sizes: null pointer");
@@ -216,6 +254,27 @@ int whvi_layer_loss_f32(const float* x, int64_t x_sample_stride, const float* g,
         return fail(WHVI_E_ALIGN, "layer_loss: pointers must be 16-byte aligned");
     LayerLossCall c{x, g, s1, s2, bias, target, dx, dg, ds1, ds2, dbias, sq_partials, static_cast<float*>(workspace),
                     workspace_bytes, x_sample_stride, S, B, flags & WHVI_LAYER_RELU_IN, nullptr, nullptr};
+    return launch_layer_loss(c, D, static_cast<cudaStream_t>(stream));
+}
+
+int whvi_layer_loss_bf16(const void* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2,
+                         const float* bias, const float* target, void* dx, float* dg, float* ds1, float* ds2, float* dbias,
+                         float* sq_partials, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int flags,
+                         whvi_stream_t stream)
+{
+    if (int rc = check_layer_shape("layer_loss_bf16", S, B, D, x_sample_stride, 4096)) return rc;
+    if (D < 128) return fail(WHVI_E_SHAPE, "layer_loss_bf16: D = %lld outside [128, 4096]", (long long)D);
+    if (flags & ~WHVI_LAYER_RELU_IN) return fail(WHVI_E_MODE, "layer_loss_bf16: unknown flags %d", flags);
+    if (S == 0 || B == 0) return fail(WHVI_E_SHAPE, "layer_loss_bf16: empty batch");
+    if (!x || !g || !s1 || !s2 || !target || !dg || !ds1 || !ds2 || !sq_partials || (bias && !dbias))
+        return fail(WHVI_E_NULL, "layer_loss_bf16: null pointer");
+    if (!aligned16(g) || !aligned16(s1) || !aligned16(s2) || !aligned16(bias) || !aligned16(target) || !aligned16(workspace))
+        return fail(WHVI_E_ALIGN, "layer_loss_bf16: fp32 pointers must be 16-byte aligned");
+    if (!aligned16(x) || (reinterpret_cast<uintptr_t>(dx) & 7u))
+        return fail(WHVI_E_ALIGN, "layer_loss_bf16: x must be 16-byte aligned, dx 8-byte aligned");
+    LayerLossCall c{static_cast<const float*>(x), g, s1, s2, bias, target, static_cast<float*>(dx), dg, ds1, ds2, dbias, sq_partials,
+                    static_cast<float*>(workspace), workspace_bytes, x_sample_stride, S, B, flags & WHVI_LAYER_RELU_IN, nullptr, nullptr};
+    c.bf16 = 1;
     return launch_layer_loss(c, D, static_cast<cudaStream_t>(stream));
 }
 

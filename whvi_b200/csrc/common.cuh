@@ -78,6 +78,7 @@ struct LayerBwdCall {
     int relu_in;
     size_t* need_only;  // query mode: workspace bytes
     int64_t groups = 1, pstride = 0;  // grouped launch (see LayerFwdCall): ds1 / ds2 / dbias are (groups, D)
+    int bf16 = 0;             // x, dy and dx are bf16 in HBM (behind the float pointers; arithmetic and workspace stay fp32)
 };
 struct LayerLossCall {  // fused last layer: forward + Gaussian-MNLL residual + backward in one pass
     const float *x, *g, *s1, *s2, *bias, *target;
@@ -87,6 +88,7 @@ struct LayerLossCall {  // fused last layer: forward + Gaussian-MNLL residual + 
     int relu_in;
     size_t* need_ws;      // query mode
     int64_t* need_sq;     // query mode
+    int bf16 = 0;         // x and dx are bf16 in HBM (behind the float pointers); target, parameters and arithmetic stay fp32
 };
 int launch_layer_loss(const LayerLossCall& c, int64_t D, cudaStream_t stream);
 int launch_bwd_reduce(float* ws, float* dg, float* ds1, float* ds2, float* dbias, int64_t S, int slabs_per_sample,

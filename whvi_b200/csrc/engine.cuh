@@ -79,6 +79,9 @@ template <>
 struct Io<float> {
     static __device__ __forceinline__ float4 ld4(const float* p) { return ldg_stream(p); }
     static __device__ __forceinline__ void st4(float* p, const float4& v) { stg_stream(p, v); }
+    // shared-memory side (bulk-copy staged tiles): read four elements widened to fp32, zero four elements
+    static __device__ __forceinline__ float4 lds4(const float* p) { return *reinterpret_cast<const float4*>(p); }
+    static __device__ __forceinline__ void sts_zero4(float* p) { *reinterpret_cast<float4*>(p) = make_float4(0.f, 0.f, 0.f, 0.f); }
 };
 template <>
 struct Io<__nv_bfloat16> {
@@ -96,6 +99,13 @@ struct Io<__nv_bfloat16> {
         asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(b) : "f"(v.w), "f"(v.z));
         asm volatile("st.global.L1::no_allocate.v2.b32 [%0], {%1,%2};" ::"l"(p), "r"(a), "r"(b) : "memory");
     }
+    static __device__ __forceinline__ float4 lds4(const __nv_bfloat16* p)
+    {
+        const uint2 u = *reinterpret_cast<const uint2*>(p);
+        return make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xFFFF0000u), __uint_as_float(u.y << 16),
+                           __uint_as_float(u.y & 0xFFFF0000u));
+    }
+    static __device__ __forceinline__ void sts_zero4(__nv_bfloat16* p) { *reinterpret_cast<uint2*>(p) = make_uint2(0u, 0u); }
 };
 
 // Barrier among the T threads of one tile group.

@@ -79,9 +79,14 @@ struct BwdArgs {
 // 64-float variant and a single-barrier stash exchange were measured and dropped
 // (profiles/r01_bwd_notes.md, items 5, 8, 10).
 // Shared memory per pair: NS x (x tile + dy tile) + X scratch + Y scratch + stash (1 tile).
-template <int N, int C, int KT, int PAIRS, int MINB, int NS, bool SINGLE, bool ALIAS, int PREG, int ROUNDS, bool WANT_DBIAS, bool RESID>
+// IO: the activations' type in HBM (x, dy, dx; see layer_fwd_kernel).  bf16 tiles are staged in the first half of their
+// fp32-sized slots (the plan, shared memory and partial-sum order are the fp32 instance's), widened on every read, and dx
+// is rounded once at the store.  The workspace, the parameters and all arithmetic stay fp32; RESID is fp32 only.
+template <int N, int C, int KT, int PAIRS, int MINB, int NS, bool SINGLE, bool ALIAS, int PREG, int ROUNDS, bool WANT_DBIAS, bool RESID,
+          class IO = float>
 __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_kernel(const BwdArgs p)
 {
+    static_assert(std::is_same_v<IO, float> || !RESID, "RESID (saved output + target) is fp32 only");
     constexpr int T = 1 << (N - C);
     constexpr int E = 1 << C;
     constexpr int H = E / 2;               // floats per thread per half-stream
@@ -112,10 +117,10 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
     const int s = blockIdx.x % p.n_samples;
     const int cta_in_sample = blockIdx.x / p.n_samples;
     const int grp = s / p.spg;   // parameter group (Stacked block); the group's virtual samples read the inputs of samples 0 .. spg-1
-    const float* __restrict__ xbase = p.x + int64_t(s - grp * p.spg) * p.x_sample_stride;
+    const IO* __restrict__ xbase = reinterpret_cast<const IO*>(p.x) + int64_t(s - grp * p.spg) * p.x_sample_stride;
     const float* __restrict__ s1p = p.s1 + int64_t(grp) * p.pstride;
     const float* __restrict__ s2p = p.s2 + int64_t(grp) * p.pstride;
-    const float* __restrict__ dybase = p.dy + int64_t(s) * p.sample_elems;
+    const IO* __restrict__ dybase = reinterpret_cast<const IO*>(p.dy) + int64_t(s) * p.sample_elems;
 
     if (threadIdx.x == 0) {
         for (int q = 0; q < PAIRS; ++q)
@@ -143,7 +148,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
         const int st = it % NS;
         if (it >= NS) mbar_wait(&empty_bar[pr][st], ((it / NS) & 1) ^ 1);
         const int64_t left = p.sample_elems - e0;
-        const uint32_t bytes = static_cast<uint32_t>((left < TILE ? left : TILE) * sizeof(float));
+        const uint32_t bytes = static_cast<uint32_t>((left < TILE ? left : TILE) * sizeof(IO));
         float* stage = smem + size_t(pr) * PAIR_FLOATS + size_t(st) * SPT * TILE;
         mbar_arrive_expect_tx(&full_bar[pr][st], SPT * bytes);
         bulk_g2s(stage, xbase + e0, bytes, &full_bar[pr][st]);
@@ -279,15 +284,15 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
                 constexpr int m = decltype(m_)::value;
                 const uint32_t off = off_f + tile_reg_offset<N, C, V_FIRST>(m);
                 if (off >= left) {
-                    *reinterpret_cast<float4*>(stage_x + off) = make_float4(0.f, 0.f, 0.f, 0.f);
-                    *reinterpret_cast<float4*>(stage_x + TILE + off) = make_float4(0.f, 0.f, 0.f, 0.f);
+                    Io<IO>::sts_zero4(reinterpret_cast<IO*>(stage_x) + off);
+                    Io<IO>::sts_zero4(reinterpret_cast<IO*>(stage_x + TILE) + off);
                     if constexpr (STAGE_TGT) *reinterpret_cast<float4*>(stage_x + 2 * TILE + off) = make_float4(0.f, 0.f, 0.f, 0.f);
                 }
             });
         }
     };
     auto raw4 = [&](const float* stage_tile, uint32_t off) -> float4 {
-        return *reinterpret_cast<const float4*>(stage_tile + off);
+        return Io<IO>::lds4(reinterpret_cast<const IO*>(stage_tile) + off);
     };
     // RESID: dy = coef * (saved output - target); the target tile is read from global memory
     // (it is shared by all samples, so it stays L2-resident), zero beyond the valid part
@@ -440,7 +445,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
             apply_g(b, gr);
             from_mid(b);  // b = dt1 (FIRST layout)
             const bool want_dx = p.dx != nullptr;
-            float* __restrict__ dxs = p.dx + int64_t(s) * p.sample_elems + e0;
+            IO* __restrict__ dxs = reinterpret_cast<IO*>(p.dx) + int64_t(s) * p.sample_elems + e0;
             for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t off, uint32_t coord) {
                 constexpr int m = decltype(m_)::value;
                 const float4 q = raw4(stage_x, off);
@@ -448,7 +453,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
                 fma4(acc_2 + 4 * m, q, b + 4 * m);
                 const float4 o = make_float4(q.x > relu_thr ? b[4 * m] * w.x : 0.f, q.y > relu_thr ? b[4 * m + 1] * w.y : 0.f,
                                              q.z > relu_thr ? b[4 * m + 2] * w.z : 0.f, q.w > relu_thr ? b[4 * m + 3] * w.w : 0.f);
-                if (want_dx && (left >= TILE || off < left)) stg_stream(dxs + off, o);
+                if (want_dx && (left >= TILE || off < left)) Io<IO>::st4(dxs + off, o);
             });
             mbar_arrive(&empty_bar[pair][st]);
         }
@@ -481,9 +486,10 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
 //   [4E,5E) s2 (Y) | [5E,5E+H) t2 upper half X->Y | [5E+H,6E) dt3 lower half Y->X | [6E,7E) the same for odd tiles |
 //   [7E,8E) dbias (X)
 // Everything else (bulk-copy staging ring, roles, workspace layout, second-stage reduction) is the kernel above.
-template <int N, int C, int KT, int ROUNDS, bool WANT_DBIAS, bool RESID>
+template <int N, int C, int KT, int ROUNDS, bool WANT_DBIAS, bool RESID, class IO = float>
 __global__ void __launch_bounds__(256, 1) layer_bwd_tm_kernel(const BwdArgs p)
 {
+    static_assert(std::is_same_v<IO, float> || !RESID, "RESID (saved output + target) is fp32 only");
     constexpr int T = 1 << (N - C);
     constexpr int E = 1 << C;
     constexpr int H = E / 2;
@@ -510,10 +516,10 @@ __global__ void __launch_bounds__(256, 1) layer_bwd_tm_kernel(const BwdArgs p)
     const int s = blockIdx.x % p.n_samples;   // sample-minor CTA order
     const int cta_in_sample = blockIdx.x / p.n_samples;
     const int grp = s / p.spg;   // parameter group (Stacked block); the group's virtual samples read the inputs of samples 0 .. spg-1
-    const float* __restrict__ xbase = p.x + int64_t(s - grp * p.spg) * p.x_sample_stride;
+    const IO* __restrict__ xbase = reinterpret_cast<const IO*>(p.x) + int64_t(s - grp * p.spg) * p.x_sample_stride;
     const float* __restrict__ s1p = p.s1 + int64_t(grp) * p.pstride;
     const float* __restrict__ s2p = p.s2 + int64_t(grp) * p.pstride;
-    const float* __restrict__ dybase = p.dy + int64_t(s) * p.sample_elems;
+    const IO* __restrict__ dybase = reinterpret_cast<const IO*>(p.dy) + int64_t(s) * p.sample_elems;
 
     if (threadIdx.x == 0) {
         for (int q = 0; q < PAIRS; ++q)
@@ -540,7 +546,7 @@ __global__ void __launch_bounds__(256, 1) layer_bwd_tm_kernel(const BwdArgs p)
         const int st = it % NS;
         if (it >= NS) mbar_wait(&empty_bar[pr][st], ((it / NS) & 1) ^ 1);
         const int64_t left = p.sample_elems - e0;
-        const uint32_t bytes = static_cast<uint32_t>((left < TILE ? left : TILE) * sizeof(float));
+        const uint32_t bytes = static_cast<uint32_t>((left < TILE ? left : TILE) * sizeof(IO));
         float* stage = smem + size_t(pr) * PAIR_FLOATS + size_t(st) * 2 * TILE;
         mbar_arrive_expect_tx(&full_bar[pr][st], 2 * bytes);
         bulk_g2s(stage, xbase + e0, bytes, &full_bar[pr][st]);
@@ -637,14 +643,14 @@ __global__ void __launch_bounds__(256, 1) layer_bwd_tm_kernel(const BwdArgs p)
                 constexpr int m = decltype(m_)::value;
                 const uint32_t off = off_f + tile_reg_offset<N, C, V_FIRST>(m);
                 if (off >= left) {
-                    *reinterpret_cast<float4*>(stage_x + off) = make_float4(0.f, 0.f, 0.f, 0.f);
-                    *reinterpret_cast<float4*>(stage_x + TILE + off) = make_float4(0.f, 0.f, 0.f, 0.f);
+                    Io<IO>::sts_zero4(reinterpret_cast<IO*>(stage_x) + off);
+                    Io<IO>::sts_zero4(reinterpret_cast<IO*>(stage_x + TILE) + off);
                 }
             });
         }
     };
     auto raw4 = [&](const float* stage_tile, uint32_t off) -> float4 {
-        return *reinterpret_cast<const float4*>(stage_tile + off);
+        return Io<IO>::lds4(reinterpret_cast<const IO*>(stage_tile) + off);
     };
     // RESID: dy = coef * (saved output - target); the target (shared by all samples, L2-resident) is read from
     // global memory, zero beyond the valid part of a partial tile
@@ -817,7 +823,7 @@ __global__ void __launch_bounds__(256, 1) layer_bwd_tm_kernel(const BwdArgs p)
         float acc0[32];
         from_mid(v, acc0);  // X: t4, Y: dt1 (FIRST layout); acc0 = running-sum chunk 0, load in flight
         const bool want_dx = p.dx != nullptr;
-        float* __restrict__ dxs = p.dx + int64_t(s) * p.sample_elems + e0;
+        IO* __restrict__ dxs = reinterpret_cast<IO*>(p.dx) + int64_t(s) * p.sample_elems + e0;
 #pragma unroll
         for (int c = 0; c < 2; ++c) {   // end product, 32 registers at a time
             float acc1[32];
@@ -857,7 +863,7 @@ __global__ void __launch_bounds__(256, 1) layer_bwd_tm_kernel(const BwdArgs p)
                     const float* bb = v + 32 * c + 4 * j;
                     const float4 o = make_float4(q[j].x > relu_thr ? bb[0] * w[4 * j] : 0.f, q[j].y > relu_thr ? bb[1] * w[4 * j + 1] : 0.f,
                                                  q[j].z > relu_thr ? bb[2] * w[4 * j + 2] : 0.f, q[j].w > relu_thr ? bb[3] * w[4 * j + 3] : 0.f);
-                    if (want_dx && (left >= TILE || off < left)) stg_stream(dxs + off, o);
+                    if (want_dx && (left >= TILE || off < left)) Io<IO>::st4(dxs + off, o);
                 });
             } else if constexpr (WANT_DBIAS) {
                 float ab[32];
@@ -1022,7 +1028,7 @@ int launch_bwd_reduce(float* ws, float* dg, float* ds1, float* ds2, float* dbias
 template <int N, int C, int KT, int PAIRS, int MINB, int NS, bool SINGLE, bool ALIAS = false, int PREG = 0, int ROUNDS = 3>
 static int launch_bwd_tma_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
 {
-    static unsigned char smem_ok[4][64] = {};
+    static unsigned char smem_ok[6][64] = {};
     constexpr int threads = (2 << (N - C)) * PAIRS;
     constexpr size_t tile = size_t(1) << N;
     constexpr bool gtab = ROUNDS == 2 && !PREG;
@@ -1054,7 +1060,13 @@ static int launch_bwd_tma_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
     };
     const bool db = c.dbias != nullptr, rs = c.target != nullptr;
     int rc;
-    if (db && rs) rc = go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, true>, 0);
+    if (c.bf16) {
+        if (rs) return fail(WHVI_E_MODE, "layer_bwd: bf16 activations cannot be combined with a target");
+        // D >= 2048 runs the tensor-memory kernel; these configurations serve WHVI_BWD_LEGACY builds, which take fp32 only
+        if constexpr (N > 10) return fail(WHVI_E_MODE, "layer_bwd: bf16 activations at D = %lld need the tensor-memory backward", (long long)D);
+        else rc = db ? go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, false, __nv_bfloat16>, 4)
+                     : go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, false, false, __nv_bfloat16>, 5);
+    } else if (db && rs) rc = go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, true>, 0);
     else if (db) rc = go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, false>, 1);
     else if (rs) rc = go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, false, true>, 2);
     else rc = go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, false, false>, 3);
@@ -1065,7 +1077,7 @@ static int launch_bwd_tma_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
 template <int N, int C, int KT, int ROUNDS>
 static int launch_bwd_tm_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
 {
-    static unsigned char smem_ok[4][64] = {};
+    static unsigned char smem_ok[6][64] = {};
     constexpr int T = 1 << (N - C);
     constexpr int PAIRS = 128 / T;
     constexpr size_t tile = size_t(1) << N;
@@ -1096,7 +1108,11 @@ static int launch_bwd_tm_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
     };
     const bool db = c.dbias != nullptr, rs = c.target != nullptr;
     int rc;
-    if (db && rs) rc = go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, true, true>, 0);
+    if (c.bf16) {
+        if (rs) return fail(WHVI_E_MODE, "layer_bwd: bf16 activations cannot be combined with a target");
+        rc = db ? go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, true, false, __nv_bfloat16>, 4)
+                : go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, false, false, __nv_bfloat16>, 5);
+    } else if (db && rs) rc = go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, true, true>, 0);
     else if (db) rc = go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, true, false>, 1);
     else if (rs) rc = go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, false, true>, 2);
     else rc = go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, false, false>, 3);

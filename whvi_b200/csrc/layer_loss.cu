@@ -38,7 +38,9 @@
 namespace whvi {
 
 
-template <int N, int C, int KT, int PAIRS, int NS, bool SINGLE, int PREG, int ROUNDS, bool HAS_BIAS>
+// IO: the type of x and dx in HBM (see layer_bwd_tma_kernel): a bf16 x tile is staged in the first half of its fp32-sized
+// slot and widened on every read, dx is rounded once at the store; the target ring, r, t2 and all arithmetic stay fp32.
+template <int N, int C, int KT, int PAIRS, int NS, bool SINGLE, int PREG, int ROUNDS, bool HAS_BIAS, class IO = float>
 __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, 1) layer_loss_kernel(const LossArgs p)
 {
     constexpr int T = 1 << (N - C);
@@ -58,7 +60,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, 1) layer_loss_kernel(c
     const uint32_t cmask = (1u << k) - 1u;
     const int s = blockIdx.x % p.n_samples;  // sample-minor CTA order: the target tile is reused out of L2
     const int cta_in_sample = blockIdx.x / p.n_samples;
-    const float* __restrict__ xbase = p.x + int64_t(s) * p.x_sample_stride;
+    const IO* __restrict__ xbase = reinterpret_cast<const IO*>(p.x) + int64_t(s) * p.x_sample_stride;
 
     if (threadIdx.x == 0) {
         for (int q = 0; q < PAIRS; ++q)
@@ -81,10 +83,17 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, 1) layer_loss_kernel(c
         const int st = it % NS;
         if (it >= NS) mbar_wait(&empty_bar[pr][st], ((it / NS) & 1) ^ 1);
         const int64_t left = p.sample_elems - e0;
-        const uint32_t bytes = static_cast<uint32_t>((left < TILE ? left : TILE) * sizeof(float));
+        const int64_t n = left < TILE ? left : TILE;
+        const uint32_t bytes = static_cast<uint32_t>(n * sizeof(float));
         float* stage = smem + size_t(pr) * PAIR_FLOATS + size_t(st) * 2 * TILE;
-        mbar_arrive_expect_tx(&full_bar[pr][st], 2 * bytes);
-        bulk_g2s(stage, xbase + e0, bytes, &full_bar[pr][st]);
+        if constexpr (std::is_same_v<IO, float>) {
+            mbar_arrive_expect_tx(&full_bar[pr][st], 2 * bytes);
+            bulk_g2s(stage, xbase + e0, bytes, &full_bar[pr][st]);
+        } else {
+            const uint32_t xbytes = static_cast<uint32_t>(n * sizeof(IO));
+            mbar_arrive_expect_tx(&full_bar[pr][st], xbytes + bytes);
+            bulk_g2s(stage, xbase + e0, xbytes, &full_bar[pr][st]);
+        }
         bulk_g2s(stage + TILE, p.target + e0, bytes, &full_bar[pr][st]);
     };
 
@@ -214,7 +223,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, 1) layer_loss_kernel(c
                     constexpr int m = decltype(m_)::value;
                     const uint32_t off = off_f + tile_reg_offset<N, C, V_FIRST>(m);
                     if (off >= left) {
-                        *reinterpret_cast<float4*>(stage_x + off) = make_float4(0.f, 0.f, 0.f, 0.f);
+                        Io<IO>::sts_zero4(reinterpret_cast<IO*>(stage_x) + off);
                         *reinterpret_cast<float4*>(stage_t + off) = make_float4(0.f, 0.f, 0.f, 0.f);
                     }
                 });
@@ -222,7 +231,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, 1) layer_loss_kernel(c
             float a[E];
             for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t off, uint32_t coord) {
                 constexpr int m = decltype(m_)::value;
-                const float4 q = *reinterpret_cast<const float4*>(stage_x + off);
+                const float4 q = Io<IO>::lds4(reinterpret_cast<const IO*>(stage_x) + off);
                 mul4(a + 4 * m, q, first_param(s2r, p.s2, m, coord, PREG > 0));
             });
             to_mid(a);  // a = t2
@@ -297,15 +306,15 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, 1) layer_loss_kernel(c
             apply_g(b, gr);
             from_mid(b);  // b = dt1 (FIRST layout)
             const bool want_dx = p.dx != nullptr;
-            float* __restrict__ dxs = p.dx + int64_t(s) * p.sample_elems + e0;
+            IO* __restrict__ dxs = reinterpret_cast<IO*>(p.dx) + int64_t(s) * p.sample_elems + e0;
             for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t off, uint32_t coord) {
                 constexpr int m = decltype(m_)::value;
-                const float4 q = *reinterpret_cast<const float4*>(stage_x + off);
+                const float4 q = Io<IO>::lds4(reinterpret_cast<const IO*>(stage_x) + off);
                 const float4 w = first_param(s2r, p.s2, m, coord, PREG == 2);
                 fma4(acc_2 + 4 * m, q, b + 4 * m);
                 const float4 o = make_float4(q.x > relu_thr ? b[4 * m] * w.x : 0.f, q.y > relu_thr ? b[4 * m + 1] * w.y : 0.f,
                                              q.z > relu_thr ? b[4 * m + 2] * w.z : 0.f, q.w > relu_thr ? b[4 * m + 3] * w.w : 0.f);
-                if (want_dx && (left >= TILE || off < left)) stg_stream(dxs + off, o);
+                if (want_dx && (left >= TILE || off < left)) Io<IO>::st4(dxs + off, o);
             });
             mbar_arrive(&empty_bar[pair][st]);
         }
@@ -332,7 +341,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, 1) layer_loss_kernel(c
 template <int N, int C, int KT, int PAIRS, int NS, bool SINGLE, int PREG, int ROUNDS>
 static int launch_loss_cfg(const LayerLossCall& c, int k, cudaStream_t stream)
 {
-    static unsigned char smem_ok[2][64] = {};
+    static unsigned char smem_ok[4][64] = {};
     constexpr int T = 1 << (N - C);
     constexpr int threads = 2 * T * PAIRS;
     constexpr size_t tile = size_t(1) << N;
@@ -359,7 +368,9 @@ static int launch_loss_cfg(const LayerLossCall& c, int k, cudaStream_t stream)
         kernel<<<static_cast<unsigned>(ctas), threads, smem, stream>>>(a);
         return check_launch("layer_loss_kernel");
     };
-    const int rc = c.bias ? go(layer_loss_kernel<N, C, KT, PAIRS, NS, SINGLE, PREG, ROUNDS, true>, 0)
+    const int rc = c.bf16 ? (c.bias ? go(layer_loss_kernel<N, C, KT, PAIRS, NS, SINGLE, PREG, ROUNDS, true, __nv_bfloat16>, 2)
+                                    : go(layer_loss_kernel<N, C, KT, PAIRS, NS, SINGLE, PREG, ROUNDS, false, __nv_bfloat16>, 3))
+                 : c.bias ? go(layer_loss_kernel<N, C, KT, PAIRS, NS, SINGLE, PREG, ROUNDS, true>, 0)
                           : go(layer_loss_kernel<N, C, KT, PAIRS, NS, SINGLE, PREG, ROUNDS, false>, 1);
     if (rc) return rc;
     return launch_bwd_reduce(c.ws, c.dg, c.ds1, c.ds2, c.bias ? c.dbias : nullptr, c.S, plan.ctas_per_sample * PAIRS, int64_t(tile), D, stream);

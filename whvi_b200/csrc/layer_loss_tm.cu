@@ -20,7 +20,8 @@
 
 namespace whvi {
 
-template <int N, int C, int KT>
+// IO: the type of x and dx in HBM (see layer_loss_kernel): bf16 x tiles fill the first half of their fp32-sized slots.
+template <int N, int C, int KT, class IO = float>
 __global__ void __launch_bounds__(256, 1) layer_loss_tm_kernel(const LossArgs p)
 {
     constexpr int T = 1 << (N - C);
@@ -42,7 +43,7 @@ __global__ void __launch_bounds__(256, 1) layer_loss_tm_kernel(const LossArgs p)
     const uint32_t cmask = (1u << k) - 1u;
     const int s = blockIdx.x % p.n_samples;  // sample-minor CTA order: the target tile is reused out of L2
     const int cta_in_sample = blockIdx.x / p.n_samples;
-    const float* __restrict__ xbase = p.x + int64_t(s) * p.x_sample_stride;
+    const IO* __restrict__ xbase = reinterpret_cast<const IO*>(p.x) + int64_t(s) * p.x_sample_stride;
 
     if (threadIdx.x == 0) {
         for (int q = 0; q < PAIRS; ++q) {
@@ -78,7 +79,7 @@ __global__ void __launch_bounds__(256, 1) layer_loss_tm_kernel(const LossArgs p)
         return static_cast<uint32_t>((left < TILE ? left : TILE) * sizeof(float));
     };
     auto issue_x = [&](int it) {      // x tile `it` -> slot it % NX (waits for Y's release of tile it - NX)
-        const uint32_t bytes = tile_bytes(it);
+        const uint32_t bytes = tile_bytes(it) / (sizeof(float) / sizeof(IO));
         if (!bytes) return;
         const int sl = it % NX;
         if (it >= NX) mbar_wait(&x_empty[pair][sl], ((it / NX) & 1) ^ 1);
@@ -176,6 +177,22 @@ __global__ void __launch_bounds__(256, 1) layer_loss_tm_kernel(const LossArgs p)
             for (int j = 0; j < 8; ++j) mul4(v + 32 * c + 4 * j, q[j], make_float4(w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]));
         }
     };
+    // the same for the X role's x tile when x is bf16 (IO != float): widened on the read
+    auto load_scaled_io = [&](float (&v)[E], const IO* tile, uint32_t col) {
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+            float w[32];
+            tm_ld32(w, tm + col + 32 * c);
+            float4 q[8];
+            static_for<0, 8>([&](auto j_) {
+                constexpr int j = decltype(j_)::value;
+                q[j] = Io<IO>::lds4(tile + off_f + tile_reg_offset<N, C, V_FIRST>(8 * c + j));
+            });
+            tm_wait_ld();
+#pragma unroll
+            for (int j = 0; j < 8; ++j) mul4(v + 32 * c + 4 * j, q[j], make_float4(w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]));
+        }
+    };
 
     // ONE loop for both roles: the two transforms and the g multiply are the same instructions on different data, and a
     // private copy per role does not fit the instruction cache next to the other role's (39% of the warp samples of the
@@ -200,7 +217,7 @@ __global__ void __launch_bounds__(256, 1) layer_loss_tm_kernel(const LossArgs p)
                 static_for<0, E / 4>([&](auto m_) {
                     constexpr int m = decltype(m_)::value;
                     const uint32_t off = off_f + tile_reg_offset<N, C, V_FIRST>(m);
-                    if (off >= left) *reinterpret_cast<float4*>(xt + off) = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (off >= left) Io<IO>::sts_zero4(reinterpret_cast<IO*>(xt) + off);
                 });
             }
         } else {
@@ -208,7 +225,9 @@ __global__ void __launch_bounds__(256, 1) layer_loss_tm_kernel(const LossArgs p)
             tm_fence_after();
         }
         float v[E];
-        load_scaled(v, role ? tt : xt, col_in);   // X: s2 * x, Y: s1 * r
+        if constexpr (std::is_same_v<IO, float>) load_scaled(v, role ? tt : xt, col_in);   // X: s2 * x, Y: s1 * r
+        else if (role) load_scaled(v, tt, col_in);
+        else load_scaled_io(v, reinterpret_cast<const IO*>(xt), col_in);
         if (role) mbar_arrive(&t_empty[pair][it % NT]);   // r has been read: the slot may take the next target tile
         it_now = it;
         to_mid(v);  // X: t2, Y: dt3
@@ -268,7 +287,7 @@ __global__ void __launch_bounds__(256, 1) layer_loss_tm_kernel(const LossArgs p)
         } else {
             mbar_wait(&x_full[pair][it % NX], (it / NX) & 1);   // completed long ago; orders this thread after the bulk copy
             const bool want_dx = p.dx != nullptr;
-            float* __restrict__ dxs = p.dx + int64_t(s) * p.sample_elems + e0;
+            IO* __restrict__ dxs = reinterpret_cast<IO*>(p.dx) + int64_t(s) * p.sample_elems + e0;
 #pragma unroll
             for (int c = 0; c < 2; ++c) {   // ds2 += dt1 * x, dx = s2 * dt1 (masked)
                 float w[32], a2[32];
@@ -277,7 +296,7 @@ __global__ void __launch_bounds__(256, 1) layer_loss_tm_kernel(const LossArgs p)
                 float4 q[8];
                 static_for<0, 8>([&](auto j_) {
                     constexpr int j = decltype(j_)::value;
-                    q[j] = *reinterpret_cast<const float4*>(xt + off_f + tile_reg_offset<N, C, V_FIRST>(8 * c + j));
+                    q[j] = Io<IO>::lds4(reinterpret_cast<const IO*>(xt) + off_f + tile_reg_offset<N, C, V_FIRST>(8 * c + j));
                 });
                 tm_wait_ld();
                 static_for<0, 8>([&](auto j_) {
@@ -287,7 +306,7 @@ __global__ void __launch_bounds__(256, 1) layer_loss_tm_kernel(const LossArgs p)
                     fma4(a2 + 4 * j, q[j], bb);
                     const float4 o = make_float4(q[j].x > relu_thr ? bb[0] * w[4 * j] : 0.f, q[j].y > relu_thr ? bb[1] * w[4 * j + 1] : 0.f,
                                                  q[j].z > relu_thr ? bb[2] * w[4 * j + 2] : 0.f, q[j].w > relu_thr ? bb[3] * w[4 * j + 3] : 0.f);
-                    if (want_dx && (left >= TILE || off < left)) stg_stream(dxs + off, o);
+                    if (want_dx && (left >= TILE || off < left)) Io<IO>::st4(dxs + off, o);
                 });
                 tm_st32(a2, tm + COL_A2 + 32 * c);
             }
@@ -337,7 +356,7 @@ __global__ void __launch_bounds__(256, 1) layer_loss_tm_kernel(const LossArgs p)
 template <int N, int C, int KT>
 static int launch_loss_tm_cfg(const LayerLossCall& c, int k, cudaStream_t stream)
 {
-    static unsigned char smem_ok[64] = {};
+    static unsigned char smem_ok[2][64] = {};
     constexpr int T = 1 << (N - C);
     constexpr int PAIRS = 128 / T;
     constexpr size_t tile = size_t(1) << N;
@@ -359,9 +378,12 @@ static int launch_loss_tm_cfg(const LayerLossCall& c, int k, cudaStream_t stream
     if (ctas > 0x7fffffffLL) return fail(WHVI_E_SHAPE, "layer_loss: grid too large");
     LossArgs a{c.x, c.xs, c.g, c.s1, c.s2, c.bias, c.target, c.dx, c.ws, c.sq_partials, c.B * D, static_cast<int>(c.S),
                plan.ctas_per_sample, plan.iters_per_group, k, c.relu_in};
-    if (int rc = ensure_smem(layer_loss_tm_kernel<N, C, KT>, smem, smem_ok)) return rc;
-    layer_loss_tm_kernel<N, C, KT><<<static_cast<unsigned>(ctas), 256, smem, stream>>>(a);
-    if (int rc = check_launch("layer_loss_tm_kernel")) return rc;
+    auto go = [&](auto kernel, int slot) -> int {
+        if (int rc = ensure_smem(kernel, smem, smem_ok[slot])) return rc;
+        kernel<<<static_cast<unsigned>(ctas), 256, smem, stream>>>(a);
+        return check_launch("layer_loss_tm_kernel");
+    };
+    if (int rc = c.bf16 ? go(layer_loss_tm_kernel<N, C, KT, __nv_bfloat16>, 1) : go(layer_loss_tm_kernel<N, C, KT>, 0)) return rc;
     return launch_bwd_reduce(c.ws, c.dg, c.ds1, c.ds2, nullptr, c.S, plan.ctas_per_sample * PAIRS, int64_t(tile), D, stream);
 }
 

@@ -12,6 +12,7 @@ import ctypes
 import functools
 
 import torch
+import torch.nn.functional as F
 from torch.autograd import Function
 
 from . import _lib
@@ -26,7 +27,8 @@ _LAUNCHES_PER_CALL = {"whvi_fwht_f32": 1, "whvi_fwht_f64": 1, "whvi_layer_fwd_f3
                       "whvi_reparam_bwd_f32": 1, "whvi_kl_f32": 1, "whvi_mc_moments_f32": 1,
                       "whvi_mc_moments_strided_f32": 1, "whvi_adam_f32": 1, "whvi_layer_moments_f32": 1,
                       "whvi_reparam_dense_f32": 2, "whvi_reparam_dense_bwd_f32": 1, "whvi_kl_dense_f32": 2,
-                      "whvi_fwht_bf16": 1, "whvi_fwht_scaled_f32": 1, "whvi_layer_moments_add_f32": 1, "whvi_layer_fwd_bf16": 1, "whvi_column_fwd_f32": 3, "whvi_column_bwd_f32": 7, "whvi_pad_rows_f32": 1, "whvi_stacked_fwd_f32": 3, "whvi_stacked_bwd_f32": 6, "whvi_kl_grouped_f32": 1}
+                      "whvi_fwht_bf16": 1, "whvi_fwht_scaled_f32": 1, "whvi_layer_moments_add_f32": 1, "whvi_layer_fwd_bf16": 1, "whvi_column_fwd_f32": 3, "whvi_column_bwd_f32": 7, "whvi_pad_rows_f32": 1, "whvi_stacked_fwd_f32": 3, "whvi_stacked_bwd_f32": 6, "whvi_kl_grouped_f32": 1,
+                      "whvi_layer_bwd_bf16": 3, "whvi_layer_loss_bf16": 3}
 # When set to a dict {"name": [(start_event, stop_event), ...]}, the named calls are bracketed
 # by CUDA events on the launching stream (bench.py's per-kernel roofline timing).
 EVENT_SINK: dict[str, list] | None = None
@@ -107,6 +109,14 @@ def _f32c(t: torch.Tensor, name: str) -> torch.Tensor:
         raise RuntimeError(f"{name} must be a CUDA tensor")
     if t.dtype != torch.float32:
         raise RuntimeError(f"{name} must be float32 (got {t.dtype})")
+    return t.contiguous()
+
+
+def _bf16c(t: torch.Tensor, name: str) -> torch.Tensor:
+    if t.device.type != "cuda":
+        raise RuntimeError(f"{name} must be a CUDA tensor")
+    if t.dtype != torch.bfloat16:
+        raise RuntimeError(f"{name} must be bfloat16 (got {t.dtype})")
     return t.contiguous()
 
 
@@ -367,7 +377,13 @@ def layer_backward_raw(x, dy, g, s1, s2, want_dx=True, want_dbias=False, relu_in
     """Returns (dx | None, dg, ds1, ds2, dbias | None); dx is (S,B,D) even for shared x.
     ``relu_in``: x came out of a fused ReLU, dx is masked by x > 0.  ``target``/``coef``:
     ``dy`` holds the layer's saved output and the upstream gradient is
-    coef * (output - target) formed inside the kernel (coef: 0-d / 1-element CUDA tensor)."""
+    coef * (output - target) formed inside the kernel (coef: 0-d / 1-element CUDA tensor).
+    A bfloat16 ``x`` selects the bf16-activation backward (``layer_backward_bf16``)."""
+    if x.dtype == torch.bfloat16:
+        if target is not None:
+            raise RuntimeError("the backward from the saved output and a target (RESID) is fp32 only; bf16 activations "
+                               "take the unfused route")
+        return layer_backward_bf16(x, dy, g, s1, s2, want_dx, want_dbias, relu_in, dy_scale)
     x, dy, g, s1, s2 = _f32c(x, "x"), _f32c(dy, "dy"), _f32c(g, "g"), _f32c(s1, "s1"), _f32c(s2, "s2")
     S, B, D, xs = _layer_dims(x, g, s1, s2)
     if dy.shape != (S, B, D):
@@ -404,6 +420,42 @@ def layer_backward_raw(x, dy, g, s1, s2, want_dx=True, want_dbias=False, relu_in
     return dx, dg, ds1, ds2, dbias
 
 
+def layer_backward_bf16(x, dy, g, s1, s2, want_dx=True, want_dbias=False, relu_in=False, dy_scale=None):
+    """``layer_backward_raw`` with bf16 activations (``whvi_layer_bwd_bf16``): ``x``, ``dy`` and the returned dx are
+    ``torch.bfloat16``; g, s1, s2, dy_scale and dg, ds1, ds2, dbias are fp32.  Defined as the fp32 backward on the widened
+    inputs: dx = bf16(dx_f32), rounded once; the parameter gradients are bit-identical to the fp32 call's."""
+    x, dy = _bf16c(x, "x"), _bf16c(dy, "dy")
+    g, s1, s2 = _f32c(g, "g"), _f32c(s1, "s1"), _f32c(s2, "s2")
+    S, B, D, xs = _layer_dims(x, g, s1, s2)
+    if dy.shape != (S, B, D):
+        raise RuntimeError(f"dy must be {(S, B, D)}, got {tuple(dy.shape)}")
+    if dy_scale is not None:
+        dy_scale = _f32c(dy_scale, "dy_scale").reshape(1)
+    if D > FUSED_BWD_MAX_D:   # the fp32 multi-pass backward on the widened inputs, dx rounded once at the end
+        dx, dg, ds1, ds2, dbias = _layer_backward_multipass(x.float(), dy.float(), g, s1, s2, want_dx, want_dbias, relu_in,
+                                                            None, None, dy_scale)
+        return (None if dx is None else dx.to(torch.bfloat16)), dg, ds1, ds2, dbias
+    if (B * D) % 8 != 0:
+        # D = 4 with an odd B: the kernel's bulk copies move whole 16-byte units per sample; one zero row of x and dy adds
+        # zero to every parameter gradient, so the padded call is exact
+        x, dy = F.pad(x, (0, 0, 0, 1)), F.pad(dy, (0, 0, 0, 1))
+        dx, dg, ds1, ds2, dbias = layer_backward_bf16(x, dy, g, s1, s2, want_dx, want_dbias, relu_in, dy_scale)
+        return (None if dx is None else dx[:, :B].contiguous()), dg, ds1, ds2, dbias
+    dev = x.device
+    dx = torch.empty((S, B, D), dtype=torch.bfloat16, device=dev) if want_dx else None
+    dg = torch.empty((S, D), dtype=torch.float32, device=dev)
+    ds1 = torch.empty(D, dtype=torch.float32, device=dev)
+    ds2 = torch.empty(D, dtype=torch.float32, device=dev)
+    dbias = torch.empty(D, dtype=torch.float32, device=dev) if want_dbias else None
+    ws = _workspace(dev, _query("whvi_layer_bwd_workspace_bytes", S, B, D)[0])
+    with torch.cuda.device(dev), _Timed("whvi_layer_bwd_bf16", ("shared_x" if xs == 0 else "distinct_x") + ("" if want_dx else "/nodx")):
+        rc = _lib.lib().whvi_layer_bwd_bf16(x.data_ptr(), xs, dy.data_ptr(), _ptr(dy_scale), g.data_ptr(), s1.data_ptr(),
+                                            s2.data_ptr(), _ptr(dx), dg.data_ptr(), ds1.data_ptr(), ds2.data_ptr(), _ptr(dbias),
+                                            ws.data_ptr(), ws.numel(), S, B, D, 1 if relu_in else 0, _stream(dev))
+    _lib.check(rc, "whvi_layer_bwd_bf16")
+    return dx, dg, ds1, ds2, dbias
+
+
 LOSS_LAYER_MIN_D, LOSS_LAYER_MAX_D = 128, 4096
 
 class DeferredScale:
@@ -431,8 +483,11 @@ class DeferredScale:
 
 def layer_loss_raw(x, g, s1, s2, bias, target, want_dx=True, relu_in=False):
     """Fused last layer (forward + squared-error residual + backward for a unit coefficient).
-    Returns (sum r^2 as a 0-d tensor, dx | None, dg, ds1, ds2, dbias | None)."""
-    x, g, s1, s2 = _f32c(x, "x"), _f32c(g, "g"), _f32c(s1, "s1"), _f32c(s2, "s2")
+    Returns (sum r^2 as a 0-d tensor, dx | None, dg, ds1, ds2, dbias | None).
+    A bfloat16 ``x`` selects ``whvi_layer_loss_bf16``: dx is then bf16 (rounded once), everything else as in fp32."""
+    bf16 = x.dtype == torch.bfloat16
+    x = _bf16c(x, "x") if bf16 else _f32c(x, "x")
+    g, s1, s2 = _f32c(g, "g"), _f32c(s1, "s1"), _f32c(s2, "s2")
     S, B, D, xs = _layer_dims(x, g, s1, s2)
     target = _f32c(target, "target")
     if target.shape != (B, D):
@@ -444,17 +499,18 @@ def layer_loss_raw(x, g, s1, s2, bias, target, want_dx=True, relu_in=False):
     need, nsq = _query("whvi_layer_loss_sizes", S, B, D)
     ws = _workspace(dev, need)
     sqp = torch.zeros(max(nsq, 1), dtype=torch.float32, device=dev)   # an upper bound: unused entries stay zero
-    dx = torch.empty((S, B, D), dtype=torch.float32, device=dev) if want_dx else None
+    dx = torch.empty((S, B, D), dtype=x.dtype, device=dev) if want_dx else None
     dg = torch.empty((S, D), dtype=torch.float32, device=dev)
     ds1 = torch.empty(D, dtype=torch.float32, device=dev)
     ds2 = torch.empty(D, dtype=torch.float32, device=dev)
     dbias = torch.empty(D, dtype=torch.float32, device=dev) if bias is not None else None
-    with torch.cuda.device(dev), _Timed("whvi_layer_loss_f32", ("shared_x" if xs == 0 else "distinct_x") + ("" if want_dx else "/nodx")):
-        rc = L.whvi_layer_loss_f32(x.data_ptr(), xs, g.data_ptr(), s1.data_ptr(), s2.data_ptr(), _ptr(bias),
-                                   target.data_ptr(), _ptr(dx), dg.data_ptr(), ds1.data_ptr(), ds2.data_ptr(),
-                                   _ptr(dbias), sqp.data_ptr(), ws.data_ptr(), ws.numel(), S, B, D,
-                                   1 if relu_in else 0, _stream(dev))
-    _lib.check(rc, "whvi_layer_loss_f32")
+    name = "whvi_layer_loss_bf16" if bf16 else "whvi_layer_loss_f32"
+    with torch.cuda.device(dev), _Timed(name, ("shared_x" if xs == 0 else "distinct_x") + ("" if want_dx else "/nodx")):
+        rc = getattr(L, name)(x.data_ptr(), xs, g.data_ptr(), s1.data_ptr(), s2.data_ptr(), _ptr(bias),
+                              target.data_ptr(), _ptr(dx), dg.data_ptr(), ds1.data_ptr(), ds2.data_ptr(),
+                              _ptr(dbias), sqp.data_ptr(), ws.data_ptr(), ws.numel(), S, B, D,
+                              1 if relu_in else 0, _stream(dev))
+    _lib.check(rc, name)
     return sqp.sum(), dx, dg, ds1, ds2, dbias
 
 
@@ -466,11 +522,16 @@ class WHVILayerFunction(Function):
     dx by x > 0, i.e. returns the gradient w.r.t. the PRODUCER's pre-activation.  The two
     flags are set in matching pairs by ``WHVINetwork`` (producer relu_out <-> consumer
     relu_in), which is what makes the chain rule come out right without the ReLU ever
-    touching HBM."""
+    touching HBM.
+
+    A bfloat16 ``x`` runs the bf16-activation kernels (output and dx bf16, parameter gradients fp32); the shared-input
+    transform is not hoisted then, because a bf16 t2 would add a rounding the fp32 composition does not have."""
 
     @staticmethod
     def forward(ctx, x, g, s1, s2, bias, relu_out=False, relu_in=False, dy_scale_from=None):
-        if x.dim() == 2 and g.size(0) >= 4 and g.size(-1) >= 128 and g.size(0) * x.numel() >= HOIST_MIN_ELEMENTS:
+        if x.dtype == torch.bfloat16:
+            y = layer_forward_bf16(x, g, s1, s2, bias, relu_out=relu_out)
+        elif x.dim() == 2 and g.size(0) >= 4 and g.size(-1) >= 128 and g.size(0) * x.numel() >= HOIST_MIN_ELEMENTS:
             # one (B, D) input block for all samples (the first layer of a network): the first transform does not depend
             # on the sample (SURVEY 8d C5), so it is done once -- t2 = H(s2 * x), one pass over B * D elements -- and every
             # (sample, row) pair costs one transform; the output stream is the same, the kernel 12% shorter (D = 4096)
@@ -490,7 +551,7 @@ class WHVILayerFunction(Function):
         want_db = ctx.has_bias and ctx.needs_input_grad[4]
         # dy came from a fused loss layer that left its loss coefficient in the shared holder
         scale = ctx.dy_scale_from.take() if ctx.dy_scale_from is not None else None
-        dx, dg, ds1, ds2, dbias = layer_backward_raw(x, dy, g, s1, s2, want_dx=want_dx, want_dbias=want_db,
+        dx, dg, ds1, ds2, dbias = layer_backward_raw(x, dy.contiguous(), g, s1, s2, want_dx=want_dx, want_dbias=want_db,
                                                      relu_in=ctx.relu_in, dy_scale=scale)
         if dx is not None and x.dim() == 2:
             dx = dx.sum(dim=0)
@@ -562,7 +623,12 @@ class WHVILayerLossFunction(Function):
     ``dx_scale_to``: a ``DeferredScale`` shared with the fused ``WHVILayerFunction`` that produced
     ``x`` and is its ONLY consumer (set by ``WHVINetwork._run`` in matching pairs, like
     relu_out/relu_in); ``dx`` is then handed on unscaled, the coefficient goes into the holder and
-    the producer's backward kernel applies it on load, saving a pass over dx."""
+    the producer's backward kernel applies it on load, saving a pass over dx.
+
+    bf16 ``x``: dx is bf16, rounded once by the kernel for the unit coefficient.  Handed on through ``dx_scale_to`` it is
+    scaled in fp32 inside the producer's backward, so the chain rounds once per layer boundary.  Without a holder (shared
+    x, a producer without the fused ReLU, a non-square producer) the coefficient is applied here to the bf16 dx, which
+    rounds a second time: bf16(bf16(dx) * c)."""
 
     @staticmethod
     def forward(ctx, x, g, s1, s2, bias, target, relu_in=False, dx_scale_to=None):

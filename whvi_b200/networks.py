@@ -245,8 +245,9 @@ class WHVINetwork(nn.Module, WHVI):
         h = head._run(X, S) if len(modules) > 1 else X
         if h.dim() == 2 or (h.dim() == 3 and h.stride(0) == 0):   # no WHVI layer before: one input block for all samples
             hh = h if h.dim() == 2 else h[0]
-            sum_y, sum_y2, _ = last.predictive_moments(hh.contiguous(), S)
+            sum_y, sum_y2, _ = last.predictive_moments(hh.float().contiguous(), S)
             return sum_y, sum_y2, S
+        h = h.float()   # bf16 activations: the head ran in bf16; the moments kernel is fp32 (the widening is exact)
         bias = None if last.bias is None else last.bias.reshape(-1)
         g = WF.reparam(last.g_mu, last.g_rho, last._draw_eps(S))
         sum_y = torch.empty(h.shape[1:], dtype=torch.float32, device=h.device)

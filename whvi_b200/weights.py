@@ -172,7 +172,10 @@ class WHVISquarePow2Matrix(nn.Module):
     def sample_lrt(self, h, *, bias=None, relu_out=False, relu_in=False, dy_scale_from=None):
         """W h for a fresh draw of g per MC sample (local reparameterisation).  The
         keyword arguments are the kernel-side fusions (bias add, ReLU on the way out, ReLU
-        mask on the way back); they default to the reference's plain behaviour."""
+        mask on the way back); they default to the reference's plain behaviour.  A bfloat16 ``h`` gives a bfloat16
+        result (bf16 activations, fp32 parameters and arithmetic; PAPER semantics only)."""
+        if h.dtype == torch.bfloat16 and self.semantics == "reference":
+            raise RuntimeError('WHVISquarePow2Matrix: bf16 activations are not supported with semantics="reference"')
         S, squeeze = self._resolve_samples(h)
         eps = self._draw_eps(S)
         if self.semantics == "reference":
@@ -194,7 +197,11 @@ class WHVISquarePow2Matrix(nn.Module):
 
     def forward_sqerr(self, h, target, *, relu_in=False):
         """Forward pass fused with sum (y - target)^2 (see functional.WHVILayerSqErrFunction).
-        h: (B, D) or (S, B, D); target: (B, D).  Returns ((S, B, D) predictions, 0-d sum)."""
+        h: (B, D) or (S, B, D); target: (B, D).  Returns ((S, B, D) predictions, 0-d sum).
+        bf16 ``h``: the bf16 forward, and the sum in torch from the widened predictions (the fused kernel is fp32 only)."""
+        if h.dtype == torch.bfloat16:
+            y = self.sample_lrt(h, bias=self.bias, relu_in=relu_in)
+            return y, (y.float() - target).square().sum()
         S, _ = self._resolve_samples(h)
         g = self._g(self._draw_eps(S))
         bias = None if self.bias is None else self.bias.reshape(-1)
@@ -323,6 +330,8 @@ class WHVIStackedMatrix(nn.Module):
     def forward(self, x, use_lrt=True, *, relu_out=False, relu_in=False):
         """x: (..., n_in) -> (..., n_out): zero-pad to D_in, apply every block, concatenate,
         add the bias, drop the padding outputs (src/weights.py:182-208)."""
+        if x.dtype == torch.bfloat16:
+            raise RuntimeError("WHVIStackedMatrix: bf16 activations are not supported (square layers only)")
         if self.grouped:
             if x.device.type != "cuda":
                 raise RuntimeError("whvi_b200 runs on CUDA only (no CPU fallback); move the module and its inputs to a GPU")
@@ -388,6 +397,8 @@ class WHVIColumnMatrix(nn.Module):
         return self.one_launch and sub.semantics == "paper" and sub.covariance == "diag"
 
     def forward(self, x, *, relu_out=False, relu_in=False):
+        if x.dtype == torch.bfloat16:
+            raise RuntimeError("WHVIColumnMatrix: bf16 activations are not supported (square layers only)")
         sub = self.weight_submodule
         S, squeeze = sub._resolve_samples(x)
         if self.fused:
