@@ -232,6 +232,29 @@ WHVI_API int whvi_kl_dense_f32(const float* mu, const float* L, float lambda_, i
                                float grad_scale, void* workspace, size_t workspace_bytes, whvi_stream_t stream);
 
 /*
+ * Grouped dense reparameterisation and KL: G blocks at once (the square blocks of a Stacked layer; G = 1 is a square or
+ * Column layer), D <= 64 or a multiple of 128 (every power of two).  Block k's mu is read at + k * mu_stride floats and its L (D, D) at + k * L_stride
+ * (strides >= D and D * D; multiples of 4 at D >= 128); entries of L above the diagonal are ignored.  eps, g, dg: (G, S, D);
+ * dmu (G, D) and dL (G, D, D) are written densely, dL zero above the diagonal.
+ *   D <= 64   one CUDA-core launch per direction for all blocks; L_k in shared memory; fixed-order fp32 sums (j ascending
+ *             forward, s ascending backward): bit-reproducible.  No workspace.
+ *   D >= 128  the tcgen05 kernels of whvi_reparam_dense_f32 / whvi_reparam_dense_bwd_f32, one launch (sequence) per block, so
+ *             g and dL equal those calls' bit for bit; the backward writes the transposed, zero-padded GEMM operands into the
+ *             workspace itself, and dmu is a device column sum (samples ascending).
+ *   whvi_reparam_dense_grouped_workspace_bytes   bytes for either direction at (S, D) (0 below 128), reused block after block
+ *   whvi_kl_dense_grouped_f32   sum over the blocks of the whvi_kl_dense_f32 term (fp64 accumulation, fixed order); dmu (G, D),
+ *                               dL (G, D, D), both or neither; workspace: G * D doubles
+ */
+WHVI_API int whvi_reparam_dense_grouped_workspace_bytes(int64_t S, int64_t D, size_t* bytes);
+WHVI_API int whvi_reparam_dense_grouped_f32(const float* mu, int64_t mu_stride, const float* L, int64_t L_stride, const float* eps, float* g,
+                                            int64_t S, int64_t D, int64_t G, void* workspace, size_t workspace_bytes, whvi_stream_t stream);
+WHVI_API int whvi_reparam_dense_grouped_bwd_f32(const float* eps, const float* dg, float* dmu, float* dL, int64_t S, int64_t D, int64_t G,
+                                                void* workspace, size_t workspace_bytes, whvi_stream_t stream);
+WHVI_API int whvi_kl_dense_grouped_f32(const float* mu, int64_t mu_stride, const float* L, int64_t L_stride, float lambda_, int64_t D,
+                                       int64_t G, float* out_kl, float* dmu, float* dL, float grad_scale, void* workspace,
+                                       size_t workspace_bytes, whvi_stream_t stream);
+
+/*
  * WHVIStackedMatrix (src/weights.py:111-208) as ONE call per direction: the G = ceil(n_out / D) square blocks of a
  * non-square layer run as a second sample axis of the fused layer kernels instead of G launches + torch.cat (:179-180),
  * with the reparameterisation (:82-83), the bias add (:204-205), the ReLU that follows the layer, the concatenation and
@@ -256,6 +279,16 @@ WHVI_API int whvi_stacked_bwd_f32(const float* x, int64_t x_sample_stride, const
                                   float* dmu, float* drho, float* ds1, float* ds2, float* dbias, void* workspace,
                                   size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags,
                                   whvi_stream_t stream);
+/* The same layer from g (G, S, D) given, however it was drawn (e.g. whvi_reparam_dense_grouped_f32): the forward without the
+ * reparameterisation, the backward returning dg (G, S, D) in place of dmu, drho (workspace from whvi_stacked_bwd_workspace_bytes).
+ * whvi_stacked_fwd_f32 / whvi_stacked_bwd_f32 are the diagonal reparameterisation around these two. */
+WHVI_API int whvi_stacked_fwd_g_f32(const float* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2,
+                                    int64_t param_stride, const float* bias, float* y_blocks, float* y, int64_t S, int64_t B, int64_t D,
+                                    int64_t G, int64_t n_out, int flags, whvi_stream_t stream);
+WHVI_API int whvi_stacked_bwd_g_f32(const float* x, int64_t x_sample_stride, const float* dy, const float* g, const float* s1,
+                                    const float* s2, int64_t param_stride, float* dx, int64_t n_in, float* dg, float* ds1, float* ds2,
+                                    float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t G,
+                                    int64_t n_out, int flags, whvi_stream_t stream);
 /* sum of the G blocks' KL terms (WHVIStackedMatrix.kl, src/weights.py:162-164) and their gradients (G, D), one launch */
 WHVI_API int whvi_kl_grouped_f32(const float* mu, const float* rho, float lambda_, int64_t D, int64_t G, int64_t param_stride,
                                  int mode, float* out_kl, float* dmu, float* drho, float grad_scale, whvi_stream_t stream);
@@ -278,6 +311,16 @@ WHVI_API int whvi_column_bwd_f32(const float* x, int64_t x_sample_stride, const 
                                  const float* s1, const float* s2, const float* eps, float* dx, float* dmu, float* drho, float* ds1,
                                  float* ds2, float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D,
                                  int64_t n, int transposed, int flags, whvi_stream_t stream);
+/* The same layer from g (S, D) given: the forward without the reparameterisation (g is read, hg = H g written), the backward
+ * returning dg (S, D) in place of dmu, drho (workspace from whvi_column_bwd_workspace_bytes).  whvi_column_fwd_f32 /
+ * whvi_column_bwd_f32 are the diagonal reparameterisation around these two. */
+WHVI_API int whvi_column_fwd_g_f32(const float* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2,
+                                   const float* bias, float* hg, float* y, int64_t S, int64_t B, int64_t D, int64_t n, int transposed,
+                                   int flags, whvi_stream_t stream);
+WHVI_API int whvi_column_bwd_g_f32(const float* x, int64_t x_sample_stride, const float* dy, const float* hg, const float* s1,
+                                   const float* s2, float* dx, float* dg, float* ds1, float* ds2, float* dbias, void* workspace,
+                                   size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int flags,
+                                   whvi_stream_t stream);
 
 /* dmu = sum_s dg[s];  drho = (sum_s dg[s]*eps[s]) * sigmoid(rho).  accumulate != 0: += */
 WHVI_API int whvi_reparam_bwd_f32(const float* rho, const float* eps, const float* dg, float* dmu, float* drho,

@@ -54,6 +54,22 @@ SIGNATURES = {
     "whvi_reparam_dense_bwd_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p]),
     "whvi_kl_dense_f32": (c_int, [c_void_p, c_void_p, c_float, c_int64, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_size_t,
                                   c_void_p]),
+    "whvi_reparam_dense_grouped_workspace_bytes": (c_int, [c_int64, c_int64, POINTER(c_size_t)]),
+    "whvi_reparam_dense_grouped_f32": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_int64,
+                                               c_void_p, c_size_t, c_void_p]),
+    "whvi_reparam_dense_grouped_bwd_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_size_t,
+                                                   c_void_p]),
+    "whvi_kl_dense_grouped_f32": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_float, c_int64, c_int64, c_void_p, c_void_p, c_void_p,
+                                          c_float, c_void_p, c_size_t, c_void_p]),
+    "whvi_stacked_fwd_g_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64,
+                                       c_int64, c_int64, c_int64, c_int64, c_int, c_void_p]),
+    "whvi_stacked_bwd_g_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p,
+                                       c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_int64, c_int64, c_int,
+                                       c_void_p]),
+    "whvi_column_fwd_g_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64,
+                                      c_int64, c_int64, c_int, c_int, c_void_p]),
+    "whvi_column_bwd_g_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                      c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
     "whvi_pad_rows_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p]),
     "whvi_stacked_fwd_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
                                      c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_int64, c_int, c_void_p]),

@@ -337,6 +337,83 @@ int whvi_kl_dense_f32(const float* mu, const float* L, float lambda_, int64_t D,
     return launch_kl_dense(mu, L, lambda_, D, out_kl, dmu, dL, grad_scale, static_cast<double*>(workspace), static_cast<cudaStream_t>(stream));
 }
 
+static int check_dense_grouped(const char* who, int64_t S, int64_t D, int64_t G, int64_t mu_stride, int64_t L_stride)
+{
+    if (S < 0 || D < 1 || G < 1 || (D > 64 && D % 128 != 0))
+        return fail(WHVI_E_SHAPE, "%s: S=%lld D=%lld G=%lld (D <= 64 or a multiple of 128)", who, (long long)S, (long long)D, (long long)G);
+    if (G > 65535) return fail(WHVI_E_SHAPE, "%s: G=%lld above 65535", who, (long long)G);
+    if (G > 1 && (mu_stride < D || L_stride < D * D))
+        return fail(WHVI_E_SHAPE, "%s: mu_stride=%lld must be >= D and L_stride=%lld >= D * D", who, (long long)mu_stride, (long long)L_stride);
+    if (D >= 128 && G > 1 && (mu_stride % 4 != 0 || L_stride % 4 != 0))
+        return fail(WHVI_E_SHAPE, "%s: strides must be multiples of 4 at D >= 128", who);
+    if (S * G > 0x7fffffffLL) return fail(WHVI_E_SHAPE, "%s: too many samples", who);
+    return WHVI_OK;
+}
+
+int whvi_reparam_dense_grouped_workspace_bytes(int64_t S, int64_t D, size_t* bytes)
+{
+    if (!bytes) return fail(WHVI_E_NULL, "reparam_dense_grouped_workspace_bytes: null pointer");
+    if (int rc = check_dense_grouped("reparam_dense_grouped_workspace_bytes", S, D, 1, D, D * D)) return rc;
+    *bytes = reparam_dense_grouped_workspace_bytes(S, D);
+    return WHVI_OK;
+}
+
+int whvi_reparam_dense_grouped_f32(const float* mu, int64_t mu_stride, const float* L, int64_t L_stride, const float* eps, float* g, int64_t S,
+                                   int64_t D, int64_t G, void* workspace, size_t workspace_bytes, whvi_stream_t stream)
+{
+    if (int rc = check_dense_grouped("reparam_dense_grouped", S, D, G, mu_stride, L_stride)) return rc;
+    if (S == 0) return WHVI_OK;
+    if (!mu || !L || !eps || !g) return fail(WHVI_E_NULL, "reparam_dense_grouped: null pointer");
+    if (D >= 128) {
+        if (!aligned16(L) || !aligned16(eps) || !aligned16(workspace))
+            return fail(WHVI_E_ALIGN, "reparam_dense_grouped: L, eps and the workspace must be 16-byte aligned at D >= 128");
+        if (!workspace || workspace_bytes < reparam_dense_grouped_workspace_bytes(S, D))
+            return fail(WHVI_E_WORKSPACE, "reparam_dense_grouped: workspace of %zu bytes needed, %zu given", reparam_dense_grouped_workspace_bytes(S, D),
+                        workspace_bytes);
+    }
+    return launch_reparam_dense_grouped(mu, mu_stride, L, L_stride, eps, g, S, D, G, static_cast<float*>(workspace), workspace_bytes,
+                                        static_cast<cudaStream_t>(stream));
+}
+
+int whvi_reparam_dense_grouped_bwd_f32(const float* eps, const float* dg, float* dmu, float* dL, int64_t S, int64_t D, int64_t G, void* workspace,
+                                       size_t workspace_bytes, whvi_stream_t stream)
+{
+    if (int rc = check_dense_grouped("reparam_dense_grouped_bwd", S, D, G, D, D * D)) return rc;
+    if (!dmu || !dL) return fail(WHVI_E_NULL, "reparam_dense_grouped_bwd: null output pointer");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (S == 0) {
+        cudaMemsetAsync(dmu, 0, sizeof(float) * size_t(G) * D, st);
+        cudaMemsetAsync(dL, 0, sizeof(float) * size_t(G) * D * D, st);
+        return check_launch("reparam_dense_grouped_bwd(empty)");
+    }
+    if (!eps || !dg) return fail(WHVI_E_NULL, "reparam_dense_grouped_bwd: null pointer");
+    if (D >= 128) {
+        if (!aligned16(dL) || !aligned16(workspace))
+            return fail(WHVI_E_ALIGN, "reparam_dense_grouped_bwd: dL and the workspace must be 16-byte aligned at D >= 128");
+        if (!workspace || workspace_bytes < reparam_dense_grouped_workspace_bytes(S, D))
+            return fail(WHVI_E_WORKSPACE, "reparam_dense_grouped_bwd: workspace of %zu bytes needed, %zu given",
+                        reparam_dense_grouped_workspace_bytes(S, D), workspace_bytes);
+    }
+    return launch_reparam_dense_grouped_bwd(eps, dg, dmu, dL, S, D, G, static_cast<float*>(workspace), workspace_bytes, st);
+}
+
+int whvi_kl_dense_grouped_f32(const float* mu, int64_t mu_stride, const float* L, int64_t L_stride, float lambda_, int64_t D, int64_t G,
+                              float* out_kl, float* dmu, float* dL, float grad_scale, void* workspace, size_t workspace_bytes,
+                              whvi_stream_t stream)
+{
+    if (D < 1 || D > 65535 || G < 1 || G > 65535 || (G > 1 && (mu_stride < D || L_stride < D * D)))
+        return fail(WHVI_E_SHAPE, "kl_dense_grouped: D=%lld G=%lld mu_stride=%lld L_stride=%lld", (long long)D, (long long)G, (long long)mu_stride,
+                    (long long)L_stride);
+    if (!(lambda_ > 0.f)) return fail(WHVI_E_SHAPE, "kl_dense_grouped: lambda must be positive");
+    if (!mu || !L || !out_kl) return fail(WHVI_E_NULL, "kl_dense_grouped: null pointer");
+    if ((dmu == nullptr) != (dL == nullptr)) return fail(WHVI_E_NULL, "kl_dense_grouped: dmu and dL must both be given or both NULL");
+    const size_t need = sizeof(double) * size_t(G) * size_t(D);
+    if (!workspace || workspace_bytes < need || (reinterpret_cast<uintptr_t>(workspace) & 7u))
+        return fail(WHVI_E_WORKSPACE, "kl_dense_grouped: workspace of %zu bytes (8-byte aligned) needed", need);
+    return launch_kl_dense_grouped(mu, mu_stride, L, L_stride, lambda_, D, G, out_kl, dmu, dL, grad_scale, static_cast<double*>(workspace),
+                                   static_cast<cudaStream_t>(stream));
+}
+
 int whvi_reparam_bwd_f32(const float* rho, const float* eps, const float* dg, float* dmu, float* drho, int64_t S,
                          int64_t D, int mode, int accumulate, whvi_stream_t stream)
 {
@@ -378,6 +455,18 @@ int whvi_pad_rows_f32(const float* in, float* out, int64_t rows, int64_t n_in, i
     return launch_stack_split(in, out, rows, D, 1, n_in, static_cast<cudaStream_t>(stream));
 }
 
+// the layer from g (G, S, D), however g was drawn; validated by the callers
+static int stacked_fwd_g(const float* x, int64_t xs, const float* g, const float* s1, const float* s2, int64_t param_stride, const float* bias,
+                         float* y_blocks, float* y, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, cudaStream_t st)
+{
+    LayerFwdCall c{x, g, s1, s2, bias, nullptr, y_blocks, nullptr, xs, G * S, B, flags & WHVI_LAYER_RELU_OUT, nullptr};
+    c.groups = G;
+    c.pstride = param_stride;
+    c.bstride = D;
+    if (int rc = launch_layer_fwd(c, D, st)) return rc;
+    return launch_stack_concat(y_blocks, y, S * B, D, G, n_out, st);
+}
+
 int whvi_stacked_fwd_f32(const float* x, int64_t x_sample_stride, const float* mu, const float* rho, const float* s1, const float* s2,
                          int64_t param_stride, const float* eps, const float* bias, float* g, float* y_blocks, float* y, int64_t S,
                          int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, whvi_stream_t stream)
@@ -390,12 +479,21 @@ int whvi_stacked_fwd_f32(const float* x, int64_t x_sample_stride, const float* m
         return fail(WHVI_E_ALIGN, "stacked_fwd: pointers must be 16-byte aligned");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (int rc = launch_reparam_diag(mu, rho, eps, g, G * S, D, st, G, param_stride)) return rc;
-    LayerFwdCall c{x, g, s1, s2, bias, nullptr, y_blocks, nullptr, x_sample_stride, G * S, B, flags & WHVI_LAYER_RELU_OUT, nullptr};
-    c.groups = G;
-    c.pstride = param_stride;
-    c.bstride = D;
-    if (int rc = launch_layer_fwd(c, D, st)) return rc;
-    return launch_stack_concat(y_blocks, y, S * B, D, G, n_out, st);
+    return stacked_fwd_g(x, x_sample_stride, g, s1, s2, param_stride, bias, y_blocks, y, S, B, D, G, n_out, flags, st);
+}
+
+int whvi_stacked_fwd_g_f32(const float* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2, int64_t param_stride,
+                           const float* bias, float* y_blocks, float* y, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags,
+                           whvi_stream_t stream)
+{
+    if (int rc = check_stacked("stacked_fwd_g", S, B, D, G, n_out, x_sample_stride, param_stride)) return rc;
+    if (flags & ~WHVI_LAYER_RELU_OUT) return fail(WHVI_E_MODE, "stacked_fwd_g: unknown flags %d", flags);
+    if (S == 0 || B == 0) return WHVI_OK;
+    if (!x || !g || !s1 || !s2 || !y_blocks || !y) return fail(WHVI_E_NULL, "stacked_fwd_g: null pointer");
+    if (!aligned16(x) || !aligned16(s1) || !aligned16(s2) || !aligned16(bias) || !aligned16(g) || !aligned16(y_blocks))
+        return fail(WHVI_E_ALIGN, "stacked_fwd_g: pointers must be 16-byte aligned");
+    return stacked_fwd_g(x, x_sample_stride, g, s1, s2, param_stride, bias, y_blocks, y, S, B, D, G, n_out, flags,
+                         static_cast<cudaStream_t>(stream));
 }
 
 static size_t stacked_bwd_layout(int64_t S, int64_t B, int64_t D, int64_t G, int want_dx, size_t layer_ws, size_t* off_dx, size_t* off_dg,
@@ -429,6 +527,37 @@ int whvi_stacked_bwd_workspace_bytes(int64_t S, int64_t B, int64_t D, int64_t G,
     return WHVI_OK;
 }
 
+static int stacked_bwd_plan(const char* who, int64_t S, int64_t B, int64_t D, int64_t G, int want_dx, const void* workspace,
+                            size_t workspace_bytes, size_t* layer_ws, size_t* off_dx, size_t* off_dg, size_t* off_ws)
+{
+    *layer_ws = 0;
+    LayerBwdCall q{};
+    q.S = S * G;
+    q.B = B;
+    q.need_only = layer_ws;
+    if (int rc = launch_layer_bwd(q, D, nullptr)) return rc;
+    const size_t need = stacked_bwd_layout(S, B, D, G, want_dx, *layer_ws, off_dx, off_dg, off_ws);
+    if (!workspace || workspace_bytes < need) return fail(WHVI_E_WORKSPACE, "%s: workspace of %zu bytes needed, %zu given", who, need, workspace_bytes);
+    return WHVI_OK;
+}
+
+// the layer's backward from dy (S, B, n_out) down to dg (G, S, D) and the per-block dx (left in the workspace for the caller's
+// block sum); validated and planned by the callers
+static int stacked_bwd_g(const float* x, int64_t xs, const float* dy, const float* g, const float* s1, const float* s2, int64_t param_stride,
+                         float* dx, float* dg, float* ds1, float* ds2, float* dbias, void* workspace, size_t layer_ws, size_t off_dx,
+                         size_t off_ws, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, cudaStream_t st)
+{
+    char* base = static_cast<char*>(workspace);
+    float* dyb = reinterpret_cast<float*>(base);
+    float* dxb = dx ? reinterpret_cast<float*>(base + off_dx) : nullptr;
+    if (int rc = launch_stack_split(dy, dyb, S * B, D, G, n_out, st)) return rc;
+    LayerBwdCall c{x, dyb, g, s1, s2, nullptr, nullptr, nullptr, dxb, dg, ds1, ds2, dbias, reinterpret_cast<float*>(base + off_ws),
+                   layer_ws, xs, S * G, B, flags & WHVI_LAYER_RELU_IN, nullptr};
+    c.groups = G;
+    c.pstride = param_stride;
+    return launch_layer_bwd(c, D, st);
+}
+
 int whvi_stacked_bwd_f32(const float* x, int64_t x_sample_stride, const float* dy, const float* g, const float* rho, const float* s1,
                          const float* s2, int64_t param_stride, const float* eps, float* dx, int64_t n_in, float* dmu, float* drho,
                          float* ds1, float* ds2, float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D,
@@ -447,29 +576,43 @@ int whvi_stacked_bwd_f32(const float* x, int64_t x_sample_stride, const float* d
     if (!x || !dy || !g || !rho || !s1 || !s2 || !eps) return fail(WHVI_E_NULL, "stacked_bwd: null pointer");
     if (!aligned16(x) || !aligned16(g) || !aligned16(s1) || !aligned16(s2) || !aligned16(workspace))
         return fail(WHVI_E_ALIGN, "stacked_bwd: pointers must be 16-byte aligned");
-    size_t layer_ws = 0;
-    {
-        LayerBwdCall q{};
-        q.S = S * G;
-        q.B = B;
-        q.need_only = &layer_ws;
-        if (int rc = launch_layer_bwd(q, D, nullptr)) return rc;
-    }
-    size_t off_dx, off_dg, off_ws;
-    const size_t need = stacked_bwd_layout(S, B, D, G, dx != nullptr, layer_ws, &off_dx, &off_dg, &off_ws);
-    if (!workspace || workspace_bytes < need) return fail(WHVI_E_WORKSPACE, "stacked_bwd: workspace of %zu bytes needed, %zu given", need, workspace_bytes);
-    char* base = static_cast<char*>(workspace);
-    float* dyb = reinterpret_cast<float*>(base);
-    float* dxb = dx ? reinterpret_cast<float*>(base + off_dx) : nullptr;
-    float* dg = reinterpret_cast<float*>(base + off_dg);
-    if (int rc = launch_stack_split(dy, dyb, S * B, D, G, n_out, st)) return rc;
-    LayerBwdCall c{x, dyb, g, s1, s2, nullptr, nullptr, nullptr, dxb, dg, ds1, ds2, dbias, reinterpret_cast<float*>(base + off_ws),
-                   layer_ws, x_sample_stride, S * G, B, flags & WHVI_LAYER_RELU_IN, nullptr};
-    c.groups = G;
-    c.pstride = param_stride;
-    if (int rc = launch_layer_bwd(c, D, st)) return rc;
+    size_t off_dx, off_dg, off_ws, layer_ws;
+    if (int rc = stacked_bwd_plan("stacked_bwd", S, B, D, G, dx != nullptr, workspace, workspace_bytes, &layer_ws, &off_dx, &off_dg, &off_ws))
+        return rc;
+    float* dg = reinterpret_cast<float*>(static_cast<char*>(workspace) + off_dg);
+    if (int rc = stacked_bwd_g(x, x_sample_stride, dy, g, s1, s2, param_stride, dx, dg, ds1, ds2, dbias, workspace, layer_ws, off_dx,
+                               off_ws, S, B, D, G, n_out, flags, st))
+        return rc;
     if (int rc = launch_reparam_diag_bwd(rho, eps, dg, dmu, drho, S, D, 0, st, G, param_stride)) return rc;
-    if (dx) return launch_stack_sum(dxb, dx, S * B, D, G, n_in, st);
+    if (dx) return launch_stack_sum(reinterpret_cast<float*>(static_cast<char*>(workspace) + off_dx), dx, S * B, D, G, n_in, st);
+    return WHVI_OK;
+}
+
+int whvi_stacked_bwd_g_f32(const float* x, int64_t x_sample_stride, const float* dy, const float* g, const float* s1, const float* s2,
+                           int64_t param_stride, float* dx, int64_t n_in, float* dg, float* ds1, float* ds2, float* dbias, void* workspace,
+                           size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, whvi_stream_t stream)
+{
+    if (int rc = check_stacked("stacked_bwd_g", S, B, D, G, n_out, x_sample_stride, param_stride)) return rc;
+    if (flags & ~WHVI_LAYER_RELU_IN) return fail(WHVI_E_MODE, "stacked_bwd_g: unknown flags %d", flags);
+    if (dx && (n_in < 1 || n_in > D)) return fail(WHVI_E_SHAPE, "stacked_bwd_g: n_in=%lld outside [1, D]", (long long)n_in);
+    if (!dg || !ds1 || !ds2) return fail(WHVI_E_NULL, "stacked_bwd_g: null output pointer");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (S == 0 || B == 0) {
+        if (S > 0) cudaMemsetAsync(dg, 0, sizeof(float) * size_t(G) * S * D, st);
+        for (float* p : {ds1, ds2, dbias})
+            if (p) cudaMemsetAsync(p, 0, sizeof(float) * size_t(G) * D, st);
+        return check_launch("stacked_bwd_g(empty)");
+    }
+    if (!x || !dy || !g || !s1 || !s2) return fail(WHVI_E_NULL, "stacked_bwd_g: null pointer");
+    if (!aligned16(x) || !aligned16(g) || !aligned16(s1) || !aligned16(s2) || !aligned16(dg) || !aligned16(workspace))
+        return fail(WHVI_E_ALIGN, "stacked_bwd_g: pointers must be 16-byte aligned");
+    size_t off_dx, off_dg, off_ws, layer_ws;
+    if (int rc = stacked_bwd_plan("stacked_bwd_g", S, B, D, G, dx != nullptr, workspace, workspace_bytes, &layer_ws, &off_dx, &off_dg, &off_ws))
+        return rc;
+    if (int rc = stacked_bwd_g(x, x_sample_stride, dy, g, s1, s2, param_stride, dx, dg, ds1, ds2, dbias, workspace, layer_ws, off_dx,
+                               off_ws, S, B, D, G, n_out, flags, st))
+        return rc;
+    if (dx) return launch_stack_sum(reinterpret_cast<float*>(static_cast<char*>(workspace) + off_dx), dx, S * B, D, G, n_in, st);
     return WHVI_OK;
 }
 
@@ -538,6 +681,43 @@ int whvi_column_bwd_f32(const float* x, int64_t x_sample_stride, const float* dy
     if (!workspace || workspace_bytes < need) return fail(WHVI_E_WORKSPACE, "column_bwd: workspace of %zu bytes needed, %zu given", need, workspace_bytes);
     return launch_column_bwd(x, x_sample_stride, dy, hg, rho, s1, s2, eps, dx, dmu, drho, ds1, ds2, dbias, static_cast<float*>(workspace), S,
                              B, D, n, transposed, flags & WHVI_LAYER_RELU_IN, st);
+}
+
+int whvi_column_fwd_g_f32(const float* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2, const float* bias, float* hg,
+                          float* y, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int flags, whvi_stream_t stream)
+{
+    if (int rc = check_column("column_fwd_g", S, B, D, n, x_sample_stride, transposed)) return rc;
+    if (flags & ~WHVI_LAYER_RELU_OUT) return fail(WHVI_E_MODE, "column_fwd_g: unknown flags %d", flags);
+    if ((flags & WHVI_LAYER_RELU_OUT) && transposed) return fail(WHVI_E_MODE, "column_fwd_g: RELU_OUT applies to the (.., 1) -> (.., n) form only");
+    if (S == 0 || B == 0) return WHVI_OK;
+    if (!x || !g || !s1 || !s2 || !hg || !y) return fail(WHVI_E_NULL, "column_fwd_g: null pointer");
+    if (!aligned16(g) || !aligned16(hg)) return fail(WHVI_E_ALIGN, "column_fwd_g: g and hg must be 16-byte aligned");
+    return launch_column_fwd_g(x, x_sample_stride, g, s1, s2, bias, hg, y, S, B, D, n, transposed, flags & WHVI_LAYER_RELU_OUT,
+                               static_cast<cudaStream_t>(stream));
+}
+
+int whvi_column_bwd_g_f32(const float* x, int64_t x_sample_stride, const float* dy, const float* hg, const float* s1, const float* s2, float* dx,
+                          float* dg, float* ds1, float* ds2, float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D,
+                          int64_t n, int transposed, int flags, whvi_stream_t stream)
+{
+    if (int rc = check_column("column_bwd_g", S, B, D, n, x_sample_stride, transposed)) return rc;
+    if (flags & ~WHVI_LAYER_RELU_IN) return fail(WHVI_E_MODE, "column_bwd_g: unknown flags %d", flags);
+    if ((flags & WHVI_LAYER_RELU_IN) && !transposed) return fail(WHVI_E_MODE, "column_bwd_g: RELU_IN applies to the (.., n) -> (.., 1) form only");
+    if (!dg || !ds1 || !ds2) return fail(WHVI_E_NULL, "column_bwd_g: null output pointer");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (S == 0 || B == 0) {
+        if (S > 0) cudaMemsetAsync(dg, 0, sizeof(float) * size_t(S) * D, st);
+        cudaMemsetAsync(ds1, 0, sizeof(float) * size_t(D), st);
+        cudaMemsetAsync(ds2, 0, sizeof(float) * size_t(D), st);
+        if (dbias) cudaMemsetAsync(dbias, 0, sizeof(float) * size_t(transposed ? 1 : n), st);
+        return check_launch("column_bwd_g(empty)");
+    }
+    if (!x || !dy || !hg || !s1 || !s2) return fail(WHVI_E_NULL, "column_bwd_g: null pointer");
+    if (!aligned16(workspace) || !aligned16(dg)) return fail(WHVI_E_ALIGN, "column_bwd_g: workspace and dg must be 16-byte aligned");
+    const size_t need = column_bwd_workspace_bytes(S, D, n);
+    if (!workspace || workspace_bytes < need) return fail(WHVI_E_WORKSPACE, "column_bwd_g: workspace of %zu bytes needed, %zu given", need, workspace_bytes);
+    return launch_column_bwd_g(x, x_sample_stride, dy, hg, s1, s2, dx, dg, ds1, ds2, dbias, static_cast<float*>(workspace), S, B, D, n, transposed,
+                               flags & WHVI_LAYER_RELU_IN, st);
 }
 
 int whvi_layer_moments_f32(const float* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2,

@@ -187,11 +187,10 @@ static unsigned ew_grid(int64_t total)
     return static_cast<unsigned>(b < 1 ? 1 : b);
 }
 
-int launch_column_fwd(const float* x, int64_t xs, const float* mu, const float* rho, const float* s1, const float* s2, const float* eps,
-                      const float* bias, float* g, float* hg, float* y, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int relu_out,
-                      cudaStream_t st)
+// the layer from g (S, D), however g was drawn: hg = H g, then the 1-wide product
+int launch_column_fwd_g(const float* x, int64_t xs, const float* g, const float* s1, const float* s2, const float* bias, float* hg, float* y,
+                        int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int relu_out, cudaStream_t st)
 {
-    if (int rc = launch_reparam_diag(mu, rho, eps, g, S, D, st)) return rc;
     if (int rc = launch_fwht(g, hg, S, D, st)) return rc;
     if (transposed) {
         const int64_t blocks = (S * B + 7) / 8;
@@ -203,6 +202,14 @@ int launch_column_fwd(const float* x, int64_t xs, const float* mu, const float* 
     return check_launch("column_outer_kernel");
 }
 
+int launch_column_fwd(const float* x, int64_t xs, const float* mu, const float* rho, const float* s1, const float* s2, const float* eps,
+                      const float* bias, float* g, float* hg, float* y, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int relu_out,
+                      cudaStream_t st)
+{
+    if (int rc = launch_reparam_diag(mu, rho, eps, g, S, D, st)) return rc;
+    return launch_column_fwd_g(x, xs, g, s1, s2, bias, hg, y, S, B, D, n, transposed, relu_out, st);
+}
+
 static int64_t up4(int64_t v) { return (v + 3) / 4 * 4; }   // every segment starts 16-byte aligned (the FWHT reads float4s)
 
 size_t column_bwd_workspace_bytes(int64_t S, int64_t D, int64_t n)
@@ -211,13 +218,13 @@ size_t column_bwd_workspace_bytes(int64_t S, int64_t D, int64_t n)
     return sizeof(float) * size_t(2 * up4(S * D) + up4(S * n) + up4((D + 255) / 256));
 }
 
-int launch_column_bwd(const float* x, int64_t xs, const float* dy, const float* hg, const float* rho, const float* s1, const float* s2,
-                      const float* eps, float* dx, float* dmu, float* drho, float* ds1, float* ds2, float* dbias, float* ws, int64_t S,
-                      int64_t B, int64_t D, int64_t n, int transposed, int relu_in, cudaStream_t st)
+// the layer's backward down to dg (S, D); ws as column_bwd_workspace_bytes (its dg segment stays unused when dg is the caller's)
+int launch_column_bwd_g(const float* x, int64_t xs, const float* dy, const float* hg, const float* s1, const float* s2, float* dx, float* dg,
+                        float* ds1, float* ds2, float* dbias, float* ws, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int relu_in,
+                        cudaStream_t st)
 {
     float* dhg = ws;
-    float* dg = dhg + up4(S * D);
-    float* dwp = dg + up4(S * D);
+    float* dwp = dhg + 2 * up4(S * D);
     float* part = dwp + up4(S * n);
     const int Di = static_cast<int>(D), ni = static_cast<int>(n);
     const dim3 dwgrid(static_cast<unsigned>((n + 31) / 32), static_cast<unsigned>(S));
@@ -246,7 +253,15 @@ int launch_column_bwd(const float* x, int64_t xs, const float* dy, const float* 
     if (int rc = check_launch("column_param_kernel")) return rc;
     column_ds1_kernel<<<1, 256, 0, st>>>(part, nparts, ds1, Di);
     if (int rc = check_launch("column_ds1_kernel")) return rc;
-    if (int rc = launch_fwht(dhg, dg, S, D, st)) return rc;   // dg = H dhg (H is symmetric)
+    return launch_fwht(dhg, dg, S, D, st);   // dg = H dhg (H is symmetric)
+}
+
+int launch_column_bwd(const float* x, int64_t xs, const float* dy, const float* hg, const float* rho, const float* s1, const float* s2,
+                      const float* eps, float* dx, float* dmu, float* drho, float* ds1, float* ds2, float* dbias, float* ws, int64_t S,
+                      int64_t B, int64_t D, int64_t n, int transposed, int relu_in, cudaStream_t st)
+{
+    float* dg = ws + up4(S * D);
+    if (int rc = launch_column_bwd_g(x, xs, dy, hg, s1, s2, dx, dg, ds1, ds2, dbias, ws, S, B, D, n, transposed, relu_in, st)) return rc;
     return launch_reparam_diag_bwd(rho, eps, dg, dmu, drho, S, D, 0, st);
 }
 

@@ -104,6 +104,18 @@ int launch_reparam_dense(const float* mu, const float* L, const float* eps, floa
 int launch_reparam_dense_bwd(const float* dgT, const float* eT, float* dL, int64_t Sp, int64_t D, cudaStream_t stream);
 int launch_kl_dense(const float* mu, const float* L, float lambda_, int64_t D, float* out, float* dmu, float* dL, float grad_scale,
                     double* row_sq, cudaStream_t stream);
+size_t reparam_dense_grouped_workspace_bytes(int64_t S, int64_t D);
+int launch_reparam_dense_grouped(const float* mu, int64_t mu_stride, const float* L, int64_t L_stride, const float* eps, float* g, int64_t S,
+                                 int64_t D, int64_t G, float* ws, size_t ws_bytes, cudaStream_t stream);
+int launch_reparam_dense_grouped_bwd(const float* eps, const float* dg, float* dmu, float* dL, int64_t S, int64_t D, int64_t G, float* ws,
+                                     size_t ws_bytes, cudaStream_t stream);
+int launch_kl_dense_grouped(const float* mu, int64_t mu_stride, const float* L, int64_t L_stride, float lambda_, int64_t D, int64_t G, float* out,
+                            float* dmu, float* dL, float grad_scale, double* row_sq, cudaStream_t stream);
+int launch_column_fwd_g(const float* x, int64_t xs, const float* g, const float* s1, const float* s2, const float* bias, float* hg, float* y,
+                        int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int relu_out, cudaStream_t st);
+int launch_column_bwd_g(const float* x, int64_t xs, const float* dy, const float* hg, const float* s1, const float* s2, float* dx, float* dg,
+                        float* ds1, float* ds2, float* dbias, float* ws, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int relu_in,
+                        cudaStream_t st);
 int launch_reparam_diag_bwd(const float* rho, const float* eps, const float* dg, float* dmu, float* drho, int64_t S,
                             int64_t D, int accumulate, cudaStream_t stream, int64_t groups = 1, int64_t pstride = 0);
 int launch_stack_split(const float* in, float* blocks, int64_t R, int64_t D, int64_t G, int64_t n_out, cudaStream_t stream);

@@ -454,4 +454,253 @@ int launch_kl_dense(const float* mu, const float* L, float lambda_, int64_t D, f
     return check_launch("kl_dense_final_kernel");
 }
 
+// ---- grouped forms: G blocks (the square blocks of a Stacked layer), block k's mu at + k * mu_stride floats and its L at
+// + k * L_stride; eps, g, dg: (G, S, D); dmu (G, D) and dL (G, D, D) are written densely.
+//
+// D <= 64: one CUDA-core kernel per direction for all blocks.  L_k (at most 64 x 64) sits in shared memory with a padded row
+// (no bank conflicts on the column walk); every output is one fp32 chain in a fixed order (j ascending forward, s ascending
+// backward), so the results are bit-reproducible.  The tcgen05 GEMM above cannot take these widths (its tile is 128 rows).
+constexpr int RDS_THREADS = 256;
+constexpr int RDS_MAX_D = 64;
+
+// grid (ceil(S / ST), G), ST = samples per CTA
+__global__ void __launch_bounds__(RDS_THREADS)
+reparam_dense_small_kernel(const float* __restrict__ mu, int64_t mu_stride, const float* __restrict__ L, int64_t L_stride,
+                           const float* __restrict__ eps, float* __restrict__ g, int S, int D, int ST)
+{
+    __shared__ float Ls[RDS_MAX_D * (RDS_MAX_D + 1)];
+    __shared__ float es[RDS_THREADS * 16];   // ST * D <= 4096
+    const int k = blockIdx.y, s0 = blockIdx.x * ST;
+    const int ns = min(ST, S - s0);
+    const float* Lk = L + size_t(k) * L_stride;
+    const float* muk = mu + size_t(k) * mu_stride;
+    for (int e = threadIdx.x; e < D * D; e += RDS_THREADS) {
+        const int i = e / D, j = e - i * D;
+        Ls[i * (D + 1) + j] = j <= i ? Lk[e] : 0.f;
+    }
+    const float* ek = eps + (size_t(k) * S + s0) * D;
+    for (int e = threadIdx.x; e < ns * D; e += RDS_THREADS) es[e] = ek[e];
+    __syncthreads();
+    float* gk = g + (size_t(k) * S + s0) * D;
+    for (int e = threadIdx.x; e < ns * D; e += RDS_THREADS) {
+        const int s = e / D, i = e - s * D;
+        const float* lr = Ls + i * (D + 1);
+        const float* er = es + s * D;
+        float acc = 0.f;
+        for (int j = 0; j <= i; ++j) acc = fmaf(lr[j], er[j], acc);
+        gk[e] = muk[i] + acc;
+    }
+}
+
+// dL_k[i, j] = sum_s dg[k, s, i] eps[k, s, j] (j <= i, 0 above), dmu_k[i] = sum_s dg[k, s, i].  Thread e of the block's
+// D * D + D outputs: e < D * D is entry (e / D, e % D) of dL_k, the rest dmu_k.  grid (ceil((D * D + D) / 256), G); the samples
+// pass through shared memory in tiles of RDS_TILE_S rows.
+constexpr int RDS_TILE_S = 32;
+__global__ void __launch_bounds__(RDS_THREADS)
+reparam_dense_small_bwd_kernel(const float* __restrict__ eps, const float* __restrict__ dg, float* __restrict__ dmu, float* __restrict__ dL,
+                               int S, int D)
+{
+    __shared__ float dgs[RDS_TILE_S * RDS_MAX_D], es[RDS_TILE_S * RDS_MAX_D];
+    const int k = blockIdx.y;
+    const int e = blockIdx.x * RDS_THREADS + threadIdx.x;
+    const int DD = D * D;
+    int i = 0, j = -1;   // j = -1: dmu entry
+    bool active = false;
+    if (e < DD) {
+        i = e / D, j = e - (e / D) * D;
+        active = j <= i;
+    } else if (e < DD + D) {
+        i = e - DD;
+        active = true;
+    }
+    const float* dgk = dg + size_t(k) * S * D;
+    const float* ek = eps + size_t(k) * S * D;
+    float acc = 0.f;
+    for (int s0 = 0; s0 < S; s0 += RDS_TILE_S) {
+        const int ns = min(RDS_TILE_S, S - s0);
+        __syncthreads();
+        for (int t = threadIdx.x; t < ns * D; t += RDS_THREADS) {
+            dgs[t] = dgk[size_t(s0) * D + t];
+            es[t] = ek[size_t(s0) * D + t];
+        }
+        __syncthreads();
+        if (active) {
+            if (j >= 0)
+                for (int s = 0; s < ns; ++s) acc = fmaf(dgs[s * D + i], es[s * D + j], acc);
+            else
+                for (int s = 0; s < ns; ++s) acc += dgs[s * D + i];
+        }
+    }
+    if (e < DD)
+        dL[size_t(k) * DD + e] = acc;   // 0 above the diagonal
+    else if (e < DD + D)
+        dmu[size_t(k) * D + i] = acc;
+}
+
+// D >= 128: the K-major operands of the dL GEMM for block k, dgT / eT (D, Sp) = the transposes of dg / eps (S, D), zero past
+// S.  32 x 32 tiles through shared memory; grid (Sp / 32, D / 32).
+__global__ void __launch_bounds__(256)
+dense_transpose_pad_kernel(const float* __restrict__ dg, const float* __restrict__ eps, float* __restrict__ dgT, float* __restrict__ eT,
+                           int S, int D, int Sp)
+{
+    __shared__ float ta[32][33], tb[32][33];
+    const int s0 = blockIdx.x * 32, i0 = blockIdx.y * 32;
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    for (int r = ty; r < 32; r += 8) {
+        const int s = s0 + r;
+        ta[r][tx] = s < S ? dg[size_t(s) * D + i0 + tx] : 0.f;
+        tb[r][tx] = s < S ? eps[size_t(s) * D + i0 + tx] : 0.f;
+    }
+    __syncthreads();
+    for (int r = ty; r < 32; r += 8) {
+        dgT[size_t(i0 + r) * Sp + s0 + tx] = ta[tx][r];
+        eT[size_t(i0 + r) * Sp + s0 + tx] = tb[tx][r];
+    }
+}
+
+// dmu[k, i] = sum_s dg[k, s, i], samples ascending
+__global__ void __launch_bounds__(256)
+dense_colsum_kernel(const float* __restrict__ dg, float* __restrict__ dmu, int S, int D)
+{
+    const int k = blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= D) return;
+    const float* p = dg + size_t(k) * S * D + i;
+    float acc = 0.f;
+    for (int s = 0; s < S; ++s) acc += p[size_t(s) * D];
+    dmu[size_t(k) * D + i] = acc;
+}
+
+static int64_t round_up(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
+
+size_t reparam_dense_grouped_workspace_bytes(int64_t S, int64_t D)
+{
+    if (D < DG_BM) return 0;
+    const size_t fwd = reparam_dense_workspace_bytes(S, D);
+    const size_t bwd = sizeof(float) * 2 * size_t(D) * size_t(round_up(S < 1 ? 1 : S, DG_BK));
+    return fwd > bwd ? fwd : bwd;
+}
+
+int launch_reparam_dense_grouped(const float* mu, int64_t mu_stride, const float* L, int64_t L_stride, const float* eps, float* g, int64_t S,
+                                 int64_t D, int64_t G, float* ws, size_t ws_bytes, cudaStream_t stream)
+{
+    if (D <= RDS_MAX_D) {
+        const int ST = static_cast<int>(D >= 16 ? 4096 / D : 256);
+        const dim3 grid(static_cast<unsigned>((S + ST - 1) / ST), static_cast<unsigned>(G));
+        reparam_dense_small_kernel<<<grid, RDS_THREADS, 0, stream>>>(mu, mu_stride, L, L_stride, eps, g, static_cast<int>(S), static_cast<int>(D), ST);
+        return check_launch("reparam_dense_small_kernel");
+    }
+    for (int64_t k = 0; k < G; ++k)   // one tcgen05 reparameterisation per block (G = ceil(n_out / D) is small)
+        if (int rc = launch_reparam_dense(mu + k * mu_stride, L + k * L_stride, eps + k * S * D, g + k * S * D, S, D, ws, ws_bytes, stream))
+            return rc;
+    return WHVI_OK;
+}
+
+int launch_reparam_dense_grouped_bwd(const float* eps, const float* dg, float* dmu, float* dL, int64_t S, int64_t D, int64_t G, float* ws,
+                                     size_t ws_bytes, cudaStream_t stream)
+{
+    if (D <= RDS_MAX_D) {
+        const dim3 grid(static_cast<unsigned>((D * D + D + RDS_THREADS - 1) / RDS_THREADS), static_cast<unsigned>(G));
+        reparam_dense_small_bwd_kernel<<<grid, RDS_THREADS, 0, stream>>>(eps, dg, dmu, dL, static_cast<int>(S), static_cast<int>(D));
+        return check_launch("reparam_dense_small_bwd_kernel");
+    }
+    if (ws == nullptr || ws_bytes < reparam_dense_grouped_workspace_bytes(S, D))
+        return fail(WHVI_E_WORKSPACE, "reparam_bwd(dense, grouped): workspace of %zu bytes needed, %zu given",
+                    reparam_dense_grouped_workspace_bytes(S, D), ws_bytes);
+    const int64_t Sp = round_up(S, DG_BK);
+    float* dgT = ws;
+    float* eT = ws + D * Sp;
+    // the GEMM writes the tiles on and below the diagonal only
+    if (cudaMemsetAsync(dL, 0, sizeof(float) * size_t(G) * D * D, stream) != cudaSuccess) return check_launch("reparam_bwd(dense): memset");
+    for (int64_t k = 0; k < G; ++k) {
+        const dim3 tgrid(static_cast<unsigned>(Sp / 32), static_cast<unsigned>(D / 32));
+        dense_transpose_pad_kernel<<<tgrid, 256, 0, stream>>>(dg + k * S * D, eps + k * S * D, dgT, eT, static_cast<int>(S), static_cast<int>(D),
+                                                              static_cast<int>(Sp));
+        if (int rc = check_launch("dense_transpose_pad_kernel")) return rc;
+        if (int rc = launch_reparam_dense_bwd(dgT, eT, dL + k * D * D, Sp, D, stream)) return rc;
+    }
+    const dim3 cgrid(static_cast<unsigned>((D + 255) / 256), static_cast<unsigned>(G));
+    dense_colsum_kernel<<<cgrid, 256, 0, stream>>>(dg, dmu, static_cast<int>(S), static_cast<int>(D));
+    return check_launch("dense_colsum_kernel");
+}
+
+// Sum over G blocks of the dense KL: the row kernel with a block axis (grid (D, G)), then one CTA that adds the rows' squares,
+// the log-diagonals and |mu|^2 in a fixed order (blocks ascending inside every thread's strided walk).
+__global__ void __launch_bounds__(256)
+kl_dense_grouped_rows_kernel(const float* __restrict__ L, int64_t L_stride, float lambda_, int D, float* __restrict__ dL, float grad_scale,
+                             double* __restrict__ row_sq)
+{
+    __shared__ double red[8];
+    const int i = blockIdx.x, k = blockIdx.y;
+    const float* Lk = L + size_t(k) * L_stride;
+    float* dLk = dL ? dL + size_t(k) * D * D : nullptr;
+    const float inv_l = 1.f / lambda_;
+    double acc = 0.0;
+    for (int j = threadIdx.x; j < D; j += blockDim.x) {
+        const float v = j <= i ? Lk[size_t(i) * D + j] : 0.f;
+        acc += double(v) * double(v);
+        if (dLk) {
+            float gr = grad_scale * v * inv_l;
+            if (j == i) gr -= grad_scale / v;
+            dLk[size_t(i) * D + j] = gr;
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double tot = 0.0;
+        for (int w = 0; w < int(blockDim.x >> 5); ++w) tot += red[w];
+        row_sq[size_t(k) * D + i] = tot;
+    }
+}
+__global__ void __launch_bounds__(1024)
+kl_dense_grouped_final_kernel(const float* __restrict__ mu, int64_t mu_stride, const float* __restrict__ L, int64_t L_stride, float lambda_,
+                              int D, int G, const double* __restrict__ row_sq, float* __restrict__ out, float* __restrict__ dmu, float grad_scale)
+{
+    __shared__ double red[3][32];
+    double s_sq = 0.0, s_log = 0.0, s_mu = 0.0;
+    const float inv_l = 1.f / lambda_;
+    for (int k = 0; k < G; ++k) {
+        const float* Lk = L + size_t(k) * L_stride;
+        const float* muk = mu + size_t(k) * mu_stride;
+        for (int i = threadIdx.x; i < D; i += blockDim.x) {
+            s_sq += row_sq[size_t(k) * D + i];
+            s_log += log(double(Lk[size_t(i) * D + i]));
+            const float m = muk[i];
+            s_mu += double(m) * double(m);
+            if (dmu) dmu[size_t(k) * D + i] = grad_scale * m * inv_l;
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        s_sq += __shfl_xor_sync(0xffffffffu, s_sq, o);
+        s_log += __shfl_xor_sync(0xffffffffu, s_log, o);
+        s_mu += __shfl_xor_sync(0xffffffffu, s_mu, o);
+    }
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (lane == 0) red[0][warp] = s_sq, red[1][warp] = s_log, red[2][warp] = s_mu;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double a = 0.0, b = 0.0, c = 0.0;
+        for (int w = 0; w < int(blockDim.x >> 5); ++w) a += red[0][w], b += red[1][w], c += red[2][w];
+        const double n = double(D) * double(G), lam = double(lambda_);
+        out[0] = static_cast<float>(0.5 * (n * log(lam) - 2.0 * b - n + a / lam + c / lam));
+    }
+}
+
+int launch_kl_dense_grouped(const float* mu, int64_t mu_stride, const float* L, int64_t L_stride, float lambda_, int64_t D, int64_t G, float* out,
+                            float* dmu, float* dL, float grad_scale, double* row_sq /* G * D doubles */, cudaStream_t stream)
+{
+    const int threads = D >= 256 ? 256 : 32;
+    kl_dense_grouped_rows_kernel<<<dim3(static_cast<unsigned>(D), static_cast<unsigned>(G)), threads, 0, stream>>>(
+        L, L_stride, lambda_, static_cast<int>(D), dL, grad_scale, row_sq);
+    if (int rc = check_launch("kl_dense_grouped_rows_kernel")) return rc;
+    int ft = 32;
+    while (ft < D && ft < 1024) ft <<= 1;
+    kl_dense_grouped_final_kernel<<<1, ft, 0, stream>>>(mu, mu_stride, L, L_stride, lambda_, static_cast<int>(D), static_cast<int>(G), row_sq, out,
+                                                        dmu, grad_scale);
+    return check_launch("kl_dense_grouped_final_kernel");
+}
+
 }  // namespace whvi

@@ -28,7 +28,10 @@ _LAUNCHES_PER_CALL = {"whvi_fwht_f32": 1, "whvi_fwht_f64": 1, "whvi_layer_fwd_f3
                       "whvi_mc_moments_strided_f32": 1, "whvi_adam_f32": 1, "whvi_layer_moments_f32": 1,
                       "whvi_reparam_dense_f32": 2, "whvi_reparam_dense_bwd_f32": 1, "whvi_kl_dense_f32": 2,
                       "whvi_fwht_bf16": 1, "whvi_fwht_scaled_f32": 1, "whvi_layer_moments_add_f32": 1, "whvi_layer_fwd_bf16": 1, "whvi_column_fwd_f32": 3, "whvi_column_bwd_f32": 7, "whvi_pad_rows_f32": 1, "whvi_stacked_fwd_f32": 3, "whvi_stacked_bwd_f32": 6, "whvi_kl_grouped_f32": 1,
-                      "whvi_layer_bwd_bf16": 3, "whvi_layer_loss_bf16": 3}
+                      "whvi_layer_bwd_bf16": 3, "whvi_layer_loss_bf16": 3,
+                      # dense grouped calls: the counts at D <= 64; at D >= 128 they run the tcgen05 sequence once per block
+                      "whvi_reparam_dense_grouped_f32": 1, "whvi_reparam_dense_grouped_bwd_f32": 1, "whvi_kl_dense_grouped_f32": 2,
+                      "whvi_stacked_fwd_g_f32": 2, "whvi_stacked_bwd_g_f32": 5, "whvi_column_fwd_g_f32": 2, "whvi_column_bwd_g_f32": 6}
 # When set to a dict {"name": [(start_event, stop_event), ...]}, the named calls are bracketed
 # by CUDA events on the launching stream (bench.py's per-kernel roofline timing).
 EVENT_SINK: dict[str, list] | None = None
@@ -275,7 +278,7 @@ def mc_moments_into(y, in_y, in_y2, out_y, out_y2):
 
 @torch.no_grad()
 def predictive_moments(x, mu, rho, s1, s2, bias=None, n_samples=64, chunk_samples=16, eps=None, generator=None,
-                       sample_range=None, out=None, t2=None, scatter_to=None):
+                       sample_range=None, out=None, t2=None, scatter_to=None, L=None):
     """MC predictive mean and variance of one square WHVI layer (PAPER semantics) for inputs
     ``x`` (B, D) -- BASELINE config 5, what ``WHVIRegression.eval_model`` reduces
     ``WHVINetwork.forward``'s (B, out, S) output to (src/networks.py:36-54, :131-132) --
@@ -294,7 +297,10 @@ def predictive_moments(x, mu, rho, s1, s2, bias=None, n_samples=64, chunk_sample
     ``scatter_to``: [(row_lo, row_hi, out_y, out_y2), ...] covering all rows -- the LAST sample
     chunk's reduction writes its totals there instead of into the local sums (peer-GPU buffers of
     the ranks that own those rows; the experiment in ``tools/peer_moments.py`` uses it).
+    ``L``: the dense posterior's lower-triangular factor (D, D) in place of ``rho``: g = mu + L eps per chunk
+    (``reparam_dense``); the moments kernels are the same.
     """
+    draw = (lambda e: ReparamFunction.apply(mu, rho, e)) if L is None else (lambda e: reparam_dense(mu, L, e))
     from .fwht import fwht_
     x = _f32c(x if t2 is None else t2, "x")
     if x.dim() != 2:
@@ -312,14 +318,14 @@ def predictive_moments(x, mu, rho, s1, s2, bias=None, n_samples=64, chunk_sample
     if FUSED_MOMENTS_MIN_D <= D <= FUSED_MOMENTS_MAX_D and scatter_to is None and hi > lo:
         # one kernel for all samples: running sums in tensor memory, nothing but the two results goes to HBM
         e = eps[lo:hi] if eps is not None else torch.randn((hi - lo, D), device=x.device, generator=generator)
-        g = ReparamFunction.apply(mu, rho, e.contiguous())
+        g = draw(e.contiguous())
         layer_moments_raw(t2, g, s1, s2, bias, sum_y, sum_y2, from_t2=True, accumulate=False)
         return sum_y, sum_y2, hi - lo
     ybuf = torch.empty((min(chunk_samples, max(hi - lo, 1)), B, D), dtype=torch.float32, device=x.device)
     for s0 in range(lo, hi, chunk_samples):
         s1_ = min(s0 + chunk_samples, hi)
         e = eps[s0:s1_] if eps is not None else torch.randn((s1_ - s0, D), device=x.device, generator=generator)
-        g = ReparamFunction.apply(mu, rho, e.contiguous())
+        g = draw(e.contiguous())
         y = layer_forward_raw(t2, g, s1, s2, bias, out=ybuf[: s1_ - s0], from_t2=True)
         if scatter_to is not None and s1_ == hi:
             for r0, r1, oy, oy2 in scatter_to:
@@ -694,24 +700,43 @@ def reparam(mu, rho, eps):
     return ReparamFunction.apply(mu, rho, eps)
 
 
+def _blocks(tensors, name):
+    """(base, stride): G blocks' parameters read where they lie when evenly spaced (FlatParams, a module's own packing),
+    else a stacked copy."""
+    base = _f32c(tensors[0], name)
+    if len(tensors) == 1:
+        return base.detach(), base.numel()
+    stride = uniform_stride(tensors)
+    if stride is None or any(t.dtype != torch.float32 for t in tensors):
+        return torch.stack([_f32c(t, name).detach() for t in tensors]), base.numel()
+    return base.detach(), stride
+
+
 class ReparamDenseFunction(Function):
-    """g[s] = mu + L eps[s] with a dense lower-triangular L (D, D), D a multiple of 128: superset of the reference (whose
-    posterior is diagonal, SURVEY F5).  Forward AND backward are the hand-written tcgen05 GEMM of ``csrc/reparam_dense.cu``
-    (TMA-fed, 3xTF32 operand split, TMEM accumulators): g = mu + E L^T, dL = tril(dg^T E); dmu is a column sum."""
+    """g[k, s] = mu_k + L_k eps[k, s] for G blocks with dense lower-triangular L_k (D, D), D <= 64 or a multiple of 128: superset of the
+    reference (whose posterior is diagonal, SURVEY F5).  ``eps`` (G, S, D); ``params`` = G x mu, G x L (the blocks' own
+    parameters).  One C call per direction (``whvi_reparam_dense_grouped_f32`` / ``..._bwd_f32``): the CUDA-core kernels at
+    D <= 64, the tcgen05 GEMMs of ``csrc/reparam_dense.cu`` block after block at D >= 128 (g = mu + E L^T, dL = tril(dg^T E)),
+    dmu a device column sum."""
 
     @staticmethod
-    def forward(ctx, mu, L, eps):
-        mu, L, eps = _f32c(mu, "g_mu"), _f32c(L, "g_L"), _f32c(eps, "eps")
-        S, D = eps.shape
-        if L.shape != (D, D):
-            raise RuntimeError(f"L must be {(D, D)}, got {tuple(L.shape)}")
+    def forward(ctx, eps, *params):
+        G = len(params) // 2
+        eps = _f32c(eps, "eps")
+        if eps.dim() != 3 or eps.size(0) != G:
+            raise RuntimeError(f"eps must be ({G}, S, D), got {tuple(eps.shape)}")
+        _, S, D = eps.shape
+        if any(m.numel() != D for m in params[:G]) or any(tuple(l.shape) != (D, D) for l in params[G:]):
+            raise RuntimeError(f"every g_mu must have {D} elements and every g_L be {(D, D)}")
+        mu, mu_stride = _blocks(params[:G], "g_mu")
+        L, L_stride = _blocks(params[G:], "g_L")
         g = torch.empty_like(eps)
-        lib = _lib.lib()
-        ws = _workspace(eps.device, _query("whvi_reparam_dense_workspace_bytes", S, D)[0])
-        with torch.cuda.device(eps.device), _Timed("whvi_reparam_dense_f32"):
-            rc = lib.whvi_reparam_dense_f32(mu.data_ptr(), L.data_ptr(), eps.data_ptr(), g.data_ptr(), S, D, ws.data_ptr(),
-                                            ws.numel(), _stream(eps.device))
-        _lib.check(rc, "whvi_reparam_dense_f32")
+        with torch.cuda.device(eps.device):
+            ws = _workspace(eps.device, _query("whvi_reparam_dense_grouped_workspace_bytes", S, D)[0])
+            with _Timed("whvi_reparam_dense_grouped_f32", f"D={D},G={G}"):
+                rc = _lib.lib().whvi_reparam_dense_grouped_f32(mu.data_ptr(), mu_stride, L.data_ptr(), L_stride, eps.data_ptr(), g.data_ptr(),
+                                                               S, D, G, ws.data_ptr(), ws.numel(), _stream(eps.device))
+        _lib.check(rc, "whvi_reparam_dense_grouped_f32")
         ctx.save_for_backward(eps)
         return g
 
@@ -719,22 +744,26 @@ class ReparamDenseFunction(Function):
     def backward(ctx, dg):
         (eps,) = ctx.saved_tensors
         dg = _f32c(dg, "dg")
-        S, D = eps.shape
-        Sp = (S + 31) // 32 * 32
-        # K-major operands for the tensor core: the transposes, zero-padded to a multiple of the 32-wide K block
-        dgT = torch.zeros((D, Sp), dtype=torch.float32, device=eps.device)
-        eT = torch.zeros((D, Sp), dtype=torch.float32, device=eps.device)
-        dgT[:, :S].copy_(dg.t())
-        eT[:, :S].copy_(eps.t())
-        dL = torch.zeros((D, D), dtype=torch.float32, device=eps.device)   # tiles above the diagonal are not written
-        with torch.cuda.device(eps.device), _Timed("whvi_reparam_dense_bwd_f32"):
-            rc = _lib.lib().whvi_reparam_dense_bwd_f32(dgT.data_ptr(), eT.data_ptr(), dL.data_ptr(), Sp, D, _stream(eps.device))
-        _lib.check(rc, "whvi_reparam_dense_bwd_f32")
-        return dg.sum(dim=0), dL, None
+        G, S, D = eps.shape
+        dmu = torch.empty((G, D), dtype=torch.float32, device=eps.device)
+        dL = torch.empty((G, D, D), dtype=torch.float32, device=eps.device)
+        with torch.cuda.device(eps.device):
+            ws = _workspace(eps.device, _query("whvi_reparam_dense_grouped_workspace_bytes", S, D)[0])
+            with _Timed("whvi_reparam_dense_grouped_bwd_f32", f"D={D},G={G}"):
+                rc = _lib.lib().whvi_reparam_dense_grouped_bwd_f32(eps.data_ptr(), dg.data_ptr(), dmu.data_ptr(), dL.data_ptr(), S, D, G,
+                                                                   ws.data_ptr(), ws.numel(), _stream(eps.device))
+        _lib.check(rc, "whvi_reparam_dense_grouped_bwd_f32")
+        return (None, *dmu.unbind(0), *dL.unbind(0))
+
+
+def reparam_dense_grouped(mus, Ls, eps):
+    """(G, S, D) samples of G dense blocks for noise ``eps`` (G, S, D)."""
+    return ReparamDenseFunction.apply(eps, *mus, *Ls)
 
 
 def reparam_dense(mu, L, eps):
-    return ReparamDenseFunction.apply(mu, L, eps)
+    """g[s] = mu + L eps[s] for one block: eps, g (S, D)."""
+    return ReparamDenseFunction.apply(eps.unsqueeze(0), mu, L)[0]
 
 
 class KLDenseFunction(Function):
@@ -770,6 +799,40 @@ def kl_gaussian_dense(mu, L, lambda_):
     return KLDenseFunction.apply(mu, L, lambda_)
 
 
+class KLDenseGroupedFunction(Function):
+    """Sum over G blocks of the dense KL term with all gradients, one C call (``whvi_kl_dense_grouped_f32``)."""
+
+    @staticmethod
+    def forward(ctx, lambda_, *params):
+        G = len(params) // 2
+        mu, mu_stride = _blocks(params[:G], "g_mu")
+        L, L_stride = _blocks(params[G:], "g_L")
+        D = params[0].numel()
+        dev = mu.device
+        out = torch.empty(1, dtype=torch.float32, device=dev)
+        need_grad = any(ctx.needs_input_grad[1:])
+        dmu = torch.empty((G, D), dtype=torch.float32, device=dev) if need_grad else None
+        dL = torch.empty((G, D, D), dtype=torch.float32, device=dev) if need_grad else None
+        ws = torch.empty(G * D, dtype=torch.float64, device=dev)
+        with torch.cuda.device(dev), _Timed("whvi_kl_dense_grouped_f32", f"D={D},G={G}"):
+            rc = _lib.lib().whvi_kl_dense_grouped_f32(mu.data_ptr(), mu_stride, L.data_ptr(), L_stride, float(lambda_), D, G, out.data_ptr(),
+                                                      _ptr(dmu), _ptr(dL), 1.0, ws.data_ptr(), ws.numel() * 8, _stream(dev))
+        _lib.check(rc, "whvi_kl_dense_grouped_f32")
+        ctx.G = G
+        if need_grad:
+            ctx.save_for_backward(dmu, dL)
+        return out.reshape(())
+
+    @staticmethod
+    def backward(ctx, dkl):
+        dmu, dL = ctx.saved_tensors
+        return (None, *(dmu * dkl).unbind(0), *(dL * dkl).unbind(0))
+
+
+def kl_gaussian_dense_grouped(mus, Ls, lambda_):
+    return KLDenseGroupedFunction.apply(lambda_, *mus, *Ls)
+
+
 # ---------------------------------------------------------------------------------------------- Stacked layer, one call per direction
 def uniform_stride(tensors) -> int | None:
     """Floats between consecutive tensors' first elements when they are evenly spaced in memory (stride >= numel, a multiple
@@ -785,6 +848,42 @@ def uniform_stride(tensors) -> int | None:
         if t.data_ptr() != p0 + k * step or not t.is_contiguous():
             return None
     return step // 4
+
+
+def _stacked_input(x, S, D):
+    """(x zero-padded to D columns, B, x_sample_stride) for a Stacked call (src/weights.py:197-198)."""
+    n_in = x.size(-1)
+    if n_in < D:
+        xp = torch.empty(x.shape[:-1] + (D,), dtype=torch.float32, device=x.device)
+        with _Timed("whvi_pad_rows_f32"):
+            _lib.check(_lib.lib().whvi_pad_rows_f32(x.data_ptr(), xp.data_ptr(), x.numel() // n_in, n_in, D, _stream(x.device)),
+                       "whvi_pad_rows_f32")
+    else:
+        xp = x
+    if xp.dim() == 2:
+        return xp, xp.size(0), 0
+    if xp.dim() == 3 and xp.size(0) == S:
+        return xp, xp.size(1), xp.size(1) * D
+    raise RuntimeError(f"x must be (B, n_in) or (S, B, n_in) with S = {S}; got {tuple(x.shape)}")
+
+
+def _stacked_vectors(groups, D):
+    """The blocks' (D,) parameter vectors, one list of G tensors per kind, as one base tensor per kind and ONE stride shared
+    by all kinds: read where they lie when they are evenly spaced alike, else a (kinds, G, D) copy."""
+    strides = [uniform_stride(g_) for g_ in groups]
+    if any(v is None for v in strides) or len(set(strides)) != 1:
+        packed = torch.stack([torch.stack([t.detach().reshape(-1) for t in g_]) for g_ in groups])
+        return list(packed.unbind(0)), D
+    return [g_[0].detach() for g_ in groups], strides[0]
+
+
+def _stacked_bias(bias, G, D):
+    if bias is None:
+        return None
+    bias = _f32c(bias, "bias").reshape(-1)
+    if bias.numel() != G * D:
+        raise RuntimeError("stacked bias must have G * D elements")
+    return bias
 
 
 class WHVIStackedFunction(Function):
@@ -804,31 +903,9 @@ class WHVIStackedFunction(Function):
         dev = x.device
         st = _stream(dev)
         with torch.cuda.device(dev):
-            if n_in < D:  # src/weights.py:197-198
-                xp = torch.empty(x.shape[:-1] + (D,), dtype=torch.float32, device=dev)
-                with _Timed("whvi_pad_rows_f32"):
-                    _lib.check(lib.whvi_pad_rows_f32(x.data_ptr(), xp.data_ptr(), x.numel() // n_in, n_in, D, st), "whvi_pad_rows_f32")
-            else:
-                xp = x
-            if xp.dim() == 2:
-                B, xs = xp.size(0), 0
-            elif xp.dim() == 3 and xp.size(0) == S:
-                B, xs = xp.size(1), xp.size(1) * D
-            else:
-                raise RuntimeError(f"x must be (B, n_in) or (S, B, n_in) with S = {S}; got {tuple(x.shape)}")
-            groups = [params[i * G:(i + 1) * G] for i in range(4)]
-            strides = [uniform_stride(g_) for g_ in groups]
-            if any(v is None for v in strides) or len(set(strides)) != 1:
-                packed = torch.stack([torch.stack([t.detach().reshape(-1) for t in g_]) for g_ in groups])   # (4, G, D) copy
-                s1p, s2p, mup, rhop = packed[0], packed[1], packed[2], packed[3]
-                stride = D
-            else:
-                s1p, s2p, mup, rhop = (g_[0].detach() for g_ in groups)
-                stride = strides[0]
-            if bias is not None:
-                bias = _f32c(bias, "bias").reshape(-1)
-                if bias.numel() != G * D:
-                    raise RuntimeError("stacked bias must have G * D elements")
+            xp, B, xs = _stacked_input(x, S, D)
+            (s1p, s2p, mup, rhop), stride = _stacked_vectors([params[i * G:(i + 1) * G] for i in range(4)], D)
+            bias = _stacked_bias(bias, G, D)
             g = torch.empty((G, S, D), dtype=torch.float32, device=dev)
             yb = torch.empty((G, S, B, D), dtype=torch.float32, device=dev)
             y = torch.empty((S, B, n_out), dtype=torch.float32, device=dev)
@@ -868,6 +945,60 @@ class WHVIStackedFunction(Function):
 
 def whvi_stacked(x, eps, bias, n_out, blocks_s1, blocks_s2, blocks_mu, blocks_rho, relu_out=False, relu_in=False):
     return WHVIStackedFunction.apply(x, eps, bias, n_out, relu_out, relu_in, *blocks_s1, *blocks_s2, *blocks_mu, *blocks_rho)
+
+
+class WHVIStackedGFunction(Function):
+    """The Stacked layer from g (G, S, D) given, however it was drawn (``whvi_stacked_fwd_g_f32`` / ``whvi_stacked_bwd_g_f32``):
+    the dense posterior's path, g from ``reparam_dense_grouped``.  ``params`` = G x s1, G x s2; the backward returns dg."""
+
+    @staticmethod
+    def forward(ctx, x, g, bias, n_out, relu_out, relu_in, *params):
+        G = len(params) // 2
+        g = _f32c(g, "g")
+        _, S, D = g.shape
+        x = _f32c(x, "x")
+        n_in = x.size(-1)
+        dev = x.device
+        with torch.cuda.device(dev):
+            xp, B, xs = _stacked_input(x, S, D)
+            (s1p, s2p), stride = _stacked_vectors([params[:G], params[G:]], D)
+            bias = _stacked_bias(bias, G, D)
+            yb = torch.empty((G, S, B, D), dtype=torch.float32, device=dev)
+            y = torch.empty((S, B, n_out), dtype=torch.float32, device=dev)
+            with _Timed("whvi_stacked_fwd_g_f32"):
+                rc = _lib.lib().whvi_stacked_fwd_g_f32(xp.data_ptr(), xs, g.data_ptr(), s1p.data_ptr(), s2p.data_ptr(), stride, _ptr(bias),
+                                                       yb.data_ptr(), y.data_ptr(), S, B, D, G, n_out, 1 if relu_out else 0, _stream(dev))
+            _lib.check(rc, "whvi_stacked_fwd_g_f32")
+        ctx.save_for_backward(xp, g, s1p, s2p)
+        ctx.meta = (S, B, D, G, xs, n_in, n_out, stride, bool(relu_in), bias is not None, x.dim())
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        xp, g, s1p, s2p = ctx.saved_tensors
+        S, B, D, G, xs, n_in, n_out, stride, relu_in, has_bias, xdim = ctx.meta
+        dy = _f32c(dy, "dy")
+        dev = dy.device
+        want_dx = ctx.needs_input_grad[0]
+        with torch.cuda.device(dev):
+            ws = _workspace(dev, _query("whvi_stacked_bwd_workspace_bytes", S, B, D, G, 1 if want_dx else 0)[0])
+            dg = torch.empty((G, S, D), dtype=torch.float32, device=dev)
+            out = torch.empty((3 if has_bias else 2, G, D), dtype=torch.float32, device=dev)   # ds1, ds2, [dbias]
+            dx = torch.empty((S, B, n_in), dtype=torch.float32, device=dev) if want_dx else None
+            with _Timed("whvi_stacked_bwd_g_f32"):
+                rc = _lib.lib().whvi_stacked_bwd_g_f32(xp.data_ptr(), xs, dy.data_ptr(), g.data_ptr(), s1p.data_ptr(), s2p.data_ptr(), stride,
+                                                       _ptr(dx), n_in, dg.data_ptr(), out[0].data_ptr(), out[1].data_ptr(),
+                                                       out[2].data_ptr() if has_bias else None, ws.data_ptr(), ws.numel(), S, B, D, G, n_out,
+                                                       1 if relu_in else 0, _stream(dev))
+            _lib.check(rc, "whvi_stacked_bwd_g_f32")
+        if want_dx and xdim == 2:
+            dx = dx.sum(dim=0)
+        dbias = out[2].reshape(1, G * D) if has_bias and ctx.needs_input_grad[2] else None
+        return (dx, dg, dbias, None, None, None, *out[0].unbind(0), *out[1].unbind(0))
+
+
+def whvi_stacked_g(x, g, bias, n_out, blocks_s1, blocks_s2, relu_out=False, relu_in=False):
+    return WHVIStackedGFunction.apply(x, g, bias, n_out, relu_out, relu_in, *blocks_s1, *blocks_s2)
 
 
 class WHVIColumnFunction(Function):
@@ -930,6 +1061,63 @@ class WHVIColumnFunction(Function):
 
 def whvi_column(x, eps, mu, rho, s1, s2, bias, n, transposed, relu_out=False, relu_in=False):
     return WHVIColumnFunction.apply(x, eps, mu, rho, s1, s2, bias, n, transposed, relu_out, relu_in)
+
+
+class WHVIColumnGFunction(Function):
+    """The Column layer from g (S, D) given, however it was drawn (``whvi_column_fwd_g_f32`` / ``whvi_column_bwd_g_f32``): the
+    dense posterior's path, g from ``reparam_dense``.  The backward returns dg."""
+
+    @staticmethod
+    def forward(ctx, x, g, s1, s2, bias, n, transposed, relu_out, relu_in):
+        x, g, s1, s2 = _f32c(x, "x"), _f32c(g, "g"), _f32c(s1, "s1"), _f32c(s2, "s2")
+        S, D = g.shape
+        width = n if transposed else 1
+        if x.size(-1) != width:
+            raise RuntimeError(f"last dimension of x must be {width}, got {x.size(-1)}")
+        if x.dim() == 2:
+            B, xs = x.size(0), 0
+        elif x.dim() == 3 and x.size(0) == S:
+            B, xs = x.size(1), x.size(1) * width
+        else:
+            raise RuntimeError(f"x must be (B, {width}) or (S, B, {width}) with S = {S}; got {tuple(x.shape)}")
+        if bias is not None:
+            bias = _f32c(bias, "bias").reshape(-1)
+        dev = x.device
+        hg = torch.empty((S, D), dtype=torch.float32, device=dev)
+        y = torch.empty((S, B, 1 if transposed else n), dtype=torch.float32, device=dev)
+        with torch.cuda.device(dev), _Timed("whvi_column_fwd_g_f32"):
+            rc = _lib.lib().whvi_column_fwd_g_f32(x.data_ptr(), xs, g.data_ptr(), s1.data_ptr(), s2.data_ptr(), _ptr(bias), hg.data_ptr(),
+                                                  y.data_ptr(), S, B, D, n, 1 if transposed else 0, 1 if relu_out else 0, _stream(dev))
+        _lib.check(rc, "whvi_column_fwd_g_f32")
+        ctx.save_for_backward(x, hg, s1, s2)
+        ctx.meta = (S, B, D, n, xs, bool(transposed), bool(relu_in), bias is not None)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        x, hg, s1, s2 = ctx.saved_tensors
+        S, B, D, n, xs, transposed, relu_in, has_bias = ctx.meta
+        dy = _f32c(dy, "dy")
+        dev = dy.device
+        want_dx = ctx.needs_input_grad[0]
+        with torch.cuda.device(dev):
+            ws = _workspace(dev, _query("whvi_column_bwd_workspace_bytes", S, D, n)[0])
+            dg = torch.empty((S, D), dtype=torch.float32, device=dev)
+            out = torch.empty((2, D), dtype=torch.float32, device=dev)   # ds1, ds2
+            dbias = torch.empty((1, 1 if transposed else n), dtype=torch.float32, device=dev) if has_bias else None
+            dx = torch.empty((S, B, n if transposed else 1), dtype=torch.float32, device=dev) if want_dx else None
+            with _Timed("whvi_column_bwd_g_f32"):
+                rc = _lib.lib().whvi_column_bwd_g_f32(x.data_ptr(), xs, dy.data_ptr(), hg.data_ptr(), s1.data_ptr(), s2.data_ptr(), _ptr(dx),
+                                                      dg.data_ptr(), out[0].data_ptr(), out[1].data_ptr(), _ptr(dbias), ws.data_ptr(),
+                                                      ws.numel(), S, B, D, n, 1 if transposed else 0, 1 if relu_in else 0, _stream(dev))
+            _lib.check(rc, "whvi_column_bwd_g_f32")
+        if want_dx and xs == 0:
+            dx = dx.sum(dim=0)
+        return dx, dg, out[0], out[1], dbias, None, None, None, None
+
+
+def whvi_column_g(x, g, s1, s2, bias, n, transposed, relu_out=False, relu_in=False):
+    return WHVIColumnGFunction.apply(x, g, s1, s2, bias, n, transposed, relu_out, relu_in)
 
 
 class KLGroupedFunction(Function):

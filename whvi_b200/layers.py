@@ -16,7 +16,7 @@ class WHVI:
 
 
 class WHVILinear(nn.Module, WHVI):
-    def __init__(self, n_in, n_out, lambda_=1e-5, bias=False, *, semantics="paper", kl_mode=0):
+    def __init__(self, n_in, n_out, lambda_=1e-5, bias=False, *, semantics="paper", kl_mode=0, covariance="diag"):
         """WHVI feed-forward layer.
 
         :param int n_in: input dimensionality.
@@ -24,9 +24,11 @@ class WHVILinear(nn.Module, WHVI):
         :param float lambda_: prior variance.
         :param boolean bias: add an optimised (non-variational) bias after the linear map.
         :param str semantics: "paper" | "reference", see ``whvi_b200.weights``.
+        :param str covariance: "diag" (the reference's posterior) | "dense" (g = mu + L eps with a lower-triangular L per
+            square block, the paper's full-covariance posterior; PAPER semantics), see ``WHVISquarePow2Matrix``.
         """
         super().__init__()
-        kw = dict(lambda_=lambda_, bias=bias, semantics=semantics, kl_mode=kl_mode)
+        kw = dict(lambda_=lambda_, bias=bias, semantics=semantics, kl_mode=kl_mode, covariance=covariance)
         if n_in == 1:
             self.weight_submodule = WHVIColumnMatrix(n_out, **kw)
         elif n_out == 1:

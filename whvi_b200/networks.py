@@ -249,7 +249,7 @@ class WHVINetwork(nn.Module, WHVI):
             return sum_y, sum_y2, S
         h = h.float()   # bf16 activations: the head ran in bf16; the moments kernel is fp32 (the widening is exact)
         bias = None if last.bias is None else last.bias.reshape(-1)
-        g = WF.reparam(last.g_mu, last.g_rho, last._draw_eps(S))
+        g = last._g(last._draw_eps(S))
         sum_y = torch.empty(h.shape[1:], dtype=torch.float32, device=h.device)
         sum_y2 = torch.empty_like(sum_y)
         if WF.FUSED_MOMENTS_MIN_D <= last.D <= WF.FUSED_MOMENTS_MAX_D:

@@ -76,8 +76,9 @@ class WHVISquarePow2Matrix(nn.Module):
             src/utils.py:49-71), 1 = the statistically consistent sigma^2 form.
         :param str covariance: "diag" -- the reference's posterior, g = mu + softplus(rho) * eps (src/weights.py:43-50);
             "dense" -- superset: g = mu + L eps with a lower-triangular ``g_L`` (D, D) parameter in place of ``g_rho``
-            (D a multiple of 128, PAPER semantics), reparameterisation / its backward / the KL with log-determinant on
-            the tcgen05 kernels of ``csrc/reparam_dense.cu``.  Not in the reference: state_dicts differ (``g_L``).
+            (PAPER semantics), reparameterisation / its backward / the KL with log-determinant on the kernels of
+            ``csrc/reparam_dense.cu`` (tcgen05 GEMMs at D >= 128, CUDA cores below).  Not in the reference: state_dicts
+            differ (``g_L``).
         """
         super().__init__()
         if D < 1 or D & (D - 1):
@@ -89,8 +90,8 @@ class WHVISquarePow2Matrix(nn.Module):
         self.padding = 0
         if covariance not in ("diag", "dense"):
             raise ValueError('covariance must be "diag" or "dense"')
-        if covariance == "dense" and (semantics != "paper" or D % 128 != 0):
-            raise ValueError('covariance="dense" needs semantics="paper" and D a multiple of 128')
+        if covariance == "dense" and semantics != "paper":
+            raise ValueError('covariance="dense" needs semantics="paper"')
         self.semantics = semantics
         self.kl_mode = kl_mode
         self.covariance = covariance
@@ -219,13 +220,14 @@ class WHVISquarePow2Matrix(nn.Module):
                            scatter_to=None):
         """MC predictive sums (sum_s y, sum_s y^2, samples done) for inputs x (B, D) without the
         (S, B, D) tensor: see functional.predictive_moments (BASELINE config 5, SURVEY 8f N1)."""
-        if self.semantics != "paper" or self.covariance != "diag":
-            raise RuntimeError("predictive_moments implements the PAPER formula with the diagonal posterior only")
+        if self.semantics != "paper":
+            raise RuntimeError("predictive_moments implements the PAPER formula")
         eps = self._eps_queue.pop(0).to(device=self.g_mu.device, dtype=torch.float32) if self._eps_queue else None
         bias = None if self.bias is None else self.bias.reshape(-1)
-        return WF.predictive_moments(x, self.g_mu, self.g_rho, self.s1, self.s2, bias, n_samples=n_samples,
+        dense = self.covariance == "dense"
+        return WF.predictive_moments(x, self.g_mu, None if dense else self.g_rho, self.s1, self.s2, bias, n_samples=n_samples,
                                      chunk_samples=chunk_samples, eps=eps, sample_range=sample_range, out=out,
-                                     generator=generator, t2=t2, scatter_to=scatter_to)
+                                     generator=generator, t2=t2, scatter_to=scatter_to, L=self.g_L if dense else None)
 
     @property
     def loss_fusable(self):
@@ -248,15 +250,16 @@ class WHVISquarePow2Matrix(nn.Module):
 
 
 class WHVIStackedMatrix(nn.Module):
-    def __init__(self, n_in, n_out, lambda_=1e-5, bias=False, *, semantics="paper", kl_mode=0):
-        """Non-square WHVI matrix as a stack of square blocks (src/weights.py:111-133)."""
+    def __init__(self, n_in, n_out, lambda_=1e-5, bias=False, *, semantics="paper", kl_mode=0, covariance="diag"):
+        """Non-square WHVI matrix as a stack of square blocks (src/weights.py:111-133).  ``covariance`` as for
+        ``WHVISquarePow2Matrix``, applied to every block: "dense" gives each block its own ``g_L``."""
         super().__init__()
         self.n_in = n_in
         self.n_out = n_out
         self.lambda_ = lambda_
         self.D_in, self.D_out, self.padding, self.stack = self.setup_dimensions(n_in, n_out)
         self.weight_matrices = nn.ModuleList([
-            WHVISquarePow2Matrix(self.D_in, lambda_=lambda_, semantics=semantics, kl_mode=kl_mode)
+            WHVISquarePow2Matrix(self.D_in, lambda_=lambda_, semantics=semantics, kl_mode=kl_mode, covariance=covariance)
             for _ in range(self.stack)
         ])
         self.bias = nn.Parameter(torch.zeros(1, self.D_out)) if bias else None
@@ -283,10 +286,11 @@ class WHVIStackedMatrix(nn.Module):
     # ------------------------------------------------------------------ one-launch path
     @property
     def grouped(self):
-        """True when all blocks run as ONE grouped launch per direction (functional.WHVIStackedFunction): PAPER semantics,
-        diagonal posterior, block size inside the fused kernels' range.  Otherwise block after block, as the reference does."""
+        """True when all blocks run as ONE grouped call per direction (functional.WHVIStackedFunction; with the dense posterior
+        the grouped dense reparameterisation and functional.WHVIStackedGFunction): PAPER semantics, block size inside the fused
+        kernels' range.  Otherwise block after block, as the reference does."""
         w = self.weight_matrices[0]
-        return self.one_launch and w.semantics == "paper" and w.covariance == "diag" and w.fusable
+        return self.one_launch and w.semantics == "paper" and w.fusable
 
     fusable = grouped   # WHVINetwork folds a following nn.ReLU into the grouped launch
     loss_fusable = False
@@ -294,8 +298,24 @@ class WHVIStackedMatrix(nn.Module):
     def _pack(self):
         """Re-home the blocks' parameters into one (G, 4, D) buffer so that the kernels read them where they lie (evenly
         spaced); a no-op when they already are (after the first call, or once FlatParams owns them).  Same values, same
-        Parameter objects, same state_dict -- only ``.data`` moves, like FlatParams does."""
+        Parameter objects, same state_dict -- only ``.data`` moves, like FlatParams does.  Dense blocks: s1, s2, g_mu and
+        g_L of block k lie together, each segment on a 16-byte boundary (FlatParams' layout of one block)."""
         ws = self.weight_matrices
+        if ws[0].covariance == "dense":
+            vec_strides = {WF.uniform_stride([getattr(w, n) for w in ws]) for n in ("s1", "s2", "g_mu")}
+            if None not in vec_strides and len(vec_strides) == 1 and WF.uniform_stride([w.g_L for w in ws]) is not None:
+                return
+            D = self.D_in
+            v4, l4 = (D + 3) // 4 * 4, (D * D + 3) // 4 * 4
+            with torch.no_grad():
+                store = torch.empty((len(ws), 3 * v4 + l4), dtype=torch.float32, device=ws[0].s1.device)
+                for k, w in enumerate(ws):
+                    for i, n in enumerate(("s1", "s2", "g_mu", "g_L")):
+                        p = getattr(w, n)
+                        dst = store[k, i * v4:i * v4 + p.numel()].view(p.shape)
+                        dst.copy_(p)
+                        p.data = dst
+            return
         names = ("s1", "s2", "g_mu", "g_rho")
         strides = [WF.uniform_stride([getattr(w, n) for w in ws]) for n in names]
         if None not in strides and len(set(strides)) == 1:
@@ -318,6 +338,8 @@ class WHVIStackedMatrix(nn.Module):
     def kl(self):
         ws = self.weight_matrices
         if self.grouped and ws[0].g_mu.device.type == "cuda":
+            if ws[0].covariance == "dense":
+                return WF.kl_gaussian_dense_grouped([w.g_mu for w in ws], [w.g_L for w in ws], self.lambda_)
             return WF.kl_gaussian_grouped([w.g_mu for w in ws], [w.g_rho for w in ws], self.lambda_, ws[0].kl_mode)
         return sum(weight.kl for weight in ws)
 
@@ -338,8 +360,12 @@ class WHVIStackedMatrix(nn.Module):
             ws = self.weight_matrices
             S, squeeze = ws[0]._resolve_samples(x)
             self._pack()
-            y = WF.whvi_stacked(x, self._eps_blocks(S), self.bias, self.n_out, [w.s1 for w in ws], [w.s2 for w in ws],
-                                [w.g_mu for w in ws], [w.g_rho for w in ws], relu_out, relu_in)
+            if ws[0].covariance == "dense":
+                g = WF.reparam_dense_grouped([w.g_mu for w in ws], [w.g_L for w in ws], self._eps_blocks(S))
+                y = WF.whvi_stacked_g(x, g, self.bias, self.n_out, [w.s1 for w in ws], [w.s2 for w in ws], relu_out, relu_in)
+            else:
+                y = WF.whvi_stacked(x, self._eps_blocks(S), self.bias, self.n_out, [w.s1 for w in ws], [w.s2 for w in ws],
+                                    [w.g_mu for w in ws], [w.g_rho for w in ws], relu_out, relu_in)
             return y[0] if squeeze else y
         x_padded = F.pad(x, (0, self.D_in - self.n_in)) if self.D_in != self.n_in else x
         output = self.sample_lrt(x_padded)
@@ -350,13 +376,14 @@ class WHVIStackedMatrix(nn.Module):
 
 
 class WHVIColumnMatrix(nn.Module):
-    def __init__(self, n_out, lambda_=1e-5, bias=False, transposed=False, *, semantics="paper", kl_mode=0):
-        """Single-column (or, transposed, single-row) WHVI matrix (src/weights.py:211-229)."""
+    def __init__(self, n_out, lambda_=1e-5, bias=False, transposed=False, *, semantics="paper", kl_mode=0, covariance="diag"):
+        """Single-column (or, transposed, single-row) WHVI matrix (src/weights.py:211-229).  ``covariance`` as for
+        ``WHVISquarePow2Matrix``, applied to the square block."""
         super().__init__()
         self.D = n_out
         self.D_adjusted = _next_pow2(n_out)
         self.weight_submodule = WHVISquarePow2Matrix(self.D_adjusted, lambda_=lambda_, semantics=semantics,
-                                                     kl_mode=kl_mode)
+                                                     kl_mode=kl_mode, covariance=covariance)
         self.transposed = transposed
         self.bias = nn.Parameter(torch.zeros(1, 1 if transposed else n_out)) if bias else None
         self.one_launch = True   # False: the op chain of round 1 (FWHT of g + torch products); tests compare the two
@@ -383,8 +410,7 @@ class WHVIColumnMatrix(nn.Module):
         if sub.semantics == "reference":
             rows = [sub.w_bar(sub.g_mu + sub.g_sigma * eps[s]).reshape(-1)[:self.D] for s in range(S)]
             return torch.stack(rows)
-        g = WF.reparam(sub.g_mu, sub.g_rho, eps)
-        return (sub.s1[0] * sub.s2 * FWHTFunction.apply(g))[:, :self.D]
+        return (sub.s1[0] * sub.s2 * FWHTFunction.apply(sub._g(eps)))[:, :self.D]
 
     def sample(self):
         w = self._weights(1)[0].reshape(-1, 1)
@@ -392,9 +418,10 @@ class WHVIColumnMatrix(nn.Module):
 
     @property
     def fused(self):
-        """True when the layer runs as one C-ABI call per direction (functional.WHVIColumnFunction): PAPER semantics."""
+        """True when the layer runs as one C-ABI call per direction (functional.WHVIColumnFunction; with the dense posterior
+        the dense reparameterisation and functional.WHVIColumnGFunction): PAPER semantics."""
         sub = self.weight_submodule
-        return self.one_launch and sub.semantics == "paper" and sub.covariance == "diag"
+        return self.one_launch and sub.semantics == "paper"
 
     def forward(self, x, *, relu_out=False, relu_in=False):
         if x.dtype == torch.bfloat16:
@@ -404,8 +431,12 @@ class WHVIColumnMatrix(nn.Module):
         if self.fused:
             if x.device.type != "cuda":
                 raise RuntimeError("whvi_b200 runs on CUDA only (no CPU fallback); move the module and its inputs to a GPU")
-            y = WF.whvi_column(x, sub._draw_eps(S), sub.g_mu, sub.g_rho, sub.s1, sub.s2, self.bias, self.D, self.transposed,
-                               relu_out, relu_in)
+            if sub.covariance == "dense":
+                y = WF.whvi_column_g(x, sub._g(sub._draw_eps(S)), sub.s1, sub.s2, self.bias, self.D, self.transposed, relu_out,
+                                     relu_in)
+            else:
+                y = WF.whvi_column(x, sub._draw_eps(S), sub.g_mu, sub.g_rho, sub.s1, sub.s2, self.bias, self.D, self.transposed,
+                                   relu_out, relu_in)
             return y[0] if squeeze else y
         if relu_in:
             raise RuntimeError("relu_in needs the fused Column path")
