@@ -289,6 +289,35 @@ WHVI_API int whvi_stacked_bwd_g_f32(const float* x, int64_t x_sample_stride, con
                                     const float* s2, int64_t param_stride, float* dx, int64_t n_in, float* dg, float* ds1, float* ds2,
                                     float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t G,
                                     int64_t n_out, int flags, whvi_stream_t stream);
+/*
+ * bf16 activations for the Stacked layer: the same arguments with x, y_blocks, y, dy and dx bf16 (void*); g, the parameters,
+ * their gradients, the workspace and all arithmetic stay fp32.  Each call is its fp32 twin on the widened inputs:
+ *   forward   y = bf16(y of the fp32 call on float(x)), bit for bit;
+ *   backward  dmu, drho (dg), ds1, ds2, dbias bit-identical to the fp32 call on float(x), float(dy); dx = bf16(dx_f32), rounded
+ *             ONCE: the per-block dx are kept fp32, summed in the fp32 call's block order, then rounded.
+ * whvi_pad_rows_bf16 is whvi_pad_rows_f32 on bf16 rows.  The workspace is the fp32 call's (whvi_stacked_bwd_workspace_bytes: the
+ * bf16 dy blocks use the first half of its dy-block region).  Alignment: fp32 pointers as the fp32 twins; forward x and y_blocks
+ * 8 bytes; backward x 16 bytes and B * D % 8 == 0 (the padded x and the block-layout dy reach the layer kernel by bulk copy, as
+ * in whvi_layer_bwd_bf16; D = 4 with an odd B is rejected with WHVI_E_SHAPE, pad B with a zero row of x and dy); other bf16
+ * pointers 2 bytes.
+ */
+WHVI_API int whvi_pad_rows_bf16(const void* in, void* out, int64_t rows, int64_t n_in, int64_t D, whvi_stream_t stream);
+WHVI_API int whvi_stacked_fwd_bf16(const void* x, int64_t x_sample_stride, const float* mu, const float* rho, const float* s1,
+                                   const float* s2, int64_t param_stride, const float* eps, const float* bias, float* g,
+                                   void* y_blocks, void* y, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags,
+                                   whvi_stream_t stream);
+WHVI_API int whvi_stacked_fwd_g_bf16(const void* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2,
+                                     int64_t param_stride, const float* bias, void* y_blocks, void* y, int64_t S, int64_t B, int64_t D,
+                                     int64_t G, int64_t n_out, int flags, whvi_stream_t stream);
+WHVI_API int whvi_stacked_bwd_bf16(const void* x, int64_t x_sample_stride, const void* dy, const float* g, const float* rho,
+                                   const float* s1, const float* s2, int64_t param_stride, const float* eps, void* dx, int64_t n_in,
+                                   float* dmu, float* drho, float* ds1, float* ds2, float* dbias, void* workspace,
+                                   size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags,
+                                   whvi_stream_t stream);
+WHVI_API int whvi_stacked_bwd_g_bf16(const void* x, int64_t x_sample_stride, const void* dy, const float* g, const float* s1,
+                                     const float* s2, int64_t param_stride, void* dx, int64_t n_in, float* dg, float* ds1, float* ds2,
+                                     float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t G,
+                                     int64_t n_out, int flags, whvi_stream_t stream);
 /* sum of the G blocks' KL terms (WHVIStackedMatrix.kl, src/weights.py:162-164) and their gradients (G, D), one launch */
 WHVI_API int whvi_kl_grouped_f32(const float* mu, const float* rho, float lambda_, int64_t D, int64_t G, int64_t param_stride,
                                  int mode, float* out_kl, float* dmu, float* drho, float grad_scale, whvi_stream_t stream);
@@ -321,6 +350,28 @@ WHVI_API int whvi_column_bwd_g_f32(const float* x, int64_t x_sample_stride, cons
                                    const float* s2, float* dx, float* dg, float* ds1, float* ds2, float* dbias, void* workspace,
                                    size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int flags,
                                    whvi_stream_t stream);
+/*
+ * bf16 activations for the Column layer: the same arguments with the activations bf16 (void*): x and dx always; y and dy in the
+ * plain form (1 -> n) only.  The transposed form (n -> 1) keeps y (S, B, 1) and dy fp32: they are 1/n of the input's bytes, they
+ * hold the predictions of a regression network, and rounding them to 8 significant bits would put that error straight into the
+ * loss.  g, hg, the parameters, their gradients, the workspace (whvi_column_bwd_workspace_bytes) and all arithmetic stay fp32.
+ * Each call is its fp32 twin on the widened inputs with the same reduction orders: the parameter gradients (and dg) are
+ * bit-identical to the fp32 call's, and every bf16 output is the fp32 output rounded once.  bf16 pointers: 2-byte aligned.
+ */
+WHVI_API int whvi_column_fwd_bf16(const void* x, int64_t x_sample_stride, const float* mu, const float* rho, const float* s1,
+                                  const float* s2, const float* eps, const float* bias, float* g, float* hg, void* y, int64_t S,
+                                  int64_t B, int64_t D, int64_t n, int transposed, int flags, whvi_stream_t stream);
+WHVI_API int whvi_column_fwd_g_bf16(const void* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2,
+                                    const float* bias, float* hg, void* y, int64_t S, int64_t B, int64_t D, int64_t n, int transposed,
+                                    int flags, whvi_stream_t stream);
+WHVI_API int whvi_column_bwd_bf16(const void* x, int64_t x_sample_stride, const void* dy, const float* hg, const float* rho,
+                                  const float* s1, const float* s2, const float* eps, void* dx, float* dmu, float* drho, float* ds1,
+                                  float* ds2, float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D,
+                                  int64_t n, int transposed, int flags, whvi_stream_t stream);
+WHVI_API int whvi_column_bwd_g_bf16(const void* x, int64_t x_sample_stride, const void* dy, const float* hg, const float* s1,
+                                    const float* s2, void* dx, float* dg, float* ds1, float* ds2, float* dbias, void* workspace,
+                                    size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int flags,
+                                    whvi_stream_t stream);
 
 /* dmu = sum_s dg[s];  drho = (sum_s dg[s]*eps[s]) * sigmoid(rho).  accumulate != 0: += */
 WHVI_API int whvi_reparam_bwd_f32(const float* rho, const float* eps, const float* dg, float* dmu, float* drho,

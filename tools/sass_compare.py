@@ -4,11 +4,17 @@
 
 OLD_OBJ_DIR / NEW_OBJ_DIR hold the per-translation-unit objects of ``python -m whvi_b200.build`` (whvi_b200/_obj).  Every
 kernel of every object is disassembled with ``cuobjdump -sass`` and keyed by its demangled name (``cu++filt``).  A template
-parameter added with a default changes the mangled names of the existing instances, so ``--strip-arg KERNEL`` drops a
-trailing ``, float`` template argument of the NEW build's KERNEL instances before the names are matched (default: the four
-kernels that gained an activation-type parameter for bf16 training).  Each old instance must have a new instance of the
-same name whose instructions AND encodings (scheduling control words included) are identical, line for line; only the
-instruction addresses are ignored.  New instances without an old counterpart are listed.  Exit status 1 on any difference.
+parameter added with a default changes the mangled names of the existing instances, so before the names are matched:
+  * ``--strip-dup KERNEL`` drops a trailing type argument of KERNEL when it repeats the one before it (the dx
+    type of the backward kernels, which defaults to the activation type: ``<..., float, float>`` and
+    ``<..., __nv_bfloat16, __nv_bfloat16>`` are the older ``<..., float>`` and ``<..., __nv_bfloat16>``);
+  * ``--strip-arg KERNEL`` then drops a trailing ``, float`` template argument that follows a non-type argument, in both builds
+    (default: the four kernels that gained an activation-type parameter for bf16 training, so that builds from before it match);
+  * ``--untemplate KERNEL`` keys a kernel that became a template on its element types by its bare name in BOTH builds, where
+    every template argument is ``float`` (the plain kernel of the older build); other instances keep their arguments.
+Each old instance must have a new instance of the same name whose instructions AND encodings (scheduling control words
+included) are identical, line for line; only the instruction addresses are ignored.  New instances without an old counterpart
+are listed.  Exit status 1 on any difference.
 """
 from __future__ import annotations
 
@@ -20,6 +26,9 @@ from pathlib import Path
 
 CUDA_BIN = Path("/usr/local/cuda/bin")
 DEFAULT_STRIP = ("layer_bwd_tma_kernel", "layer_bwd_tm_kernel", "layer_loss_kernel", "layer_loss_tm_kernel")
+DEFAULT_STRIP_DUP = ("layer_bwd_tma_kernel", "layer_bwd_tm_kernel")
+DEFAULT_UNTEMPLATE = ("stack_split_kernel", "stack_concat_kernel", "stack_sum_kernel", "column_dot_kernel", "column_outer_kernel",
+                      "column_dot_dx_kernel", "column_dw_kernel", "column_outer_dx_kernel", "column_dbias_kernel")
 _ADDR = re.compile(r"/\*[0-9a-f]{4,}\*/")
 
 
@@ -50,20 +59,30 @@ def demangle(names: list[str]) -> dict[str, str]:
     return dict(zip(names, out.splitlines()))
 
 
-def normalise(name: str, strip: tuple[str, ...]) -> str:
-    for k in strip:
-        if re.search(rf"\b{k}<", name) and re.search(r", float>\(", name):
-            return re.sub(r", float>\(", ">(", name, count=1)
+def normalise(name: str, strip: tuple[str, ...], strip_dup: tuple[str, ...] = (), untemplate: tuple[str, ...] = ()) -> str:
+    m = re.match(r"(?:void )?whvi::(\w+)(?:<([^()]*)>)?\(", name)
+    if m and m.group(1) in untemplate:
+        args = m.group(2)
+        if args is None or all(a.strip() == "float" for a in args.split(",")):
+            return f"whvi::{m.group(1)}"
+        return f"whvi::{m.group(1)}<{args}>"
+    for k in strip_dup:
+        if re.search(rf"\b{k}<", name):
+            name = re.sub(r", (float|__nv_bfloat16), \1>\(", r", \1>(", name, count=1)
+    for k in strip:   # only a ``float`` that follows a non-type argument: ``<..., __nv_bfloat16, float>`` is a distinct instance
+        if re.search(rf"\b{k}<", name):
+            return re.sub(r"(\(\w+\)-?\d+), float>\(", r"\1>(", name, count=1)
     return name
 
 
-def collect(obj_dir: Path, strip: tuple[str, ...]) -> dict[str, tuple[str, list[str]]]:
+def collect(obj_dir: Path, strip: tuple[str, ...], strip_dup: tuple[str, ...] = (), untemplate: tuple[str, ...] = ()
+            ) -> dict[str, tuple[str, list[str]]]:
     res: dict[str, tuple[str, list[str]]] = {}
     for obj in sorted(obj_dir.glob("*.o")):
         funcs = kernels(obj)
         dm = demangle(list(funcs))
         for mangled, sass in funcs.items():
-            res[normalise(dm[mangled], strip)] = (obj.name, sass)
+            res[normalise(dm[mangled], strip, strip_dup, untemplate)] = (obj.name, sass)
     return res
 
 
@@ -72,9 +91,12 @@ def main() -> int:
     ap.add_argument("old", type=Path)
     ap.add_argument("new", type=Path)
     ap.add_argument("--strip-arg", nargs="*", default=list(DEFAULT_STRIP))
+    ap.add_argument("--strip-dup", nargs="*", default=list(DEFAULT_STRIP_DUP))
+    ap.add_argument("--untemplate", nargs="*", default=list(DEFAULT_UNTEMPLATE))
     a = ap.parse_args()
-    strip = tuple(a.strip_arg)
-    old, new = collect(a.old, ()), collect(a.new, strip)
+    untemplate = tuple(a.untemplate)
+    strip, strip_dup = tuple(a.strip_arg), tuple(a.strip_dup)
+    old, new = collect(a.old, strip, strip_dup, untemplate), collect(a.new, strip, strip_dup, untemplate)
     same, differ, missing = 0, [], []
     for name, (obj, sass) in sorted(old.items()):
         if name not in new:

@@ -96,6 +96,27 @@ SIGNATURES = {
     "whvi_layer_loss_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                      c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_int,
                                      c_void_p]),
+    # bf16 twins of the Stacked and Column calls: the fp32 signatures with void* activations
+    "whvi_pad_rows_bf16": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p]),
+    "whvi_stacked_fwd_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
+                                      c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_int64, c_int, c_void_p]),
+    "whvi_stacked_fwd_g_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64,
+                                        c_int64, c_int64, c_int64, c_int64, c_int, c_void_p]),
+    "whvi_stacked_bwd_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
+                                      c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64,
+                                      c_int64, c_int64, c_int64, c_int, c_void_p]),
+    "whvi_stacked_bwd_g_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p,
+                                        c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_int64, c_int64, c_int,
+                                        c_void_p]),
+    "whvi_column_fwd_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_int64, c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
+    "whvi_column_fwd_g_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64,
+                                       c_int64, c_int64, c_int, c_int, c_void_p]),
+    "whvi_column_bwd_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_int64,
+                                     c_int, c_int, c_void_p]),
+    "whvi_column_bwd_g_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                       c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
     "whvi_fwht_f64": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p]),
     "whvi_mc_moments_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p]),
     "whvi_mc_moments_strided_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64,

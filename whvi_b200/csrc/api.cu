@@ -446,54 +446,93 @@ static int check_stacked(const char* who, int64_t S, int64_t B, int64_t D, int64
     return WHVI_OK;
 }
 
+static int pad_rows(const char* who, const void* in, void* out, int64_t rows, int64_t n_in, int64_t D, int bf16, whvi_stream_t stream)
+{
+    if (rows < 0 || n_in < 1 || D < n_in || D % 4 != 0) return fail(WHVI_E_SHAPE, "%s: rows=%lld n_in=%lld D=%lld", who, (long long)rows, (long long)n_in, (long long)D);
+    if (rows == 0) return WHVI_OK;
+    if (!in || !out) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (!aligned16(out)) return fail(WHVI_E_ALIGN, "%s: out must be 16-byte aligned", who);
+    if (bf16 && (reinterpret_cast<uintptr_t>(in) & 1u)) return fail(WHVI_E_ALIGN, "%s: in must be 2-byte aligned", who);
+    return launch_stack_split(static_cast<const float*>(in), static_cast<float*>(out), rows, D, 1, n_in, static_cast<cudaStream_t>(stream), bf16);
+}
+
 int whvi_pad_rows_f32(const float* in, float* out, int64_t rows, int64_t n_in, int64_t D, whvi_stream_t stream)
 {
-    if (rows < 0 || n_in < 1 || D < n_in || D % 4 != 0) return fail(WHVI_E_SHAPE, "pad_rows: rows=%lld n_in=%lld D=%lld", (long long)rows, (long long)n_in, (long long)D);
-    if (rows == 0) return WHVI_OK;
-    if (!in || !out) return fail(WHVI_E_NULL, "pad_rows: null pointer");
-    if (!aligned16(out)) return fail(WHVI_E_ALIGN, "pad_rows: out must be 16-byte aligned");
-    return launch_stack_split(in, out, rows, D, 1, n_in, static_cast<cudaStream_t>(stream));
+    return pad_rows("pad_rows", in, out, rows, n_in, D, 0, stream);
 }
+
+int whvi_pad_rows_bf16(const void* in, void* out, int64_t rows, int64_t n_in, int64_t D, whvi_stream_t stream)
+{
+    return pad_rows("pad_rows_bf16", in, out, rows, n_in, D, 1, stream);
+}
+
+// bf16 activations (x, y_blocks, y, dy, dx) behind the float pointers of the internal calls: a pointer of 2-byte elements must be
+// 2-byte aligned; the padded x and the block-layout dy of the backward arrive by bulk copy (see check_bf16_io)
+static bool odd(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 1u) != 0; }
 
 // the layer from g (G, S, D), however g was drawn; validated by the callers
 static int stacked_fwd_g(const float* x, int64_t xs, const float* g, const float* s1, const float* s2, int64_t param_stride, const float* bias,
-                         float* y_blocks, float* y, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, cudaStream_t st)
+                         float* y_blocks, float* y, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, cudaStream_t st, int bf16 = 0)
 {
     LayerFwdCall c{x, g, s1, s2, bias, nullptr, y_blocks, nullptr, xs, G * S, B, flags & WHVI_LAYER_RELU_OUT, nullptr};
     c.groups = G;
     c.pstride = param_stride;
     c.bstride = D;
+    c.bf16 = bf16;
     if (int rc = launch_layer_fwd(c, D, st)) return rc;
-    return launch_stack_concat(y_blocks, y, S * B, D, G, n_out, st);
+    return launch_stack_concat(y_blocks, y, S * B, D, G, n_out, st, bf16);
+}
+
+// a Stacked forward: from (mu, rho, eps) drawn here, or -- from_g -- from g given (then mu, rho, eps are unused)
+static int stacked_fwd(const char* who, int from_g, const void* x, int64_t x_sample_stride, const float* mu, const float* rho, const float* s1,
+                       const float* s2, int64_t param_stride, const float* eps, const float* bias, float* g, void* y_blocks, void* y, int64_t S,
+                       int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, int bf16, whvi_stream_t stream)
+{
+    if (int rc = check_stacked(who, S, B, D, G, n_out, x_sample_stride, param_stride)) return rc;
+    if (flags & ~WHVI_LAYER_RELU_OUT) return fail(WHVI_E_MODE, "%s: unknown flags %d", who, flags);
+    if (S == 0 || B == 0) return WHVI_OK;
+    if (!x || (!from_g && (!mu || !rho || !eps)) || !s1 || !s2 || !g || !y_blocks || !y) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (!aligned16(s1) || !aligned16(s2) || !aligned16(bias) || !aligned16(g))
+        return fail(WHVI_E_ALIGN, "%s: pointers must be 16-byte aligned", who);
+    if (bf16 ? ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y_blocks)) & 7u) || odd(y) : !aligned16(x) || !aligned16(y_blocks))
+        return fail(WHVI_E_ALIGN, bf16 ? "%s: x and y_blocks must be 8-byte aligned, y 2-byte aligned" : "%s: pointers must be 16-byte aligned", who);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (!from_g)
+        if (int rc = launch_reparam_diag(mu, rho, eps, g, G * S, D, st, G, param_stride)) return rc;
+    return stacked_fwd_g(static_cast<const float*>(x), x_sample_stride, g, s1, s2, param_stride, bias, static_cast<float*>(y_blocks),
+                         static_cast<float*>(y), S, B, D, G, n_out, flags, st, bf16);
 }
 
 int whvi_stacked_fwd_f32(const float* x, int64_t x_sample_stride, const float* mu, const float* rho, const float* s1, const float* s2,
                          int64_t param_stride, const float* eps, const float* bias, float* g, float* y_blocks, float* y, int64_t S,
                          int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, whvi_stream_t stream)
 {
-    if (int rc = check_stacked("stacked_fwd", S, B, D, G, n_out, x_sample_stride, param_stride)) return rc;
-    if (flags & ~WHVI_LAYER_RELU_OUT) return fail(WHVI_E_MODE, "stacked_fwd: unknown flags %d", flags);
-    if (S == 0 || B == 0) return WHVI_OK;
-    if (!x || !mu || !rho || !s1 || !s2 || !eps || !g || !y_blocks || !y) return fail(WHVI_E_NULL, "stacked_fwd: null pointer");
-    if (!aligned16(x) || !aligned16(s1) || !aligned16(s2) || !aligned16(bias) || !aligned16(g) || !aligned16(y_blocks))
-        return fail(WHVI_E_ALIGN, "stacked_fwd: pointers must be 16-byte aligned");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (int rc = launch_reparam_diag(mu, rho, eps, g, G * S, D, st, G, param_stride)) return rc;
-    return stacked_fwd_g(x, x_sample_stride, g, s1, s2, param_stride, bias, y_blocks, y, S, B, D, G, n_out, flags, st);
+    return stacked_fwd("stacked_fwd", 0, x, x_sample_stride, mu, rho, s1, s2, param_stride, eps, bias, g, y_blocks, y, S, B, D, G, n_out, flags, 0,
+                       stream);
+}
+
+int whvi_stacked_fwd_bf16(const void* x, int64_t x_sample_stride, const float* mu, const float* rho, const float* s1, const float* s2,
+                          int64_t param_stride, const float* eps, const float* bias, float* g, void* y_blocks, void* y, int64_t S,
+                          int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, whvi_stream_t stream)
+{
+    return stacked_fwd("stacked_fwd_bf16", 0, x, x_sample_stride, mu, rho, s1, s2, param_stride, eps, bias, g, y_blocks, y, S, B, D, G, n_out, flags,
+                       1, stream);
 }
 
 int whvi_stacked_fwd_g_f32(const float* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2, int64_t param_stride,
                            const float* bias, float* y_blocks, float* y, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags,
                            whvi_stream_t stream)
 {
-    if (int rc = check_stacked("stacked_fwd_g", S, B, D, G, n_out, x_sample_stride, param_stride)) return rc;
-    if (flags & ~WHVI_LAYER_RELU_OUT) return fail(WHVI_E_MODE, "stacked_fwd_g: unknown flags %d", flags);
-    if (S == 0 || B == 0) return WHVI_OK;
-    if (!x || !g || !s1 || !s2 || !y_blocks || !y) return fail(WHVI_E_NULL, "stacked_fwd_g: null pointer");
-    if (!aligned16(x) || !aligned16(s1) || !aligned16(s2) || !aligned16(bias) || !aligned16(g) || !aligned16(y_blocks))
-        return fail(WHVI_E_ALIGN, "stacked_fwd_g: pointers must be 16-byte aligned");
-    return stacked_fwd_g(x, x_sample_stride, g, s1, s2, param_stride, bias, y_blocks, y, S, B, D, G, n_out, flags,
-                         static_cast<cudaStream_t>(stream));
+    return stacked_fwd("stacked_fwd_g", 1, x, x_sample_stride, nullptr, nullptr, s1, s2, param_stride, nullptr, bias, const_cast<float*>(g),
+                       y_blocks, y, S, B, D, G, n_out, flags, 0, stream);
+}
+
+int whvi_stacked_fwd_g_bf16(const void* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2, int64_t param_stride,
+                            const float* bias, void* y_blocks, void* y, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags,
+                            whvi_stream_t stream)
+{
+    return stacked_fwd("stacked_fwd_g_bf16", 1, x, x_sample_stride, nullptr, nullptr, s1, s2, param_stride, nullptr, bias, const_cast<float*>(g),
+                       y_blocks, y, S, B, D, G, n_out, flags, 1, stream);
 }
 
 static size_t stacked_bwd_layout(int64_t S, int64_t B, int64_t D, int64_t G, int want_dx, size_t layer_ws, size_t* off_dx, size_t* off_dg,
@@ -542,20 +581,60 @@ static int stacked_bwd_plan(const char* who, int64_t S, int64_t B, int64_t D, in
 }
 
 // the layer's backward from dy (S, B, n_out) down to dg (G, S, D) and the per-block dx (left in the workspace for the caller's
-// block sum); validated and planned by the callers
+// block sum); validated and planned by the callers.  bf16: dy is split into the first half of the (fp32-sized) dy-block region,
+// and the per-block dx stay fp32 (summed and rounded once by stack_sum)
 static int stacked_bwd_g(const float* x, int64_t xs, const float* dy, const float* g, const float* s1, const float* s2, int64_t param_stride,
                          float* dx, float* dg, float* ds1, float* ds2, float* dbias, void* workspace, size_t layer_ws, size_t off_dx,
-                         size_t off_ws, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, cudaStream_t st)
+                         size_t off_ws, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, cudaStream_t st, int bf16 = 0)
 {
     char* base = static_cast<char*>(workspace);
     float* dyb = reinterpret_cast<float*>(base);
     float* dxb = dx ? reinterpret_cast<float*>(base + off_dx) : nullptr;
-    if (int rc = launch_stack_split(dy, dyb, S * B, D, G, n_out, st)) return rc;
+    if (int rc = launch_stack_split(dy, dyb, S * B, D, G, n_out, st, bf16)) return rc;
     LayerBwdCall c{x, dyb, g, s1, s2, nullptr, nullptr, nullptr, dxb, dg, ds1, ds2, dbias, reinterpret_cast<float*>(base + off_ws),
                    layer_ws, xs, S * G, B, flags & WHVI_LAYER_RELU_IN, nullptr};
     c.groups = G;
     c.pstride = param_stride;
+    c.bf16 = bf16;
+    c.dx_f32 = bf16;
     return launch_layer_bwd(c, D, st);
+}
+
+// a Stacked backward: down to (dmu, drho) through the diagonal reparameterisation, or -- from_g -- to dg (G, S, D) in the caller's
+// buffer g_out (then rho, eps, dmu and drho are unused)
+static int stacked_bwd(const char* who, int from_g, float* g_out, const void* x, int64_t x_sample_stride, const void* dy, const float* g, const float* rho,
+                       const float* s1, const float* s2, int64_t param_stride, const float* eps, void* dx, int64_t n_in, float* dmu, float* drho,
+                       float* ds1, float* ds2, float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t G,
+                       int64_t n_out, int flags, int bf16, whvi_stream_t stream)
+{
+    if (int rc = check_stacked(who, S, B, D, G, n_out, x_sample_stride, param_stride)) return rc;
+    if (flags & ~WHVI_LAYER_RELU_IN) return fail(WHVI_E_MODE, "%s: unknown flags %d", who, flags);
+    if (dx && (n_in < 1 || n_in > D)) return fail(WHVI_E_SHAPE, "%s: n_in=%lld outside [1, D]", who, (long long)n_in);
+    if ((from_g ? !g_out : (!dmu || !drho)) || !ds1 || !ds2) return fail(WHVI_E_NULL, "%s: null output pointer", who);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (S == 0 || B == 0) {
+        if (from_g && S > 0) cudaMemsetAsync(g_out, 0, sizeof(float) * size_t(G) * S * D, st);
+        for (float* p : {dmu, drho, ds1, ds2, dbias})
+            if (p) cudaMemsetAsync(p, 0, sizeof(float) * size_t(G) * D, st);
+        return check_launch(from_g ? "stacked_bwd_g(empty)" : "stacked_bwd(empty)");
+    }
+    if (!x || !dy || !g || (!from_g && (!rho || !eps)) || !s1 || !s2) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (!aligned16(x) || !aligned16(g) || !aligned16(s1) || !aligned16(s2) || !aligned16(g_out) || !aligned16(workspace))
+        return fail(WHVI_E_ALIGN, "%s: pointers must be 16-byte aligned", who);
+    if (bf16 && (B * D) % 8 != 0)   // the padded x and the block-layout dy reach the backward kernel by bulk copy (check_bf16_io)
+        return fail(WHVI_E_SHAPE, "%s: B * D = %lld must be a multiple of 8 for bf16 activations (pad B)", who, (long long)(B * D));
+    if (bf16 && (odd(dy) || odd(dx))) return fail(WHVI_E_ALIGN, "%s: dy and dx must be 2-byte aligned", who);
+    size_t off_dx, off_dg, off_ws, layer_ws;
+    if (int rc = stacked_bwd_plan(who, S, B, D, G, dx != nullptr, workspace, workspace_bytes, &layer_ws, &off_dx, &off_dg, &off_ws)) return rc;
+    float* dg = from_g ? g_out : reinterpret_cast<float*>(static_cast<char*>(workspace) + off_dg);
+    if (int rc = stacked_bwd_g(static_cast<const float*>(x), x_sample_stride, static_cast<const float*>(dy), g, s1, s2, param_stride,
+                               static_cast<float*>(dx), dg, ds1, ds2, dbias, workspace, layer_ws, off_dx, off_ws, S, B, D, G, n_out, flags, st, bf16))
+        return rc;
+    if (!from_g)
+        if (int rc = launch_reparam_diag_bwd(rho, eps, dg, dmu, drho, S, D, 0, st, G, param_stride)) return rc;
+    if (dx)
+        return launch_stack_sum(reinterpret_cast<float*>(static_cast<char*>(workspace) + off_dx), static_cast<float*>(dx), S * B, D, G, n_in, st, bf16);
+    return WHVI_OK;
 }
 
 int whvi_stacked_bwd_f32(const float* x, int64_t x_sample_stride, const float* dy, const float* g, const float* rho, const float* s1,
@@ -563,59 +642,34 @@ int whvi_stacked_bwd_f32(const float* x, int64_t x_sample_stride, const float* d
                          float* ds1, float* ds2, float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D,
                          int64_t G, int64_t n_out, int flags, whvi_stream_t stream)
 {
-    if (int rc = check_stacked("stacked_bwd", S, B, D, G, n_out, x_sample_stride, param_stride)) return rc;
-    if (flags & ~WHVI_LAYER_RELU_IN) return fail(WHVI_E_MODE, "stacked_bwd: unknown flags %d", flags);
-    if (dx && (n_in < 1 || n_in > D)) return fail(WHVI_E_SHAPE, "stacked_bwd: n_in=%lld outside [1, D]", (long long)n_in);
-    if (!dmu || !drho || !ds1 || !ds2) return fail(WHVI_E_NULL, "stacked_bwd: null output pointer");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (S == 0 || B == 0) {
-        for (float* p : {dmu, drho, ds1, ds2, dbias})
-            if (p) cudaMemsetAsync(p, 0, sizeof(float) * size_t(G) * D, st);
-        return check_launch("stacked_bwd(empty)");
-    }
-    if (!x || !dy || !g || !rho || !s1 || !s2 || !eps) return fail(WHVI_E_NULL, "stacked_bwd: null pointer");
-    if (!aligned16(x) || !aligned16(g) || !aligned16(s1) || !aligned16(s2) || !aligned16(workspace))
-        return fail(WHVI_E_ALIGN, "stacked_bwd: pointers must be 16-byte aligned");
-    size_t off_dx, off_dg, off_ws, layer_ws;
-    if (int rc = stacked_bwd_plan("stacked_bwd", S, B, D, G, dx != nullptr, workspace, workspace_bytes, &layer_ws, &off_dx, &off_dg, &off_ws))
-        return rc;
-    float* dg = reinterpret_cast<float*>(static_cast<char*>(workspace) + off_dg);
-    if (int rc = stacked_bwd_g(x, x_sample_stride, dy, g, s1, s2, param_stride, dx, dg, ds1, ds2, dbias, workspace, layer_ws, off_dx,
-                               off_ws, S, B, D, G, n_out, flags, st))
-        return rc;
-    if (int rc = launch_reparam_diag_bwd(rho, eps, dg, dmu, drho, S, D, 0, st, G, param_stride)) return rc;
-    if (dx) return launch_stack_sum(reinterpret_cast<float*>(static_cast<char*>(workspace) + off_dx), dx, S * B, D, G, n_in, st);
-    return WHVI_OK;
+    return stacked_bwd("stacked_bwd", 0, nullptr, x, x_sample_stride, dy, g, rho, s1, s2, param_stride, eps, dx, n_in, dmu, drho, ds1, ds2, dbias,
+                       workspace, workspace_bytes, S, B, D, G, n_out, flags, 0, stream);
+}
+
+int whvi_stacked_bwd_bf16(const void* x, int64_t x_sample_stride, const void* dy, const float* g, const float* rho, const float* s1,
+                          const float* s2, int64_t param_stride, const float* eps, void* dx, int64_t n_in, float* dmu, float* drho,
+                          float* ds1, float* ds2, float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D,
+                          int64_t G, int64_t n_out, int flags, whvi_stream_t stream)
+{
+    return stacked_bwd("stacked_bwd_bf16", 0, nullptr, x, x_sample_stride, dy, g, rho, s1, s2, param_stride, eps, dx, n_in, dmu, drho, ds1, ds2, dbias,
+                       workspace, workspace_bytes, S, B, D, G, n_out, flags, 1, stream);
 }
 
 int whvi_stacked_bwd_g_f32(const float* x, int64_t x_sample_stride, const float* dy, const float* g, const float* s1, const float* s2,
                            int64_t param_stride, float* dx, int64_t n_in, float* dg, float* ds1, float* ds2, float* dbias, void* workspace,
                            size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, whvi_stream_t stream)
 {
-    if (int rc = check_stacked("stacked_bwd_g", S, B, D, G, n_out, x_sample_stride, param_stride)) return rc;
-    if (flags & ~WHVI_LAYER_RELU_IN) return fail(WHVI_E_MODE, "stacked_bwd_g: unknown flags %d", flags);
-    if (dx && (n_in < 1 || n_in > D)) return fail(WHVI_E_SHAPE, "stacked_bwd_g: n_in=%lld outside [1, D]", (long long)n_in);
-    if (!dg || !ds1 || !ds2) return fail(WHVI_E_NULL, "stacked_bwd_g: null output pointer");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (S == 0 || B == 0) {
-        if (S > 0) cudaMemsetAsync(dg, 0, sizeof(float) * size_t(G) * S * D, st);
-        for (float* p : {ds1, ds2, dbias})
-            if (p) cudaMemsetAsync(p, 0, sizeof(float) * size_t(G) * D, st);
-        return check_launch("stacked_bwd_g(empty)");
-    }
-    if (!x || !dy || !g || !s1 || !s2) return fail(WHVI_E_NULL, "stacked_bwd_g: null pointer");
-    if (!aligned16(x) || !aligned16(g) || !aligned16(s1) || !aligned16(s2) || !aligned16(dg) || !aligned16(workspace))
-        return fail(WHVI_E_ALIGN, "stacked_bwd_g: pointers must be 16-byte aligned");
-    size_t off_dx, off_dg, off_ws, layer_ws;
-    if (int rc = stacked_bwd_plan("stacked_bwd_g", S, B, D, G, dx != nullptr, workspace, workspace_bytes, &layer_ws, &off_dx, &off_dg, &off_ws))
-        return rc;
-    if (int rc = stacked_bwd_g(x, x_sample_stride, dy, g, s1, s2, param_stride, dx, dg, ds1, ds2, dbias, workspace, layer_ws, off_dx,
-                               off_ws, S, B, D, G, n_out, flags, st))
-        return rc;
-    if (dx) return launch_stack_sum(reinterpret_cast<float*>(static_cast<char*>(workspace) + off_dx), dx, S * B, D, G, n_in, st);
-    return WHVI_OK;
+    return stacked_bwd("stacked_bwd_g", 1, dg, x, x_sample_stride, dy, g, nullptr, s1, s2, param_stride, nullptr, dx, n_in, nullptr, nullptr, ds1,
+                       ds2, dbias, workspace, workspace_bytes, S, B, D, G, n_out, flags, 0, stream);
 }
 
+int whvi_stacked_bwd_g_bf16(const void* x, int64_t x_sample_stride, const void* dy, const float* g, const float* s1, const float* s2,
+                            int64_t param_stride, void* dx, int64_t n_in, float* dg, float* ds1, float* ds2, float* dbias, void* workspace,
+                            size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t G, int64_t n_out, int flags, whvi_stream_t stream)
+{
+    return stacked_bwd("stacked_bwd_g_bf16", 1, dg, x, x_sample_stride, dy, g, nullptr, s1, s2, param_stride, nullptr, dx, n_in, nullptr, nullptr,
+                       ds1, ds2, dbias, workspace, workspace_bytes, S, B, D, G, n_out, flags, 1, stream);
+}
 int whvi_kl_grouped_f32(const float* mu, const float* rho, float lambda_, int64_t D, int64_t G, int64_t param_stride, int mode,
                         float* out_kl, float* dmu, float* drho, float grad_scale, whvi_stream_t stream)
 {
@@ -637,18 +691,53 @@ static int check_column(const char* who, int64_t S, int64_t B, int64_t D, int64_
     return WHVI_OK;
 }
 
+// a Column forward: from (mu, rho, eps) drawn here into g, or -- from_g -- from g given (then mu, rho, eps are unused).  bf16: x and
+// the plain form's y are bf16; the transposed form's y (S, B, 1) stays fp32
+static int column_fwd(const char* who, int from_g, const void* x, int64_t x_sample_stride, const float* mu, const float* rho, const float* s1,
+                      const float* s2, const float* eps, const float* bias, float* g, float* hg, void* y, int64_t S, int64_t B, int64_t D, int64_t n,
+                      int transposed, int flags, int bf16, whvi_stream_t stream)
+{
+    if (int rc = check_column(who, S, B, D, n, x_sample_stride, transposed)) return rc;
+    if (flags & ~WHVI_LAYER_RELU_OUT) return fail(WHVI_E_MODE, "%s: unknown flags %d", who, flags);
+    if ((flags & WHVI_LAYER_RELU_OUT) && transposed) return fail(WHVI_E_MODE, "%s: RELU_OUT applies to the (.., 1) -> (.., n) form only", who);
+    if (S == 0 || B == 0) return WHVI_OK;
+    if (!x || (!from_g && (!mu || !rho || !eps)) || !s1 || !s2 || !g || !hg || !y) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (!aligned16(g) || !aligned16(hg)) return fail(WHVI_E_ALIGN, "%s: g and hg must be 16-byte aligned", who);
+    if (bf16 && (odd(x) || (!transposed && odd(y)))) return fail(WHVI_E_ALIGN, "%s: bf16 pointers must be 2-byte aligned", who);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (from_g)
+        return launch_column_fwd_g(static_cast<const float*>(x), x_sample_stride, g, s1, s2, bias, hg, static_cast<float*>(y), S, B, D, n,
+                                   transposed, flags & WHVI_LAYER_RELU_OUT, st, bf16);
+    return launch_column_fwd(static_cast<const float*>(x), x_sample_stride, mu, rho, s1, s2, eps, bias, g, hg, static_cast<float*>(y), S, B, D, n,
+                             transposed, flags & WHVI_LAYER_RELU_OUT, st, bf16);
+}
+
 int whvi_column_fwd_f32(const float* x, int64_t x_sample_stride, const float* mu, const float* rho, const float* s1, const float* s2,
                         const float* eps, const float* bias, float* g, float* hg, float* y, int64_t S, int64_t B, int64_t D, int64_t n,
                         int transposed, int flags, whvi_stream_t stream)
 {
-    if (int rc = check_column("column_fwd", S, B, D, n, x_sample_stride, transposed)) return rc;
-    if (flags & ~WHVI_LAYER_RELU_OUT) return fail(WHVI_E_MODE, "column_fwd: unknown flags %d", flags);
-    if ((flags & WHVI_LAYER_RELU_OUT) && transposed) return fail(WHVI_E_MODE, "column_fwd: RELU_OUT applies to the (.., 1) -> (.., n) form only");
-    if (S == 0 || B == 0) return WHVI_OK;
-    if (!x || !mu || !rho || !s1 || !s2 || !eps || !g || !hg || !y) return fail(WHVI_E_NULL, "column_fwd: null pointer");
-    if (!aligned16(g) || !aligned16(hg)) return fail(WHVI_E_ALIGN, "column_fwd: g and hg must be 16-byte aligned");
-    return launch_column_fwd(x, x_sample_stride, mu, rho, s1, s2, eps, bias, g, hg, y, S, B, D, n, transposed, flags & WHVI_LAYER_RELU_OUT,
-                             static_cast<cudaStream_t>(stream));
+    return column_fwd("column_fwd", 0, x, x_sample_stride, mu, rho, s1, s2, eps, bias, g, hg, y, S, B, D, n, transposed, flags, 0, stream);
+}
+
+int whvi_column_fwd_bf16(const void* x, int64_t x_sample_stride, const float* mu, const float* rho, const float* s1, const float* s2,
+                         const float* eps, const float* bias, float* g, float* hg, void* y, int64_t S, int64_t B, int64_t D, int64_t n,
+                         int transposed, int flags, whvi_stream_t stream)
+{
+    return column_fwd("column_fwd_bf16", 0, x, x_sample_stride, mu, rho, s1, s2, eps, bias, g, hg, y, S, B, D, n, transposed, flags, 1, stream);
+}
+
+int whvi_column_fwd_g_f32(const float* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2, const float* bias, float* hg,
+                          float* y, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int flags, whvi_stream_t stream)
+{
+    return column_fwd("column_fwd_g", 1, x, x_sample_stride, nullptr, nullptr, s1, s2, nullptr, bias, const_cast<float*>(g), hg, y, S, B, D, n,
+                      transposed, flags, 0, stream);
+}
+
+int whvi_column_fwd_g_bf16(const void* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2, const float* bias, float* hg,
+                           void* y, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int flags, whvi_stream_t stream)
+{
+    return column_fwd("column_fwd_g_bf16", 1, x, x_sample_stride, nullptr, nullptr, s1, s2, nullptr, bias, const_cast<float*>(g), hg, y, S, B, D, n,
+                      transposed, flags, 1, stream);
 }
 
 int whvi_column_bwd_workspace_bytes(int64_t S, int64_t D, int64_t n, size_t* bytes)
@@ -659,65 +748,70 @@ int whvi_column_bwd_workspace_bytes(int64_t S, int64_t D, int64_t n, size_t* byt
     return WHVI_OK;
 }
 
+// a Column backward: down to (dmu, drho) through the diagonal reparameterisation, or -- from_g -- to dg (S, D) (then rho, eps, dmu and
+// drho are unused).  bf16: x, dx and the plain form's dy are bf16; the transposed form's dy (S, B, 1) stays fp32
+static int column_bwd(const char* who, int from_g, const void* x, int64_t x_sample_stride, const void* dy, const float* hg, const float* rho,
+                      const float* s1, const float* s2, const float* eps, void* dx, float* dg, float* dmu, float* drho, float* ds1, float* ds2,
+                      float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int flags,
+                      int bf16, whvi_stream_t stream)
+{
+    if (int rc = check_column(who, S, B, D, n, x_sample_stride, transposed)) return rc;
+    if (flags & ~WHVI_LAYER_RELU_IN) return fail(WHVI_E_MODE, "%s: unknown flags %d", who, flags);
+    if ((flags & WHVI_LAYER_RELU_IN) && !transposed) return fail(WHVI_E_MODE, "%s: RELU_IN applies to the (.., n) -> (.., 1) form only", who);
+    if ((from_g ? !dg : (!dmu || !drho)) || !ds1 || !ds2) return fail(WHVI_E_NULL, "%s: null output pointer", who);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (S == 0 || B == 0) {
+        if (from_g && S > 0) cudaMemsetAsync(dg, 0, sizeof(float) * size_t(S) * D, st);
+        for (float* p : {dmu, drho, ds1, ds2})
+            if (p) cudaMemsetAsync(p, 0, sizeof(float) * size_t(D), st);
+        if (dbias) cudaMemsetAsync(dbias, 0, sizeof(float) * size_t(transposed ? 1 : n), st);
+        return check_launch(from_g ? "column_bwd_g(empty)" : "column_bwd(empty)");
+    }
+    if (!x || !dy || !hg || (!from_g && (!rho || !eps)) || !s1 || !s2) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (from_g ? !aligned16(workspace) || !aligned16(dg) : !aligned16(workspace))
+        return fail(WHVI_E_ALIGN, from_g ? "%s: workspace and dg must be 16-byte aligned" : "%s: workspace must be 16-byte aligned", who);
+    if (bf16 && (odd(x) || odd(dx) || (!transposed && odd(dy)))) return fail(WHVI_E_ALIGN, "%s: bf16 pointers must be 2-byte aligned", who);
+    const size_t need = column_bwd_workspace_bytes(S, D, n);
+    if (!workspace || workspace_bytes < need) return fail(WHVI_E_WORKSPACE, "%s: workspace of %zu bytes needed, %zu given", who, need, workspace_bytes);
+    if (from_g)
+        return launch_column_bwd_g(static_cast<const float*>(x), x_sample_stride, static_cast<const float*>(dy), hg, s1, s2, static_cast<float*>(dx),
+                                   dg, ds1, ds2, dbias, static_cast<float*>(workspace), S, B, D, n, transposed, flags & WHVI_LAYER_RELU_IN, st, bf16);
+    return launch_column_bwd(static_cast<const float*>(x), x_sample_stride, static_cast<const float*>(dy), hg, rho, s1, s2, eps, static_cast<float*>(dx),
+                             dmu, drho, ds1, ds2, dbias, static_cast<float*>(workspace), S, B, D, n, transposed, flags & WHVI_LAYER_RELU_IN, st, bf16);
+}
+
 int whvi_column_bwd_f32(const float* x, int64_t x_sample_stride, const float* dy, const float* hg, const float* rho, const float* s1,
                         const float* s2, const float* eps, float* dx, float* dmu, float* drho, float* ds1, float* ds2, float* dbias,
                         void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int flags,
                         whvi_stream_t stream)
 {
-    if (int rc = check_column("column_bwd", S, B, D, n, x_sample_stride, transposed)) return rc;
-    if (flags & ~WHVI_LAYER_RELU_IN) return fail(WHVI_E_MODE, "column_bwd: unknown flags %d", flags);
-    if ((flags & WHVI_LAYER_RELU_IN) && !transposed) return fail(WHVI_E_MODE, "column_bwd: RELU_IN applies to the (.., n) -> (.., 1) form only");
-    if (!dmu || !drho || !ds1 || !ds2) return fail(WHVI_E_NULL, "column_bwd: null output pointer");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (S == 0 || B == 0) {
-        for (float* p : {dmu, drho, ds1, ds2})
-            cudaMemsetAsync(p, 0, sizeof(float) * size_t(D), st);
-        if (dbias) cudaMemsetAsync(dbias, 0, sizeof(float) * size_t(transposed ? 1 : n), st);
-        return check_launch("column_bwd(empty)");
-    }
-    if (!x || !dy || !hg || !rho || !s1 || !s2 || !eps) return fail(WHVI_E_NULL, "column_bwd: null pointer");
-    if (!aligned16(workspace)) return fail(WHVI_E_ALIGN, "column_bwd: workspace must be 16-byte aligned");
-    const size_t need = column_bwd_workspace_bytes(S, D, n);
-    if (!workspace || workspace_bytes < need) return fail(WHVI_E_WORKSPACE, "column_bwd: workspace of %zu bytes needed, %zu given", need, workspace_bytes);
-    return launch_column_bwd(x, x_sample_stride, dy, hg, rho, s1, s2, eps, dx, dmu, drho, ds1, ds2, dbias, static_cast<float*>(workspace), S,
-                             B, D, n, transposed, flags & WHVI_LAYER_RELU_IN, st);
+    return column_bwd("column_bwd", 0, x, x_sample_stride, dy, hg, rho, s1, s2, eps, dx, nullptr, dmu, drho, ds1, ds2, dbias, workspace,
+                      workspace_bytes, S, B, D, n, transposed, flags, 0, stream);
 }
 
-int whvi_column_fwd_g_f32(const float* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2, const float* bias, float* hg,
-                          float* y, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int flags, whvi_stream_t stream)
+int whvi_column_bwd_bf16(const void* x, int64_t x_sample_stride, const void* dy, const float* hg, const float* rho, const float* s1,
+                         const float* s2, const float* eps, void* dx, float* dmu, float* drho, float* ds1, float* ds2, float* dbias,
+                         void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int flags,
+                         whvi_stream_t stream)
 {
-    if (int rc = check_column("column_fwd_g", S, B, D, n, x_sample_stride, transposed)) return rc;
-    if (flags & ~WHVI_LAYER_RELU_OUT) return fail(WHVI_E_MODE, "column_fwd_g: unknown flags %d", flags);
-    if ((flags & WHVI_LAYER_RELU_OUT) && transposed) return fail(WHVI_E_MODE, "column_fwd_g: RELU_OUT applies to the (.., 1) -> (.., n) form only");
-    if (S == 0 || B == 0) return WHVI_OK;
-    if (!x || !g || !s1 || !s2 || !hg || !y) return fail(WHVI_E_NULL, "column_fwd_g: null pointer");
-    if (!aligned16(g) || !aligned16(hg)) return fail(WHVI_E_ALIGN, "column_fwd_g: g and hg must be 16-byte aligned");
-    return launch_column_fwd_g(x, x_sample_stride, g, s1, s2, bias, hg, y, S, B, D, n, transposed, flags & WHVI_LAYER_RELU_OUT,
-                               static_cast<cudaStream_t>(stream));
+    return column_bwd("column_bwd_bf16", 0, x, x_sample_stride, dy, hg, rho, s1, s2, eps, dx, nullptr, dmu, drho, ds1, ds2, dbias, workspace,
+                      workspace_bytes, S, B, D, n, transposed, flags, 1, stream);
 }
 
 int whvi_column_bwd_g_f32(const float* x, int64_t x_sample_stride, const float* dy, const float* hg, const float* s1, const float* s2, float* dx,
                           float* dg, float* ds1, float* ds2, float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D,
                           int64_t n, int transposed, int flags, whvi_stream_t stream)
 {
-    if (int rc = check_column("column_bwd_g", S, B, D, n, x_sample_stride, transposed)) return rc;
-    if (flags & ~WHVI_LAYER_RELU_IN) return fail(WHVI_E_MODE, "column_bwd_g: unknown flags %d", flags);
-    if ((flags & WHVI_LAYER_RELU_IN) && !transposed) return fail(WHVI_E_MODE, "column_bwd_g: RELU_IN applies to the (.., n) -> (.., 1) form only");
-    if (!dg || !ds1 || !ds2) return fail(WHVI_E_NULL, "column_bwd_g: null output pointer");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (S == 0 || B == 0) {
-        if (S > 0) cudaMemsetAsync(dg, 0, sizeof(float) * size_t(S) * D, st);
-        cudaMemsetAsync(ds1, 0, sizeof(float) * size_t(D), st);
-        cudaMemsetAsync(ds2, 0, sizeof(float) * size_t(D), st);
-        if (dbias) cudaMemsetAsync(dbias, 0, sizeof(float) * size_t(transposed ? 1 : n), st);
-        return check_launch("column_bwd_g(empty)");
-    }
-    if (!x || !dy || !hg || !s1 || !s2) return fail(WHVI_E_NULL, "column_bwd_g: null pointer");
-    if (!aligned16(workspace) || !aligned16(dg)) return fail(WHVI_E_ALIGN, "column_bwd_g: workspace and dg must be 16-byte aligned");
-    const size_t need = column_bwd_workspace_bytes(S, D, n);
-    if (!workspace || workspace_bytes < need) return fail(WHVI_E_WORKSPACE, "column_bwd_g: workspace of %zu bytes needed, %zu given", need, workspace_bytes);
-    return launch_column_bwd_g(x, x_sample_stride, dy, hg, s1, s2, dx, dg, ds1, ds2, dbias, static_cast<float*>(workspace), S, B, D, n, transposed,
-                               flags & WHVI_LAYER_RELU_IN, st);
+    return column_bwd("column_bwd_g", 1, x, x_sample_stride, dy, hg, nullptr, s1, s2, nullptr, dx, dg, nullptr, nullptr, ds1, ds2, dbias, workspace,
+                      workspace_bytes, S, B, D, n, transposed, flags, 0, stream);
+}
+
+int whvi_column_bwd_g_bf16(const void* x, int64_t x_sample_stride, const void* dy, const float* hg, const float* s1, const float* s2, void* dx,
+                           float* dg, float* ds1, float* ds2, float* dbias, void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t D,
+                           int64_t n, int transposed, int flags, whvi_stream_t stream)
+{
+    return column_bwd("column_bwd_g_bf16", 1, x, x_sample_stride, dy, hg, nullptr, s1, s2, nullptr, dx, dg, nullptr, nullptr, ds1, ds2, dbias,
+                      workspace, workspace_bytes, S, B, D, n, transposed, flags, 1, stream);
 }
 
 int whvi_layer_moments_f32(const float* x, int64_t x_sample_stride, const float* g, const float* s1, const float* s2,

@@ -79,6 +79,7 @@ struct LayerBwdCall {
     size_t* need_only;  // query mode: workspace bytes
     int64_t groups = 1, pstride = 0;  // grouped launch (see LayerFwdCall): ds1 / ds2 / dbias are (groups, D)
     int bf16 = 0;             // x, dy and dx are bf16 in HBM (behind the float pointers; arithmetic and workspace stay fp32)
+    int dx_f32 = 0;           // with bf16: dx stays fp32 (the grouped backward's per-block dx, summed and rounded once by the caller)
 };
 struct LayerLossCall {  // fused last layer: forward + Gaussian-MNLL residual + backward in one pass
     const float *x, *g, *s1, *s2, *bias, *target;
@@ -111,23 +112,26 @@ int launch_reparam_dense_grouped_bwd(const float* eps, const float* dg, float* d
                                      size_t ws_bytes, cudaStream_t stream);
 int launch_kl_dense_grouped(const float* mu, int64_t mu_stride, const float* L, int64_t L_stride, float lambda_, int64_t D, int64_t G, float* out,
                             float* dmu, float* dL, float grad_scale, double* row_sq, cudaStream_t stream);
+// Column layer; bf16 != 0: x, dx and the plain form's y / dy are bf16 behind the float pointers (column.cu)
 int launch_column_fwd_g(const float* x, int64_t xs, const float* g, const float* s1, const float* s2, const float* bias, float* hg, float* y,
-                        int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int relu_out, cudaStream_t st);
+                        int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int relu_out, cudaStream_t st, int bf16 = 0);
 int launch_column_bwd_g(const float* x, int64_t xs, const float* dy, const float* hg, const float* s1, const float* s2, float* dx, float* dg,
                         float* ds1, float* ds2, float* dbias, float* ws, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int relu_in,
-                        cudaStream_t st);
+                        cudaStream_t st, int bf16 = 0);
 int launch_reparam_diag_bwd(const float* rho, const float* eps, const float* dg, float* dmu, float* drho, int64_t S,
                             int64_t D, int accumulate, cudaStream_t stream, int64_t groups = 1, int64_t pstride = 0);
-int launch_stack_split(const float* in, float* blocks, int64_t R, int64_t D, int64_t G, int64_t n_out, cudaStream_t stream);
-int launch_stack_concat(const float* blocks, float* out, int64_t R, int64_t D, int64_t G, int64_t n_out, cudaStream_t stream);
-int launch_stack_sum(const float* dxb, float* dx, int64_t R, int64_t D, int64_t G, int64_t n_in, cudaStream_t stream);
+// the Stacked interleave kernels; bf16 != 0: the activation side (in / out / dx) is bf16 behind the float pointers (the blocks of
+// split and concat are bf16 too, stack_sum's dxb stays fp32 and its output is rounded once)
+int launch_stack_split(const float* in, float* blocks, int64_t R, int64_t D, int64_t G, int64_t n_out, cudaStream_t stream, int bf16 = 0);
+int launch_stack_concat(const float* blocks, float* out, int64_t R, int64_t D, int64_t G, int64_t n_out, cudaStream_t stream, int bf16 = 0);
+int launch_stack_sum(const float* dxb, float* dx, int64_t R, int64_t D, int64_t G, int64_t n_in, cudaStream_t stream, int bf16 = 0);
 int launch_column_fwd(const float* x, int64_t xs, const float* mu, const float* rho, const float* s1, const float* s2, const float* eps,
                       const float* bias, float* g, float* hg, float* y, int64_t S, int64_t B, int64_t D, int64_t n, int transposed, int relu_out,
-                      cudaStream_t st);
+                      cudaStream_t st, int bf16 = 0);
 size_t column_bwd_workspace_bytes(int64_t S, int64_t D, int64_t n);
 int launch_column_bwd(const float* x, int64_t xs, const float* dy, const float* hg, const float* rho, const float* s1, const float* s2,
                       const float* eps, float* dx, float* dmu, float* drho, float* ds1, float* ds2, float* dbias, float* ws, int64_t S,
-                      int64_t B, int64_t D, int64_t n, int transposed, int relu_in, cudaStream_t st);
+                      int64_t B, int64_t D, int64_t n, int transposed, int relu_in, cudaStream_t st, int bf16 = 0);
 int launch_layer_moments(const float* x, int64_t xs, const float* g, const float* s1, const float* s2, const float* bias, float* sum_y,
                          float* sum_y2, int64_t S, int64_t B, int64_t D, int from_t2, int accumulate, int reserve_sms, cudaStream_t stream,
                          const float* in_y = nullptr, const float* in_y2 = nullptr);

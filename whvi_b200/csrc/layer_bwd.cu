@@ -82,8 +82,10 @@ struct BwdArgs {
 // IO: the activations' type in HBM (x, dy, dx; see layer_fwd_kernel).  bf16 tiles are staged in the first half of their
 // fp32-sized slots (the plan, shared memory and partial-sum order are the fp32 instance's), widened on every read, and dx
 // is rounded once at the store.  The workspace, the parameters and all arithmetic stay fp32; RESID is fp32 only.
+// DX: the type dx is stored as (IO by default).  bf16 x and dy with an fp32 dx serve the grouped (Stacked) backward, whose
+// per-block dx are summed in fp32 and rounded once by the caller.
 template <int N, int C, int KT, int PAIRS, int MINB, int NS, bool SINGLE, bool ALIAS, int PREG, int ROUNDS, bool WANT_DBIAS, bool RESID,
-          class IO = float>
+          class IO = float, class DX = IO>
 __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_kernel(const BwdArgs p)
 {
     static_assert(std::is_same_v<IO, float> || !RESID, "RESID (saved output + target) is fp32 only");
@@ -445,7 +447,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
             apply_g(b, gr);
             from_mid(b);  // b = dt1 (FIRST layout)
             const bool want_dx = p.dx != nullptr;
-            IO* __restrict__ dxs = reinterpret_cast<IO*>(p.dx) + int64_t(s) * p.sample_elems + e0;
+            DX* __restrict__ dxs = reinterpret_cast<DX*>(p.dx) + int64_t(s) * p.sample_elems + e0;
             for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t off, uint32_t coord) {
                 constexpr int m = decltype(m_)::value;
                 const float4 q = raw4(stage_x, off);
@@ -453,7 +455,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
                 fma4(acc_2 + 4 * m, q, b + 4 * m);
                 const float4 o = make_float4(q.x > relu_thr ? b[4 * m] * w.x : 0.f, q.y > relu_thr ? b[4 * m + 1] * w.y : 0.f,
                                              q.z > relu_thr ? b[4 * m + 2] * w.z : 0.f, q.w > relu_thr ? b[4 * m + 3] * w.w : 0.f);
-                if (want_dx && (left >= TILE || off < left)) Io<IO>::st4(dxs + off, o);
+                if (want_dx && (left >= TILE || off < left)) Io<DX>::st4(dxs + off, o);
             });
             mbar_arrive(&empty_bar[pair][st]);
         }
@@ -486,7 +488,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
 //   [4E,5E) s2 (Y) | [5E,5E+H) t2 upper half X->Y | [5E+H,6E) dt3 lower half Y->X | [6E,7E) the same for odd tiles |
 //   [7E,8E) dbias (X)
 // Everything else (bulk-copy staging ring, roles, workspace layout, second-stage reduction) is the kernel above.
-template <int N, int C, int KT, int ROUNDS, bool WANT_DBIAS, bool RESID, class IO = float>
+template <int N, int C, int KT, int ROUNDS, bool WANT_DBIAS, bool RESID, class IO = float, class DX = IO>   // IO, DX: as above
 __global__ void __launch_bounds__(256, 1) layer_bwd_tm_kernel(const BwdArgs p)
 {
     static_assert(std::is_same_v<IO, float> || !RESID, "RESID (saved output + target) is fp32 only");
@@ -823,7 +825,7 @@ __global__ void __launch_bounds__(256, 1) layer_bwd_tm_kernel(const BwdArgs p)
         float acc0[32];
         from_mid(v, acc0);  // X: t4, Y: dt1 (FIRST layout); acc0 = running-sum chunk 0, load in flight
         const bool want_dx = p.dx != nullptr;
-        IO* __restrict__ dxs = reinterpret_cast<IO*>(p.dx) + int64_t(s) * p.sample_elems + e0;
+        DX* __restrict__ dxs = reinterpret_cast<DX*>(p.dx) + int64_t(s) * p.sample_elems + e0;
 #pragma unroll
         for (int c = 0; c < 2; ++c) {   // end product, 32 registers at a time
             float acc1[32];
@@ -863,7 +865,7 @@ __global__ void __launch_bounds__(256, 1) layer_bwd_tm_kernel(const BwdArgs p)
                     const float* bb = v + 32 * c + 4 * j;
                     const float4 o = make_float4(q[j].x > relu_thr ? bb[0] * w[4 * j] : 0.f, q[j].y > relu_thr ? bb[1] * w[4 * j + 1] : 0.f,
                                                  q[j].z > relu_thr ? bb[2] * w[4 * j + 2] : 0.f, q[j].w > relu_thr ? bb[3] * w[4 * j + 3] : 0.f);
-                    if (want_dx && (left >= TILE || off < left)) Io<IO>::st4(dxs + off, o);
+                    if (want_dx && (left >= TILE || off < left)) Io<DX>::st4(dxs + off, o);
                 });
             } else if constexpr (WANT_DBIAS) {
                 float ab[32];
@@ -1028,7 +1030,7 @@ int launch_bwd_reduce(float* ws, float* dg, float* ds1, float* ds2, float* dbias
 template <int N, int C, int KT, int PAIRS, int MINB, int NS, bool SINGLE, bool ALIAS = false, int PREG = 0, int ROUNDS = 3>
 static int launch_bwd_tma_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
 {
-    static unsigned char smem_ok[6][64] = {};
+    static unsigned char smem_ok[8][64] = {};
     constexpr int threads = (2 << (N - C)) * PAIRS;
     constexpr size_t tile = size_t(1) << N;
     constexpr bool gtab = ROUNDS == 2 && !PREG;
@@ -1064,6 +1066,9 @@ static int launch_bwd_tma_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
         if (rs) return fail(WHVI_E_MODE, "layer_bwd: bf16 activations cannot be combined with a target");
         // D >= 2048 runs the tensor-memory kernel; these configurations serve WHVI_BWD_LEGACY builds, which take fp32 only
         if constexpr (N > 10) return fail(WHVI_E_MODE, "layer_bwd: bf16 activations at D = %lld need the tensor-memory backward", (long long)D);
+        else if (c.dx_f32)
+            rc = db ? go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, false, __nv_bfloat16, float>, 6)
+                    : go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, false, false, __nv_bfloat16, float>, 7);
         else rc = db ? go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, false, __nv_bfloat16>, 4)
                      : go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, false, false, __nv_bfloat16>, 5);
     } else if (db && rs) rc = go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, true>, 0);
@@ -1077,7 +1082,7 @@ static int launch_bwd_tma_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
 template <int N, int C, int KT, int ROUNDS>
 static int launch_bwd_tm_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
 {
-    static unsigned char smem_ok[6][64] = {};
+    static unsigned char smem_ok[8][64] = {};
     constexpr int T = 1 << (N - C);
     constexpr int PAIRS = 128 / T;
     constexpr size_t tile = size_t(1) << N;
@@ -1110,8 +1115,11 @@ static int launch_bwd_tm_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
     int rc;
     if (c.bf16) {
         if (rs) return fail(WHVI_E_MODE, "layer_bwd: bf16 activations cannot be combined with a target");
-        rc = db ? go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, true, false, __nv_bfloat16>, 4)
-                : go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, false, false, __nv_bfloat16>, 5);
+        if (c.dx_f32)
+            rc = db ? go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, true, false, __nv_bfloat16, float>, 6)
+                    : go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, false, false, __nv_bfloat16, float>, 7);
+        else rc = db ? go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, true, false, __nv_bfloat16>, 4)
+                     : go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, false, false, __nv_bfloat16>, 5);
     } else if (db && rs) rc = go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, true, true>, 0);
     else if (db) rc = go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, true, false>, 1);
     else if (rs) rc = go(layer_bwd_tm_kernel<N, C, KT, ROUNDS, false, true>, 2);

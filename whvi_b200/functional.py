@@ -31,7 +31,11 @@ _LAUNCHES_PER_CALL = {"whvi_fwht_f32": 1, "whvi_fwht_f64": 1, "whvi_layer_fwd_f3
                       "whvi_layer_bwd_bf16": 3, "whvi_layer_loss_bf16": 3,
                       # dense grouped calls: the counts at D <= 64; at D >= 128 they run the tcgen05 sequence once per block
                       "whvi_reparam_dense_grouped_f32": 1, "whvi_reparam_dense_grouped_bwd_f32": 1, "whvi_kl_dense_grouped_f32": 2,
-                      "whvi_stacked_fwd_g_f32": 2, "whvi_stacked_bwd_g_f32": 5, "whvi_column_fwd_g_f32": 2, "whvi_column_bwd_g_f32": 6}
+                      "whvi_stacked_fwd_g_f32": 2, "whvi_stacked_bwd_g_f32": 5, "whvi_column_fwd_g_f32": 2, "whvi_column_bwd_g_f32": 6,
+                      # bf16 twins of the Stacked and Column calls: the fp32 calls' launches
+                      "whvi_pad_rows_bf16": 1, "whvi_stacked_fwd_bf16": 3, "whvi_stacked_fwd_g_bf16": 2, "whvi_stacked_bwd_bf16": 6,
+                      "whvi_stacked_bwd_g_bf16": 5, "whvi_column_fwd_bf16": 3, "whvi_column_fwd_g_bf16": 2, "whvi_column_bwd_bf16": 7,
+                      "whvi_column_bwd_g_bf16": 6}
 # When set to a dict {"name": [(start_event, stop_event), ...]}, the named calls are bracketed
 # by CUDA events on the launching stream (bench.py's per-kernel roofline timing).
 EVENT_SINK: dict[str, list] | None = None
@@ -850,14 +854,19 @@ def uniform_stride(tensors) -> int | None:
     return step // 4
 
 
+def _act(t: torch.Tensor, name: str) -> torch.Tensor:
+    """A contiguous fp32 or bf16 CUDA activation (the Stacked and Column calls take either, dispatching on the dtype)."""
+    return _bf16c(t, name) if t.dtype == torch.bfloat16 else _f32c(t, name)
+
+
 def _stacked_input(x, S, D):
-    """(x zero-padded to D columns, B, x_sample_stride) for a Stacked call (src/weights.py:197-198)."""
+    """(x zero-padded to D columns, B, x_sample_stride) for a Stacked call (src/weights.py:197-198); fp32 or bf16, as x."""
     n_in = x.size(-1)
     if n_in < D:
-        xp = torch.empty(x.shape[:-1] + (D,), dtype=torch.float32, device=x.device)
-        with _Timed("whvi_pad_rows_f32"):
-            _lib.check(_lib.lib().whvi_pad_rows_f32(x.data_ptr(), xp.data_ptr(), x.numel() // n_in, n_in, D, _stream(x.device)),
-                       "whvi_pad_rows_f32")
+        name = "whvi_pad_rows_bf16" if x.dtype == torch.bfloat16 else "whvi_pad_rows_f32"
+        xp = torch.empty(x.shape[:-1] + (D,), dtype=x.dtype, device=x.device)
+        with _Timed(name):
+            _lib.check(getattr(_lib.lib(), name)(x.data_ptr(), xp.data_ptr(), x.numel() // n_in, n_in, D, _stream(x.device)), name)
     else:
         xp = x
     if xp.dim() == 2:
@@ -877,6 +886,16 @@ def _stacked_vectors(groups, D):
     return [g_[0].detach() for g_ in groups], strides[0]
 
 
+def _stacked_bwd_rows(xp, xs, dy, B, D):
+    """bf16 at D = 4 with an odd B: the backward's bulk copies move whole 16-byte units per sample, so the call gets one zero row
+    of the padded x and of dy (as ``layer_backward_bf16``), which adds zero to every gradient; the caller drops dx's extra row.
+    Returns (xp, xs, dy, B) for the call."""
+    if xp.dtype != torch.bfloat16 or (B * D) % 8 == 0:
+        return xp, xs, dy, B
+    xp = F.pad(xp, (0, 0, 0, 1))
+    return xp, (0 if xs == 0 else (B + 1) * D), F.pad(dy, (0, 0, 0, 1)), B + 1
+
+
 def _stacked_bias(bias, G, D):
     if bias is None:
         return None
@@ -890,14 +909,18 @@ class WHVIStackedFunction(Function):
     """WHVIStackedMatrix.forward (src/weights.py:182-208) for all G blocks in one C-ABI call per direction
     (``whvi_stacked_fwd_f32`` / ``whvi_stacked_bwd_f32``): pad, reparameterisation, G x S virtual samples through the fused layer
     kernel, bias, optional ReLU, concatenation, slice.  ``params`` = G x s1, G x s2, G x g_mu, G x g_rho (the blocks' own
-    parameters, so autograd routes the gradients); ``eps`` (G, S, D)."""
+    parameters, so autograd routes the gradients); ``eps`` (G, S, D).
+
+    A bfloat16 ``x`` runs the bf16 twins (``whvi_stacked_fwd_bf16`` / ``whvi_stacked_bwd_bf16``): y and dx are bf16, the fp32
+    calls on the widened inputs rounded once; the parameter gradients are fp32 and bit-identical to the fp32 calls'."""
 
     @staticmethod
     def forward(ctx, x, eps, bias, n_out, relu_out, relu_in, *params):
         G = len(params) // 4
         eps = _f32c(eps, "eps")
         _, S, D = eps.shape
-        x = _f32c(x, "x")
+        x = _act(x, "x")
+        name = "whvi_stacked_fwd_bf16" if x.dtype == torch.bfloat16 else "whvi_stacked_fwd_f32"
         n_in = x.size(-1)
         lib = _lib.lib()
         dev = x.device
@@ -907,13 +930,13 @@ class WHVIStackedFunction(Function):
             (s1p, s2p, mup, rhop), stride = _stacked_vectors([params[i * G:(i + 1) * G] for i in range(4)], D)
             bias = _stacked_bias(bias, G, D)
             g = torch.empty((G, S, D), dtype=torch.float32, device=dev)
-            yb = torch.empty((G, S, B, D), dtype=torch.float32, device=dev)
-            y = torch.empty((S, B, n_out), dtype=torch.float32, device=dev)
-            with _Timed("whvi_stacked_fwd_f32"):
-                rc = lib.whvi_stacked_fwd_f32(xp.data_ptr(), xs, mup.data_ptr(), rhop.data_ptr(), s1p.data_ptr(), s2p.data_ptr(), stride,
-                                              eps.data_ptr(), _ptr(bias), g.data_ptr(), yb.data_ptr(), y.data_ptr(), S, B, D, G, n_out,
-                                              1 if relu_out else 0, st)
-            _lib.check(rc, "whvi_stacked_fwd_f32")
+            yb = torch.empty((G, S, B, D), dtype=x.dtype, device=dev)
+            y = torch.empty((S, B, n_out), dtype=x.dtype, device=dev)
+            with _Timed(name):
+                rc = getattr(lib, name)(xp.data_ptr(), xs, mup.data_ptr(), rhop.data_ptr(), s1p.data_ptr(), s2p.data_ptr(), stride,
+                                        eps.data_ptr(), _ptr(bias), g.data_ptr(), yb.data_ptr(), y.data_ptr(), S, B, D, G, n_out,
+                                        1 if relu_out else 0, st)
+            _lib.check(rc, name)
         ctx.save_for_backward(xp, eps, g, s1p, s2p, rhop)
         ctx.meta = (S, B, D, G, xs, n_in, n_out, stride, bool(relu_in), bias is not None, x.dim())
         return y
@@ -922,20 +945,25 @@ class WHVIStackedFunction(Function):
     def backward(ctx, dy):
         xp, eps, g, s1p, s2p, rhop = ctx.saved_tensors
         S, B, D, G, xs, n_in, n_out, stride, relu_in, has_bias, xdim = ctx.meta
-        dy = _f32c(dy, "dy")
+        bf16 = xp.dtype == torch.bfloat16
+        dy = _bf16c(dy, "dy") if bf16 else _f32c(dy, "dy")
+        name = "whvi_stacked_bwd_bf16" if bf16 else "whvi_stacked_bwd_f32"
         dev = dy.device
         lib = _lib.lib()
         want_dx = ctx.needs_input_grad[0]
+        xp, xs, dy, Bc = _stacked_bwd_rows(xp, xs, dy, B, D)
         with torch.cuda.device(dev):
-            ws = _workspace(dev, _query("whvi_stacked_bwd_workspace_bytes", S, B, D, G, 1 if want_dx else 0)[0])
+            ws = _workspace(dev, _query("whvi_stacked_bwd_workspace_bytes", S, Bc, D, G, 1 if want_dx else 0)[0])
             out = torch.empty((5 if has_bias else 4, G, D), dtype=torch.float32, device=dev)   # dmu, drho, ds1, ds2, [dbias]
-            dx = torch.empty((S, B, n_in), dtype=torch.float32, device=dev) if want_dx else None
-            with _Timed("whvi_stacked_bwd_f32"):
-                rc = lib.whvi_stacked_bwd_f32(xp.data_ptr(), xs, dy.data_ptr(), g.data_ptr(), rhop.data_ptr(), s1p.data_ptr(), s2p.data_ptr(),
-                                              stride, eps.data_ptr(), _ptr(dx), n_in, out[0].data_ptr(), out[1].data_ptr(),
-                                              out[2].data_ptr(), out[3].data_ptr(), out[4].data_ptr() if has_bias else None,
-                                              ws.data_ptr(), ws.numel(), S, B, D, G, n_out, 1 if relu_in else 0, _stream(dev))
-            _lib.check(rc, "whvi_stacked_bwd_f32")
+            dx = torch.empty((S, Bc, n_in), dtype=xp.dtype, device=dev) if want_dx else None
+            with _Timed(name):
+                rc = getattr(lib, name)(xp.data_ptr(), xs, dy.data_ptr(), g.data_ptr(), rhop.data_ptr(), s1p.data_ptr(), s2p.data_ptr(),
+                                        stride, eps.data_ptr(), _ptr(dx), n_in, out[0].data_ptr(), out[1].data_ptr(),
+                                        out[2].data_ptr(), out[3].data_ptr(), out[4].data_ptr() if has_bias else None,
+                                        ws.data_ptr(), ws.numel(), S, Bc, D, G, n_out, 1 if relu_in else 0, _stream(dev))
+            _lib.check(rc, name)
+        if want_dx and Bc != B:
+            dx = dx[:, :B]
         if want_dx and xdim == 2:
             dx = dx.sum(dim=0)
         dbias = out[4].reshape(1, G * D) if has_bias and ctx.needs_input_grad[2] else None
@@ -949,26 +977,28 @@ def whvi_stacked(x, eps, bias, n_out, blocks_s1, blocks_s2, blocks_mu, blocks_rh
 
 class WHVIStackedGFunction(Function):
     """The Stacked layer from g (G, S, D) given, however it was drawn (``whvi_stacked_fwd_g_f32`` / ``whvi_stacked_bwd_g_f32``):
-    the dense posterior's path, g from ``reparam_dense_grouped``.  ``params`` = G x s1, G x s2; the backward returns dg."""
+    the dense posterior's path, g from ``reparam_dense_grouped``.  ``params`` = G x s1, G x s2; the backward returns dg.  A bfloat16
+    ``x`` runs the bf16 twins, as ``WHVIStackedFunction``."""
 
     @staticmethod
     def forward(ctx, x, g, bias, n_out, relu_out, relu_in, *params):
         G = len(params) // 2
         g = _f32c(g, "g")
         _, S, D = g.shape
-        x = _f32c(x, "x")
+        x = _act(x, "x")
+        name = "whvi_stacked_fwd_g_bf16" if x.dtype == torch.bfloat16 else "whvi_stacked_fwd_g_f32"
         n_in = x.size(-1)
         dev = x.device
         with torch.cuda.device(dev):
             xp, B, xs = _stacked_input(x, S, D)
             (s1p, s2p), stride = _stacked_vectors([params[:G], params[G:]], D)
             bias = _stacked_bias(bias, G, D)
-            yb = torch.empty((G, S, B, D), dtype=torch.float32, device=dev)
-            y = torch.empty((S, B, n_out), dtype=torch.float32, device=dev)
-            with _Timed("whvi_stacked_fwd_g_f32"):
-                rc = _lib.lib().whvi_stacked_fwd_g_f32(xp.data_ptr(), xs, g.data_ptr(), s1p.data_ptr(), s2p.data_ptr(), stride, _ptr(bias),
-                                                       yb.data_ptr(), y.data_ptr(), S, B, D, G, n_out, 1 if relu_out else 0, _stream(dev))
-            _lib.check(rc, "whvi_stacked_fwd_g_f32")
+            yb = torch.empty((G, S, B, D), dtype=x.dtype, device=dev)
+            y = torch.empty((S, B, n_out), dtype=x.dtype, device=dev)
+            with _Timed(name):
+                rc = getattr(_lib.lib(), name)(xp.data_ptr(), xs, g.data_ptr(), s1p.data_ptr(), s2p.data_ptr(), stride, _ptr(bias),
+                                               yb.data_ptr(), y.data_ptr(), S, B, D, G, n_out, 1 if relu_out else 0, _stream(dev))
+            _lib.check(rc, name)
         ctx.save_for_backward(xp, g, s1p, s2p)
         ctx.meta = (S, B, D, G, xs, n_in, n_out, stride, bool(relu_in), bias is not None, x.dim())
         return y
@@ -977,20 +1007,25 @@ class WHVIStackedGFunction(Function):
     def backward(ctx, dy):
         xp, g, s1p, s2p = ctx.saved_tensors
         S, B, D, G, xs, n_in, n_out, stride, relu_in, has_bias, xdim = ctx.meta
-        dy = _f32c(dy, "dy")
+        bf16 = xp.dtype == torch.bfloat16
+        dy = _bf16c(dy, "dy") if bf16 else _f32c(dy, "dy")
+        name = "whvi_stacked_bwd_g_bf16" if bf16 else "whvi_stacked_bwd_g_f32"
         dev = dy.device
         want_dx = ctx.needs_input_grad[0]
+        xp, xs, dy, Bc = _stacked_bwd_rows(xp, xs, dy, B, D)
         with torch.cuda.device(dev):
-            ws = _workspace(dev, _query("whvi_stacked_bwd_workspace_bytes", S, B, D, G, 1 if want_dx else 0)[0])
+            ws = _workspace(dev, _query("whvi_stacked_bwd_workspace_bytes", S, Bc, D, G, 1 if want_dx else 0)[0])
             dg = torch.empty((G, S, D), dtype=torch.float32, device=dev)
             out = torch.empty((3 if has_bias else 2, G, D), dtype=torch.float32, device=dev)   # ds1, ds2, [dbias]
-            dx = torch.empty((S, B, n_in), dtype=torch.float32, device=dev) if want_dx else None
-            with _Timed("whvi_stacked_bwd_g_f32"):
-                rc = _lib.lib().whvi_stacked_bwd_g_f32(xp.data_ptr(), xs, dy.data_ptr(), g.data_ptr(), s1p.data_ptr(), s2p.data_ptr(), stride,
-                                                       _ptr(dx), n_in, dg.data_ptr(), out[0].data_ptr(), out[1].data_ptr(),
-                                                       out[2].data_ptr() if has_bias else None, ws.data_ptr(), ws.numel(), S, B, D, G, n_out,
-                                                       1 if relu_in else 0, _stream(dev))
-            _lib.check(rc, "whvi_stacked_bwd_g_f32")
+            dx = torch.empty((S, Bc, n_in), dtype=xp.dtype, device=dev) if want_dx else None
+            with _Timed(name):
+                rc = getattr(_lib.lib(), name)(xp.data_ptr(), xs, dy.data_ptr(), g.data_ptr(), s1p.data_ptr(), s2p.data_ptr(), stride,
+                                               _ptr(dx), n_in, dg.data_ptr(), out[0].data_ptr(), out[1].data_ptr(),
+                                               out[2].data_ptr() if has_bias else None, ws.data_ptr(), ws.numel(), S, Bc, D, G, n_out,
+                                               1 if relu_in else 0, _stream(dev))
+            _lib.check(rc, name)
+        if want_dx and Bc != B:
+            dx = dx[:, :B]
         if want_dx and xdim == 2:
             dx = dx.sum(dim=0)
         dbias = out[2].reshape(1, G * D) if has_bias and ctx.needs_input_grad[2] else None
@@ -1004,11 +1039,14 @@ def whvi_stacked_g(x, g, bias, n_out, blocks_s1, blocks_s2, relu_out=False, relu
 class WHVIColumnFunction(Function):
     """WHVIColumnMatrix.forward (src/weights.py:231-251, PAPER semantics) in one C-ABI call per direction
     (``whvi_column_fwd_f32`` / ``whvi_column_bwd_f32``): reparameterisation, ONE FWHT of g per MC sample, the 1-wide product,
-    the bias.  ``x``: (B, n) / (S, B, n) when ``transposed`` (-> (S, B, 1)), (B, 1) / (S, B, 1) otherwise (-> (S, B, n))."""
+    the bias.  ``x``: (B, n) / (S, B, n) when ``transposed`` (-> (S, B, 1)), (B, 1) / (S, B, 1) otherwise (-> (S, B, n)).
+
+    A bfloat16 ``x`` runs the bf16 twins: x and dx are bf16, and so are y and dy of the plain form; the transposed form's output
+    (S, B, 1) stays fp32 (``include/whvi_b200.h``).  The parameter gradients are fp32, bit-identical to the fp32 calls'."""
 
     @staticmethod
     def forward(ctx, x, eps, mu, rho, s1, s2, bias, n, transposed, relu_out, relu_in):
-        x, eps = _f32c(x, "x"), _f32c(eps, "eps")
+        x, eps = _act(x, "x"), _f32c(eps, "eps")
         mu, rho, s1, s2 = _f32c(mu, "g_mu"), _f32c(rho, "g_rho"), _f32c(s1, "s1"), _f32c(s2, "s2")
         S, D = eps.shape
         width = n if transposed else 1
@@ -1025,12 +1063,13 @@ class WHVIColumnFunction(Function):
         dev = x.device
         g = torch.empty((S, D), dtype=torch.float32, device=dev)
         hg = torch.empty((S, D), dtype=torch.float32, device=dev)    # H g, kept for the backward
-        y = torch.empty((S, B, 1 if transposed else n), dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev), _Timed("whvi_column_fwd_f32"):
-            rc = _lib.lib().whvi_column_fwd_f32(x.data_ptr(), xs, mu.data_ptr(), rho.data_ptr(), s1.data_ptr(), s2.data_ptr(), eps.data_ptr(),
-                                                _ptr(bias), g.data_ptr(), hg.data_ptr(), y.data_ptr(), S, B, D, n, 1 if transposed else 0,
-                                                1 if relu_out else 0, _stream(dev))
-        _lib.check(rc, "whvi_column_fwd_f32")
+        y = torch.empty((S, B, 1 if transposed else n), dtype=torch.float32 if transposed else x.dtype, device=dev)
+        name = "whvi_column_fwd_bf16" if x.dtype == torch.bfloat16 else "whvi_column_fwd_f32"
+        with torch.cuda.device(dev), _Timed(name):
+            rc = getattr(_lib.lib(), name)(x.data_ptr(), xs, mu.data_ptr(), rho.data_ptr(), s1.data_ptr(), s2.data_ptr(), eps.data_ptr(),
+                                           _ptr(bias), g.data_ptr(), hg.data_ptr(), y.data_ptr(), S, B, D, n, 1 if transposed else 0,
+                                           1 if relu_out else 0, _stream(dev))
+        _lib.check(rc, name)
         ctx.save_for_backward(x, eps, hg, rho, s1, s2)
         ctx.meta = (S, B, D, n, xs, bool(transposed), bool(relu_in), bias is not None)
         return y
@@ -1039,7 +1078,9 @@ class WHVIColumnFunction(Function):
     def backward(ctx, dy):
         x, eps, hg, rho, s1, s2 = ctx.saved_tensors
         S, B, D, n, xs, transposed, relu_in, has_bias = ctx.meta
-        dy = _f32c(dy, "dy")
+        bf16 = x.dtype == torch.bfloat16
+        dy = _bf16c(dy, "dy") if bf16 and not transposed else _f32c(dy, "dy")
+        name = "whvi_column_bwd_bf16" if bf16 else "whvi_column_bwd_f32"
         dev = dy.device
         lib = _lib.lib()
         want_dx = ctx.needs_input_grad[0]
@@ -1047,13 +1088,13 @@ class WHVIColumnFunction(Function):
             ws = _workspace(dev, _query("whvi_column_bwd_workspace_bytes", S, D, n)[0])
             out = torch.empty((4, D), dtype=torch.float32, device=dev)   # dmu, drho, ds1, ds2
             dbias = torch.empty((1, 1 if transposed else n), dtype=torch.float32, device=dev) if has_bias else None
-            dx = torch.empty((S, B, n if transposed else 1), dtype=torch.float32, device=dev) if want_dx else None
-            with _Timed("whvi_column_bwd_f32"):
-                rc = lib.whvi_column_bwd_f32(x.data_ptr(), xs, dy.data_ptr(), hg.data_ptr(), rho.data_ptr(), s1.data_ptr(), s2.data_ptr(),
-                                             eps.data_ptr(), _ptr(dx), out[0].data_ptr(), out[1].data_ptr(), out[2].data_ptr(),
-                                             out[3].data_ptr(), _ptr(dbias), ws.data_ptr(), ws.numel(), S, B, D, n, 1 if transposed else 0,
-                                             1 if relu_in else 0, _stream(dev))
-            _lib.check(rc, "whvi_column_bwd_f32")
+            dx = torch.empty((S, B, n if transposed else 1), dtype=x.dtype, device=dev) if want_dx else None
+            with _Timed(name):
+                rc = getattr(lib, name)(x.data_ptr(), xs, dy.data_ptr(), hg.data_ptr(), rho.data_ptr(), s1.data_ptr(), s2.data_ptr(),
+                                        eps.data_ptr(), _ptr(dx), out[0].data_ptr(), out[1].data_ptr(), out[2].data_ptr(),
+                                        out[3].data_ptr(), _ptr(dbias), ws.data_ptr(), ws.numel(), S, B, D, n, 1 if transposed else 0,
+                                        1 if relu_in else 0, _stream(dev))
+            _lib.check(rc, name)
         if want_dx and xs == 0:
             dx = dx.sum(dim=0)
         return dx, None, out[0], out[1], out[2], out[3], dbias, None, None, None, None
@@ -1065,11 +1106,12 @@ def whvi_column(x, eps, mu, rho, s1, s2, bias, n, transposed, relu_out=False, re
 
 class WHVIColumnGFunction(Function):
     """The Column layer from g (S, D) given, however it was drawn (``whvi_column_fwd_g_f32`` / ``whvi_column_bwd_g_f32``): the
-    dense posterior's path, g from ``reparam_dense``.  The backward returns dg."""
+    dense posterior's path, g from ``reparam_dense``.  The backward returns dg.  A bfloat16 ``x`` runs the bf16 twins, as
+    ``WHVIColumnFunction``."""
 
     @staticmethod
     def forward(ctx, x, g, s1, s2, bias, n, transposed, relu_out, relu_in):
-        x, g, s1, s2 = _f32c(x, "x"), _f32c(g, "g"), _f32c(s1, "s1"), _f32c(s2, "s2")
+        x, g, s1, s2 = _act(x, "x"), _f32c(g, "g"), _f32c(s1, "s1"), _f32c(s2, "s2")
         S, D = g.shape
         width = n if transposed else 1
         if x.size(-1) != width:
@@ -1084,11 +1126,12 @@ class WHVIColumnGFunction(Function):
             bias = _f32c(bias, "bias").reshape(-1)
         dev = x.device
         hg = torch.empty((S, D), dtype=torch.float32, device=dev)
-        y = torch.empty((S, B, 1 if transposed else n), dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev), _Timed("whvi_column_fwd_g_f32"):
-            rc = _lib.lib().whvi_column_fwd_g_f32(x.data_ptr(), xs, g.data_ptr(), s1.data_ptr(), s2.data_ptr(), _ptr(bias), hg.data_ptr(),
-                                                  y.data_ptr(), S, B, D, n, 1 if transposed else 0, 1 if relu_out else 0, _stream(dev))
-        _lib.check(rc, "whvi_column_fwd_g_f32")
+        y = torch.empty((S, B, 1 if transposed else n), dtype=torch.float32 if transposed else x.dtype, device=dev)
+        name = "whvi_column_fwd_g_bf16" if x.dtype == torch.bfloat16 else "whvi_column_fwd_g_f32"
+        with torch.cuda.device(dev), _Timed(name):
+            rc = getattr(_lib.lib(), name)(x.data_ptr(), xs, g.data_ptr(), s1.data_ptr(), s2.data_ptr(), _ptr(bias), hg.data_ptr(),
+                                           y.data_ptr(), S, B, D, n, 1 if transposed else 0, 1 if relu_out else 0, _stream(dev))
+        _lib.check(rc, name)
         ctx.save_for_backward(x, hg, s1, s2)
         ctx.meta = (S, B, D, n, xs, bool(transposed), bool(relu_in), bias is not None)
         return y
@@ -1097,7 +1140,9 @@ class WHVIColumnGFunction(Function):
     def backward(ctx, dy):
         x, hg, s1, s2 = ctx.saved_tensors
         S, B, D, n, xs, transposed, relu_in, has_bias = ctx.meta
-        dy = _f32c(dy, "dy")
+        bf16 = x.dtype == torch.bfloat16
+        dy = _bf16c(dy, "dy") if bf16 and not transposed else _f32c(dy, "dy")
+        name = "whvi_column_bwd_g_bf16" if bf16 else "whvi_column_bwd_g_f32"
         dev = dy.device
         want_dx = ctx.needs_input_grad[0]
         with torch.cuda.device(dev):
@@ -1105,12 +1150,12 @@ class WHVIColumnGFunction(Function):
             dg = torch.empty((S, D), dtype=torch.float32, device=dev)
             out = torch.empty((2, D), dtype=torch.float32, device=dev)   # ds1, ds2
             dbias = torch.empty((1, 1 if transposed else n), dtype=torch.float32, device=dev) if has_bias else None
-            dx = torch.empty((S, B, n if transposed else 1), dtype=torch.float32, device=dev) if want_dx else None
-            with _Timed("whvi_column_bwd_g_f32"):
-                rc = _lib.lib().whvi_column_bwd_g_f32(x.data_ptr(), xs, dy.data_ptr(), hg.data_ptr(), s1.data_ptr(), s2.data_ptr(), _ptr(dx),
-                                                      dg.data_ptr(), out[0].data_ptr(), out[1].data_ptr(), _ptr(dbias), ws.data_ptr(),
-                                                      ws.numel(), S, B, D, n, 1 if transposed else 0, 1 if relu_in else 0, _stream(dev))
-            _lib.check(rc, "whvi_column_bwd_g_f32")
+            dx = torch.empty((S, B, n if transposed else 1), dtype=x.dtype, device=dev) if want_dx else None
+            with _Timed(name):
+                rc = getattr(_lib.lib(), name)(x.data_ptr(), xs, dy.data_ptr(), hg.data_ptr(), s1.data_ptr(), s2.data_ptr(), _ptr(dx),
+                                               dg.data_ptr(), out[0].data_ptr(), out[1].data_ptr(), _ptr(dbias), ws.data_ptr(),
+                                               ws.numel(), S, B, D, n, 1 if transposed else 0, 1 if relu_in else 0, _stream(dev))
+            _lib.check(rc, name)
         if want_dx and xs == 0:
             dx = dx.sum(dim=0)
         return dx, dg, out[0], out[1], dbias, None, None, None, None

@@ -351,9 +351,14 @@ class WHVIStackedMatrix(nn.Module):
 
     def forward(self, x, use_lrt=True, *, relu_out=False, relu_in=False):
         """x: (..., n_in) -> (..., n_out): zero-pad to D_in, apply every block, concatenate,
-        add the bias, drop the padding outputs (src/weights.py:182-208)."""
+        add the bias, drop the padding outputs (src/weights.py:182-208).  A bfloat16 ``x`` gives a bfloat16 result (bf16
+        activations, fp32 parameters and arithmetic) on the grouped path."""
         if x.dtype == torch.bfloat16:
-            raise RuntimeError("WHVIStackedMatrix: bf16 activations are not supported (square layers only)")
+            if x.device.type != "cuda":
+                raise RuntimeError("WHVIStackedMatrix: bf16 activations run on CUDA only; move the module and its inputs to a GPU")
+            if not self.grouped:
+                raise RuntimeError('WHVIStackedMatrix: bf16 activations need the grouped path (semantics="paper", '
+                                   f"4 <= D_in <= {WF.FUSED_BWD_MAX_D}, one_launch)")
         if self.grouped:
             if x.device.type != "cuda":
                 raise RuntimeError("whvi_b200 runs on CUDA only (no CPU fallback); move the module and its inputs to a GPU")
@@ -424,8 +429,13 @@ class WHVIColumnMatrix(nn.Module):
         return self.one_launch and sub.semantics == "paper"
 
     def forward(self, x, *, relu_out=False, relu_in=False):
+        """A bfloat16 ``x`` runs the fused path with bf16 activations: the plain form (1 -> n) returns bfloat16, the transposed
+        form (n -> 1) float32 -- its (S, B, 1) output holds the network's predictions, which are not rounded to bf16."""
         if x.dtype == torch.bfloat16:
-            raise RuntimeError("WHVIColumnMatrix: bf16 activations are not supported (square layers only)")
+            if x.device.type != "cuda":
+                raise RuntimeError("WHVIColumnMatrix: bf16 activations run on CUDA only; move the module and its inputs to a GPU")
+            if not self.fused:
+                raise RuntimeError('WHVIColumnMatrix: bf16 activations need the fused path (semantics="paper", one_launch)')
         sub = self.weight_submodule
         S, squeeze = sub._resolve_samples(x)
         if self.fused:
