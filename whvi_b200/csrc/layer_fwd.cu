@@ -109,7 +109,16 @@ __global__ void __launch_bounds__((1 << (N - C)) * GROUPS, MINB) layer_fwd_kerne
             const int64_t e1 = e0 + GROUPS * TILE;
             if (e1 < a.sample_elems) {
                 const int64_t left1 = a.sample_elems - e1;
-                l2_prefetch_bulk(xs + GROUPS * TILE, static_cast<uint32_t>((left1 < TILE ? left1 : TILE) * sizeof(IO)));
+                const uint32_t bytes = static_cast<uint32_t>((left1 < TILE ? left1 : TILE) * sizeof(IO));
+                if constexpr (sizeof(IO) < sizeof(float)) {
+                    // a bulk prefetch takes a 16-byte-aligned address and whole 16-byte units; a bf16 sample of B * D % 8 != 0
+                    // elements (D = 4 with an odd B) starts 8 bytes off and ends on half a unit: prefetch the whole units
+                    // of aligned tiles only
+                    const bool aligned = (reinterpret_cast<uintptr_t>(xs + GROUPS * TILE) & 15u) == 0;
+                    if (aligned && bytes >= 16) l2_prefetch_bulk(xs + GROUPS * TILE, bytes & ~15u);
+                } else {
+                    l2_prefetch_bulk(xs + GROUPS * TILE, bytes);
+                }
             }
         }
 
