@@ -432,6 +432,39 @@ WHVI_API int whvi_mc_moments_strided_f32(const float* y, int64_t y_sample_stride
                                          int64_t n, whvi_stream_t stream);
 
 /*
+ * Categorical (softmax) likelihood of a classifier (not in the reference, whose networks only regress).  logits: (S, B, K)
+ * sample-major rows r = s * B + b, fp32 or bf16 (the _bf16 calls: the fp32 calls on the widened logits, same plan and order, so
+ * bit-identical; a bf16 dz is the fp32 dz rounded once).  labels: (B) int64, shared by the samples.  2 <= K <= 65536, any K.
+ *   whvi_categorical_sizes       bytes of workspace whvi_categorical_nll_* needs for R = S * B rows of K classes
+ *   whvi_categorical_nll_*       lse[r] = log sum_k exp(z[r, k]) (max-subtracted; lse may be NULL) and
+ *                                total[0] = sum_r (lse[r] - z[r, y_b]): fp64 per-CTA partials in the workspace, summed in a fixed
+ *                                order.  The caller applies the estimator's coefficient n / (m S).
+ *   whvi_categorical_nll_bwd_*   dz[r, k] = c[0] (exp(z[r, k] - lse[r]) - [k = y_b]), c a device scalar (NULL = 1), lse the forward's
+ *   whvi_categorical_predictive_*  prob_sum[b, k] (+)= sum_s softmax(z[s, b])[k] and, with labels, loglik_sum[b] (+)=
+ *                                sum_s log softmax(z[s, b])[y_b]; (B, K) and (B) fp32, s ascending.  Sample s's rows are read at
+ *                                logits + s * sample_stride (>= B * K, so a sample chunk may be a slice of a larger tensor);
+ *                                flags & WHVI_CATEGORICAL_ACCUMULATE adds to the existing sums in the order one call over all
+ *                                samples would (chunks give that call's bits).  labels and loglik_sum both or neither.
+ * A label outside [0, K) is never used as an index: that row's loss (so the total), its log p and its dz row are NaN.
+ * Every reduction has a fixed order: repeated calls are bit-identical.  Alignment: the element size of each pointer's type
+ * (rows need no more: the loads are element-wise); workspace 8 bytes.
+ */
+#define WHVI_CATEGORICAL_ACCUMULATE 1
+WHVI_API int whvi_categorical_sizes(int64_t R, int64_t K, size_t* workspace_bytes);
+WHVI_API int whvi_categorical_nll_f32(const float* logits, const int64_t* labels, float* lse, float* total, void* workspace,
+                                      size_t workspace_bytes, int64_t S, int64_t B, int64_t K, whvi_stream_t stream);
+WHVI_API int whvi_categorical_nll_bf16(const void* logits, const int64_t* labels, float* lse, float* total, void* workspace,
+                                       size_t workspace_bytes, int64_t S, int64_t B, int64_t K, whvi_stream_t stream);
+WHVI_API int whvi_categorical_nll_bwd_f32(const float* logits, const int64_t* labels, const float* lse, const float* c, float* dz,
+                                          int64_t S, int64_t B, int64_t K, whvi_stream_t stream);
+WHVI_API int whvi_categorical_nll_bwd_bf16(const void* logits, const int64_t* labels, const float* lse, const float* c, void* dz,
+                                           int64_t S, int64_t B, int64_t K, whvi_stream_t stream);
+WHVI_API int whvi_categorical_predictive_f32(const float* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum,
+                                             float* loglik_sum, int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream);
+WHVI_API int whvi_categorical_predictive_bf16(const void* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum,
+                                              float* loglik_sum, int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream);
+
+/*
  * One Adam step over a flat fp32 parameter buffer (the optimizer.step() of the reference's training loop,
  * src/networks.py:80-82, :92-94, which the reference runs as torch.optim.Adam: src/evaluation.py:15-27), in
  * torch.optim.Adam's arithmetic (weight_decay = 0, amsgrad = False):

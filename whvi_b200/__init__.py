@@ -2,11 +2,11 @@
 reference's Python surface.  See DESIGN.md for the path, INTEGRATION.md for the C ABI."""
 from .fwht import FWHT, FWHTFunction, fwht_  # noqa: F401
 from .layers import WHVI, WHVILinear  # noqa: F401
-from .likelihoods import GaussianLikelihood, Likelihood  # noqa: F401
-from .networks import WHVINetwork, WHVIRegression  # noqa: F401
+from .likelihoods import CategoricalLikelihood, GaussianLikelihood, Likelihood  # noqa: F401
+from .networks import WHVIClassification, WHVINetwork, WHVIRegression  # noqa: F401
 from .optim import FlatAdam, FlatParams  # noqa: F401
 from .utils import Cosine  # noqa: F401
 from .weights import WHVIColumnMatrix, WHVISquarePow2Matrix, WHVIStackedMatrix  # noqa: F401
 
-__all__ = ["Cosine", "FWHT", "FWHTFunction", "fwht_", "WHVI", "WHVILinear", "GaussianLikelihood", "Likelihood",
-           "WHVINetwork", "WHVIRegression", "FlatAdam", "FlatParams", "WHVIColumnMatrix", "WHVISquarePow2Matrix", "WHVIStackedMatrix"]
+__all__ = ["Cosine", "FWHT", "FWHTFunction", "fwht_", "WHVI", "WHVILinear", "CategoricalLikelihood", "GaussianLikelihood",
+           "Likelihood", "WHVIClassification", "WHVINetwork", "WHVIRegression", "FlatAdam", "FlatParams", "WHVIColumnMatrix", "WHVISquarePow2Matrix", "WHVIStackedMatrix"]

@@ -127,6 +127,16 @@ SIGNATURES = {
                               c_float, c_float, c_float, c_void_p]),
     "whvi_kl_f32": (c_int, [c_void_p, c_void_p, c_float, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_float, c_int,
                             c_void_p]),
+    # categorical likelihood: the _bf16 twins have the fp32 signatures with void* logits / dz
+    "whvi_categorical_sizes": (c_int, [c_int64, c_int64, POINTER(c_size_t)]),
+    "whvi_categorical_nll_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_void_p]),
+    "whvi_categorical_nll_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_void_p]),
+    "whvi_categorical_nll_bwd_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p]),
+    "whvi_categorical_nll_bwd_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p]),
+    "whvi_categorical_predictive_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int,
+                                                c_void_p]),
+    "whvi_categorical_predictive_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int,
+                                                 c_void_p]),
 }
 
 _lib = None

@@ -877,4 +877,101 @@ int whvi_mc_moments_strided_f32(const float* y, int64_t y_sample_stride, const f
     return launch_mc_moments(y, y_sample_stride, in_sum_y, in_sum_y2, out_sum_y, out_sum_y2, S, n, static_cast<cudaStream_t>(stream));
 }
 
+// ---- categorical likelihood (csrc/categorical.cu) -----------------------------------------------------------------------
+static bool aligned(const void* p, uintptr_t bytes) { return (reinterpret_cast<uintptr_t>(p) & (bytes - 1)) == 0; }
+
+static int check_categorical(const char* who, int64_t S, int64_t B, int64_t K)
+{
+    if (S < 0 || B < 0) return fail(WHVI_E_SHAPE, "%s: S=%lld B=%lld", who, (long long)S, (long long)B);
+    if (K < 2 || K > 65536) return fail(WHVI_E_SHAPE, "%s: K = %lld outside [2, 65536]", who, (long long)K);
+    if (B > (int64_t(1) << 46) || (S > 0 && B > (int64_t(1) << 46) / S)) return fail(WHVI_E_SHAPE, "%s: S * B too large", who);
+    return WHVI_OK;
+}
+
+int whvi_categorical_sizes(int64_t R, int64_t K, size_t* workspace_bytes)
+{
+    if (!workspace_bytes) return fail(WHVI_E_NULL, "categorical_sizes: null pointer");
+    if (int rc = check_categorical("categorical_sizes", R, 1, K)) return rc;
+    *workspace_bytes = categorical_workspace_bytes(R, K);
+    return WHVI_OK;
+}
+
+static int categorical_nll(const char* who, const void* logits, size_t elem, const int64_t* labels, float* lse, float* total, void* workspace,
+                           size_t workspace_bytes, int64_t S, int64_t B, int64_t K, whvi_stream_t stream)
+{
+    if (int rc = check_categorical(who, S, B, K)) return rc;
+    if (!total || (S * B > 0 && (!logits || !labels))) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (!aligned(logits, elem) || !aligned(labels, 8) || !aligned(lse, 4) || !aligned(total, 4))
+        return fail(WHVI_E_ALIGN, "%s: logits, labels, lse and total must be aligned to their element size", who);
+    const size_t need = categorical_workspace_bytes(S * B, K);
+    if (!workspace || workspace_bytes < need || !aligned(workspace, 8))
+        return fail(WHVI_E_WORKSPACE, "%s: workspace of %zu bytes (8-byte aligned) needed, %zu given", who, need, workspace_bytes);
+    return launch_categorical_nll(logits, labels, lse, total, workspace, S, B, K, elem == 2, static_cast<cudaStream_t>(stream));
+}
+
+int whvi_categorical_nll_f32(const float* logits, const int64_t* labels, float* lse, float* total, void* workspace, size_t workspace_bytes,
+                             int64_t S, int64_t B, int64_t K, whvi_stream_t stream)
+{
+    return categorical_nll("categorical_nll_f32", logits, 4, labels, lse, total, workspace, workspace_bytes, S, B, K, stream);
+}
+
+int whvi_categorical_nll_bf16(const void* logits, const int64_t* labels, float* lse, float* total, void* workspace, size_t workspace_bytes,
+                              int64_t S, int64_t B, int64_t K, whvi_stream_t stream)
+{
+    return categorical_nll("categorical_nll_bf16", logits, 2, labels, lse, total, workspace, workspace_bytes, S, B, K, stream);
+}
+
+static int categorical_nll_bwd(const char* who, const void* logits, size_t elem, const int64_t* labels, const float* lse, const float* c,
+                               void* dz, int64_t S, int64_t B, int64_t K, whvi_stream_t stream)
+{
+    if (int rc = check_categorical(who, S, B, K)) return rc;
+    if (S * B == 0) return WHVI_OK;
+    if (!logits || !labels || !lse || !dz) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (!aligned(logits, elem) || !aligned(dz, elem) || !aligned(labels, 8) || !aligned(lse, 4) || !aligned(c, 4))
+        return fail(WHVI_E_ALIGN, "%s: logits, dz, labels, lse and c must be aligned to their element size", who);
+    return launch_categorical_nll_bwd(logits, labels, lse, c, dz, S, B, K, elem == 2, static_cast<cudaStream_t>(stream));
+}
+
+int whvi_categorical_nll_bwd_f32(const float* logits, const int64_t* labels, const float* lse, const float* c, float* dz, int64_t S,
+                                 int64_t B, int64_t K, whvi_stream_t stream)
+{
+    return categorical_nll_bwd("categorical_nll_bwd_f32", logits, 4, labels, lse, c, dz, S, B, K, stream);
+}
+
+int whvi_categorical_nll_bwd_bf16(const void* logits, const int64_t* labels, const float* lse, const float* c, void* dz, int64_t S,
+                                  int64_t B, int64_t K, whvi_stream_t stream)
+{
+    return categorical_nll_bwd("categorical_nll_bwd_bf16", logits, 2, labels, lse, c, dz, S, B, K, stream);
+}
+
+static int categorical_predictive(const char* who, const void* logits, size_t elem, int64_t sample_stride, const int64_t* labels,
+                                  float* prob_sum, float* loglik_sum, int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream)
+{
+    if (int rc = check_categorical(who, S, B, K)) return rc;
+    if (flags & ~WHVI_CATEGORICAL_ACCUMULATE) return fail(WHVI_E_MODE, "%s: unknown flags %d", who, flags);
+    if (S > 1 && sample_stride < B * K)
+        return fail(WHVI_E_SHAPE, "%s: sample_stride=%lld below B * K = %lld", who, (long long)sample_stride, (long long)(B * K));
+    if (S > 1 && sample_stride > (int64_t(1) << 62) / S) return fail(WHVI_E_SHAPE, "%s: sample_stride too large", who);
+    if ((labels == nullptr) != (loglik_sum == nullptr)) return fail(WHVI_E_NULL, "%s: labels and loglik_sum must both be given or both NULL", who);
+    if (B == 0) return WHVI_OK;
+    if (!prob_sum || (S > 0 && !logits)) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (!aligned(logits, elem) || !aligned(labels, 8) || !aligned(prob_sum, 4) || !aligned(loglik_sum, 4))
+        return fail(WHVI_E_ALIGN, "%s: logits, labels, prob_sum and loglik_sum must be aligned to their element size", who);
+    return launch_categorical_predictive(logits, sample_stride, labels, prob_sum, loglik_sum, S, B, K, flags & WHVI_CATEGORICAL_ACCUMULATE,
+                                         elem == 2, static_cast<cudaStream_t>(stream));
+}
+
+int whvi_categorical_predictive_f32(const float* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,
+                                    int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream)
+{
+    return categorical_predictive("categorical_predictive_f32", logits, 4, sample_stride, labels, prob_sum, loglik_sum, S, B, K, flags, stream);
+}
+
+int whvi_categorical_predictive_bf16(const void* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,
+                                     int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream)
+{
+    return categorical_predictive("categorical_predictive_bf16", logits, 2, sample_stride, labels, prob_sum, loglik_sum, S, B, K, flags,
+                                  stream);
+}
+
 }  // extern "C"

@@ -141,5 +141,13 @@ int launch_adam(float* p, const float* g, float* m, float* v, int64_t n, float l
                 float b1, float b2, float eps, float grad_scale, cudaStream_t stream);
 int launch_kl(const float* mu, const float* rho, float lambda_, int64_t D, int mode, float* out, float* dmu, float* drho,
               float grad_scale, int accumulate, cudaStream_t stream, int64_t groups = 1, int64_t pstride = 0);
+// categorical likelihood (categorical.cu); bf16 != 0: the logits and dz are bf16 behind the void pointers
+size_t categorical_workspace_bytes(int64_t R, int64_t K);
+int launch_categorical_nll(const void* z, const int64_t* labels, float* lse, float* total, void* ws, int64_t S, int64_t B, int64_t K,
+                           int bf16, cudaStream_t st);
+int launch_categorical_nll_bwd(const void* z, const int64_t* labels, const float* lse, const float* c, void* dz, int64_t S, int64_t B,
+                               int64_t K, int bf16, cudaStream_t st);
+int launch_categorical_predictive(const void* z, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,
+                                  int64_t S, int64_t B, int64_t K, int accumulate, int bf16, cudaStream_t st);
 
 }  // namespace whvi

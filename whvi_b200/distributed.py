@@ -92,3 +92,15 @@ def reduce_predictive_moments(sum_y: torch.Tensor, sum_y2: torch.Tensor, n_local
     mean = sum_y / count
     var = sum_y2 / count - mean * mean
     return mean, var
+
+
+def reduce_predictive_probs(prob_sum: torch.Tensor, loglik_sum: torch.Tensor | None, n_local: int, group=None):
+    """Classification evaluation sharded by MC sample: combine per-rank sum_s softmax(z_s) (B, K) and sum_s log p_s(y) (B,)
+    (``WHVIClassification.predictive_prob_sums``; ``loglik_sum`` may be None) into the MC-mean probabilities and the mean
+    log-likelihood per input over all samples.  The test MNLL with n = m is minus the mean of the latter."""
+    count = torch.tensor([float(n_local)], device=prob_sum.device)
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        for t in (prob_sum, loglik_sum, count):
+            if t is not None:
+                dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+    return prob_sum / count, None if loglik_sum is None else loglik_sum / count

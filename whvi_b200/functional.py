@@ -35,7 +35,10 @@ _LAUNCHES_PER_CALL = {"whvi_fwht_f32": 1, "whvi_fwht_f64": 1, "whvi_layer_fwd_f3
                       # bf16 twins of the Stacked and Column calls: the fp32 calls' launches
                       "whvi_pad_rows_bf16": 1, "whvi_stacked_fwd_bf16": 3, "whvi_stacked_fwd_g_bf16": 2, "whvi_stacked_bwd_bf16": 6,
                       "whvi_stacked_bwd_g_bf16": 5, "whvi_column_fwd_bf16": 3, "whvi_column_fwd_g_bf16": 2, "whvi_column_bwd_bf16": 7,
-                      "whvi_column_bwd_g_bf16": 6}
+                      "whvi_column_bwd_g_bf16": 6,
+                      # categorical likelihood: the forward is the row kernel + the fixed-order sum of its per-CTA partials
+                      "whvi_categorical_nll_f32": 2, "whvi_categorical_nll_bf16": 2, "whvi_categorical_nll_bwd_f32": 1,
+                      "whvi_categorical_nll_bwd_bf16": 1, "whvi_categorical_predictive_f32": 1, "whvi_categorical_predictive_bf16": 1}
 # When set to a dict {"name": [(start_event, stop_event), ...]}, the named calls are bracketed
 # by CUDA events on the launching stream (bench.py's per-kernel roofline timing).
 EVENT_SINK: dict[str, list] | None = None
@@ -1232,3 +1235,93 @@ class KLFunction(Function):
 
 def kl_gaussian(mu, rho, lambda_, mode=0):
     return KLFunction.apply(mu, rho, lambda_, mode)
+
+
+# ---------------------------------------------------------------------------------------------- categorical likelihood
+def _categorical_args(logits, labels):
+    """(logits, labels, S, B, K) for the categorical calls.  Shapes and dtypes are checked before the device, so every misuse
+    gets its own message; nothing here reads the labels (a device sync would break CUDA-graph capture): labels outside
+    [0, K) come back as NaN from the kernels."""
+    if logits.dim() != 3:
+        raise RuntimeError(f"logits must be (S, B, K), got {tuple(logits.shape)}")
+    S, B, K = logits.shape
+    if labels.dim() != 1 or labels.size(0) != B:
+        raise RuntimeError(f"labels must be ({B},) for logits {tuple(logits.shape)}, got {tuple(labels.shape)}")
+    if logits.dtype not in (torch.float32, torch.bfloat16):
+        raise RuntimeError(f"logits must be float32 or bfloat16 (got {logits.dtype})")
+    if labels.dtype != torch.int64:
+        raise RuntimeError(f"labels must be int64 (got {labels.dtype})")
+    if logits.device.type != "cuda" or labels.device != logits.device:
+        raise RuntimeError("logits and labels must be CUDA tensors on one device")
+    return logits.contiguous(), labels.contiguous(), S, B, K
+
+
+class CategoricalNLLFunction(Function):
+    """sum_{s,b} -log softmax(z[s, b])[y_b] for (S, B, K) logits (fp32 or bf16) and (B,) int64 labels, as a 0-d fp32 tensor
+    (``whvi_categorical_nll_*``: max-subtracted log-sum-exp per row, fixed-order fp64 reduction).  The backward is
+    ``whvi_categorical_nll_bwd_*`` with the incoming gradient read from the device (no sync, graph-capturable); dz has the
+    logits' dtype."""
+
+    @staticmethod
+    def forward(ctx, logits, labels):
+        logits, labels, S, B, K = _categorical_args(logits, labels)
+        bf16 = logits.dtype == torch.bfloat16
+        name = "whvi_categorical_nll_bf16" if bf16 else "whvi_categorical_nll_f32"
+        dev = logits.device
+        want_grad = ctx.needs_input_grad[0]
+        lse = torch.empty((S, B), dtype=torch.float32, device=dev) if want_grad else None
+        total = torch.empty(1, dtype=torch.float32, device=dev)
+        with torch.cuda.device(dev):
+            ws = _workspace(dev, _query("whvi_categorical_sizes", S * B, K)[0])
+            with _Timed(name, f"K={K}"):
+                rc = getattr(_lib.lib(), name)(logits.data_ptr(), labels.data_ptr(), _ptr(lse), total.data_ptr(), ws.data_ptr(), ws.numel(),
+                                               S, B, K, _stream(dev))
+        _lib.check(rc, name)
+        if want_grad:
+            ctx.save_for_backward(logits, labels, lse)
+        return total.reshape(())
+
+    @staticmethod
+    def backward(ctx, d_total):
+        logits, labels, lse = ctx.saved_tensors
+        S, B, K = logits.shape
+        c = _f32c(d_total, "grad_output").reshape(1)
+        dz = torch.empty_like(logits)
+        name = "whvi_categorical_nll_bwd_bf16" if logits.dtype == torch.bfloat16 else "whvi_categorical_nll_bwd_f32"
+        with torch.cuda.device(logits.device), _Timed(name, f"K={K}"):
+            rc = getattr(_lib.lib(), name)(logits.data_ptr(), labels.data_ptr(), lse.data_ptr(), c.data_ptr(), dz.data_ptr(), S, B, K,
+                                           _stream(logits.device))
+        _lib.check(rc, name)
+        return dz, None
+
+
+def categorical_nll(logits, labels):
+    return CategoricalNLLFunction.apply(logits, labels)
+
+
+def categorical_predictive_(logits, labels, prob_sum, loglik_sum=None, accumulate=False):
+    """prob_sum (+)= sum_s softmax(logits[s]) (B, K) and, with ``labels``, loglik_sum (+)= sum_s log softmax(logits[s])[labels]
+    (B,), samples ascending (``whvi_categorical_predictive_*``).  ``logits`` (S, B, K) fp32 or bf16 may be a sample-slice of a
+    larger tensor (rows contiguous, any sample stride); ``accumulate`` continues the sums of earlier sample chunks in the order
+    of one call over all samples, so chunked evaluation gives the same bits.  No autograd."""
+    if logits.dim() != 3:
+        raise RuntimeError(f"logits must be (S, B, K), got {tuple(logits.shape)}")
+    S, B, K = logits.shape
+    if labels is not None:
+        labels = _categorical_args(logits[:0], labels)[1]
+    elif logits.dtype not in (torch.float32, torch.bfloat16) or logits.device.type != "cuda":
+        raise RuntimeError("logits must be a float32 or bfloat16 CUDA tensor")
+    if (labels is None) != (loglik_sum is None):
+        raise RuntimeError("labels and loglik_sum go together")
+    if logits.stride(2) != 1 or logits.stride(1) != K:
+        logits = logits.contiguous()
+    stride = logits.stride(0) if S > 1 else B * K
+    for t, name, n in ((prob_sum, "prob_sum", B * K), (loglik_sum, "loglik_sum", B)):
+        if t is not None and (t.dtype != torch.float32 or not t.is_contiguous() or t.numel() != n or t.device != logits.device):
+            raise RuntimeError(f"{name} must be a contiguous float32 tensor with {n} elements on {logits.device}")
+    name = "whvi_categorical_predictive_bf16" if logits.dtype == torch.bfloat16 else "whvi_categorical_predictive_f32"
+    with torch.cuda.device(logits.device), _Timed(name, f"K={K}"):
+        rc = getattr(_lib.lib(), name)(logits.data_ptr(), stride, _ptr(labels), prob_sum.data_ptr(), _ptr(loglik_sum), S, B, K,
+                                       1 if accumulate else 0, _stream(logits.device))
+    _lib.check(rc, name)
+    return prob_sum, loglik_sum

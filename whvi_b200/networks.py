@@ -18,7 +18,7 @@ import torch.nn.functional as F
 
 from . import functional as WF
 from .layers import WHVI, WHVILinear
-from .likelihoods import GaussianLikelihood, Likelihood
+from .likelihoods import CategoricalLikelihood, GaussianLikelihood, Likelihood
 
 try:  # progress bars exactly like the reference when tqdm is around
     from tqdm import tqdm
@@ -183,6 +183,10 @@ class WHVINetwork(nn.Module, WHVI):
             n_samples = self.train_samples if self.training else self.eval_samples
             _, sq = self._run(x, n_samples, sqerr_target=y.contiguous().float())
             self.current_mnll = self.likelihood.mnll_from_sq_error(sq, m=y.size(0), n_out=y.size(1), n_mc=n_samples, n=n)
+        elif isinstance(self.likelihood, CategoricalLikelihood):
+            # the (S, B, K) logits as the last module leaves them: no (B, K, S) permute copy
+            n_samples = self.train_samples if self.training else self.eval_samples
+            self.current_mnll = self.likelihood.mnll_from_logits(y, self._run(x, n_samples), n)
         else:
             self.current_mnll = self.likelihood.mnll_batch_estimate(y, self(x), n)
         self.current_kl = self.kl
@@ -295,3 +299,48 @@ class WHVIRegression(WHVINetwork):
                 mnll = self.likelihood.mnll_from_sq_error(sq.to(torch.float32), m=m, n_out=n_out, n_mc=S, n=m)
                 return float(rmse), float(mnll)
         return super().eval_model(X_test, y_test, loss)
+
+
+class WHVIClassification(WHVINetwork):
+    def __init__(self, modules: Iterable[nn.Module], **kwargs):
+        """WHVI network for classification: the last module's K outputs are the logits of a softmax likelihood
+        (``CategoricalLikelihood``); targets are (batch,) int64 class labels on the GPU."""
+        super().__init__(modules, likelihood=CategoricalLikelihood(), **kwargs)
+
+    @torch.no_grad()
+    def predictive_prob_sums(self, X: torch.Tensor, y: torch.Tensor | None = None, n_samples: int | None = None,
+                        chunk_samples: int | None = None):
+        """(sum_s softmax(z_s) (batch, K) fp32, sum_s log softmax(z_s)[y] (batch,) fp32 or None without ``y``, S) over the MC
+        samples.  The network runs ``chunk_samples`` samples at a time (default 16) and the ``whvi_categorical_predictive``
+        kernel continues the sums chunk after chunk in sample order, so the (S, batch, K) logits never exist at once and the
+        result does not depend on the chunking."""
+        S = int(n_samples if n_samples is not None else (self.train_samples if self.training else self.eval_samples))
+        chunk = max(1, int(chunk_samples if chunk_samples is not None else 16))
+        prob_sum = loglik_sum = None
+        for s0 in range(0, S, chunk):
+            logits = self._run(X, min(chunk, S - s0))
+            if prob_sum is None:
+                prob_sum = torch.empty(logits.shape[1:], dtype=torch.float32, device=logits.device)
+                loglik_sum = None if y is None else torch.empty(logits.shape[1], dtype=torch.float32, device=logits.device)
+            WF.categorical_predictive_(logits, y, prob_sum, loglik_sum, accumulate=s0 > 0)
+        if prob_sum is None:
+            raise RuntimeError("predictive_prob_sums needs n_samples >= 1")
+        return prob_sum, loglik_sum, S
+
+    @torch.no_grad()
+    def predict_proba(self, X: torch.Tensor, n_samples: int | None = None, chunk_samples: int | None = None) -> torch.Tensor:
+        """MC-mean class probabilities (batch, K): 1/S sum_s softmax(z_s), ``chunk_samples`` samples at a time."""
+        prob_sum, _, S = self.predictive_prob_sums(X, None, n_samples, chunk_samples)
+        return prob_sum / S
+
+    def eval_model(self, X_test: torch.Tensor, y_test: torch.Tensor, loss=None) -> Tuple[float, float]:
+        """Error rate of the MC-mean prediction and test MNLL (the training estimator with n = m).  Both come from the
+        chunked predictive sums; a user-supplied ``loss(y_pred, y_true)`` gets the (batch, K, S) logits of ``forward()``
+        instead, as in ``WHVINetwork.eval_model``."""
+        self.eval()
+        if loss is not None:
+            return super().eval_model(X_test, y_test, loss)
+        prob_sum, loglik_sum, S = self.predictive_prob_sums(X_test, y_test)
+        error = (prob_sum.argmax(dim=1) != y_test).to(torch.float64).mean()
+        mnll = -loglik_sum.to(torch.float64).sum() / S   # n / (m S) * sum_{b,s} -log p with n = m
+        return float(error), float(mnll)
