@@ -465,6 +465,39 @@ WHVI_API int whvi_categorical_predictive_bf16(const void* logits, int64_t sample
                                               float* loglik_sum, int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream);
 
 /*
+ * Patch gather and scatter of a convolutional WHVI layer (WHVIConv2d; not in the reference).  Activations are channels-last:
+ * x and dx are (S|1, B, H, W, C), the patch matrix is (S|1, B * Ho * Wo, ld) with its rows in (b, oh, ow) order, i.e. the rows a
+ * layer call takes.  Column order: tap (i, j) and channel c go to column (i * kw + j) * C + c (channels fastest), so a WHVI
+ * weight W (C_out, C * kh * kw) is the torch filter W.reshape(C_out, kh, kw, C).permute(0, 3, 1, 2).
+ *   Ho = (H + 2 pad_h - dil_h (kh - 1) - 1) / stride_h + 1, Wo likewise (floor); Ho <= 0 or Wo <= 0 is WHVI_E_SHAPE.
+ *   whvi_im2col_*   patches[s, (b, oh, ow), (i kw + j) C + c] = x[s, b, oh stride_h - pad_h + i dil_h, ow stride_w - pad_w + j dil_w, c]
+ *                   and 0 for taps outside the image and for the columns n_in ... ld - 1 (n_in = C kh kw <= ld, else
+ *                   WHVI_E_SHAPE): every element of the (S, B Ho Wo, ld) output is written, so ld = D of a Stacked or square
+ *                   layer gives that call's padded input directly.  x_sample_stride: 0 (one (B, H, W, C) image batch for all S
+ *                   samples; patches are still written per sample) or B H W C.  A copy: the bf16 call moves the same bits.
+ *   whvi_col2im_*   the adjoint: dx[s, b, h, w, c] = sum of the dpatches elements that im2col took from x[s, b, h, w, c], taps
+ *                   i ascending then j ascending, fp32 accumulation (a bf16 dx is rounded once).  No atomics: bit-reproducible.
+ *                   flags & WHVI_COL2IM_SUM_SAMPLES: dx is ONE (B, H, W, C) block, the per-sample sums added over s ascending
+ *                   (the gradient of an input shared by the samples; S = 0 writes zeros); otherwise dx is (S, B, H, W, C).
+ * Limits: H, W, C, kernel, stride, dilation in [1, 2^24), padding in [0, 2^24), dil (k - 1) + 1 < 2^24, C kh kw and ld below
+ * 2^31, elements below 2^62 (int64 indexing: rows may exceed 65535 and elements 2^31).  Alignment: the element size of each
+ * pointer's type; 16-byte aligned pointers with C and ld multiples of 4 (fp32) or 8 (bf16) take 16-byte moves.
+ */
+#define WHVI_COL2IM_SUM_SAMPLES 1
+WHVI_API int whvi_im2col_f32(const float* x, int64_t x_sample_stride, float* patches, int64_t S, int64_t B, int64_t H, int64_t W,
+                             int64_t C, int64_t kh, int64_t kw, int64_t stride_h, int64_t stride_w, int64_t pad_h, int64_t pad_w,
+                             int64_t dil_h, int64_t dil_w, int64_t ld, whvi_stream_t stream);
+WHVI_API int whvi_im2col_bf16(const void* x, int64_t x_sample_stride, void* patches, int64_t S, int64_t B, int64_t H, int64_t W,
+                              int64_t C, int64_t kh, int64_t kw, int64_t stride_h, int64_t stride_w, int64_t pad_h, int64_t pad_w,
+                              int64_t dil_h, int64_t dil_w, int64_t ld, whvi_stream_t stream);
+WHVI_API int whvi_col2im_f32(const float* dpatches, int64_t ld, float* dx, int64_t S, int64_t B, int64_t H, int64_t W, int64_t C,
+                             int64_t kh, int64_t kw, int64_t stride_h, int64_t stride_w, int64_t pad_h, int64_t pad_w, int64_t dil_h,
+                             int64_t dil_w, int flags, whvi_stream_t stream);
+WHVI_API int whvi_col2im_bf16(const void* dpatches, int64_t ld, void* dx, int64_t S, int64_t B, int64_t H, int64_t W, int64_t C,
+                              int64_t kh, int64_t kw, int64_t stride_h, int64_t stride_w, int64_t pad_h, int64_t pad_w, int64_t dil_h,
+                              int64_t dil_w, int flags, whvi_stream_t stream);
+
+/*
  * One Adam step over a flat fp32 parameter buffer (the optimizer.step() of the reference's training loop,
  * src/networks.py:80-82, :92-94, which the reference runs as torch.optim.Adam: src/evaluation.py:15-27), in
  * torch.optim.Adam's arithmetic (weight_decay = 0, amsgrad = False):

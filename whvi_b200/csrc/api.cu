@@ -974,4 +974,92 @@ int whvi_categorical_predictive_bf16(const void* logits, int64_t sample_stride, 
                                   stream);
 }
 
+// ---- convolution patches (csrc/conv.cu) ---------------------------------------------------------------------------------
+static int check_conv(const char* who, int64_t S, int64_t B, int64_t H, int64_t W, int64_t C, int64_t kh, int64_t kw, int64_t sh,
+                      int64_t sw, int64_t ph, int64_t pw, int64_t dh, int64_t dw, int64_t ld, ConvGeom* g)
+{
+    constexpr int64_t kLim = int64_t(1) << 24;
+    if (S < 0 || B < 0) return fail(WHVI_E_SHAPE, "%s: S=%lld B=%lld", who, (long long)S, (long long)B);
+    const int64_t pos[] = {H, W, C, kh, kw, sh, sw, dh, dw};
+    for (int64_t v : pos)
+        if (v < 1 || v >= kLim) return fail(WHVI_E_SHAPE, "%s: H, W, C, kernel, stride and dilation must lie in [1, 2^24)", who);
+    if (ph < 0 || pw < 0 || ph >= kLim || pw >= kLim) return fail(WHVI_E_SHAPE, "%s: padding must lie in [0, 2^24)", who);
+    const int64_t ext_h = dh * (kh - 1) + 1, ext_w = dw * (kw - 1) + 1;
+    if (ext_h >= kLim || ext_w >= kLim) return fail(WHVI_E_SHAPE, "%s: dilated kernel extent must be below 2^24", who);
+    const int64_t num_h = H + 2 * ph - ext_h, num_w = W + 2 * pw - ext_w;
+    if (num_h < 0 || num_w < 0)
+        return fail(WHVI_E_SHAPE, "%s: the dilated kernel (%lld x %lld) exceeds the padded image (%lld x %lld): Ho or Wo <= 0", who,
+                    (long long)ext_h, (long long)ext_w, (long long)(H + 2 * ph), (long long)(W + 2 * pw));
+    const int64_t Ho = num_h / sh + 1, Wo = num_w / sw + 1;
+    if (kh * kw > (int64_t(1) << 31) / C || ld > INT32_MAX)
+        return fail(WHVI_E_SHAPE, "%s: C * kh * kw and ld must stay below 2^31", who);
+    const int64_t n_in = C * kh * kw;
+    if (ld < n_in) return fail(WHVI_E_SHAPE, "%s: ld=%lld below n_in = C * kh * kw = %lld", who, (long long)ld, (long long)n_in);
+    // the larger side, S * B * max(Ho * Wo * ld, H * W * C) elements, must stay below 2^62 (Ho * Wo and H * W are below 2^52)
+    constexpr int64_t kMaxElems = int64_t(1) << 62;
+    if (Ho * Wo > kMaxElems / ld || H * W > kMaxElems / C) return fail(WHVI_E_SHAPE, "%s: too many elements", who);
+    const int64_t per = Ho * Wo * ld > H * W * C ? Ho * Wo * ld : H * W * C;
+    if ((B > 0 && S > kMaxElems / B) || (S * B > 0 && S * B > kMaxElems / per)) return fail(WHVI_E_SHAPE, "%s: too many elements", who);
+    *g = ConvGeom{S, B, int(H), int(W), int(C), int(kh), int(kw), int(sh), int(sw), int(ph), int(pw), int(dh), int(dw), int(Ho), int(Wo)};
+    return WHVI_OK;
+}
+
+static int im2col(const char* who, const void* x, int64_t x_sample_stride, void* patches, size_t elem, int64_t S, int64_t B, int64_t H,
+                  int64_t W, int64_t C, int64_t kh, int64_t kw, int64_t sh, int64_t sw, int64_t ph, int64_t pw, int64_t dh, int64_t dw,
+                  int64_t ld, whvi_stream_t stream)
+{
+    ConvGeom g;
+    if (int rc = check_conv(who, S, B, H, W, C, kh, kw, sh, sw, ph, pw, dh, dw, ld, &g)) return rc;
+    if (x_sample_stride != 0 && x_sample_stride != B * H * W * C)
+        return fail(WHVI_E_SHAPE, "%s: x_sample_stride must be 0 or B*H*W*C", who);
+    if (S * B == 0) return WHVI_OK;
+    if (!x || !patches) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (!aligned(x, elem) || !aligned(patches, elem)) return fail(WHVI_E_ALIGN, "%s: x and patches must be aligned to their element size", who);
+    return launch_im2col(x, x_sample_stride, patches, g, ld, elem == 2, static_cast<cudaStream_t>(stream));
+}
+
+int whvi_im2col_f32(const float* x, int64_t x_sample_stride, float* patches, int64_t S, int64_t B, int64_t H, int64_t W, int64_t C,
+                    int64_t kh, int64_t kw, int64_t stride_h, int64_t stride_w, int64_t pad_h, int64_t pad_w, int64_t dil_h,
+                    int64_t dil_w, int64_t ld, whvi_stream_t stream)
+{
+    return im2col("im2col_f32", x, x_sample_stride, patches, 4, S, B, H, W, C, kh, kw, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w,
+                  ld, stream);
+}
+
+int whvi_im2col_bf16(const void* x, int64_t x_sample_stride, void* patches, int64_t S, int64_t B, int64_t H, int64_t W, int64_t C,
+                     int64_t kh, int64_t kw, int64_t stride_h, int64_t stride_w, int64_t pad_h, int64_t pad_w, int64_t dil_h,
+                     int64_t dil_w, int64_t ld, whvi_stream_t stream)
+{
+    return im2col("im2col_bf16", x, x_sample_stride, patches, 2, S, B, H, W, C, kh, kw, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w,
+                  ld, stream);
+}
+
+static int col2im(const char* who, const void* dpatches, int64_t ld, void* dx, size_t elem, int64_t S, int64_t B, int64_t H, int64_t W,
+                  int64_t C, int64_t kh, int64_t kw, int64_t sh, int64_t sw, int64_t ph, int64_t pw, int64_t dh, int64_t dw, int flags,
+                  whvi_stream_t stream)
+{
+    ConvGeom g;
+    if (int rc = check_conv(who, S, B, H, W, C, kh, kw, sh, sw, ph, pw, dh, dw, ld, &g)) return rc;
+    if (flags & ~WHVI_COL2IM_SUM_SAMPLES) return fail(WHVI_E_MODE, "%s: unknown flags %d", who, flags);
+    const int sum = flags & WHVI_COL2IM_SUM_SAMPLES;
+    if ((sum ? 1 : S) * B == 0) return WHVI_OK;
+    if (!dx || (S > 0 && !dpatches)) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (!aligned(dpatches, elem) || !aligned(dx, elem)) return fail(WHVI_E_ALIGN, "%s: dpatches and dx must be aligned to their element size", who);
+    return launch_col2im(dpatches, ld, dx, g, sum, elem == 2, static_cast<cudaStream_t>(stream));
+}
+
+int whvi_col2im_f32(const float* dpatches, int64_t ld, float* dx, int64_t S, int64_t B, int64_t H, int64_t W, int64_t C, int64_t kh,
+                    int64_t kw, int64_t stride_h, int64_t stride_w, int64_t pad_h, int64_t pad_w, int64_t dil_h, int64_t dil_w, int flags,
+                    whvi_stream_t stream)
+{
+    return col2im("col2im_f32", dpatches, ld, dx, 4, S, B, H, W, C, kh, kw, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, flags, stream);
+}
+
+int whvi_col2im_bf16(const void* dpatches, int64_t ld, void* dx, int64_t S, int64_t B, int64_t H, int64_t W, int64_t C, int64_t kh,
+                     int64_t kw, int64_t stride_h, int64_t stride_w, int64_t pad_h, int64_t pad_w, int64_t dil_h, int64_t dil_w, int flags,
+                     whvi_stream_t stream)
+{
+    return col2im("col2im_bf16", dpatches, ld, dx, 2, S, B, H, W, C, kh, kw, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, flags, stream);
+}
+
 }  // extern "C"

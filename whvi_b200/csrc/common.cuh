@@ -149,5 +149,12 @@ int launch_categorical_nll_bwd(const void* z, const int64_t* labels, const float
                                int64_t K, int bf16, cudaStream_t st);
 int launch_categorical_predictive(const void* z, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,
                                   int64_t S, int64_t B, int64_t K, int accumulate, int bf16, cudaStream_t st);
+// patch gather / scatter of WHVIConv2d (conv.cu); validated geometry, every spatial quantity below 2^24
+struct ConvGeom {
+    int64_t S, B;
+    int H, W, C, kh, kw, sh, sw, ph, pw, dh, dw, Ho, Wo;
+};
+int launch_im2col(const void* x, int64_t xs, void* out, const ConvGeom& g, int64_t ld, int bf16, cudaStream_t st);
+int launch_col2im(const void* dp, int64_t ld, void* dx, const ConvGeom& g, int sum_samples, int bf16, cudaStream_t st);
 
 }  // namespace whvi

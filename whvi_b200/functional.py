@@ -38,7 +38,8 @@ _LAUNCHES_PER_CALL = {"whvi_fwht_f32": 1, "whvi_fwht_f64": 1, "whvi_layer_fwd_f3
                       "whvi_column_bwd_g_bf16": 6,
                       # categorical likelihood: the forward is the row kernel + the fixed-order sum of its per-CTA partials
                       "whvi_categorical_nll_f32": 2, "whvi_categorical_nll_bf16": 2, "whvi_categorical_nll_bwd_f32": 1,
-                      "whvi_categorical_nll_bwd_bf16": 1, "whvi_categorical_predictive_f32": 1, "whvi_categorical_predictive_bf16": 1}
+                      "whvi_categorical_nll_bwd_bf16": 1, "whvi_categorical_predictive_f32": 1, "whvi_categorical_predictive_bf16": 1,
+                      "whvi_im2col_f32": 1, "whvi_im2col_bf16": 1, "whvi_col2im_f32": 1, "whvi_col2im_bf16": 1}
 # When set to a dict {"name": [(start_event, stop_event), ...]}, the named calls are bracketed
 # by CUDA events on the launching stream (bench.py's per-kernel roofline timing).
 EVENT_SINK: dict[str, list] | None = None
@@ -1325,3 +1326,75 @@ def categorical_predictive_(logits, labels, prob_sum, loglik_sum=None, accumulat
                                        1 if accumulate else 0, _stream(logits.device))
     _lib.check(rc, name)
     return prob_sum, loglik_sum
+
+
+# ---------------------------------------------------------------------------------------------- convolution patches
+def conv_output_size(n: int, k: int, stride: int, pad: int, dil: int) -> int:
+    """Output length of a convolution along one spatial axis (torch.nn.Conv2d's formula, floor)."""
+    return (n + 2 * pad - dil * (k - 1) - 1) // stride + 1
+
+
+def _image_dims(x):
+    """(S or None, B, H, W, C, x_sample_stride) of a channels-last (B, H, W, C) or (S, B, H, W, C) image batch."""
+    if x.dim() == 4:
+        return (None, *x.shape, 0)
+    if x.dim() == 5:
+        return (x.size(0), *x.shape[1:], x[0].numel())
+    raise RuntimeError(f"images must be (B, H, W, C) or (S, B, H, W, C) channels-last, got {tuple(x.shape)}")
+
+
+def im2col_(x, geom, ld):
+    """Patch matrix of a channels-last image batch (``whvi_im2col_*``): ``x`` (B, H, W, C) -> (B Ho Wo, ld), or (S, B, H, W, C)
+    -> (S, B Ho Wo, ld), fp32 or bf16 as ``x``.  ``geom`` = (kh, kw, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w).  Column
+    (i kw + j) C + c holds tap (i, j) of channel c; columns from C kh kw to ld - 1 are zero.  No autograd."""
+    x = _act(x, "x")
+    S, B, H, W, C, xs = _image_dims(x)
+    kh, kw, sh, sw, ph, pw, dh, dw = geom
+    Ho, Wo = conv_output_size(H, kh, sh, ph, dh), conv_output_size(W, kw, sw, pw, dw)
+    out = torch.empty(((B * Ho * Wo, ld) if S is None else (S, B * Ho * Wo, ld)), dtype=x.dtype, device=x.device)
+    name = "whvi_im2col_bf16" if x.dtype == torch.bfloat16 else "whvi_im2col_f32"
+    with torch.cuda.device(x.device), _Timed(name):
+        rc = getattr(_lib.lib(), name)(x.data_ptr(), xs, out.data_ptr(), 1 if S is None else S, B, H, W, C, *geom, ld, _stream(x.device))
+    _lib.check(rc, name)
+    return out
+
+
+def col2im_(dpatches, geom, image_shape, sum_samples=False):
+    """Adjoint of ``im2col_`` (``whvi_col2im_*``): the (B Ho Wo, ld) or (S, B Ho Wo, ld) patch gradient scattered back to the
+    channels-last image of ``image_shape`` (B, H, W, C), each input element summing its taps i ascending, j ascending in fp32.
+    ``sum_samples``: a (S, B Ho Wo, ld) gradient is reduced over s ascending into one (B, H, W, C) block, the gradient of an
+    input shared by the samples; otherwise the result has the sample axis of ``dpatches``.  No autograd."""
+    dp = _act(dpatches, "dpatches")
+    B, H, W, C = image_shape
+    S = 1 if dp.dim() == 2 else dp.size(0)
+    ld = dp.size(-1)
+    shape = (B, H, W, C) if dp.dim() == 2 or sum_samples else (S, B, H, W, C)
+    dx = torch.empty(shape, dtype=dp.dtype, device=dp.device)
+    name = "whvi_col2im_bf16" if dp.dtype == torch.bfloat16 else "whvi_col2im_f32"
+    with torch.cuda.device(dp.device), _Timed(name):
+        rc = getattr(_lib.lib(), name)(dp.data_ptr(), ld, dx.data_ptr(), S, B, H, W, C, *geom, 1 if sum_samples else 0, _stream(dp.device))
+    _lib.check(rc, name)
+    return dx
+
+
+class Im2ColFunction(Function):
+    """``im2col_`` with its adjoint as the backward: the patch gather of ``WHVIConv2d``.  A layer call on the patch matrix
+    follows it, and autograd composes the two, so every parameter gradient comes from the layer's own kernels.  For an input
+    shared by the samples the patches are one (B Ho Wo, ld) block, which the layer reads for every sample and whose gradient
+    it returns already summed over the samples; col2im then scatters that one block.  The backward is skipped when ``x``
+    needs no gradient."""
+
+    @staticmethod
+    def forward(ctx, x, geom, ld):
+        ctx.geom, ctx.image_shape = geom, tuple(x.shape[-4:])
+        return im2col_(x, geom, ld)
+
+    @staticmethod
+    def backward(ctx, dpatches):
+        if not ctx.needs_input_grad[0]:
+            return None, None, None
+        return col2im_(dpatches, ctx.geom, ctx.image_shape), None, None
+
+
+def im2col(x, geom, ld):
+    return Im2ColFunction.apply(x, geom, ld)

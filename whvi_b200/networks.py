@@ -17,7 +17,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import functional as WF
-from .layers import WHVI, WHVILinear
+from .layers import WHVI, WHVIConv2d, WHVILinear
 from .likelihoods import CategoricalLikelihood, GaussianLikelihood, Likelihood
 
 try:  # progress bars exactly like the reference when tqdm is around
@@ -60,7 +60,7 @@ class WHVINetwork(nn.Module, WHVI):
         return sum([m.kl for m in self.sequential.children() if 'kl' in dir(m)])
 
     def _whvi_layers(self):
-        return [m for m in self.sequential.children() if isinstance(m, WHVILinear)]
+        return [m for m in self.sequential.children() if isinstance(m, (WHVILinear, WHVIConv2d))]
 
     def _predraw_reference_order(self, n_samples: int) -> None:
         blocks = [b for layer in self._whvi_layers() for b in layer.square_blocks()]
@@ -98,7 +98,8 @@ class WHVINetwork(nn.Module, WHVI):
         (S, B, out) activations, or -- with ``sqerr_target`` and a fusable last layer --
         ``(activations, sum of squared errors)`` with the reduction done in the last
         layer's kernel.  ``[Square WHVI layer, nn.ReLU, Square WHVI layer]`` runs are executed
-        with the ReLU folded into the two kernels (``self.fuse``)."""
+        with the ReLU folded into the two kernels (``self.fuse``).  Foreign modules before the first WHVI layer see the
+        input as it is (e.g. a (B, C, H, W) image batch); after it, the sample axis folded into the batch."""
         modules = list(self.sequential.children())
         layers = self._whvi_layers()
         if self.rng_mode == "reference":
@@ -108,9 +109,12 @@ class WHVINetwork(nn.Module, WHVI):
         sq = None
         try:
             h, i, relu_in, scale_holder = x, 0, False, None
+            sampled = False   # a WHVI layer has run: h carries the sample axis
             while i < len(modules):
                 module = modules[i]
                 last = i == len(modules) - 1
+                whvi_layer = isinstance(module, (WHVILinear, WHVIConv2d))
+                sampled = sampled or whvi_layer
                 if self.fuse and self._fusable_stacked(module):
                     # all blocks of the Stacked layer in one grouped launch, the following ReLU folded in when the
                     # consumer's kernels can apply the mask on the way back
@@ -147,7 +151,7 @@ class WHVINetwork(nn.Module, WHVI):
                     relu_in = relu_out
                     i += 2 if relu_out else 1
                     continue
-                if isinstance(module, WHVILinear) or h.dim() == 2:
+                if whvi_layer or not sampled:
                     h = module(h)
                 else:  # foreign module: fold the sample axis into the batch
                     S, B = h.shape[0], h.shape[1]
@@ -157,13 +161,13 @@ class WHVINetwork(nn.Module, WHVI):
         finally:
             for layer in layers:
                 layer.mc_samples = None
-        if h is not None and h.dim() == 2:  # no WHVI layer introduced a sample axis: S identical predictions
+        if h is not None and not sampled:  # no WHVI layer introduced a sample axis: S identical predictions
             h = h.unsqueeze(0).expand(n_samples, *h.shape)
         return (h, sq) if sqerr_target is not None else h
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
-        """x: (batch_size, in_dim) -> (batch_size, out_dim, n_samples)."""
-        assert x.dim() == 2, "Input shape must be (batch_size, in_dim)"
+        """x: (batch_size, in_dim) or an image batch (batch_size, C, H, W) -> (batch_size, out_dim, n_samples)."""
+        assert x.dim() in (2, 4), "Input shape must be (batch_size, in_dim) or (batch_size, C, H, W)"
         batch_size = x.size()[0]
         n_samples = self.train_samples if self.training else self.eval_samples
         h = self._run(x, n_samples)
