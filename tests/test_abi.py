@@ -87,6 +87,24 @@ def test_argument_validation_without_a_gpu():
     assert L.whvi_mc_moments_f32(a, None, a, 2, 8, 0, None) == E_NULL
 
 
+def test_stacked_rejects_more_than_65535_groups_without_a_gpu():
+    """G > 65535 would be the grouped reparameterisation backward's grid.y: every Stacked entry point rejects it with
+    WHVI_E_SHAPE before any CUDA call (null pointers: the shape check comes first)."""
+    from whvi_b200 import _lib
+    L = _lib.lib()
+    E_SHAPE = -2
+    G, D, S, B = 65536, 4, 1, 1
+    ws = ctypes.c_size_t(0)
+    assert L.whvi_stacked_bwd_workspace_bytes(S, B, D, G, 0, ctypes.byref(ws)) == E_SHAPE
+    assert b"above 65535" in L.whvi_last_error()
+    assert L.whvi_stacked_fwd_f32(None, 0, None, None, None, None, D, None, None, None, None, None, S, B, D, G, G * D, 0,
+                                  None) == E_SHAPE
+    assert L.whvi_stacked_bwd_f32(None, 0, None, None, None, None, None, D, None, None, D, None, None, None, None, None, None, 0,
+                                  S, B, D, G, G * D, 0, None) == E_SHAPE
+    assert b"above 65535" in L.whvi_last_error()
+    assert L.whvi_stacked_bwd_workspace_bytes(S, B, D, 65535, 0, ctypes.byref(ws)) == 0   # the limit itself is fine
+
+
 def test_shim_and_ctypes_reach_the_same_entry_points():
     """The CPython shim (csrc_host/fastcall.c) is a second way INTO the C ABI, not around it: for the all-integer entry points
     it hands out, the status codes and error messages equal what the ctypes binding of the same function returns (argument

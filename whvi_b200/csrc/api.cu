@@ -440,6 +440,7 @@ static int check_stacked(const char* who, int64_t S, int64_t B, int64_t D, int64
     if (int rc = check_layer_shape(who, S, B, D, xs)) return rc;
     if (G < 1 || n_out <= (G - 1) * D || n_out > G * D)
         return fail(WHVI_E_SHAPE, "%s: G=%lld blocks of D=%lld do not match n_out=%lld", who, (long long)G, (long long)D, (long long)n_out);
+    if (G > 65535) return fail(WHVI_E_SHAPE, "%s: G=%lld above 65535", who, (long long)G);   // the grouped reparam backward's grid.y
     if (G > 1 && (pstride < D || pstride % 4 != 0))
         return fail(WHVI_E_SHAPE, "%s: param_stride=%lld must be >= D and a multiple of 4", who, (long long)pstride);
     if (S * G > 0x7fffffffLL) return fail(WHVI_E_SHAPE, "%s: too many virtual samples", who);

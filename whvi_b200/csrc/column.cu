@@ -84,26 +84,29 @@ column_dot_dx_kernel(const float* __restrict__ dy, const A* __restrict__ x, int6
 }
 
 // dwp[s, j] = sum_b u[s, b] * v[s, b, j] over the batch: transposed u = dy (S, B), v = x (S, B, n); plain u = x (S, B), v = dy (S, B, n).
-// 32 columns x 8 batch slices per CTA, slices combined in a fixed order.  grid (ceil(n / 32), S).  U, V: the activation types of u, v.
+// 32 columns x 8 batch slices per CTA, slices combined in a fixed order.  grid (ceil(n / 32), min(S, 65535)); a CTA takes samples
+// blockIdx.y, + gridDim.y, ...  U, V: the activation types of u, v.
 template <class U, class V>
 __global__ void __launch_bounds__(256)
-column_dw_kernel(const U* __restrict__ u, int64_t us, const V* __restrict__ v, int64_t vs, float* __restrict__ dwp, int64_t B, int n)
+column_dw_kernel(const U* __restrict__ u, int64_t us, const V* __restrict__ v, int64_t vs, float* __restrict__ dwp, int64_t S, int64_t B, int n)
 {
     __shared__ float red[8][32];
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
     const int j = blockIdx.x * 32 + tx;
-    const int64_t s = blockIdx.y;
-    const U* up = u + s * us;
-    const V* vp = v + s * vs;
-    float acc = 0.f;
-    if (j < n)
-        for (int64_t b = ty; b < B; b += 8) acc = fmaf(widen(up[b]), widen(vp[b * n + j]), acc);
-    red[ty][tx] = acc;
-    __syncthreads();
-    if (ty == 0 && j < n) {
+    for (int64_t s = blockIdx.y; s < S; s += gridDim.y) {
+        const U* up = u + s * us;
+        const V* vp = v + s * vs;
+        float acc = 0.f;
+        if (j < n)
+            for (int64_t b = ty; b < B; b += 8) acc = fmaf(widen(up[b]), widen(vp[b * n + j]), acc);
+        red[ty][tx] = acc;
+        __syncthreads();
+        if (ty == 0 && j < n) {
 #pragma unroll
-        for (int q = 1; q < 8; ++q) acc += red[q][tx];
-        dwp[s * n + j] = acc;
+            for (int q = 1; q < 8; ++q) acc += red[q][tx];
+            dwp[s * n + j] = acc;
+        }
+        __syncthreads();   // red is refilled for the next sample
     }
 }
 
@@ -258,13 +261,13 @@ static int column_bwd_products(const float* x, int64_t xs, const float* dy, cons
     const A* xa = reinterpret_cast<const A*>(x);
     A* dxa = reinterpret_cast<A*>(dx);
     const int Di = static_cast<int>(D), ni = static_cast<int>(n);
-    const dim3 dwgrid(static_cast<unsigned>((n + 31) / 32), static_cast<unsigned>(S));
+    const dim3 dwgrid(static_cast<unsigned>((n + 31) / 32), static_cast<unsigned>(S < 65535 ? S : 65535));   // grid.y <= 65535
     if (transposed) {   // dy (S, B) is fp32
         if (dx) {
             column_dot_dx_kernel<A><<<ew_grid(S * B * n), 256, 0, st>>>(dy, xa, xs, hg, s1, s2, dxa, S, B, Di, ni, relu_in);
             if (int rc = check_launch("column_dot_dx_kernel")) return rc;
         }
-        column_dw_kernel<float, A><<<dwgrid, 256, 0, st>>>(dy, B, xa, xs, dwp, B, ni);   // u = dy (S, B), v = x (stride xs: 0 when shared)
+        column_dw_kernel<float, A><<<dwgrid, 256, 0, st>>>(dy, B, xa, xs, dwp, S, B, ni);   // u = dy (S, B), v = x (stride xs: 0 when shared)
     } else {
         const A* dya = reinterpret_cast<const A*>(dy);
         if (dx) {
@@ -272,7 +275,7 @@ static int column_bwd_products(const float* x, int64_t xs, const float* dy, cons
             column_outer_dx_kernel<A><<<static_cast<unsigned>(blocks), 256, 0, st>>>(dya, hg, s1, s2, dxa, S, B, Di, ni);
             if (int rc = check_launch("column_outer_dx_kernel")) return rc;
         }
-        column_dw_kernel<A, A><<<dwgrid, 256, 0, st>>>(xa, xs, dya, B * n, dwp, B, ni);  // u = x (S, B) (stride xs), v = dy (S, B, n)
+        column_dw_kernel<A, A><<<dwgrid, 256, 0, st>>>(xa, xs, dya, B * n, dwp, S, B, ni);  // u = x (S, B) (stride xs), v = dy (S, B, n)
     }
     if (int rc = check_launch("column_dw_kernel")) return rc;
     if (dbias) {

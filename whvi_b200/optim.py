@@ -130,5 +130,31 @@ class FlatAdam(torch.optim.Optimizer):
         _lib.check(rc, "whvi_adam_f32")
         return loss
 
+    def load_state_dict(self, state_dict) -> None:
+        """``torch.optim.Optimizer.load_state_dict``, then the loaded step count and moments copied into the buffers the kernel
+        reads, which stay this optimizer's state.  A tensor ``lr`` receives the loaded value in place and stays in the
+        param group.  Everything is copied in place, so a ``graphs.GraphedTrainStep`` captured before the load stays valid."""
+        groups = state_dict["param_groups"]
+        pid = groups[0]["params"][0] if len(groups) == 1 and groups[0]["params"] else None
+        saved = state_dict["state"].get(pid, {})
+        n = self.flat.numel
+        for key, size in (("step", 1), ("exp_avg", n), ("exp_avg_sq", n)):
+            got = saved.get(key)
+            if got is None or torch.as_tensor(got).numel() != size:
+                have = "missing" if got is None else f"{torch.as_tensor(got).numel()} elements"
+                raise ValueError(f"FlatAdam.load_state_dict: state '{key}' must have {size} elements "
+                                 f"(this optimizer's flat buffer), got {have}")
+        lr = self.param_groups[0]["lr"]
+        super().load_state_dict(state_dict)
+        loaded = self.state[self.flat.params[0]]
+        with torch.no_grad():
+            self.step_t.copy_(torch.as_tensor(loaded["step"]).reshape(1))
+            self.exp_avg.copy_(loaded["exp_avg"].reshape(-1))
+            self.exp_avg_sq.copy_(loaded["exp_avg_sq"].reshape(-1))
+            if torch.is_tensor(lr):
+                lr.copy_(torch.as_tensor(self.param_groups[0]["lr"]).reshape(lr.shape))
+                self.param_groups[0]["lr"] = lr
+        self.state[self.flat.params[0]] = {"step": self.step_t, "exp_avg": self.exp_avg, "exp_avg_sq": self.exp_avg_sq}
+
     def zero_grad(self, set_to_none: bool = False) -> None:  # noqa: ARG002 -- the views must survive
         self.flat.zero_grad()
