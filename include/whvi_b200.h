@@ -445,7 +445,17 @@ WHVI_API int whvi_mc_moments_strided_f32(const float* y, int64_t y_sample_stride
  *                                logits + s * sample_stride (>= B * K, so a sample chunk may be a slice of a larger tensor);
  *                                flags & WHVI_CATEGORICAL_ACCUMULATE adds to the existing sums in the order one call over all
  *                                samples would (chunks give that call's bits).  labels and loglik_sum both or neither.
- * A label outside [0, K) is never used as an index: that row's loss (so the total), its log p and its dz row are NaN.
+ *   whvi_categorical_uncertainty_*  the predictive's prob_sum and loglik_sum, bit for bit, and in the same pass
+ *                                ent_sum[b] (+)= sum_s H_s with H_s = sum_k p_k (lse_s - z[s, b, k]), the entropy of sample s's
+ *                                softmax (every term >= 0; a class with p_k = 0 adds 0), and, with labels,
+ *                                logpred[b] = log sum_s p_s(y_b), a running logaddexp of log p_s(y_b) over s ascending (no
+ *                                underflow when a confident model is wrong; with WHVI_CATEGORICAL_ACCUMULATE continued from
+ *                                the stored value, so chunks give one call's bits; S = 0 without it gives -inf).  (B) fp32 each.
+ *                                prob_sum and ent_sum required; labels, loglik_sum and logpred all or none; otherwise validated
+ *                                as the predictive.  The test NLL of the MC predictive is log S - logpred[b]; the mutual
+ *                                information is H[prob_sum / S] - ent_sum / S.
+ * A label outside [0, K) is never used as an index: that row's loss (so the total), its log p (loglik_sum, logpred) and its dz
+ * row are NaN.
  * Every reduction has a fixed order: repeated calls are bit-identical.  Alignment: the element size of each pointer's type
  * (rows need no more: the loads are element-wise); workspace 8 bytes.
  */
@@ -463,6 +473,12 @@ WHVI_API int whvi_categorical_predictive_f32(const float* logits, int64_t sample
                                              float* loglik_sum, int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream);
 WHVI_API int whvi_categorical_predictive_bf16(const void* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum,
                                               float* loglik_sum, int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream);
+WHVI_API int whvi_categorical_uncertainty_f32(const float* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum,
+                                              float* loglik_sum, float* logpred, float* ent_sum, int64_t S, int64_t B, int64_t K,
+                                              int flags, whvi_stream_t stream);
+WHVI_API int whvi_categorical_uncertainty_bf16(const void* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum,
+                                               float* loglik_sum, float* logpred, float* ent_sum, int64_t S, int64_t B, int64_t K,
+                                               int flags, whvi_stream_t stream);
 
 /*
  * Patch gather and scatter of a convolutional WHVI layer (WHVIConv2d; not in the reference).  Activations are channels-last:

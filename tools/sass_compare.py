@@ -11,7 +11,11 @@ parameter added with a default changes the mangled names of the existing instanc
   * ``--strip-arg KERNEL`` then drops a trailing ``, float`` template argument that follows a non-type argument, in both builds
     (default: the four kernels that gained an activation-type parameter for bf16 training, so that builds from before it match);
   * ``--untemplate KERNEL`` keys a kernel that became a template on its element types by its bare name in BOTH builds, where
-    every template argument is ``float`` (the plain kernel of the older build); other instances keep their arguments.
+    every template argument is ``float`` (the plain kernel of the older build); other instances keep their arguments;
+  * ``--strip-false KERNEL`` drops a trailing ``, false`` template argument of KERNEL (a ``bool`` flag added last, whose
+    ``false`` instances are the older ones) and keys KERNEL's instances without their parameter list, since the flag came
+    with extra trailing parameters that the ``false`` instances never read (default: ``categorical_predictive_kernel``, whose
+    ``true`` instances add the uncertainty sums).
 Each old instance must have a new instance of the same name whose instructions AND encodings (scheduling control words
 included) are identical, line for line; only the instruction addresses are ignored.  New instances without an old counterpart
 are listed.  Exit status 1 on any difference.
@@ -29,6 +33,7 @@ DEFAULT_STRIP = ("layer_bwd_tma_kernel", "layer_bwd_tm_kernel", "layer_loss_kern
 DEFAULT_STRIP_DUP = ("layer_bwd_tma_kernel", "layer_bwd_tm_kernel")
 DEFAULT_UNTEMPLATE = ("stack_split_kernel", "stack_concat_kernel", "stack_sum_kernel", "column_dot_kernel", "column_outer_kernel",
                       "column_dot_dx_kernel", "column_dw_kernel", "column_outer_dx_kernel", "column_dbias_kernel")
+DEFAULT_STRIP_FALSE = ("categorical_predictive_kernel",)
 _ADDR = re.compile(r"/\*[0-9a-f]{4,}\*/")
 
 
@@ -59,7 +64,12 @@ def demangle(names: list[str]) -> dict[str, str]:
     return dict(zip(names, out.splitlines()))
 
 
-def normalise(name: str, strip: tuple[str, ...], strip_dup: tuple[str, ...] = (), untemplate: tuple[str, ...] = ()) -> str:
+def normalise(name: str, strip: tuple[str, ...], strip_dup: tuple[str, ...] = (), untemplate: tuple[str, ...] = (),
+              strip_false: tuple[str, ...] = ()) -> str:
+    for k in strip_false:   # cu++filt prints the flag as ``(bool)0``; the parameter list is dropped too (see --strip-false)
+        if re.search(rf"\b{k}<", name):
+            name = re.sub(r", (?:false|\(bool\)0)>\(", ">(", name, count=1)
+            return name[:name.index(">(") + 1]
     m = re.match(r"(?:void )?whvi::(\w+)(?:<([^()]*)>)?\(", name)
     if m and m.group(1) in untemplate:
         args = m.group(2)
@@ -75,14 +85,14 @@ def normalise(name: str, strip: tuple[str, ...], strip_dup: tuple[str, ...] = ()
     return name
 
 
-def collect(obj_dir: Path, strip: tuple[str, ...], strip_dup: tuple[str, ...] = (), untemplate: tuple[str, ...] = ()
-            ) -> dict[str, tuple[str, list[str]]]:
+def collect(obj_dir: Path, strip: tuple[str, ...], strip_dup: tuple[str, ...] = (), untemplate: tuple[str, ...] = (),
+            strip_false: tuple[str, ...] = ()) -> dict[str, tuple[str, list[str]]]:
     res: dict[str, tuple[str, list[str]]] = {}
     for obj in sorted(obj_dir.glob("*.o")):
         funcs = kernels(obj)
         dm = demangle(list(funcs))
         for mangled, sass in funcs.items():
-            res[normalise(dm[mangled], strip, strip_dup, untemplate)] = (obj.name, sass)
+            res[normalise(dm[mangled], strip, strip_dup, untemplate, strip_false)] = (obj.name, sass)
     return res
 
 
@@ -93,10 +103,12 @@ def main() -> int:
     ap.add_argument("--strip-arg", nargs="*", default=list(DEFAULT_STRIP))
     ap.add_argument("--strip-dup", nargs="*", default=list(DEFAULT_STRIP_DUP))
     ap.add_argument("--untemplate", nargs="*", default=list(DEFAULT_UNTEMPLATE))
+    ap.add_argument("--strip-false", nargs="*", default=list(DEFAULT_STRIP_FALSE))
     a = ap.parse_args()
-    untemplate = tuple(a.untemplate)
+    untemplate, strip_false = tuple(a.untemplate), tuple(a.strip_false)
     strip, strip_dup = tuple(a.strip_arg), tuple(a.strip_dup)
-    old, new = collect(a.old, strip, strip_dup, untemplate), collect(a.new, strip, strip_dup, untemplate)
+    old = collect(a.old, strip, strip_dup, untemplate, strip_false)
+    new = collect(a.new, strip, strip_dup, untemplate, strip_false)
     same, differ, missing = 0, [], []
     for name, (obj, sass) in sorted(old.items()):
         if name not in new:

@@ -137,6 +137,10 @@ SIGNATURES = {
                                                 c_void_p]),
     "whvi_categorical_predictive_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int,
                                                  c_void_p]),
+    "whvi_categorical_uncertainty_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64,
+                                                 c_int64, c_int, c_void_p]),
+    "whvi_categorical_uncertainty_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64,
+                                                  c_int64, c_int, c_void_p]),
     # convolution patches: geometry (S, B, H, W, C, kh, kw, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w) as int64
     "whvi_im2col_f32": (c_int, [c_void_p, c_int64, c_void_p] + [c_int64] * 14 + [c_void_p]),
     "whvi_im2col_bf16": (c_int, [c_void_p, c_int64, c_void_p] + [c_int64] * 14 + [c_void_p]),

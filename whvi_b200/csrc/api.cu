@@ -945,34 +945,56 @@ int whvi_categorical_nll_bwd_bf16(const void* logits, const int64_t* labels, con
     return categorical_nll_bwd("categorical_nll_bwd_bf16", logits, 2, labels, lse, c, dz, S, B, K, stream);
 }
 
+// unc: the uncertainty call, which also takes logpred (with labels and loglik_sum) and ent_sum (required, like prob_sum)
 static int categorical_predictive(const char* who, const void* logits, size_t elem, int64_t sample_stride, const int64_t* labels,
-                                  float* prob_sum, float* loglik_sum, int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream)
+                                  float* prob_sum, float* loglik_sum, float* logpred, float* ent_sum, bool unc, int64_t S, int64_t B,
+                                  int64_t K, int flags, whvi_stream_t stream)
 {
     if (int rc = check_categorical(who, S, B, K)) return rc;
     if (flags & ~WHVI_CATEGORICAL_ACCUMULATE) return fail(WHVI_E_MODE, "%s: unknown flags %d", who, flags);
     if (S > 1 && sample_stride < B * K)
         return fail(WHVI_E_SHAPE, "%s: sample_stride=%lld below B * K = %lld", who, (long long)sample_stride, (long long)(B * K));
     if (S > 1 && sample_stride > (int64_t(1) << 62) / S) return fail(WHVI_E_SHAPE, "%s: sample_stride too large", who);
-    if ((labels == nullptr) != (loglik_sum == nullptr)) return fail(WHVI_E_NULL, "%s: labels and loglik_sum must both be given or both NULL", who);
+    if (!unc && (labels == nullptr) != (loglik_sum == nullptr))
+        return fail(WHVI_E_NULL, "%s: labels and loglik_sum must both be given or both NULL", who);
+    if (unc && ((labels == nullptr) != (loglik_sum == nullptr) || (labels == nullptr) != (logpred == nullptr)))
+        return fail(WHVI_E_NULL, "%s: labels, loglik_sum and logpred must all be given or all NULL", who);
     if (B == 0) return WHVI_OK;
-    if (!prob_sum || (S > 0 && !logits)) return fail(WHVI_E_NULL, "%s: null pointer", who);
+    if (!prob_sum || (unc && !ent_sum) || (S > 0 && !logits)) return fail(WHVI_E_NULL, "%s: null pointer", who);
     if (!aligned(logits, elem) || !aligned(labels, 8) || !aligned(prob_sum, 4) || !aligned(loglik_sum, 4))
         return fail(WHVI_E_ALIGN, "%s: logits, labels, prob_sum and loglik_sum must be aligned to their element size", who);
-    return launch_categorical_predictive(logits, sample_stride, labels, prob_sum, loglik_sum, S, B, K, flags & WHVI_CATEGORICAL_ACCUMULATE,
-                                         elem == 2, static_cast<cudaStream_t>(stream));
+    if (!aligned(logpred, 4) || !aligned(ent_sum, 4)) return fail(WHVI_E_ALIGN, "%s: logpred and ent_sum must be 4-byte aligned", who);
+    return launch_categorical_predictive(logits, sample_stride, labels, prob_sum, loglik_sum, logpred, ent_sum, S, B, K,
+                                         flags & WHVI_CATEGORICAL_ACCUMULATE, elem == 2, static_cast<cudaStream_t>(stream));
 }
 
 int whvi_categorical_predictive_f32(const float* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,
                                     int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream)
 {
-    return categorical_predictive("categorical_predictive_f32", logits, 4, sample_stride, labels, prob_sum, loglik_sum, S, B, K, flags, stream);
+    return categorical_predictive("categorical_predictive_f32", logits, 4, sample_stride, labels, prob_sum, loglik_sum, nullptr, nullptr,
+                                  false, S, B, K, flags, stream);
 }
 
 int whvi_categorical_predictive_bf16(const void* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,
                                      int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream)
 {
-    return categorical_predictive("categorical_predictive_bf16", logits, 2, sample_stride, labels, prob_sum, loglik_sum, S, B, K, flags,
-                                  stream);
+    return categorical_predictive("categorical_predictive_bf16", logits, 2, sample_stride, labels, prob_sum, loglik_sum, nullptr, nullptr,
+                                  false, S, B, K, flags, stream);
+}
+
+int whvi_categorical_uncertainty_f32(const float* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,
+                                     float* logpred, float* ent_sum, int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream)
+{
+    return categorical_predictive("categorical_uncertainty_f32", logits, 4, sample_stride, labels, prob_sum, loglik_sum, logpred, ent_sum,
+                                  true, S, B, K, flags, stream);
+}
+
+int whvi_categorical_uncertainty_bf16(const void* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum,
+                                      float* loglik_sum, float* logpred, float* ent_sum, int64_t S, int64_t B, int64_t K, int flags,
+                                      whvi_stream_t stream)
+{
+    return categorical_predictive("categorical_uncertainty_bf16", logits, 2, sample_stride, labels, prob_sum, loglik_sum, logpred, ent_sum,
+                                  true, S, B, K, flags, stream);
 }
 
 // ---- convolution patches (csrc/conv.cu) ---------------------------------------------------------------------------------

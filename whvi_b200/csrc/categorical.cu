@@ -3,6 +3,8 @@
 //                            total = sum_r loss_r: fp64 per-CTA partials, then one CTA sums them in a fixed order
 //   categorical_nll_bwd      dz_rk = c (exp(z_rk - lse_r) - [k = y_b]),  c a device scalar
 //   categorical_predictive   prob_sum[b, :] (+)= sum_s softmax(z_{s,b}),  loglik_sum[b] (+)= sum_s log p_s(y_b),  s ascending
+//     <UNC = true> also      ent_sum[b] (+)= sum_s H_s,  H_s = sum_k p_k (lse - z_k)  (every term >= 0; p_k = 0 adds nothing),
+//                            logpred[b] = logaddexp over s of log p_s(y_b), continued from the stored value with accumulate
 // Rows r = s * B + b of the (S, B, K) logits, labels (B) int64.
 //
 // Work split: a GROUP of TPR threads owns a row.  K <= 32: TPR = next_pow2(K), so a warp holds 32 / TPR rows; K <= 2048:
@@ -80,6 +82,35 @@ __device__ __forceinline__ float row_lse(const T* row, int K, int lane, bool val
     return a.m + logf(a.s);
 }
 
+// sum of v over the group in every thread, in a fixed order (butterfly, then for a CTA the warps ascending).  Same calling
+// rules as row_lse: every lane of the warp takes part, and TPR == kThreads synchronises the CTA.
+template <int TPR>
+__device__ __forceinline__ float group_sum(float v)
+{
+    constexpr int width = TPR < 32 ? TPR : 32;
+#pragma unroll
+    for (int o = width / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);   // a + b == b + a: every lane agrees
+    if constexpr (TPR > 32) {
+        __shared__ float warps[TPR / 32];
+        if ((threadIdx.x & 31) == 0) warps[threadIdx.x >> 5] = v;
+        __syncthreads();
+        v = warps[0];
+#pragma unroll
+        for (int w = 1; w < TPR / 32; ++w) v += warps[w];
+        __syncthreads();
+    }
+    return v;
+}
+
+// log(exp(a) + exp(b)); -inf with -inf is -inf, and a NaN argument gives NaN (fmaxf alone would drop it)
+__device__ __forceinline__ float logaddexp(float a, float b)
+{
+    if (a != a || b != b) return qnan();
+    const float m = fmaxf(a, b);
+    if (m == -INFINITY) return m;
+    return m + log1pf(expf(fminf(a, b) - m));
+}
+
 template <int TPR, typename T>
 __global__ void __launch_bounds__(kThreads)
 categorical_nll_kernel(const T* __restrict__ z, const int64_t* __restrict__ labels, float* __restrict__ lse_out,
@@ -149,11 +180,12 @@ categorical_nll_bwd_kernel(const T* __restrict__ z, const int64_t* __restrict__ 
     }
 }
 
-template <int TPR, typename T>
+// UNC = false: the predictive sums.  UNC = true: the same sums (same bits) plus ent_sum and, with labels, logpred.
+template <int TPR, typename T, bool UNC>
 __global__ void __launch_bounds__(kThreads)
 categorical_predictive_kernel(const T* __restrict__ z, int64_t sample_stride, const int64_t* __restrict__ labels,
                               float* __restrict__ prob_sum, float* __restrict__ loglik_sum, int64_t S, int64_t B, int K,
-                              int accumulate)
+                              int accumulate, float* __restrict__ logpred, float* __restrict__ ent_sum)
 {
     constexpr int G = kThreads / TPR;
     const int g = threadIdx.x / TPR, lane = threadIdx.x % TPR;
@@ -170,9 +202,39 @@ categorical_predictive_kernel(const T* __restrict__ z, int64_t sample_stride, co
             ok = y >= 0 && y < K;
         }
         float ll = (accumulate && valid && loglik_sum) ? loglik_sum[b] : 0.f;
+        float ent = 0.f, lp = -INFINITY;
+        if constexpr (UNC) {
+            if (accumulate && valid) {
+                ent = ent_sum[b];
+                if (logpred) lp = logpred[b];
+            }
+        }
         for (int64_t s = 0; s < S; ++s) {
             const T* row = z + s * sample_stride + off;
             const float l = row_lse<TPR>(row, K, lane, valid);
+            if constexpr (UNC) {
+                float h = 0.f;   // this lane's share of H_s; an invalid group adds zeros but still joins the group sum
+                if (valid) {
+                    const bool fresh = s == 0 && !accumulate;
+                    for (int k = lane; k < K; k += TPR) {
+                        const float zk = ldz(row, k);
+                        prow[k] = (fresh ? 0.f : prow[k]) + expf(zk - l);
+                        // the entropy's p_k from its own exp2: sharing expf's result would keep the compiler from fusing
+                        // expf's last multiply into the add above, and prob_sum would lose the predictive's bits
+                        const float p = exp2f((zk - l) * 1.44269504f);
+                        h += p != 0.f ? p * (l - zk) : 0.f;   // p = 0 (z_k = -inf, underflow): no 0 * inf
+                    }
+                }
+                h = group_sum<TPR>(h);
+                if (!valid) continue;
+                ent += h;
+                if (labels && lane == 0) {
+                    const float lpy = ok ? ldz(row, y) - l : qnan();
+                    ll += lpy;
+                    lp = logaddexp(lp, lpy);
+                }
+                continue;
+            }
             if (!valid) continue;
             const bool fresh = s == 0 && !accumulate;
             for (int k = lane; k < K; k += TPR) prow[k] = (fresh ? 0.f : prow[k]) + expf(ldz(row, k) - l);
@@ -182,6 +244,12 @@ categorical_predictive_kernel(const T* __restrict__ z, int64_t sample_stride, co
         if (S == 0 && !accumulate)
             for (int k = lane; k < K; k += TPR) prow[k] = 0.f;
         if (loglik_sum && lane == 0) loglik_sum[b] = ll;
+        if constexpr (UNC) {
+            if (lane == 0) {
+                ent_sum[b] = ent;
+                if (logpred) logpred[b] = lp;
+            }
+        }
     }
 }
 
@@ -244,15 +312,18 @@ int nll_bwd_t(const void* z, const int64_t* labels, const float* lse, const floa
     return check_launch("categorical_nll_bwd_kernel");
 }
 
+// ent_sum != NULL selects the UNC instance
 template <typename T>
-int predictive_t(const void* z, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum, int64_t S, int64_t B,
-                 int64_t K, int accumulate, cudaStream_t st)
+int predictive_t(const void* z, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum, float* logpred,
+                 float* ent_sum, int64_t S, int64_t B, int64_t K, int accumulate, cudaStream_t st)
 {
     if (B == 0) return WHVI_OK;
     const Plan p = plan(B, K);
     with_tpr(p.tpr, [&](auto tpr) {
-        categorical_predictive_kernel<decltype(tpr)::value, T><<<static_cast<unsigned>(p.ctas), kThreads, 0, st>>>(
-            static_cast<const T*>(z), sample_stride, labels, prob_sum, loglik_sum, S, B, static_cast<int>(K), accumulate);
+        constexpr int TPR = decltype(tpr)::value;
+        auto kernel = ent_sum ? categorical_predictive_kernel<TPR, T, true> : categorical_predictive_kernel<TPR, T, false>;
+        kernel<<<static_cast<unsigned>(p.ctas), kThreads, 0, st>>>(static_cast<const T*>(z), sample_stride, labels, prob_sum, loglik_sum,
+                                                                   S, B, static_cast<int>(K), accumulate, logpred, ent_sum);
     });
     return check_launch("categorical_predictive_kernel");
 }
@@ -274,10 +345,11 @@ int launch_categorical_nll_bwd(const void* z, const int64_t* labels, const float
 }
 
 int launch_categorical_predictive(const void* z, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,
-                                  int64_t S, int64_t B, int64_t K, int accumulate, int bf16, cudaStream_t st)
+                                  float* logpred, float* ent_sum, int64_t S, int64_t B, int64_t K, int accumulate, int bf16,
+                                  cudaStream_t st)
 {
-    return bf16 ? predictive_t<__nv_bfloat16>(z, sample_stride, labels, prob_sum, loglik_sum, S, B, K, accumulate, st)
-                : predictive_t<float>(z, sample_stride, labels, prob_sum, loglik_sum, S, B, K, accumulate, st);
+    return bf16 ? predictive_t<__nv_bfloat16>(z, sample_stride, labels, prob_sum, loglik_sum, logpred, ent_sum, S, B, K, accumulate, st)
+                : predictive_t<float>(z, sample_stride, labels, prob_sum, loglik_sum, logpred, ent_sum, S, B, K, accumulate, st);
 }
 
 }  // namespace whvi

@@ -147,8 +147,10 @@ int launch_categorical_nll(const void* z, const int64_t* labels, float* lse, flo
                            int bf16, cudaStream_t st);
 int launch_categorical_nll_bwd(const void* z, const int64_t* labels, const float* lse, const float* c, void* dz, int64_t S, int64_t B,
                                int64_t K, int bf16, cudaStream_t st);
+// ent_sum != NULL: the uncertainty sums as well (logpred with the labels, else NULL)
 int launch_categorical_predictive(const void* z, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,
-                                  int64_t S, int64_t B, int64_t K, int accumulate, int bf16, cudaStream_t st);
+                                  float* logpred, float* ent_sum, int64_t S, int64_t B, int64_t K, int accumulate, int bf16,
+                                  cudaStream_t st);
 // patch gather / scatter of WHVIConv2d (conv.cu); validated geometry, every spatial quantity below 2^24
 struct ConvGeom {
     int64_t S, B;

@@ -104,3 +104,33 @@ def reduce_predictive_probs(prob_sum: torch.Tensor, loglik_sum: torch.Tensor | N
             if t is not None:
                 dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
     return prob_sum / count, None if loglik_sum is None else loglik_sum / count
+
+
+def reduce_predictive_uncertainty(prob_sum: torch.Tensor, ent_sum: torch.Tensor, logpred: torch.Tensor | None,
+                                  loglik_sum: torch.Tensor | None, n_local: int, group=None):
+    """Classification uncertainty with evaluation sharded by MC sample: combine each rank's sums of
+    ``functional.categorical_uncertainty_`` (``WHVIClassification.predictive_uncertainty_sums``) over all samples.  prob_sum,
+    ent_sum and loglik_sum are added across ranks (in place); logpred = log sum_s p_s(y) is combined as a log-sum-exp across
+    ranks in fp64 (an all-reduce MAX, then a SUM of exp(l - max)): a row that is -inf on every rank stays -inf, and a NaN row on
+    any rank (a label outside [0, K)) stays NaN.  Returns (``uncertainty.CategoricalUncertainty`` over all samples, the mean
+    log-likelihood per input or None); logpred and loglik_sum may be None together.  Works in a single process too."""
+    from .uncertainty import categorical_uncertainty
+    count = torch.tensor([float(n_local)], dtype=torch.float64, device=prob_sum.device)
+    logpred = None if logpred is None else logpred.to(torch.float64)
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        for t in (prob_sum, ent_sum, loglik_sum, count):
+            if t is not None:
+                dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+        if logpred is not None:
+            nan = torch.isnan(logpred)
+            finite = torch.where(nan, float("-inf"), logpred)
+            m = finite.clone()
+            dist.all_reduce(m, op=dist.ReduceOp.MAX, group=group)
+            shift = torch.where(m == float("-inf"), 0.0, m)   # -inf everywhere: exp(-inf - 0) = 0, no -inf - -inf
+            e = torch.exp(finite - shift)
+            dist.all_reduce(e, op=dist.ReduceOp.SUM, group=group)
+            any_nan = nan.to(torch.float64)
+            dist.all_reduce(any_nan, op=dist.ReduceOp.SUM, group=group)
+            logpred = torch.where(any_nan > 0, float("nan"), torch.log(e) + shift)
+    S = int(count.item())
+    return categorical_uncertainty(prob_sum, ent_sum, logpred, S), None if loglik_sum is None else loglik_sum / count.to(loglik_sum.dtype)

@@ -39,6 +39,7 @@ _LAUNCHES_PER_CALL = {"whvi_fwht_f32": 1, "whvi_fwht_f64": 1, "whvi_layer_fwd_f3
                       # categorical likelihood: the forward is the row kernel + the fixed-order sum of its per-CTA partials
                       "whvi_categorical_nll_f32": 2, "whvi_categorical_nll_bf16": 2, "whvi_categorical_nll_bwd_f32": 1,
                       "whvi_categorical_nll_bwd_bf16": 1, "whvi_categorical_predictive_f32": 1, "whvi_categorical_predictive_bf16": 1,
+                      "whvi_categorical_uncertainty_f32": 1, "whvi_categorical_uncertainty_bf16": 1,
                       "whvi_im2col_f32": 1, "whvi_im2col_bf16": 1, "whvi_col2im_f32": 1, "whvi_col2im_bf16": 1}
 # When set to a dict {"name": [(start_event, stop_event), ...]}, the named calls are bracketed
 # by CUDA events on the launching stream (bench.py's per-kernel roofline timing).
@@ -1305,6 +1306,40 @@ def categorical_predictive_(logits, labels, prob_sum, loglik_sum=None, accumulat
     (B,), samples ascending (``whvi_categorical_predictive_*``).  ``logits`` (S, B, K) fp32 or bf16 may be a sample-slice of a
     larger tensor (rows contiguous, any sample stride); ``accumulate`` continues the sums of earlier sample chunks in the order
     of one call over all samples, so chunked evaluation gives the same bits.  No autograd."""
+    logits, labels, S, B, K, stride = _predictive_args(logits, labels)
+    if (labels is None) != (loglik_sum is None):
+        raise RuntimeError("labels and loglik_sum go together")
+    _check_sums(logits, (prob_sum, "prob_sum", B * K), (loglik_sum, "loglik_sum", B))
+    name = "whvi_categorical_predictive_bf16" if logits.dtype == torch.bfloat16 else "whvi_categorical_predictive_f32"
+    with torch.cuda.device(logits.device), _Timed(name, f"K={K}"):
+        rc = getattr(_lib.lib(), name)(logits.data_ptr(), stride, _ptr(labels), prob_sum.data_ptr(), _ptr(loglik_sum), S, B, K,
+                                       1 if accumulate else 0, _stream(logits.device))
+    _lib.check(rc, name)
+    return prob_sum, loglik_sum
+
+
+def categorical_uncertainty_(logits, labels, prob_sum, ent_sum, loglik_sum=None, logpred=None, accumulate=False):
+    """``categorical_predictive_``'s prob_sum and loglik_sum (the same bits) and, from the same pass over the logits,
+    ent_sum (+)= sum_s H[softmax(logits[s])] (B,) and, with ``labels``, logpred = log sum_s softmax(logits[s])[labels] (B,), kept as a
+    running log-sum-exp over the samples so that it does not underflow (``whvi_categorical_uncertainty_*``).  ``labels``,
+    ``loglik_sum`` and ``logpred`` go together.  Same input handling as ``categorical_predictive_``: fp32 or bf16 logits, any
+    sample stride, and ``accumulate`` continues every sum of earlier sample chunks with one call's bits.  No autograd."""
+    logits, labels, S, B, K, stride = _predictive_args(logits, labels)
+    if not ((labels is None) == (loglik_sum is None) == (logpred is None)):
+        raise RuntimeError("labels, loglik_sum and logpred go together")
+    if prob_sum is None or ent_sum is None:
+        raise RuntimeError("prob_sum and ent_sum are required")
+    _check_sums(logits, (prob_sum, "prob_sum", B * K), (ent_sum, "ent_sum", B), (loglik_sum, "loglik_sum", B), (logpred, "logpred", B))
+    name = "whvi_categorical_uncertainty_bf16" if logits.dtype == torch.bfloat16 else "whvi_categorical_uncertainty_f32"
+    with torch.cuda.device(logits.device), _Timed(name, f"K={K}"):
+        rc = getattr(_lib.lib(), name)(logits.data_ptr(), stride, _ptr(labels), prob_sum.data_ptr(), _ptr(loglik_sum), _ptr(logpred),
+                                       ent_sum.data_ptr(), S, B, K, 1 if accumulate else 0, _stream(logits.device))
+    _lib.check(rc, name)
+    return prob_sum, ent_sum, loglik_sum, logpred
+
+
+def _predictive_args(logits, labels):
+    """(logits with rows contiguous, labels, S, B, K, sample stride) for the predictive calls; checked before the device."""
     if logits.dim() != 3:
         raise RuntimeError(f"logits must be (S, B, K), got {tuple(logits.shape)}")
     S, B, K = logits.shape
@@ -1312,20 +1347,16 @@ def categorical_predictive_(logits, labels, prob_sum, loglik_sum=None, accumulat
         labels = _categorical_args(logits[:0], labels)[1]
     elif logits.dtype not in (torch.float32, torch.bfloat16) or logits.device.type != "cuda":
         raise RuntimeError("logits must be a float32 or bfloat16 CUDA tensor")
-    if (labels is None) != (loglik_sum is None):
-        raise RuntimeError("labels and loglik_sum go together")
     if logits.stride(2) != 1 or logits.stride(1) != K:
         logits = logits.contiguous()
-    stride = logits.stride(0) if S > 1 else B * K
-    for t, name, n in ((prob_sum, "prob_sum", B * K), (loglik_sum, "loglik_sum", B)):
+    return logits, labels, S, B, K, (logits.stride(0) if S > 1 else B * K)
+
+
+def _check_sums(logits, *sums):
+    """Each (tensor or None, name, elements) given must be a contiguous fp32 tensor of that size on the logits' device."""
+    for t, name, n in sums:
         if t is not None and (t.dtype != torch.float32 or not t.is_contiguous() or t.numel() != n or t.device != logits.device):
             raise RuntimeError(f"{name} must be a contiguous float32 tensor with {n} elements on {logits.device}")
-    name = "whvi_categorical_predictive_bf16" if logits.dtype == torch.bfloat16 else "whvi_categorical_predictive_f32"
-    with torch.cuda.device(logits.device), _Timed(name, f"K={K}"):
-        rc = getattr(_lib.lib(), name)(logits.data_ptr(), stride, _ptr(labels), prob_sum.data_ptr(), _ptr(loglik_sum), S, B, K,
-                                       1 if accumulate else 0, _stream(logits.device))
-    _lib.check(rc, name)
-    return prob_sum, loglik_sum
 
 
 # ---------------------------------------------------------------------------------------------- convolution patches

@@ -19,6 +19,8 @@ import torch.nn.functional as F
 from . import functional as WF
 from .layers import WHVI, WHVIConv2d, WHVILinear
 from .likelihoods import CategoricalLikelihood, GaussianLikelihood, Likelihood
+from .uncertainty import (CategoricalUncertainty, RegressionUncertainty, brier_score, categorical_uncertainty,
+                          expected_calibration_error)
 
 try:  # progress bars exactly like the reference when tqdm is around
     from tqdm import tqdm
@@ -304,6 +306,24 @@ class WHVIRegression(WHVINetwork):
                 return float(rmse), float(mnll)
         return super().eval_model(X_test, y_test, loss)
 
+    @torch.no_grad()
+    def predictive_uncertainty(self, X: torch.Tensor, n_samples: int | None = None) -> RegressionUncertainty:
+        """The MC mean of the predictions, their variance over the samples (epistemic; biased, 1/S) and the Gaussian
+        likelihood's noise variance sigma^2 (aleatoric), each (batch, out) fp64.  A network that ends in a square WHVI layer
+        takes both moments from ``predictive_sums`` (reduced inside that layer's kernel, no (S, batch, out) tensor); any other
+        reduces the (S, batch, out) predictions in fp64.  The variance from the sums is sum_y2 / S - mean^2, not clamped."""
+        S = int(n_samples if n_samples is not None else (self.train_samples if self.training else self.eval_samples))
+        sums = None if self.rng_mode == "reference" else self.predictive_sums(X, S)
+        if sums is not None:
+            sum_y, sum_y2, S = sums
+            mean = sum_y.to(torch.float64) / S
+            var = sum_y2.to(torch.float64) / S - mean * mean
+        else:
+            y = self._run(X, S).reshape(S, X.size(0), -1).to(torch.float64)
+            mean, var = y.mean(0), y.var(0, unbiased=False)
+        noise = (self.likelihood.sigma.detach().to(torch.float64) ** 2).expand_as(mean)
+        return RegressionUncertainty(mean, var, noise, S)
+
 
 class WHVIClassification(WHVINetwork):
     def __init__(self, modules: Iterable[nn.Module], **kwargs):
@@ -318,11 +338,9 @@ class WHVIClassification(WHVINetwork):
         samples.  The network runs ``chunk_samples`` samples at a time (default 16) and the ``whvi_categorical_predictive``
         kernel continues the sums chunk after chunk in sample order, so the (S, batch, K) logits never exist at once and the
         result does not depend on the chunking."""
-        S = int(n_samples if n_samples is not None else (self.train_samples if self.training else self.eval_samples))
-        chunk = max(1, int(chunk_samples if chunk_samples is not None else 16))
+        S, chunks = self._sample_chunks(X, n_samples, chunk_samples)
         prob_sum = loglik_sum = None
-        for s0 in range(0, S, chunk):
-            logits = self._run(X, min(chunk, S - s0))
+        for s0, logits in chunks:
             if prob_sum is None:
                 prob_sum = torch.empty(logits.shape[1:], dtype=torch.float32, device=logits.device)
                 loglik_sum = None if y is None else torch.empty(logits.shape[1], dtype=torch.float32, device=logits.device)
@@ -330,6 +348,58 @@ class WHVIClassification(WHVINetwork):
         if prob_sum is None:
             raise RuntimeError("predictive_prob_sums needs n_samples >= 1")
         return prob_sum, loglik_sum, S
+
+    def _sample_chunks(self, X, n_samples, chunk_samples):
+        """S and a generator of (first sample, (n, batch, K) logits) over chunks of ``chunk_samples`` samples (default 16)."""
+        S = int(n_samples if n_samples is not None else (self.train_samples if self.training else self.eval_samples))
+        chunk = max(1, int(chunk_samples if chunk_samples is not None else 16))
+        return S, ((s0, self._run(X, min(chunk, S - s0))) for s0 in range(0, S, chunk))
+
+    @torch.no_grad()
+    def predictive_uncertainty_sums(self, X: torch.Tensor, y: torch.Tensor | None = None, n_samples: int | None = None,
+                                    chunk_samples: int | None = None):
+        """(prob_sum (batch, K), ent_sum (batch,), loglik_sum (batch,) or None, logpred (batch,) or None, S): the sums of
+        ``predictive_prob_sums`` (the same bits) and, from the same kernel pass, sum_s H[softmax(z_s)] and, with ``y``,
+        log sum_s p_s(y) as a running log-sum-exp (``whvi_categorical_uncertainty``), chunk after chunk in sample order."""
+        S, chunks = self._sample_chunks(X, n_samples, chunk_samples)
+        sums = None
+        for s0, logits in chunks:
+            if sums is None:   # prob_sum, then ent_sum, loglik_sum, logpred (the last two only with labels)
+                B, dev = logits.shape[1], logits.device
+                vecs = [torch.empty(B, dtype=torch.float32, device=dev) for _ in range(1 if y is None else 3)]
+                sums = [torch.empty(logits.shape[1:], dtype=torch.float32, device=dev)] + vecs + ([None, None] if y is None else [])
+            WF.categorical_uncertainty_(logits, y, *sums, accumulate=s0 > 0)
+        if sums is None:
+            raise RuntimeError("predictive_uncertainty needs n_samples >= 1")
+        return (*sums, S)
+
+    @torch.no_grad()
+    def predictive_uncertainty(self, X: torch.Tensor, y: torch.Tensor | None = None, n_samples: int | None = None,
+                               chunk_samples: int | None = None) -> CategoricalUncertainty:
+        """Per-input uncertainty of the MC predictive, ``chunk_samples`` samples at a time (default 16), as a
+        ``uncertainty.CategoricalUncertainty``: ``probs`` (what ``predict_proba`` returns), ``predictive_entropy`` H[probs],
+        ``expected_entropy`` (1/S) sum_s H[softmax(z_s)], ``mutual_information`` (their difference, the epistemic part used
+        for out-of-distribution detection and active learning), ``log_predictive`` log (1/S) sum_s p_s(y) with ``y`` (else
+        None; kept as a log-sum-exp, so it stays finite when a confident model is wrong) and ``S``.  The entropies and
+        log_predictive are fp64.  The mutual information is not clamped: when the samples agree, fp32 rounding of the sums can
+        make it negative by about 1e-6 log K.  Runs the network exactly as ``predict_proba`` does, with the same launches."""
+        prob_sum, ent_sum, _, logpred, S = self.predictive_uncertainty_sums(X, y, n_samples, chunk_samples)
+        return categorical_uncertainty(prob_sum, ent_sum, logpred, S)
+
+    @torch.no_grad()
+    def predictive_metrics(self, X: torch.Tensor, y: torch.Tensor, n_samples: int | None = None, chunk_samples: int | None = None,
+                           n_bins: int = 15) -> dict:
+        """Test metrics of the MC predictive from one chunked pass: ``error`` (of the argmax of the mean probabilities), ``nll``
+        (-mean_b log (1/S) sum_s p_s(y_b), the test NLL BNN papers report), ``mnll`` (``eval_model``'s estimator with n = m,
+        -(1/S) sum_{b,s} log p_s(y_b)), ``brier`` (``uncertainty.brier_score``) and ``ece`` (``uncertainty.
+        expected_calibration_error`` with ``n_bins`` equal-width confidence bins).  All in fp64 from the sums."""
+        prob_sum, ent_sum, loglik_sum, logpred, S = self.predictive_uncertainty_sums(X, y, n_samples, chunk_samples)
+        u = categorical_uncertainty(prob_sum, ent_sum, logpred, S)
+        return {"error": float((prob_sum.argmax(dim=1) != y).to(torch.float64).mean()),
+                "nll": float(-u.log_predictive.mean()),
+                "mnll": float(-loglik_sum.to(torch.float64).sum() / S),
+                "brier": brier_score(u.probs, y),
+                "ece": expected_calibration_error(u.probs, y, n_bins)}
 
     @torch.no_grad()
     def predict_proba(self, X: torch.Tensor, n_samples: int | None = None, chunk_samples: int | None = None) -> torch.Tensor:
