@@ -668,7 +668,7 @@ class WHVILayerLossFunction(Function):
             elif ctx.dx_scale_to is not None:
                 ctx.dx_scale_to.put(c.reshape(1))
             else:
-                dx = dx.mul_(c)
+                dx = dx * c   # not in place: dx is a saved tensor, and a retained graph's next backward reads it again
         return dx, dg * c, ds1 * c, ds2 * c, None if dbias is None else dbias * c, None, None, None
 
 
