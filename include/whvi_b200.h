@@ -440,6 +440,15 @@ WHVI_API int whvi_mc_moments_strided_f32(const float* y, int64_t y_sample_stride
  *                                total[0] = sum_r (lse[r] - z[r, y_b]): fp64 per-CTA partials in the workspace, summed in a fixed
  *                                order.  The caller applies the estimator's coefficient n / (m S).
  *   whvi_categorical_nll_bwd_*   dz[r, k] = c[0] (exp(z[r, k] - lse[r]) - [k = y_b]), c a device scalar (NULL = 1), lse the forward's
+ *   whvi_categorical_nll_ex_*    whvi_categorical_nll_* with torch's cross_entropy options (reduction "sum"): class weights
+ *                                weight (K) fp32 (NULL = ones), label smoothing eps in [0, 1] and, with flags &
+ *                                WHVI_CATEGORICAL_IGNORE, ignore_index: total[0] = sum_r l_r,
+ *                                l_r = (1 - eps) w_y (lse[r] - z[r, y_b]) + (eps / K) sum_k w_k (lse[r] - z[r, k]), the smoothing
+ *                                sum in a second pass over the row (every term >= 0); l_r = 0 when y_b == ignore_index (tested
+ *                                before the range, so ignore_index = -100 works).  Same workspace (whvi_categorical_sizes).
+ *   whvi_categorical_nll_bwd_ex_*  dz[r, k] = c[0] ((1 - eps) w_y (p_k - [k = y_b]) + (eps / K) (W p_k - w_k)), p = softmax(z[r]),
+ *                                W = sum_k w_k; an ignored row's dz row is 0.  Both _ex calls: eps not finite or outside [0, 1]
+ *                                WHVI_E_SHAPE, flags other than WHVI_CATEGORICAL_IGNORE WHVI_E_MODE, weight 4-byte aligned.
  *   whvi_categorical_predictive_*  prob_sum[b, k] (+)= sum_s softmax(z[s, b])[k] and, with labels, loglik_sum[b] (+)=
  *                                sum_s log softmax(z[s, b])[y_b]; (B, K) and (B) fp32, s ascending.  Sample s's rows are read at
  *                                logits + s * sample_stride (>= B * K, so a sample chunk may be a slice of a larger tensor);
@@ -460,6 +469,7 @@ WHVI_API int whvi_mc_moments_strided_f32(const float* y, int64_t y_sample_stride
  * (rows need no more: the loads are element-wise); workspace 8 bytes.
  */
 #define WHVI_CATEGORICAL_ACCUMULATE 1
+#define WHVI_CATEGORICAL_IGNORE 2
 WHVI_API int whvi_categorical_sizes(int64_t R, int64_t K, size_t* workspace_bytes);
 WHVI_API int whvi_categorical_nll_f32(const float* logits, const int64_t* labels, float* lse, float* total, void* workspace,
                                       size_t workspace_bytes, int64_t S, int64_t B, int64_t K, whvi_stream_t stream);
@@ -469,6 +479,18 @@ WHVI_API int whvi_categorical_nll_bwd_f32(const float* logits, const int64_t* la
                                           int64_t S, int64_t B, int64_t K, whvi_stream_t stream);
 WHVI_API int whvi_categorical_nll_bwd_bf16(const void* logits, const int64_t* labels, const float* lse, const float* c, void* dz,
                                            int64_t S, int64_t B, int64_t K, whvi_stream_t stream);
+WHVI_API int whvi_categorical_nll_ex_f32(const float* logits, const int64_t* labels, float* lse, float* total, void* workspace,
+                                         size_t workspace_bytes, int64_t S, int64_t B, int64_t K, const float* weight,
+                                         float label_smoothing, int64_t ignore_index, int flags, whvi_stream_t stream);
+WHVI_API int whvi_categorical_nll_ex_bf16(const void* logits, const int64_t* labels, float* lse, float* total, void* workspace,
+                                          size_t workspace_bytes, int64_t S, int64_t B, int64_t K, const float* weight,
+                                          float label_smoothing, int64_t ignore_index, int flags, whvi_stream_t stream);
+WHVI_API int whvi_categorical_nll_bwd_ex_f32(const float* logits, const int64_t* labels, const float* lse, const float* c, float* dz,
+                                             int64_t S, int64_t B, int64_t K, const float* weight, float label_smoothing,
+                                             int64_t ignore_index, int flags, whvi_stream_t stream);
+WHVI_API int whvi_categorical_nll_bwd_ex_bf16(const void* logits, const int64_t* labels, const float* lse, const float* c, void* dz,
+                                              int64_t S, int64_t B, int64_t K, const float* weight, float label_smoothing,
+                                              int64_t ignore_index, int flags, whvi_stream_t stream);
 WHVI_API int whvi_categorical_predictive_f32(const float* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum,
                                              float* loglik_sum, int64_t S, int64_t B, int64_t K, int flags, whvi_stream_t stream);
 WHVI_API int whvi_categorical_predictive_bf16(const void* logits, int64_t sample_stride, const int64_t* labels, float* prob_sum,

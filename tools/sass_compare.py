@@ -15,7 +15,8 @@ parameter added with a default changes the mangled names of the existing instanc
   * ``--strip-false KERNEL`` drops a trailing ``, false`` template argument of KERNEL (a ``bool`` flag added last, whose
     ``false`` instances are the older ones) and keys KERNEL's instances without their parameter list, since the flag came
     with extra trailing parameters that the ``false`` instances never read (default: ``categorical_predictive_kernel``, whose
-    ``true`` instances add the uncertainty sums).
+    ``true`` instances add the uncertainty sums, and ``categorical_nll_kernel`` / ``categorical_nll_bwd_kernel``, whose ``true``
+    instances take class weights, label smoothing and ignore_index).
 Each old instance must have a new instance of the same name whose instructions AND encodings (scheduling control words
 included) are identical, line for line; only the instruction addresses are ignored.  New instances without an old counterpart
 are listed.  Exit status 1 on any difference.
@@ -33,7 +34,7 @@ DEFAULT_STRIP = ("layer_bwd_tma_kernel", "layer_bwd_tm_kernel", "layer_loss_kern
 DEFAULT_STRIP_DUP = ("layer_bwd_tma_kernel", "layer_bwd_tm_kernel")
 DEFAULT_UNTEMPLATE = ("stack_split_kernel", "stack_concat_kernel", "stack_sum_kernel", "column_dot_kernel", "column_outer_kernel",
                       "column_dot_dx_kernel", "column_dw_kernel", "column_outer_dx_kernel", "column_dbias_kernel")
-DEFAULT_STRIP_FALSE = ("categorical_predictive_kernel",)
+DEFAULT_STRIP_FALSE = ("categorical_predictive_kernel", "categorical_nll_kernel", "categorical_nll_bwd_kernel")
 _ADDR = re.compile(r"/\*[0-9a-f]{4,}\*/")
 
 

@@ -133,6 +133,15 @@ SIGNATURES = {
     "whvi_categorical_nll_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64, c_void_p]),
     "whvi_categorical_nll_bwd_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p]),
     "whvi_categorical_nll_bwd_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p]),
+    # the _ex calls: the plain arguments, then weight, label_smoothing (float: stays on ctypes), ignore_index and flags
+    "whvi_categorical_nll_ex_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64,
+                                            c_void_p, c_float, c_int64, c_int, c_void_p]),
+    "whvi_categorical_nll_ex_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int64, c_int64, c_int64,
+                                             c_void_p, c_float, c_int64, c_int, c_void_p]),
+    "whvi_categorical_nll_bwd_ex_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p,
+                                                c_float, c_int64, c_int, c_void_p]),
+    "whvi_categorical_nll_bwd_ex_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p,
+                                                 c_float, c_int64, c_int, c_void_p]),
     "whvi_categorical_predictive_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int,
                                                 c_void_p]),
     "whvi_categorical_predictive_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int,

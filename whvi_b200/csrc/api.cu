@@ -897,8 +897,20 @@ int whvi_categorical_sizes(int64_t R, int64_t K, size_t* workspace_bytes)
     return WHVI_OK;
 }
 
+static constexpr CategoricalOpts kPlainOpts{false, nullptr, 0.f, 0, 0};
+
+// the _ex calls' options, validated before any CUDA call; the plain calls' checks follow
+static int categorical_opts(const char* who, const float* weight, float eps, int64_t ignore_index, int flags, CategoricalOpts* o)
+{
+    if (!(eps >= 0.f && eps <= 1.f)) return fail(WHVI_E_SHAPE, "%s: label_smoothing = %g outside [0, 1]", who, static_cast<double>(eps));
+    if (flags & ~WHVI_CATEGORICAL_IGNORE) return fail(WHVI_E_MODE, "%s: unknown flags %d", who, flags);
+    if (!aligned(weight, 4)) return fail(WHVI_E_ALIGN, "%s: weight must be 4-byte aligned", who);
+    *o = CategoricalOpts{true, weight, eps, ignore_index, (flags & WHVI_CATEGORICAL_IGNORE) ? 1 : 0};
+    return WHVI_OK;
+}
+
 static int categorical_nll(const char* who, const void* logits, size_t elem, const int64_t* labels, float* lse, float* total, void* workspace,
-                           size_t workspace_bytes, int64_t S, int64_t B, int64_t K, whvi_stream_t stream)
+                           size_t workspace_bytes, int64_t S, int64_t B, int64_t K, const CategoricalOpts& o, whvi_stream_t stream)
 {
     if (int rc = check_categorical(who, S, B, K)) return rc;
     if (!total || (S * B > 0 && (!logits || !labels))) return fail(WHVI_E_NULL, "%s: null pointer", who);
@@ -907,42 +919,94 @@ static int categorical_nll(const char* who, const void* logits, size_t elem, con
     const size_t need = categorical_workspace_bytes(S * B, K);
     if (!workspace || workspace_bytes < need || !aligned(workspace, 8))
         return fail(WHVI_E_WORKSPACE, "%s: workspace of %zu bytes (8-byte aligned) needed, %zu given", who, need, workspace_bytes);
-    return launch_categorical_nll(logits, labels, lse, total, workspace, S, B, K, elem == 2, static_cast<cudaStream_t>(stream));
+    return launch_categorical_nll(logits, labels, lse, total, workspace, S, B, K, elem == 2, o, static_cast<cudaStream_t>(stream));
 }
 
 int whvi_categorical_nll_f32(const float* logits, const int64_t* labels, float* lse, float* total, void* workspace, size_t workspace_bytes,
                              int64_t S, int64_t B, int64_t K, whvi_stream_t stream)
 {
-    return categorical_nll("categorical_nll_f32", logits, 4, labels, lse, total, workspace, workspace_bytes, S, B, K, stream);
+    return categorical_nll("categorical_nll_f32", logits, 4, labels, lse, total, workspace, workspace_bytes, S, B, K, kPlainOpts, stream);
 }
 
 int whvi_categorical_nll_bf16(const void* logits, const int64_t* labels, float* lse, float* total, void* workspace, size_t workspace_bytes,
                               int64_t S, int64_t B, int64_t K, whvi_stream_t stream)
 {
-    return categorical_nll("categorical_nll_bf16", logits, 2, labels, lse, total, workspace, workspace_bytes, S, B, K, stream);
+    return categorical_nll("categorical_nll_bf16", logits, 2, labels, lse, total, workspace, workspace_bytes, S, B, K, kPlainOpts, stream);
+}
+
+static int categorical_nll_ex(const char* who, const void* logits, size_t elem, const int64_t* labels, float* lse, float* total,
+                              void* workspace, size_t workspace_bytes, int64_t S, int64_t B, int64_t K, const float* weight, float eps,
+                              int64_t ignore_index, int flags, whvi_stream_t stream)
+{
+    if (int rc = check_categorical(who, S, B, K)) return rc;
+    CategoricalOpts o;
+    if (int rc = categorical_opts(who, weight, eps, ignore_index, flags, &o)) return rc;
+    return categorical_nll(who, logits, elem, labels, lse, total, workspace, workspace_bytes, S, B, K, o, stream);
+}
+
+int whvi_categorical_nll_ex_f32(const float* logits, const int64_t* labels, float* lse, float* total, void* workspace,
+                                size_t workspace_bytes, int64_t S, int64_t B, int64_t K, const float* weight, float label_smoothing,
+                                int64_t ignore_index, int flags, whvi_stream_t stream)
+{
+    return categorical_nll_ex("categorical_nll_ex_f32", logits, 4, labels, lse, total, workspace, workspace_bytes, S, B, K, weight,
+                              label_smoothing, ignore_index, flags, stream);
+}
+
+int whvi_categorical_nll_ex_bf16(const void* logits, const int64_t* labels, float* lse, float* total, void* workspace,
+                                 size_t workspace_bytes, int64_t S, int64_t B, int64_t K, const float* weight, float label_smoothing,
+                                 int64_t ignore_index, int flags, whvi_stream_t stream)
+{
+    return categorical_nll_ex("categorical_nll_ex_bf16", logits, 2, labels, lse, total, workspace, workspace_bytes, S, B, K, weight,
+                              label_smoothing, ignore_index, flags, stream);
 }
 
 static int categorical_nll_bwd(const char* who, const void* logits, size_t elem, const int64_t* labels, const float* lse, const float* c,
-                               void* dz, int64_t S, int64_t B, int64_t K, whvi_stream_t stream)
+                               void* dz, int64_t S, int64_t B, int64_t K, const CategoricalOpts& o, whvi_stream_t stream)
 {
     if (int rc = check_categorical(who, S, B, K)) return rc;
     if (S * B == 0) return WHVI_OK;
     if (!logits || !labels || !lse || !dz) return fail(WHVI_E_NULL, "%s: null pointer", who);
     if (!aligned(logits, elem) || !aligned(dz, elem) || !aligned(labels, 8) || !aligned(lse, 4) || !aligned(c, 4))
         return fail(WHVI_E_ALIGN, "%s: logits, dz, labels, lse and c must be aligned to their element size", who);
-    return launch_categorical_nll_bwd(logits, labels, lse, c, dz, S, B, K, elem == 2, static_cast<cudaStream_t>(stream));
+    return launch_categorical_nll_bwd(logits, labels, lse, c, dz, S, B, K, elem == 2, o, static_cast<cudaStream_t>(stream));
 }
 
 int whvi_categorical_nll_bwd_f32(const float* logits, const int64_t* labels, const float* lse, const float* c, float* dz, int64_t S,
                                  int64_t B, int64_t K, whvi_stream_t stream)
 {
-    return categorical_nll_bwd("categorical_nll_bwd_f32", logits, 4, labels, lse, c, dz, S, B, K, stream);
+    return categorical_nll_bwd("categorical_nll_bwd_f32", logits, 4, labels, lse, c, dz, S, B, K, kPlainOpts, stream);
 }
 
 int whvi_categorical_nll_bwd_bf16(const void* logits, const int64_t* labels, const float* lse, const float* c, void* dz, int64_t S,
                                   int64_t B, int64_t K, whvi_stream_t stream)
 {
-    return categorical_nll_bwd("categorical_nll_bwd_bf16", logits, 2, labels, lse, c, dz, S, B, K, stream);
+    return categorical_nll_bwd("categorical_nll_bwd_bf16", logits, 2, labels, lse, c, dz, S, B, K, kPlainOpts, stream);
+}
+
+static int categorical_nll_bwd_ex(const char* who, const void* logits, size_t elem, const int64_t* labels, const float* lse, const float* c,
+                                  void* dz, int64_t S, int64_t B, int64_t K, const float* weight, float eps, int64_t ignore_index,
+                                  int flags, whvi_stream_t stream)
+{
+    if (int rc = check_categorical(who, S, B, K)) return rc;
+    CategoricalOpts o;
+    if (int rc = categorical_opts(who, weight, eps, ignore_index, flags, &o)) return rc;
+    return categorical_nll_bwd(who, logits, elem, labels, lse, c, dz, S, B, K, o, stream);
+}
+
+int whvi_categorical_nll_bwd_ex_f32(const float* logits, const int64_t* labels, const float* lse, const float* c, float* dz, int64_t S,
+                                    int64_t B, int64_t K, const float* weight, float label_smoothing, int64_t ignore_index, int flags,
+                                    whvi_stream_t stream)
+{
+    return categorical_nll_bwd_ex("categorical_nll_bwd_ex_f32", logits, 4, labels, lse, c, dz, S, B, K, weight, label_smoothing,
+                                  ignore_index, flags, stream);
+}
+
+int whvi_categorical_nll_bwd_ex_bf16(const void* logits, const int64_t* labels, const float* lse, const float* c, void* dz, int64_t S,
+                                     int64_t B, int64_t K, const float* weight, float label_smoothing, int64_t ignore_index, int flags,
+                                     whvi_stream_t stream)
+{
+    return categorical_nll_bwd_ex("categorical_nll_bwd_ex_bf16", logits, 2, labels, lse, c, dz, S, B, K, weight, label_smoothing,
+                                  ignore_index, flags, stream);
 }
 
 // unc: the uncertainty call, which also takes logpred (with labels and loglik_sum) and ent_sum (required, like prob_sum)

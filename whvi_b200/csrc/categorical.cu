@@ -2,6 +2,12 @@
 //   categorical_nll          lse_r = log sum_k exp(z_rk) (max-subtracted, online), loss_r = lse_r - z_{r, y_b},
 //                            total = sum_r loss_r: fp64 per-CTA partials, then one CTA sums them in a fixed order
 //   categorical_nll_bwd      dz_rk = c (exp(z_rk - lse_r) - [k = y_b]),  c a device scalar
+//     <OPT = true> (class weights w, label smoothing eps, ignore_index; torch's cross_entropy(..., reduction="sum")):
+//                            loss_r = (1 - eps) w_y (lse_r - z_ry) + (eps / K) sum_k w_k (lse_r - z_rk), the smoothing sum in a
+//                            second pass over the row once lse_r is known (every term >= 0: no W lse - sum w z cancellation);
+//                            dz_rk = c [(1 - eps) w_y (p_k - [k = y]) + (eps / K) (W p_k - w_k)],  W = sum_k w_k reduced once per
+//                            CTA before the row loop.  An ignored row (y_b == ignore_index, tested before the range) gives 0 and
+//                            a zero dz row; w = NULL is all ones
 //   categorical_predictive   prob_sum[b, :] (+)= sum_s softmax(z_{s,b}),  loglik_sum[b] (+)= sum_s log p_s(y_b),  s ascending
 //     <UNC = true> also      ent_sum[b] (+)= sum_s H_s,  H_s = sum_k p_k (lse - z_k)  (every term >= 0; p_k = 0 adds nothing),
 //                            logpred[b] = logaddexp over s of log p_s(y_b), continued from the stored value with accumulate
@@ -83,8 +89,9 @@ __device__ __forceinline__ float row_lse(const T* row, int K, int lane, bool val
 }
 
 // sum of v over the group in every thread, in a fixed order (butterfly, then for a CTA the warps ascending).  Same calling
-// rules as row_lse: every lane of the warp takes part, and TPR == kThreads synchronises the CTA.
-template <int TPR>
+// rules as row_lse: every lane of the warp takes part, and TPR == kThreads synchronises the CTA.  SLOT names the warps[] array:
+// the OPT instances use slot 1, because sharing the array with them changed the register allocation of the UNC kernels.
+template <int TPR, int SLOT = 0>
 __device__ __forceinline__ float group_sum(float v)
 {
     constexpr int width = TPR < 32 ? TPR : 32;
@@ -111,10 +118,14 @@ __device__ __forceinline__ float logaddexp(float a, float b)
     return m + log1pf(expf(fminf(a, b) - m));
 }
 
-template <int TPR, typename T>
+// weight of class k (w = NULL: 1)
+__device__ __forceinline__ float wk(const float* w, int64_t k) { return w ? __ldg(w + k) : 1.f; }
+
+template <int TPR, typename T, bool OPT>
 __global__ void __launch_bounds__(kThreads)
 categorical_nll_kernel(const T* __restrict__ z, const int64_t* __restrict__ labels, float* __restrict__ lse_out,
-                       double* __restrict__ partials, int64_t R, int64_t B, int K)
+                       double* __restrict__ partials, int64_t R, int64_t B, int K, const float* __restrict__ w, float eps,
+                       int64_t ignore_index, int ignore)
 {
     constexpr int G = kThreads / TPR;
     const int g = threadIdx.x / TPR, lane = threadIdx.x % TPR;
@@ -125,6 +136,26 @@ categorical_nll_kernel(const T* __restrict__ z, const int64_t* __restrict__ labe
         const bool valid = r < R;
         const T* row = z + (valid ? r : 0) * int64_t(K);
         const float lse = row_lse<TPR>(row, K, lane, valid);
+        if constexpr (OPT) {
+            const int64_t y = valid ? labels[r % B] : 0;
+            const bool skip = !valid || (ignore && y == ignore_index);
+            const bool ok = y >= 0 && y < K;
+            float sm = 0.f;   // this lane's share of sum_k w_k (lse - z_k); eps is grid-uniform, so is the group sum's call
+            if (eps != 0.f) {
+                if (!skip && ok) {
+#pragma unroll 4
+                    for (int k = lane; k < K; k += TPR) sm += wk(w, k) * (lse - ldz(row, k));
+                }
+                sm = group_sum<TPR, 1>(sm);
+            }
+            if (valid && lane == 0) {
+                float loss = 0.f;
+                if (!skip) loss = ok ? (1.f - eps) * wk(w, y) * (lse - ldz(row, y)) + (eps / K) * sm : qnan();
+                if (lse_out) lse_out[r] = lse;
+                acc += static_cast<double>(loss);
+            }
+            continue;
+        }
         if (valid && lane == 0) {
             const int64_t y = labels[r % B];
             const float loss = (y >= 0 && y < K) ? lse - ldz(row, y) : qnan();
@@ -156,22 +187,55 @@ __global__ void __launch_bounds__(kThreads) categorical_total_kernel(const doubl
     if (threadIdx.x == 0) total[0] = static_cast<float>(red[0]);
 }
 
-template <int TPR, typename T>
+template <int TPR, typename T, bool OPT>
 __global__ void __launch_bounds__(kThreads)
 categorical_nll_bwd_kernel(const T* __restrict__ z, const int64_t* __restrict__ labels, const float* __restrict__ lse,
-                           const float* __restrict__ coef, T* __restrict__ dz, int64_t R, int64_t B, int K)
+                           const float* __restrict__ coef, T* __restrict__ dz, int64_t R, int64_t B, int K,
+                           const float* __restrict__ w, float eps, int64_t ignore_index, int ignore)
 {
     constexpr int G = kThreads / TPR;
     const int g = threadIdx.x / TPR, lane = threadIdx.x % TPR;
     const float c = coef ? __ldg(coef) : 1.f;
+    float W = static_cast<float>(K);
+    if constexpr (OPT) {
+        // W = sum_k w_k over the whole CTA before any row (no sync in the row loop), in a fixed order; 8 independent partial
+        // sums per thread keep 8 loads in flight instead of one dependent chain.  W only enters through eps (grid-uniform)
+        if (w && eps != 0.f) {
+            float part[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+            for (int k = threadIdx.x; k < K; k += 8 * kThreads) {
+#pragma unroll
+                for (int j = 0; j < 8; ++j)
+                    if (k + j * kThreads < K) part[j] += __ldg(w + k + j * kThreads);
+            }
+            W = group_sum<kThreads, 1>(((part[0] + part[1]) + (part[2] + part[3])) + ((part[4] + part[5]) + (part[6] + part[7])));
+        }
+    }
     const int64_t blocks = (R + G - 1) / G;
     for (int64_t blk = blockIdx.x; blk < blocks; blk += gridDim.x) {
         const int64_t r = blk * G + g;
         if (r >= R) continue;
         const int64_t y = labels[r % B];
         const bool ok = y >= 0 && y < K;
-        const float l = lse[r];
         const int64_t base = r * int64_t(K);
+        if constexpr (OPT) {
+            // rows without a gradient leave the element loop: a per-element `ok ? .. : NaN` became a branch around each
+            // element's loads there, and the loop lost its batched loads (half the bandwidth at K = 65536)
+            const bool ignored = ignore && y == ignore_index;
+            if (ignored || !ok) {
+                const float v = ignored ? 0.f : qnan();
+                for (int k = lane; k < K; k += TPR) stz(dz, base + k, v);
+                continue;
+            }
+            const float l = lse[r];
+            const float a = c * (1.f - eps) * wk(w, y), e = c * (eps / K), eW = e * W;
+#pragma unroll 4
+            for (int k = lane; k < K; k += TPR) {
+                const float p = expf(ldz(z, base + k) - l);
+                stz(dz, base + k, a * (p - (k == y ? 1.f : 0.f)) + (eW * p - e * wk(w, k)));
+            }
+            continue;
+        }
+        const float l = lse[r];
 #pragma unroll 4
         for (int k = lane; k < K; k += TPR) {
             const float v = ok ? c * (expf(ldz(z, base + k) - l) - (k == y ? 1.f : 0.f)) : qnan();
@@ -283,15 +347,19 @@ void with_tpr(int tpr, F&& f)
     }
 }
 
+// o.on selects the OPT instances (the _ex calls); the plain calls pass on = false and run the OPT = false instances
 template <typename T>
-int nll_t(const void* z, const int64_t* labels, float* lse, float* total, void* ws, int64_t S, int64_t B, int64_t K, cudaStream_t st)
+int nll_t(const void* z, const int64_t* labels, float* lse, float* total, void* ws, int64_t S, int64_t B, int64_t K, const CategoricalOpts& o,
+          cudaStream_t st)
 {
     const int64_t R = S * B;
     const Plan p = plan(R, K);
     double* partials = static_cast<double*>(ws);
     with_tpr(p.tpr, [&](auto tpr) {
-        categorical_nll_kernel<decltype(tpr)::value, T><<<static_cast<unsigned>(p.ctas), kThreads, 0, st>>>(
-            static_cast<const T*>(z), labels, lse, partials, R, B, static_cast<int>(K));
+        constexpr int TPR = decltype(tpr)::value;
+        auto kernel = o.on ? categorical_nll_kernel<TPR, T, true> : categorical_nll_kernel<TPR, T, false>;
+        kernel<<<static_cast<unsigned>(p.ctas), kThreads, 0, st>>>(static_cast<const T*>(z), labels, lse, partials, R, B, static_cast<int>(K),
+                                                                   o.weight, o.eps, o.ignore_index, o.ignore);
     });
     if (int rc = check_launch("categorical_nll_kernel")) return rc;
     categorical_total_kernel<<<1, kThreads, 0, st>>>(partials, p.ctas, total);
@@ -300,14 +368,16 @@ int nll_t(const void* z, const int64_t* labels, float* lse, float* total, void* 
 
 template <typename T>
 int nll_bwd_t(const void* z, const int64_t* labels, const float* lse, const float* c, void* dz, int64_t S, int64_t B, int64_t K,
-              cudaStream_t st)
+              const CategoricalOpts& o, cudaStream_t st)
 {
     const int64_t R = S * B;
     if (R == 0) return WHVI_OK;
     const Plan p = plan(R, K);
     with_tpr(p.tpr, [&](auto tpr) {
-        categorical_nll_bwd_kernel<decltype(tpr)::value, T><<<static_cast<unsigned>(p.ctas), kThreads, 0, st>>>(
-            static_cast<const T*>(z), labels, lse, c, static_cast<T*>(dz), R, B, static_cast<int>(K));
+        constexpr int TPR = decltype(tpr)::value;
+        auto kernel = o.on ? categorical_nll_bwd_kernel<TPR, T, true> : categorical_nll_bwd_kernel<TPR, T, false>;
+        kernel<<<static_cast<unsigned>(p.ctas), kThreads, 0, st>>>(static_cast<const T*>(z), labels, lse, c, static_cast<T*>(dz), R, B,
+                                                                   static_cast<int>(K), o.weight, o.eps, o.ignore_index, o.ignore);
     });
     return check_launch("categorical_nll_bwd_kernel");
 }
@@ -333,15 +403,16 @@ int predictive_t(const void* z, int64_t sample_stride, const int64_t* labels, fl
 size_t categorical_workspace_bytes(int64_t R, int64_t K) { return sizeof(double) * static_cast<size_t>(plan(R, K).ctas); }
 
 int launch_categorical_nll(const void* z, const int64_t* labels, float* lse, float* total, void* ws, int64_t S, int64_t B, int64_t K,
-                           int bf16, cudaStream_t st)
+                           int bf16, const CategoricalOpts& o, cudaStream_t st)
 {
-    return bf16 ? nll_t<__nv_bfloat16>(z, labels, lse, total, ws, S, B, K, st) : nll_t<float>(z, labels, lse, total, ws, S, B, K, st);
+    return bf16 ? nll_t<__nv_bfloat16>(z, labels, lse, total, ws, S, B, K, o, st) : nll_t<float>(z, labels, lse, total, ws, S, B, K, o, st);
 }
 
 int launch_categorical_nll_bwd(const void* z, const int64_t* labels, const float* lse, const float* c, void* dz, int64_t S, int64_t B,
-                               int64_t K, int bf16, cudaStream_t st)
+                               int64_t K, int bf16, const CategoricalOpts& o, cudaStream_t st)
 {
-    return bf16 ? nll_bwd_t<__nv_bfloat16>(z, labels, lse, c, dz, S, B, K, st) : nll_bwd_t<float>(z, labels, lse, c, dz, S, B, K, st);
+    return bf16 ? nll_bwd_t<__nv_bfloat16>(z, labels, lse, c, dz, S, B, K, o, st)
+                : nll_bwd_t<float>(z, labels, lse, c, dz, S, B, K, o, st);
 }
 
 int launch_categorical_predictive(const void* z, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,

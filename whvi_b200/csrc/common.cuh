@@ -143,10 +143,18 @@ int launch_kl(const float* mu, const float* rho, float lambda_, int64_t D, int m
               float grad_scale, int accumulate, cudaStream_t stream, int64_t groups = 1, int64_t pstride = 0);
 // categorical likelihood (categorical.cu); bf16 != 0: the logits and dz are bf16 behind the void pointers
 size_t categorical_workspace_bytes(int64_t R, int64_t K);
+// the _ex calls' options: on = false runs the plain instances (weight NULL, eps 0, no ignore_index)
+struct CategoricalOpts {
+    bool on;
+    const float* weight;   // (K) or NULL for ones
+    float eps;             // label smoothing in [0, 1]
+    int64_t ignore_index;
+    int ignore;            // rows with y_b == ignore_index add 0 and get a zero dz row
+};
 int launch_categorical_nll(const void* z, const int64_t* labels, float* lse, float* total, void* ws, int64_t S, int64_t B, int64_t K,
-                           int bf16, cudaStream_t st);
+                           int bf16, const CategoricalOpts& o, cudaStream_t st);
 int launch_categorical_nll_bwd(const void* z, const int64_t* labels, const float* lse, const float* c, void* dz, int64_t S, int64_t B,
-                               int64_t K, int bf16, cudaStream_t st);
+                               int64_t K, int bf16, const CategoricalOpts& o, cudaStream_t st);
 // ent_sum != NULL: the uncertainty sums as well (logpred with the labels, else NULL)
 int launch_categorical_predictive(const void* z, int64_t sample_stride, const int64_t* labels, float* prob_sum, float* loglik_sum,
                                   float* logpred, float* ent_sum, int64_t S, int64_t B, int64_t K, int accumulate, int bf16,

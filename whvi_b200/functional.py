@@ -1258,17 +1258,43 @@ def _categorical_args(logits, labels):
     return logits.contiguous(), labels.contiguous(), S, B, K
 
 
+CATEGORICAL_IGNORE = 2   # WHVI_CATEGORICAL_IGNORE
+# the _ex calls launch what the plain calls do: the row kernel (+ the fixed-order total) with its options instance
+_LAUNCHES_PER_CALL.update({"whvi_categorical_nll_ex_f32": 2, "whvi_categorical_nll_ex_bf16": 2, "whvi_categorical_nll_bwd_ex_f32": 1,
+                           "whvi_categorical_nll_bwd_ex_bf16": 1})
+
+
+def _categorical_opts(logits, weight, label_smoothing, ignore_index):
+    """The _ex calls' trailing arguments (weight pointer or None, label_smoothing, ignore_index, flags), or None when every option
+    is at its default (the plain calls).  Shapes and devices are checked here; nothing reads the weights or labels."""
+    if weight is None and label_smoothing == 0.0 and ignore_index is None:
+        return None
+    K = logits.size(-1)
+    if weight is not None and (weight.dim() != 1 or weight.numel() != K or weight.dtype != torch.float32
+                               or weight.device != logits.device or not weight.is_contiguous()):
+        raise RuntimeError(f"weight must be a contiguous float32 ({K},) tensor on {logits.device}")
+    if not 0.0 <= float(label_smoothing) <= 1.0:
+        raise RuntimeError(f"label_smoothing must be in [0, 1] (got {label_smoothing})")
+    return (_ptr(weight), float(label_smoothing), 0 if ignore_index is None else int(ignore_index),
+            0 if ignore_index is None else CATEGORICAL_IGNORE)
+
+
 class CategoricalNLLFunction(Function):
     """sum_{s,b} -log softmax(z[s, b])[y_b] for (S, B, K) logits (fp32 or bf16) and (B,) int64 labels, as a 0-d fp32 tensor
     (``whvi_categorical_nll_*``: max-subtracted log-sum-exp per row, fixed-order fp64 reduction).  The backward is
     ``whvi_categorical_nll_bwd_*`` with the incoming gradient read from the device (no sync, graph-capturable); dz has the
-    logits' dtype."""
+    logits' dtype.
+
+    With ``weight`` (K,) fp32, ``label_smoothing`` in [0, 1] or ``ignore_index`` (an int, or None for none) the sum is
+    ``F.cross_entropy(z, y, weight, ignore_index=..., label_smoothing=..., reduction="sum")`` over the rows instead, from the
+    ``whvi_categorical_nll_ex_*`` / ``nll_bwd_ex_*`` calls; at their defaults the plain calls run, with the same launches."""
 
     @staticmethod
-    def forward(ctx, logits, labels):
+    def forward(ctx, logits, labels, weight=None, label_smoothing=0.0, ignore_index=None):
         logits, labels, S, B, K = _categorical_args(logits, labels)
+        opts = _categorical_opts(logits, weight, label_smoothing, ignore_index)
         bf16 = logits.dtype == torch.bfloat16
-        name = "whvi_categorical_nll_bf16" if bf16 else "whvi_categorical_nll_f32"
+        name = f"whvi_categorical_nll{'' if opts is None else '_ex'}_{'bf16' if bf16 else 'f32'}"
         dev = logits.device
         want_grad = ctx.needs_input_grad[0]
         lse = torch.empty((S, B), dtype=torch.float32, device=dev) if want_grad else None
@@ -1277,28 +1303,32 @@ class CategoricalNLLFunction(Function):
             ws = _workspace(dev, _query("whvi_categorical_sizes", S * B, K)[0])
             with _Timed(name, f"K={K}"):
                 rc = getattr(_lib.lib(), name)(logits.data_ptr(), labels.data_ptr(), _ptr(lse), total.data_ptr(), ws.data_ptr(), ws.numel(),
-                                               S, B, K, _stream(dev))
+                                               S, B, K, *(opts or ()), _stream(dev))
         _lib.check(rc, name)
         if want_grad:
-            ctx.save_for_backward(logits, labels, lse)
+            ctx.save_for_backward(logits, labels, lse, weight)
+            ctx.opts = opts
         return total.reshape(())
 
     @staticmethod
     def backward(ctx, d_total):
-        logits, labels, lse = ctx.saved_tensors
+        logits, labels, lse, _weight = ctx.saved_tensors   # the weight is saved so that it outlives the graph
         S, B, K = logits.shape
         c = _f32c(d_total, "grad_output").reshape(1)
         dz = torch.empty_like(logits)
-        name = "whvi_categorical_nll_bwd_bf16" if logits.dtype == torch.bfloat16 else "whvi_categorical_nll_bwd_f32"
+        opts = ctx.opts
+        name = f"whvi_categorical_nll_bwd{'' if opts is None else '_ex'}_{'bf16' if logits.dtype == torch.bfloat16 else 'f32'}"
         with torch.cuda.device(logits.device), _Timed(name, f"K={K}"):
             rc = getattr(_lib.lib(), name)(logits.data_ptr(), labels.data_ptr(), lse.data_ptr(), c.data_ptr(), dz.data_ptr(), S, B, K,
-                                           _stream(logits.device))
+                                           *(opts or ()), _stream(logits.device))
         _lib.check(rc, name)
-        return dz, None
+        return dz, None, None, None, None
 
 
-def categorical_nll(logits, labels):
-    return CategoricalNLLFunction.apply(logits, labels)
+def categorical_nll(logits, labels, weight=None, label_smoothing=0.0, ignore_index=None):
+    """``CategoricalNLLFunction``: the summed softmax cross-entropy of (S, B, K) logits against (B,) labels, with torch's
+    ``cross_entropy`` options (``reduction="sum"``) when any is given."""
+    return CategoricalNLLFunction.apply(logits, labels, weight, label_smoothing, ignore_index)
 
 
 def categorical_predictive_(logits, labels, prob_sum, loglik_sum=None, accumulate=False):

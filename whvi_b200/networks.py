@@ -326,10 +326,15 @@ class WHVIRegression(WHVINetwork):
 
 
 class WHVIClassification(WHVINetwork):
-    def __init__(self, modules: Iterable[nn.Module], **kwargs):
+    def __init__(self, modules: Iterable[nn.Module], *, weight=None, label_smoothing: float = 0.0, ignore_index: int | None = None,
+                 **kwargs):
         """WHVI network for classification: the last module's K outputs are the logits of a softmax likelihood
-        (``CategoricalLikelihood``); targets are (batch,) int64 class labels on the GPU."""
-        super().__init__(modules, likelihood=CategoricalLikelihood(), **kwargs)
+        (``CategoricalLikelihood``); targets are (batch,) int64 class labels on the GPU.  ``weight``, ``label_smoothing`` and
+        ``ignore_index`` are ``torch.nn.functional.cross_entropy``'s options and go to the likelihood: they shape the training
+        loss (``loss``, ``train_model``).  Evaluation (``eval_model``, ``predictive_metrics``) leaves out the rows labelled
+        ``ignore_index`` but reports the plain, unweighted and unsmoothed predictive likelihood, the test NLL BNN papers
+        report."""
+        super().__init__(modules, likelihood=CategoricalLikelihood(weight, label_smoothing, ignore_index), **kwargs)
 
     @torch.no_grad()
     def predictive_prob_sums(self, X: torch.Tensor, y: torch.Tensor | None = None, n_samples: int | None = None,
@@ -392,8 +397,12 @@ class WHVIClassification(WHVINetwork):
         """Test metrics of the MC predictive from one chunked pass: ``error`` (of the argmax of the mean probabilities), ``nll``
         (-mean_b log (1/S) sum_s p_s(y_b), the test NLL BNN papers report), ``mnll`` (``eval_model``'s estimator with n = m,
         -(1/S) sum_{b,s} log p_s(y_b)), ``brier`` (``uncertainty.brier_score``) and ``ece`` (``uncertainty.
-        expected_calibration_error`` with ``n_bins`` equal-width confidence bins).  All in fp64 from the sums."""
+        expected_calibration_error`` with ``n_bins`` equal-width confidence bins).  All in fp64 from the sums.  With the
+        likelihood's ``ignore_index``, over the rows not labelled with it; never weighted or smoothed."""
         prob_sum, ent_sum, loglik_sum, logpred, S = self.predictive_uncertainty_sums(X, y, n_samples, chunk_samples)
+        keep = self.likelihood.labelled(y)
+        if keep is not None:   # every metric over the labelled rows only (an O(B) mask on the sums)
+            prob_sum, ent_sum, loglik_sum, logpred, y = prob_sum[keep], ent_sum[keep], loglik_sum[keep], logpred[keep], y[keep]
         u = categorical_uncertainty(prob_sum, ent_sum, logpred, S)
         return {"error": float((prob_sum.argmax(dim=1) != y).to(torch.float64).mean()),
                 "nll": float(-u.log_predictive.mean()),
@@ -410,11 +419,24 @@ class WHVIClassification(WHVINetwork):
     def eval_model(self, X_test: torch.Tensor, y_test: torch.Tensor, loss=None) -> Tuple[float, float]:
         """Error rate of the MC-mean prediction and test MNLL (the training estimator with n = m).  Both come from the
         chunked predictive sums; a user-supplied ``loss(y_pred, y_true)`` gets the (batch, K, S) logits of ``forward()``
-        instead, as in ``WHVINetwork.eval_model``."""
+        instead, as in ``WHVINetwork.eval_model``.  With the likelihood's options, both are over the rows not labelled
+        ``ignore_index`` (m is their number) and the MNLL is the plain one: class weights and label smoothing shape training
+        only."""
         self.eval()
-        if loss is not None:
+        lik = self.likelihood
+        plain = lik.weight is None and lik.label_smoothing == 0.0 and lik.ignore_index is None
+        if loss is not None and plain:
             return super().eval_model(X_test, y_test, loss)
+        if loss is not None:
+            y_pred = self(X_test)
+            keep = lik.labelled(y_test)
+            logits, y = (y_pred, y_test) if keep is None else (y_pred[keep], y_test[keep])
+            mnll = WF.categorical_nll(logits.permute(2, 0, 1), y) / logits.size(2)
+            return float(loss(y_pred, y_test)), float(mnll)
         prob_sum, loglik_sum, S = self.predictive_prob_sums(X_test, y_test)
+        keep = lik.labelled(y_test)
+        if keep is not None:
+            prob_sum, loglik_sum, y_test = prob_sum[keep], loglik_sum[keep], y_test[keep]
         error = (prob_sum.argmax(dim=1) != y_test).to(torch.float64).mean()
         mnll = -loglik_sum.to(torch.float64).sum() / S   # n / (m S) * sum_{b,s} -log p with n = m
         return float(error), float(mnll)
