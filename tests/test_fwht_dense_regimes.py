@@ -536,8 +536,6 @@ KERNEL_TESTS = {
         "reparam_dense_small_kernel", "reparam_dense_small_bwd_kernel", "dense_transpose_pad_kernel", "dense_colsum_kernel",
         "kl_dense_grouped_rows_kernel", "kl_dense_grouped_final_kernel", "mc_moments_kernel")},
 }
-# layer_fwd_split.cu's kernel is dispatched only in a build with -DWHVI_FWD_SPLIT_8192=1
-CENSUS_EXCLUDED = {"layer_fwd_split.cu"}
 
 
 def kernel_census():
@@ -545,8 +543,6 @@ def kernel_census():
     __launch_bounds__(...) with nested parentheses skipped)."""
     names = set()
     for path in sorted(CSRC.glob("*.cu")) + sorted(CSRC.glob("*.cuh")):
-        if path.name in CENSUS_EXCLUDED:
-            continue
         src = re.sub(r"//[^\n]*|/\*.*?\*/", "", path.read_text(), flags=re.S)
         for m in re.finditer(r"__global__\s+void\s+", src):
             i = m.end()

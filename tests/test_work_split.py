@@ -54,24 +54,24 @@ def make_plan_waves(S, tiles_per_sample, groups, slots, min_iters, max_waves):
 
 # ------------------------------------------------------------------------------------------------- launch tables
 # Each entry: k = log2 D -> (tile bits N, groups or pairs per CTA, extra).
-# Forward, launch_layer_fwd (layer_fwd.cu:256-282): extra = min_iters of make_plan(S, tiles, GROUPS, 148 * 16, min_iters),
-# 4 for the two-view kernels (ROUNDS == 2), 2 for the three-view ones (layer_fwd.cu:221).
+# Forward, launch_layer_fwd (layer_fwd.cu:265-288): extra = min_iters of make_plan(S, tiles, GROUPS, 148 * 16, min_iters),
+# 4 for the two-view kernels (ROUNDS == 2), 2 for the three-view ones (layer_fwd.cu:230).
 FWD = {**{k: (10, 4, 2) for k in range(2, 7)},     # three views
        **{k: (10, 8, 4) for k in range(7, 11)},    # two views, one warp per 1024-float tile
        11: (12, 2, 4), 12: (12, 2, 4),             # two views, 64 floats per thread
        13: (13, 1, 2), 14: (14, 1, 2), 15: (15, 1, 2)}
 FWD_TARGET_CTAS = SMS * 16
 
-# Backward, launch_layer_bwd (layer_bwd.cu:1131-1157), the tensor-memory kernels of the default build:
+# Backward, launch_layer_bwd (layer_bwd.cu:1036-1050):
 # layer_bwd_tma_kernel N = 10 with 4 pairs for k <= 10; layer_bwd_tm_kernel with N = 12 and 128 / 64 = 2 pairs for
 # k = 11, 12, and N = 13 with 128 / 128 = 1 pair for k = 13 (launch_bwd_tm_cfg: PAIRS = 128 / T, T = 2^(N - 6)).
-# Both plan with make_plan_waves(S, tiles, PAIRS, 148, 8, 8) (layer_bwd.cu:1044, 1093).  extra = None.
+# Both plan with make_plan_waves(S, tiles, PAIRS, 148, 8, 8) (layer_bwd.cu:953, 1000).  extra = None.
 BWD = {**{k: (10, 4, None) for k in range(2, 11)}, 11: (12, 2, None), 12: (12, 2, None), 13: (13, 1, None)}
 
-# Loss layer, launch_layer_loss (layer_loss.cu:379-406) and launch_layer_loss_tm (layer_loss_tm.cu:390-396): extra = the
+# Loss layer, launch_layer_loss (layer_loss.cu:367-392) and launch_layer_loss_tm (layer_loss_tm.cu:390-396): extra = the
 # squared-error partials per slab, T / 32 with T = 2^(N - C) threads per role.  layer_loss.cu runs for k = 7..10 always and
 # for k = 11, 12 with a bias; without a bias k = 11, 12 run the tensor-memory kernel.  Both plan with make_plan_waves(S,
-# tiles, PAIRS, 148, 8, 8) (layer_loss.cu:352, layer_loss_tm.cu:367).
+# tiles, PAIRS, 148, 8, 8) (layer_loss.cu:340, layer_loss_tm.cu:367).
 LOSS = {**{k: (10, 4, 1) for k in range(7, 11)},  # N = 10, C = 5: 32 threads per role
         11: (11, 2, 2), 12: (12, 1, 4)}          # N = 11 / 12, C = 5
 LOSS_TM = {11: (12, 2, 2), 12: (12, 2, 2)}       # N = 12, C = 6
@@ -136,7 +136,7 @@ def bwd_workspace_bytes(S, B, D):
 
 def loss_sizes(S, B, D):
     """(workspace bytes, squared-error partials) as whvi_layer_loss_sizes reports them: the larger of the two kernels at
-    k = 11, 12, where the query cannot know whether the call will have a bias (layer_loss.cu:383-398)."""
+    k = 11, 12, where the query cannot know whether the call will have a bias (layer_loss.cu:370-384)."""
     k = _log2(D)
     out = []
     for tm in ([False, True] if k in LOSS_TM else [False]):
@@ -162,7 +162,7 @@ def moments_grid(B, D, reserve_sms=0):
 
 
 def reduce_branches(S, sp, D, groups=1):
-    """launch_bwd_reduce (layer_bwd.cu:1010-1028): (pass A runs, pass A's grid z, pass B's CTA-per-output branch)."""
+    """launch_bwd_reduce (layer_bwd.cu:919-937): (pass A runs, pass A's grid z, pass B's CTA-per-output branch)."""
     direct = D == sp.tile
     return sp.slabs > 1 or direct, min(S, 65535), (S // groups) * (sp.tile // D) >= 1024
 

@@ -95,7 +95,6 @@ int launch_layer_loss(const LayerLossCall& c, int64_t D, cudaStream_t stream);
 int launch_bwd_reduce(float* ws, float* dg, float* ds1, float* ds2, float* dbias, int64_t S, int slabs_per_sample,
                       int64_t tile, int64_t D, cudaStream_t stream, int64_t groups = 1);
 int launch_layer_fwd(const LayerFwdCall& c, int64_t D, cudaStream_t stream);
-int launch_layer_fwd_split(const LayerFwdCall& c, cudaStream_t stream);   // D = 8192 (layer_fwd_split.cu)
 int launch_layer_bwd(const LayerBwdCall& c, int64_t D, cudaStream_t stream);
 int launch_reparam_diag(const float* mu, const float* rho, const float* eps, float* g, int64_t S, int64_t D,
                         cudaStream_t stream, int64_t groups = 1, int64_t pstride = 0);

@@ -1,32 +1,23 @@
 // Kernel (3): the fused WHVILinear backward (see layer_fwd.cu for the math and layout notes).
-// The transposition buffers of THIS translation unit use the padded (XOR-free) layout (WHVI_PADDED_BWD, default 1;
-// measured: the backward gains ~4% at D = 1024...8192 with bit-identical outputs, the two-view forward does not,
-// profiles/r01_bwd_notes.md item 14, profiles/r02_ab_padbwd.txt); -DWHVI_PADDED_BWD=0 builds the swizzled variant.
-#ifndef WHVI_PADDED_BWD
-#define WHVI_PADDED_BWD 1   // product default since round 2: bit-identical outputs, -4% (profiles/r02_ab_padbwd.txt)
-#endif
-#if WHVI_PADDED_BWD && !defined(WHVI_PADDED)
+// The transposition buffers of THIS translation unit use the padded (XOR-free) layout: the backward gains ~4% at
+// D = 1024...8192 over the swizzled one with bit-identical outputs, the two-view forward does not
+// (profiles/r01_bwd_notes.md item 14, profiles/r02_ab_padbwd.txt).
 #define WHVI_PADDED 1
-#endif
-#include <cstdlib>
 #include "layer_common.cuh"
 #include "tmem.cuh"
 
 namespace whvi {
 
 // ------------------------------------------------------------------------------ backward
-// Does the MNLL target tile ride in the TMA stage (RESID kernels)?  One definition for the
-// kernel's shared-memory carve-up and the launcher's size computation.
-// sw = words of one transposition buffer (scratch_words(n, c); == 2^n unless WHVI_PADDED)
-constexpr size_t bwd_smem_bytes(int n, int pairs, int ns, bool single, bool alias, bool gtab, int spt, size_t sw)
+// Shared memory of layer_bwd_tma_kernel: per tile pair, 2 stages of `spt` tiles, a half-stash pair (one tile) and two
+// transposition buffers per role.  Does the MNLL target tile ride in the TMA stage (RESID kernels)?  One definition for
+// the kernel's shared-memory carve-up and the launcher's size computation.
+// sw = words of one transposition buffer (scratch_words(n, c))
+constexpr size_t bwd_smem_bytes(int n, int pairs, int spt, size_t sw)
 {
-    return sizeof(float) * (((size_t(spt) * ns + (alias ? 0 : 1)) * (size_t(1) << n) + (single ? 2 : 4) * sw) * pairs +
-                            (gtab ? sw : 0));
+    return sizeof(float) * ((size_t(spt) * 2 + 1) * (size_t(1) << n) + 4 * sw) * pairs;
 }
-constexpr bool bwd_stage_target(int n, int pairs, int ns, bool single, bool alias, bool gtab, int minb, size_t sw)
-{
-    return bwd_smem_bytes(n, pairs, ns, single, alias, gtab, 3, sw) <= size_t(minb == 2 ? 112 : 200) * 1024;
-}
+constexpr bool bwd_stage_target(int n, int pairs, size_t sw) { return bwd_smem_bytes(n, pairs, 3, sw) <= size_t(200) * 1024; }
 
 struct BwdArgs {
     const float* x;
@@ -47,13 +38,15 @@ struct BwdArgs {
     const float* coef;     // RESID: device scalar
     const float* dy_scale; // optional device scalar: the upstream gradient is dy_scale[0] * dy (deferred
                            // scaling of a producer that computed its dx for a unit loss coefficient)
-    int stagger = 0;       // layer_bwd_tm_kernel: clock cycles by which the CTA's second tile pair starts late
+    int pad = 0;           // not read: keeps spg and pstride at the parameter offsets the kernels were timed with; without
+                           // it ptxas allocates the registers of every backward instance differently (and
+                           // layer_bwd_tm_kernel's RESID instances spill more)
     int spg = 0x7fffffff;  // grouped launch (LayerFwdCall): samples per parameter group
     int pstride = 0;       // floats between consecutive groups' s1 / s2 vectors
 };
 
-// Stream-role specialised, TMA-staged backward.  Every tile is worked on by a PAIR of thread
-// sets running concurrently:
+// Stream-role specialised, TMA-staged backward, D <= 1024.  Every tile is worked on by a PAIR of
+// thread sets running concurrently:
 //   X role:  t2 = H(s2*x) -> t4 = H(g*t2) -> ds1 += dy*t4 (+ dbias += dy)
 //   Y role:  dt3 = H(s1*dy) -> dt1 = H(g*dt3) -> ds2 += dt1*x, dx = s2*dt1
 //   both:    dg += dt3*t2, half of the coordinates each (exchanged through a half-stash)
@@ -74,8 +67,8 @@ struct BwdArgs {
 //   * the dg accumulator is split between the roles (X: float4 slots 0..E/8-1, Y: the rest;
 //     each sends the other the half-stream it needs through a shared half-stash), which
 //     balances the register budgets of the two roles.
-// One CTA per SM (shared memory is the limit), so the spare registers hold this thread's s1/s2/g
-// values across tiles (PREG).  A two-CTA/SM variant with shared-memory accumulators, a two-view
+// One CTA per SM (shared memory is the limit), so the spare registers hold this thread's input-side
+// scaling (X: s2, Y: s1) and g values across tiles.  A two-CTA/SM variant with shared-memory accumulators, a two-view
 // 64-float variant and a single-barrier stash exchange were measured and dropped
 // (profiles/r01_bwd_notes.md, items 5, 8, 10).
 // Shared memory per pair: NS x (x tile + dy tile) + X scratch + Y scratch + stash (1 tile).
@@ -84,35 +77,28 @@ struct BwdArgs {
 // is rounded once at the store.  The workspace, the parameters and all arithmetic stay fp32; RESID is fp32 only.
 // DX: the type dx is stored as (IO by default).  bf16 x and dy with an fp32 dx serve the grouped (Stacked) backward, whose
 // per-block dx are summed in fp32 and rounded once by the caller.
-template <int N, int C, int KT, int PAIRS, int MINB, int NS, bool SINGLE, bool ALIAS, int PREG, int ROUNDS, bool WANT_DBIAS, bool RESID,
-          class IO = float, class DX = IO>
-__global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_kernel(const BwdArgs p)
+template <int N, int C, int KT, bool WANT_DBIAS, bool RESID, class IO = float, class DX = IO>
+__global__ void __launch_bounds__(256, 1) layer_bwd_tma_kernel(const BwdArgs p)
 {
     static_assert(std::is_same_v<IO, float> || !RESID, "RESID (saved output + target) is fp32 only");
     constexpr int T = 1 << (N - C);
     constexpr int E = 1 << C;
     constexpr int H = E / 2;               // floats per thread per half-stream
+    constexpr int PAIRS = 128 / T;
+    constexpr int NS = 2;
     constexpr int64_t TILE = int64_t(1) << N;
-    constexpr int SCR = SINGLE ? 1 : 2;      // scratch tiles per role
+    static_assert(PAIRS * T == 128, "layer_bwd_tma_kernel: 4 warps per role");
+    // Two views: FIRST + MID cover every bit, and the middle of the layer (g multiply, dg products) is
+    // the MID view -- half the transpositions of a three-view form, hence half of the dominant L1/shared wavefronts.
+    static_assert(rounds_needed(N, C, N) <= 2, "2-view kernel needs FIRST+MID to cover all bits");
+    constexpr int SW = int(scratch_words(N, C));  // one transposition buffer
     // RESID: the target tile rides in the stage too (third tile) when shared memory allows
-    // ALIAS (needs ping-pong scratch): the half-stashes live in each role's idle first scratch
-    // buffer instead of a tile of their own (every read of it precedes the barrier that followed
-    // the second buffer's write), which makes room for two CTAs per SM.
-    // ROUNDS == 3: FIRST -> MID -> LAST, the middle of the layer (g multiply, dg products) in the
-    // LAST view.  ROUNDS == 2 (configurations where FIRST + MID cover every bit): the middle is
-    // the MID view -- half the transpositions, hence half of the dominant L1/shared wavefronts.
-    static_assert(ROUNDS == 3 || rounds_needed(N, C, N) <= 2, "2-view kernel needs FIRST+MID to cover all bits");
-    static_assert(rounds_needed(N, C, N) <= 3, "FIRST+MID+LAST must cover every tile bit (e.g. 5+5+3 = 13 bits at C = 5)");
-    constexpr bool GTAB = ROUNDS == 2 && !PREG;  // g in shared memory in MID order (one table per CTA)
-    constexpr int STASH = ALIAS ? 0 : 1;
-    constexpr int SW = int(scratch_words(N, C));  // one transposition buffer (== TILE unless WHVI_PADDED)
-    constexpr bool STAGE_TGT = RESID && bwd_stage_target(N, PAIRS, NS, SINGLE, ALIAS, ROUNDS == 2 && !PREG, MINB, SW);
+    constexpr bool STAGE_TGT = RESID && bwd_stage_target(N, PAIRS, SW);
     constexpr int SPT = STAGE_TGT ? 3 : 2;   // tiles per stage
-    constexpr int PAIR_FLOATS = WHVI_PADDED ? (SPT * NS + STASH) * int(TILE) + 2 * SCR * SW : (SPT * NS + 2 * SCR + STASH) * int(TILE);
+    constexpr int PAIR_FLOATS = (SPT * NS + 1) * int(TILE) + 4 * SW;
     extern __shared__ float4 smem4[];
     __shared__ uint64_t full_bar[PAIRS][NS], empty_bar[PAIRS][NS];
-    float* gt = reinterpret_cast<float*>(smem4);                      // GTAB only
-    float* smem = reinterpret_cast<float*>(smem4) + (ROUNDS == 2 && !PREG ? (WHVI_PADDED ? size_t(SW) : (size_t(1) << N)) : 0);
+    float* smem = reinterpret_cast<float*>(smem4);
     const int k = KT >= 0 ? KT : p.k;
     const uint32_t cmask = (1u << k) - 1u;
     // sample-minor CTA order (see layer_fwd.cu): shared x / target tiles are reused out of L2
@@ -162,18 +148,11 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
     const int pair = (threadIdx.x % (T * PAIRS)) / T;
     const uint32_t tid = threadIdx.x % T;
     float* pair_smem = smem + size_t(pair) * PAIR_FLOATS;
-#if WHVI_PADDED
-    float* scratch = pair_smem + (SPT * NS) * TILE + (SCR * role) * SW;  // this role's transposition buffer(s)
-    float* scratch2 = scratch + (SINGLE ? 0 : SW);
-    float* stash_t2 = ALIAS ? pair_smem + (SPT * NS) * TILE : pair_smem + (SPT * NS) * TILE + 2 * SCR * SW;
-    float* stash_d3 = ALIAS ? pair_smem + (SPT * NS) * TILE + SCR * SW : stash_t2 + TILE / 2;
-#else
-    float* scratch = pair_smem + (SPT * NS + SCR * role) * TILE;  // this role's transposition buffer(s)
-    float* scratch2 = scratch + (SINGLE ? 0 : TILE);
+    float* scratch = pair_smem + (SPT * NS) * TILE + (2 * role) * SW;  // this role's ping-pong transposition buffers
+    float* scratch2 = scratch + SW;
     // half-stashes: X -> Y upper half of t2, Y -> X lower half of dt3
-    float* stash_t2 = ALIAS ? pair_smem + (SPT * NS) * TILE : pair_smem + (SPT * NS + 2 * SCR) * TILE;
-    float* stash_d3 = ALIAS ? pair_smem + (SPT * NS + SCR) * TILE : stash_t2 + TILE / 2;
-#endif
+    float* stash_t2 = pair_smem + (SPT * NS) * TILE + 4 * SW;
+    float* stash_d3 = stash_t2 + TILE / 2;
     const int bar_role = 1 + 3 * pair + role;
     const int bar_pair = 3 + 3 * pair;
     const float* __restrict__ gs = p.g + (int64_t(s) << k);
@@ -183,94 +162,44 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
     const float relu_thr = p.relu_in ? 0.f : -INFINITY;
 
     const uint32_t off_f = tile_thread_offset<N, C, V_FIRST>(tid);
-    const uint32_t off_l = tile_thread_offset<N, C, V_LAST>(tid);
     const uint32_t wb_fm = transpose_writer_base<N, C, V_FIRST, V_MID>(tid);
-    const uint32_t wb_ml = transpose_writer_base<N, C, V_MID, V_LAST>(tid);
-    const uint32_t wb_lm = transpose_writer_base<N, C, V_LAST, V_MID2>(tid);
-    const uint32_t wb_mf = ROUNDS == 3 ? transpose_writer_base<N, C, V_MID2, V_FIRST>(tid)
-                                       : transpose_writer_base<N, C, V_MID, V_FIRST>(tid);
-    const uint32_t mid_logical = view_tid_logical(view_mid(N, C), tid);  // ROUNDS == 2: this thread's MID-view index bits
-    uint32_t gbase = 0;
-    if constexpr (GTAB) {
-        gbase = gtab_base<N, C>(tid, k);
-        gtab_fill<N, C>(gt, gs, 2 * T * PAIRS, k);
-        __syncthreads();
-    }
+    const uint32_t wb_mf = transpose_writer_base<N, C, V_MID, V_FIRST>(tid);
+    const uint32_t mid_logical = view_tid_logical(view_mid(N, C), tid);  // this thread's MID-view index bits
     // stream -> middle layout (t2 / dt3) and back (t4 / dt1)
     auto to_mid = [&](float (&v)[E]) {
-        if constexpr (ROUNDS == 3) {
-            transform_in<N, C, KT, T, SINGLE>(v, scratch, scratch2, tid, bar_role, k, wb_fm, wb_ml);
-        } else {
-            bfly_round<N, C, KT, SEQ2_IN, 0>(v, k);
-            if constexpr (SINGLE) role_sync<T>(bar_role);
-            transpose_write<N, C, V_FIRST, V_MID>(v, scratch, wb_fm);
-            role_sync<T>(bar_role);
-            transpose_read<C>(v, scratch, tid);
-            bfly_round<N, C, KT, SEQ2_IN, 1>(v, k);
-        }
+        bfly_round<N, C, KT, SEQ2_IN, 0>(v, k);
+        transpose_write<N, C, V_FIRST, V_MID>(v, scratch, wb_fm);
+        role_sync<T>(bar_role);
+        transpose_read<C>(v, scratch, tid);
+        bfly_round<N, C, KT, SEQ2_IN, 1>(v, k);
     };
     auto from_mid = [&](float (&v)[E]) {
-        if constexpr (ROUNDS == 3) {
-            transform_out<N, C, KT, T, SINGLE>(v, scratch, scratch2, tid, bar_role, k, wb_lm, wb_mf);
-        } else {
-            bfly_round<N, C, KT, SEQ2_OUT, 0>(v, k);
-            if constexpr (SINGLE) role_sync<T>(bar_role);
-            transpose_write<N, C, V_MID, V_FIRST>(v, scratch2, wb_mf);
-            role_sync<T>(bar_role);
-            transpose_read<C>(v, scratch2, tid);
-            bfly_round<N, C, KT, SEQ2_OUT, 1>(v, k);
-        }
+        bfly_round<N, C, KT, SEQ2_OUT, 0>(v, k);
+        transpose_write<N, C, V_MID, V_FIRST>(v, scratch2, wb_mf);
+        role_sync<T>(bar_role);
+        transpose_read<C>(v, scratch2, tid);
+        bfly_round<N, C, KT, SEQ2_OUT, 1>(v, k);
     };
-    // g in the middle layout: once into registers (PREG) ...
+    // g in the middle layout, once into registers
     auto load_g_regs = [&](float* gr) {
-        if constexpr (ROUNDS == 3) {
-            for_each_vec<N, C, V_LAST>(off_l, cmask, [&](auto m_, uint32_t, uint32_t coord) {
-                constexpr int m = decltype(m_)::value;
-                const float4 w = ldg4(gs + coord);
-                gr[4 * m] = w.x, gr[4 * m + 1] = w.y, gr[4 * m + 2] = w.z, gr[4 * m + 3] = w.w;
-            });
-        } else {
-            static_for<0, E>([&](auto r_) {
-                constexpr int r = decltype(r_)::value;
-                constexpr uint32_t rl = view_reg_logical(view_mid(N, C), r);
-                gr[r] = __ldg(gs + ((mid_logical | rl) & cmask));
-            });
-        }
+        static_for<0, E>([&](auto r_) {
+            constexpr int r = decltype(r_)::value;
+            constexpr uint32_t rl = view_reg_logical(view_mid(N, C), r);
+            gr[r] = __ldg(gs + ((mid_logical | rl) & cmask));
+        });
     };
-    // ... or per tile from global memory (LAST view) / the shared-memory table (MID view)
     auto apply_g = [&](float (&v)[E], const float* gr) {
-        if constexpr (PREG) {
 #pragma unroll
-            for (int m = 0; m < E / 4; ++m) scale4(v + 4 * m, make_float4(gr[4 * m], gr[4 * m + 1], gr[4 * m + 2], gr[4 * m + 3]));
-        } else if constexpr (ROUNDS == 3) {
-            for_each_vec<N, C, V_LAST>(off_l, cmask, [&](auto m_, uint32_t, uint32_t coord) {
-                constexpr int m = decltype(m_)::value;
-                scale4(v + 4 * m, ldg4(gs + coord));
-            });
-        } else {
-            gtab_for_each<N, C>(gt, gbase, [&](auto j_, const float4 w) {
-                constexpr int j = decltype(j_)::value;
-                scale4(v + 4 * j, w);
-            });
-        }
+        for (int m = 0; m < E / 4; ++m) scale4(v + 4 * m, make_float4(gr[4 * m], gr[4 * m + 1], gr[4 * m + 2], gr[4 * m + 3]));
     };
     // this role's half of the dg partial sums -> workspace (registers [half*H, half*H + H))
     auto store_dg_half = [&](const float (&acc)[E / 2], int half_is_upper, float* dst) {
-        if constexpr (ROUNDS == 3) {
-            for_each_vec<N, C, V_LAST>(off_l, cmask, [&](auto m_, uint32_t off, uint32_t) {
-                constexpr int m = decltype(m_)::value;
-                constexpr int mh = m % (E / 8);
-                if ((m >= E / 8) == (half_is_upper != 0))
-                    *reinterpret_cast<float4*>(dst + off) = make_float4(acc[4 * mh], acc[4 * mh + 1], acc[4 * mh + 2], acc[4 * mh + 3]);
-            });
-        } else {
-            static_for<0, E / 2>([&](auto r_) {
-                constexpr int r = decltype(r_)::value;
-                constexpr uint32_t rl_lo = view_reg_logical(view_mid(N, C), r);
-                constexpr uint32_t rl_hi = view_reg_logical(view_mid(N, C), r + E / 2);
-                dst[mid_logical | (half_is_upper ? rl_hi : rl_lo)] = acc[r];
-            });
-        }
+        static_for<0, E / 2>([&](auto r_) {
+            constexpr int r = decltype(r_)::value;
+            constexpr uint32_t rl_lo = view_reg_logical(view_mid(N, C), r);
+            constexpr uint32_t rl_hi = view_reg_logical(view_mid(N, C), r + E / 2);
+            dst[mid_logical | (half_is_upper ? rl_hi : rl_lo)] = acc[r];
+        });
     };
     float* __restrict__ slab = p.ws + (((int64_t(s) * p.ctas_per_sample + cta_in_sample) * PAIRS + pair) * 4) * TILE;
     const uint32_t hs_base = tid << (C - 1);           // this thread's H floats in a half-stash
@@ -319,18 +248,16 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
 
     if (role == 0) {
         // ------------------------------------------------------------------ X role
-        // PREG: this thread's s2 and g values never change from tile to tile (its coordinates are
+        // this thread's s2 and g values never change from tile to tile (its coordinates are
         // fixed), so they are loaded once; each per-tile parameter load otherwise costs as many
         // L1 wavefronts as a raw-tile read, and the L1/shared data pipe is what bounds this kernel
-        float s2r[PREG ? E : 1], gr[PREG ? E : 1];
-        if constexpr (PREG) {
-            for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t, uint32_t coord) {
-                constexpr int m = decltype(m_)::value;
-                const float4 w = ldg4(s2p + coord);
-                s2r[4 * m] = w.x, s2r[4 * m + 1] = w.y, s2r[4 * m + 2] = w.z, s2r[4 * m + 3] = w.w;
-            });
-            load_g_regs(gr);
-        }
+        float s2r[E], gr[E];
+        for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t, uint32_t coord) {
+            constexpr int m = decltype(m_)::value;
+            const float4 w = ldg4(s2p + coord);
+            s2r[4 * m] = w.x, s2r[4 * m + 1] = w.y, s2r[4 * m + 2] = w.z, s2r[4 * m + 3] = w.w;
+        });
+        load_g_regs(gr);
         float acc_1[E];
         float acc_b[WANT_DBIAS ? E : 1];
 #pragma unroll
@@ -354,14 +281,12 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
             mbar_wait(&full_bar[pair][st], (it / NS) & 1);
             zero_tail(stage_x, left);
             float a[E];
-            for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t off, uint32_t coord) {
+            for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t off, uint32_t) {
                 constexpr int m = decltype(m_)::value;
                 const float4 q = raw4(stage_x, off);
-                const float4 w = PREG ? make_float4(s2r[4 * m], s2r[4 * m + 1], s2r[4 * m + 2], s2r[4 * m + 3]) : ldg4(s2p + coord);
-                mul4(a + 4 * m, q, w);
+                mul4(a + 4 * m, q, make_float4(s2r[4 * m], s2r[4 * m + 1], s2r[4 * m + 2], s2r[4 * m + 3]));
             });
             to_mid(a);  // a = t2 (middle layout)
-            if constexpr (ALIAS && SINGLE) role_sync<T>(bar_role);  // scratch (now the stash) is no longer being read
 #pragma unroll
             for (int jj = 0; jj < H / 4; ++jj)   // publish the upper half of t2
                 *reinterpret_cast<float4*>(stash_t2 + hs_base + ((jj ^ hs_swz) << 2)) =
@@ -397,19 +322,13 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
         store_dg_half(acc_g, 0, slab);
     } else {
         // ------------------------------------------------------------------ Y role
-        float s1r[PREG ? E : 1], s2r[PREG == 2 ? E : 1], gr[PREG ? E : 1];  // PREG == 2: s2 (for dx) as well
-        if constexpr (PREG) {
-            for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t, uint32_t coord) {
-                constexpr int m = decltype(m_)::value;
-                const float4 w = ldg4(s1p + coord);
-                s1r[4 * m] = w.x, s1r[4 * m + 1] = w.y, s1r[4 * m + 2] = w.z, s1r[4 * m + 3] = w.w;
-                if constexpr (PREG == 2) {
-                    const float4 u = ldg4(s2p + coord);
-                    s2r[4 * m] = u.x, s2r[4 * m + 1] = u.y, s2r[4 * m + 2] = u.z, s2r[4 * m + 3] = u.w;
-                }
-            });
-            load_g_regs(gr);
-        }
+        float s1r[E], gr[E];   // s2 (for dx) is read per tile
+        for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t, uint32_t coord) {
+            constexpr int m = decltype(m_)::value;
+            const float4 w = ldg4(s1p + coord);
+            s1r[4 * m] = w.x, s1r[4 * m + 1] = w.y, s1r[4 * m + 2] = w.z, s1r[4 * m + 3] = w.w;
+        });
+        load_g_regs(gr);
         float acc_2[E];
 #pragma unroll
         for (int i = 0; i < E; ++i) acc_2[i] = 0.f;
@@ -425,14 +344,12 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
             mbar_wait(&full_bar[pair][st], (it / NS) & 1);
             zero_tail(stage_x, left);
             float b[E];
-            for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t off, uint32_t coord) {
+            for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t off, uint32_t) {
                 constexpr int m = decltype(m_)::value;
                 const float4 q = to_dy(raw4(stage_dy, off), tgt, off, left);
-                const float4 w = PREG ? make_float4(s1r[4 * m], s1r[4 * m + 1], s1r[4 * m + 2], s1r[4 * m + 3]) : ldg4(s1p + coord);
-                mul4(b + 4 * m, q, w);
+                mul4(b + 4 * m, q, make_float4(s1r[4 * m], s1r[4 * m + 1], s1r[4 * m + 2], s1r[4 * m + 3]));
             });
             to_mid(b);  // b = dt3 (middle layout)
-            if constexpr (ALIAS && SINGLE) role_sync<T>(bar_role);
 #pragma unroll
             for (int jj = 0; jj < H / 4; ++jj)   // publish the lower half of dt3
                 *reinterpret_cast<float4*>(stash_d3 + hs_base + ((jj ^ hs_swz) << 2)) =
@@ -451,7 +368,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
             for_each_vec<N, C, V_FIRST>(off_f, cmask, [&](auto m_, uint32_t off, uint32_t coord) {
                 constexpr int m = decltype(m_)::value;
                 const float4 q = raw4(stage_x, off);
-                const float4 w = PREG == 2 ? make_float4(s2r[4 * m], s2r[4 * m + 1], s2r[4 * m + 2], s2r[4 * m + 3]) : ldg4(s2p + coord);
+                const float4 w = ldg4(s2p + coord);
                 fma4(acc_2 + 4 * m, q, b + 4 * m);
                 const float4 o = make_float4(q.x > relu_thr ? b[4 * m] * w.x : 0.f, q.y > relu_thr ? b[4 * m + 1] * w.y : 0.f,
                                              q.z > relu_thr ? b[4 * m + 2] * w.z : 0.f, q.w > relu_thr ? b[4 * m + 3] * w.w : 0.f);
@@ -468,7 +385,7 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, MINB) layer_bwd_tma_ke
 }
 
 // ------------------------------------------------------------------ backward, TMEM edition (round 2)
-// D >= 2048.  The three-view kernel above is bound by the L1/shared-memory data pipe (77% of its peak at 48% of
+// D >= 2048.  A three-view form of the kernel above is bound by the L1/shared-memory data pipe (77% of its peak at 48% of
 // the HBM roofline, profiles/r01_bwd_notes.md item 7): ~3260 wavefronts per 4096-element tile pair, and because
 // its single tile pair per SM runs all eight warps in lock-step, shared-memory phases and FP32 phases add up
 // instead of overlapping.  Two views (64 floats per thread, ONE transposition per transform) need 1024 + 512
@@ -738,14 +655,6 @@ __global__ void __launch_bounds__(256, 1) layer_bwd_tm_kernel(const BwdArgs p)
     const uint32_t col_pr = role ? COL_PR : COL_S2;
     if (role == 0 && tid == 0)
         for (int i = 0; i < NS - 1; ++i) issue_tile(i, pair);
-    // The CTA's tile pairs never synchronise with each other, but they start together and do identical work, so
-    // left alone they hit the shared-memory pipe at the same moments (all eight warps store, then all eight
-    // butterfly).  Starting the second pair a fraction of a phase late interleaves one pair's transpositions with the
-    // other's butterflies for the whole launch.
-    if (PAIRS > 1 && pair == 1 && p.stagger > 0) {
-        const long long t0 = clock64();
-        while (clock64() - t0 < p.stagger) {}
-    }
 #pragma unroll 1
     for (int it = 0; it < p.iters_per_group; ++it) {
         const int64_t e0 = tile_of(it, pair);
@@ -1027,18 +936,18 @@ int launch_bwd_reduce(float* ws, float* dg, float* ds1, float* ds2, float* dbias
     return check_launch("layer_bwd_reduce_fold_kernel");
 }
 
-template <int N, int C, int KT, int PAIRS, int MINB, int NS, bool SINGLE, bool ALIAS = false, int PREG = 0, int ROUNDS = 3>
+template <int N, int C, int KT>
 static int launch_bwd_tma_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
 {
     static unsigned char smem_ok[8][64] = {};
-    constexpr int threads = (2 << (N - C)) * PAIRS;
+    constexpr int T = 1 << (N - C);
+    constexpr int PAIRS = 128 / T;
     constexpr size_t tile = size_t(1) << N;
-    constexpr bool gtab = ROUNDS == 2 && !PREG;
     constexpr size_t sw = scratch_words(N, C);
-    constexpr size_t smem_plain = bwd_smem_bytes(N, PAIRS, NS, SINGLE, ALIAS, gtab, 2, sw);
-    constexpr size_t smem_tgt = bwd_smem_bytes(N, PAIRS, NS, SINGLE, ALIAS, gtab, 3, sw);  // RESID with the target staged
+    constexpr size_t smem_plain = bwd_smem_bytes(N, PAIRS, 2, sw);
+    constexpr size_t smem_tgt = bwd_smem_bytes(N, PAIRS, 3, sw);  // RESID with the target staged
     static_assert(smem_plain <= 227 * 1024, "backward kernel shared memory");
-    const size_t smem = (c.target != nullptr && bwd_stage_target(N, PAIRS, NS, SINGLE, ALIAS, gtab, MINB, sw)) ? smem_tgt : smem_plain;
+    const size_t smem = (c.target != nullptr && bwd_stage_target(N, PAIRS, sw)) ? smem_tgt : smem_plain;
     const int64_t D = int64_t(1) << k;
     const int64_t tiles_per_sample = (c.B * D + int64_t(tile) - 1) / int64_t(tile);
     const Plan plan = make_plan_waves(c.S, tiles_per_sample, PAIRS, 148, 8, 8);
@@ -1057,24 +966,22 @@ static int launch_bwd_tma_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
     a.pstride = static_cast<int>(c.pstride);
     auto go = [&](auto kernel, int slot) -> int {
         if (int rc = ensure_smem(kernel, smem, smem_ok[slot])) return rc;
-        kernel<<<static_cast<unsigned>(ctas), threads, smem, stream>>>(a);
+        kernel<<<static_cast<unsigned>(ctas), 256, smem, stream>>>(a);
         return check_launch("layer_bwd_tma_kernel");
     };
     const bool db = c.dbias != nullptr, rs = c.target != nullptr;
     int rc;
     if (c.bf16) {
         if (rs) return fail(WHVI_E_MODE, "layer_bwd: bf16 activations cannot be combined with a target");
-        // D >= 2048 runs the tensor-memory kernel; these configurations serve WHVI_BWD_LEGACY builds, which take fp32 only
-        if constexpr (N > 10) return fail(WHVI_E_MODE, "layer_bwd: bf16 activations at D = %lld need the tensor-memory backward", (long long)D);
-        else if (c.dx_f32)
-            rc = db ? go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, false, __nv_bfloat16, float>, 6)
-                    : go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, false, false, __nv_bfloat16, float>, 7);
-        else rc = db ? go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, false, __nv_bfloat16>, 4)
-                     : go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, false, false, __nv_bfloat16>, 5);
-    } else if (db && rs) rc = go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, true>, 0);
-    else if (db) rc = go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, true, false>, 1);
-    else if (rs) rc = go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, false, true>, 2);
-    else rc = go(layer_bwd_tma_kernel<N, C, KT, PAIRS, MINB, NS, SINGLE, ALIAS, PREG, ROUNDS, false, false>, 3);
+        if (c.dx_f32)
+            rc = db ? go(layer_bwd_tma_kernel<N, C, KT, true, false, __nv_bfloat16, float>, 6)
+                    : go(layer_bwd_tma_kernel<N, C, KT, false, false, __nv_bfloat16, float>, 7);
+        else rc = db ? go(layer_bwd_tma_kernel<N, C, KT, true, false, __nv_bfloat16>, 4)
+                     : go(layer_bwd_tma_kernel<N, C, KT, false, false, __nv_bfloat16>, 5);
+    } else if (db && rs) rc = go(layer_bwd_tma_kernel<N, C, KT, true, true>, 0);
+    else if (db) rc = go(layer_bwd_tma_kernel<N, C, KT, true, false>, 1);
+    else if (rs) rc = go(layer_bwd_tma_kernel<N, C, KT, false, true>, 2);
+    else rc = go(layer_bwd_tma_kernel<N, C, KT, false, false>, 3);
     if (rc) return rc;
     return launch_bwd_reduce(c.ws, c.dg, c.ds1, c.ds2, c.dbias, c.S, plan.ctas_per_sample * PAIRS, int64_t(tile), D, stream, c.groups);
 }
@@ -1104,8 +1011,6 @@ static int launch_bwd_tm_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
               c.relu_in, c.target, c.coef, c.dy_scale};
     a.spg = static_cast<int>(c.S / c.groups);
     a.pstride = static_cast<int>(c.pstride);
-    static const int stagger = [] { const char* e = std::getenv("WHVI_BWD_STAGGER"); return e ? std::atoi(e) : 0; }();
-    a.stagger = stagger;
     auto go = [&](auto kernel, int slot) -> int {
         if (int rc = ensure_smem(kernel, smem, smem_ok[slot])) return rc;
         kernel<<<static_cast<unsigned>(ctas), 256, smem, stream>>>(a);
@@ -1131,28 +1036,16 @@ static int launch_bwd_tm_cfg(const LayerBwdCall& c, int k, cudaStream_t stream)
 int launch_layer_bwd(const LayerBwdCall& c, int64_t D, cudaStream_t stream)
 {
     const int k = ilog2(D);
-    // TMA-staged kernels, one CTA per SM, NS = 2 stages, ping-pong transposition buffers where
-    // they fit, parameters register-resident where the register file allows.
-    // D <= 1024: two views (FIRST + MID cover all 10 tile bits), one warp per role, 4 pairs per CTA
-    if (k >= 2 && k <= 6) return launch_bwd_tma_cfg<10, 5, k_family(2, 6), 4, 1, 2, false, false, 1, 2>(c, k, stream);
-    if (k >= 7 && k <= 9) return launch_bwd_tma_cfg<10, 5, k_family(7, 9), 4, 1, 2, false, false, 1, 2>(c, k, stream);
-    if (k == 10) return launch_bwd_tma_cfg<10, 5, 10, 4, 1, 2, false, false, 1, 2>(c, k, stream);
-    // D >= 2048: three views (a 64-float-per-thread two-view variant measured slower at D = 4096:
-    // 1.16 ms vs 1.08 ms -- too few warps and no room for register-resident parameters)
-#ifndef WHVI_BWD_LEGACY   // -DWHVI_BWD_LEGACY=1: round 1's three-view register-only kernels (A/B builds)
+    // D <= 1024: TMA-staged kernels, one CTA per SM, NS = 2 stages, ping-pong transposition buffers, parameters
+    // register-resident, two views (FIRST + MID cover all 10 tile bits), one warp per role, 4 pairs per CTA
+    if (k >= 2 && k <= 6) return launch_bwd_tma_cfg<10, 5, k_family(2, 6)>(c, k, stream);
+    if (k >= 7 && k <= 9) return launch_bwd_tma_cfg<10, 5, k_family(7, 9)>(c, k, stream);
+    if (k == 10) return launch_bwd_tma_cfg<10, 5, 10>(c, k, stream);
     // D = 2048, 4096: two views, 64 floats per thread, running sums / g / role exchange in tensor memory
     if (k == 11) return launch_bwd_tm_cfg<12, 6, 11, 2>(c, k, stream);
     if (k == 12) return launch_bwd_tm_cfg<12, 6, 12, 2>(c, k, stream);
     // D = 8192: three views, 64 floats per thread, one tile pair per CTA, same tensor-memory residency
     if (k == 13) return launch_bwd_tm_cfg<13, 6, 13, 3>(c, k, stream);
-#endif
-    if (k == 11) return launch_bwd_tma_cfg<11, 5, 11, 2, 1, 2, false, false, 2, 3>(c, k, stream);
-    if (k == 12) return launch_bwd_tma_cfg<12, 5, 12, 1, 1, 2, false, false, 2, 3>(c, k, stream);
-#if WHVI_PADDED  // the padded scratch does not fit next to a stash tile of its own at D = 8192: alias the stash
-    if (k == 13) return launch_bwd_tma_cfg<13, 5, 13, 1, 1, 2, true, true, 0, 3>(c, k, stream);
-#else
-    if (k == 13) return launch_bwd_tma_cfg<13, 5, 13, 1, 1, 2, true, false, 0, 3>(c, k, stream);
-#endif
     return fail(WHVI_E_SHAPE, "layer_bwd: D = %lld unsupported (4 <= D <= 8192)", (long long)D);
 }
 

@@ -276,12 +276,8 @@ int launch_layer_fwd(const LayerFwdCall& c, int64_t D, cudaStream_t stream)
     if (k == 12) return launch_fwd_cfg<12, 6, 12, 2, 2, 1, 4>(c, k, stream);
     // D = 8192: three views, 32 floats per thread
     // D = 8192: three views, 64 floats per thread, one in-place buffer, 4 CTAs of 128 threads per
-    // SM (measured 68% of the HBM roofline vs 60% for 32 floats/thread with ping-pong buffers)
-#if WHVI_FWD_SPLIT_8192   // -DWHVI_FWD_SPLIT_8192=1 (A/B builds): layer_fwd_split.cu -- two 4096-float halves through the two-view
-    // engine with the other half parked in tensor memory.  Correct (whole GPU suite) but measured SLOWER than the three-view
-    // kernel below: 62% vs 68% of the HBM roofline (86% vs 99% with FROM_T2), profiles/r02_fwd_split_8192.md
-    if (k == 13) return launch_layer_fwd_split(c, stream);
-#endif
+    // SM (measured 68% of the HBM roofline vs 60% for 32 floats/thread with ping-pong buffers; two 4096-float halves
+    // through the two-view engine with the other half in tensor memory measured 62%, profiles/r02_fwd_split_8192.md)
     if (k == 13) return launch_fwd_cfg<13, 6, 13, 1, 3, 1, 4>(c, k, stream);
     // D = 16384, 32768 (forward only: MC predictive evaluation, BASELINE config 5): three views,
     // 64 floats per thread, one in-place transposition buffer (64 / 128 KB)

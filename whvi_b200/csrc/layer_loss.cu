@@ -24,15 +24,10 @@
 // released by Y one tile ago, so it does not stall, and the copy still has a whole tile of lead
 // time.  (With 2 stages and the refill at the start of an iteration X waits for Y and the two
 // roles serialise: measured 2x slower.)
-// The transposition buffers of THIS translation unit use the padded (XOR-free) layout (WHVI_PADDED_BWD, default 1;
-// measured: the backward gains ~4% at D = 1024...8192 with bit-identical outputs, the two-view forward does not,
-// profiles/r01_bwd_notes.md item 14, profiles/r02_ab_padbwd.txt); -DWHVI_PADDED_BWD=0 builds the swizzled variant.
-#ifndef WHVI_PADDED_BWD
-#define WHVI_PADDED_BWD 1   // product default since round 2: bit-identical outputs, -4% (profiles/r02_ab_padbwd.txt)
-#endif
-#if WHVI_PADDED_BWD && !defined(WHVI_PADDED)
+// The transposition buffers of THIS translation unit use the padded (XOR-free) layout, as layer_bwd.cu does: the backward
+// gains ~4% at D = 1024...8192 over the swizzled one with bit-identical outputs (profiles/r01_bwd_notes.md item 14,
+// profiles/r02_ab_padbwd.txt).
 #define WHVI_PADDED 1
-#endif
 #include "layer_common.cuh"
 
 namespace whvi {
@@ -47,9 +42,8 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, 1) layer_loss_kernel(c
     constexpr int E = 1 << C;
     constexpr int64_t TILE = int64_t(1) << N;
     constexpr int SCR = SINGLE ? 1 : 2;
-    constexpr int SW = int(scratch_words(N, C));  // one transposition buffer (== TILE unless WHVI_PADDED)
-    constexpr int PAIR_FLOATS = WHVI_PADDED ? (2 * NS + NS) * int(TILE) + 2 * SCR * SW
-                                            : (2 * NS + 2 * SCR + NS) * int(TILE);  // stages, scratch, one full t2 stash per stage
+    constexpr int SW = int(scratch_words(N, C));  // one transposition buffer
+    constexpr int PAIR_FLOATS = (2 * NS + NS) * int(TILE) + 2 * SCR * SW;  // stages, one full t2 stash per stage, scratch
     static_assert(ROUNDS == 3 || rounds_needed(N, C, N) <= 2, "2-view kernel needs FIRST+MID to cover all bits");
     static_assert(rounds_needed(N, C, N) <= 3, "FIRST+MID+LAST must cover every tile bit");
     static_assert(ROUNDS == 3 || PREG > 0, "the 2-view loss kernel keeps g in registers");
@@ -101,15 +95,9 @@ __global__ void __launch_bounds__((2 << (N - C)) * PAIRS, 1) layer_loss_kernel(c
     const int pair = (threadIdx.x % (T * PAIRS)) / T;
     const uint32_t tid = threadIdx.x % T;
     float* pair_smem = smem + size_t(pair) * PAIR_FLOATS;
-#if WHVI_PADDED
     float* scratch = pair_smem + (2 * NS) * TILE + (SCR * role) * SW;
     float* scratch2 = scratch + (SINGLE ? 0 : SW);
     float* stash0 = pair_smem + (2 * NS) * TILE + 2 * SCR * SW;       // + st * TILE
-#else
-    float* scratch = pair_smem + (2 * NS + SCR * role) * TILE;
-    float* scratch2 = scratch + (SINGLE ? 0 : TILE);
-    float* stash0 = pair_smem + (2 * NS + 2 * SCR) * TILE;       // + st * TILE
-#endif
     const int bar_role = 1 + 2 * pair + role;
     const float* __restrict__ gs = p.g + (int64_t(s) << k);
     const float relu_thr = p.relu_in ? 0.f : -INFINITY;
@@ -379,7 +367,6 @@ static int launch_loss_cfg(const LayerLossCall& c, int k, cudaStream_t stream)
 int launch_layer_loss(const LayerLossCall& c, int64_t D, cudaStream_t stream)
 {
     const int k = ilog2(D);
-#ifndef WHVI_LOSS_LEGACY   // -DWHVI_LOSS_LEGACY=1: round 1's three-view register-only kernel at D = 2048, 4096 (A/B builds)
     if ((k == 11 || k == 12) && c.need_ws) {
         // size query: the caller does not say whether there will be a bias, and the two kernels split the work
         // differently -> report the larger of each (unused sq_partials entries must be zero: see whvi_b200.h)
@@ -397,7 +384,6 @@ int launch_layer_loss(const LayerLossCall& c, int64_t D, cudaStream_t stream)
         return WHVI_OK;
     }
     if ((k == 11 || k == 12) && c.bias == nullptr) return launch_layer_loss_tm(c, D, stream);
-#endif
     if (k >= 7 && k <= 9) return launch_loss_cfg<10, 5, k_family(7, 9), 4, 3, false, 1, 2>(c, k, stream);
     if (k == 10) return launch_loss_cfg<10, 5, 10, 4, 3, false, 1, 2>(c, k, stream);
     if (k == 11) return launch_loss_cfg<11, 5, 11, 2, 3, false, 1, 3>(c, k, stream);

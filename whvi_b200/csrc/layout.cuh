@@ -29,12 +29,13 @@
 #define WHVI_HD inline
 #endif
 
-// WHVI_PADDED=1 (variant builds only: python -m whvi_b200.build --variant padded -DWHVI_PADDED=1):
+// WHVI_PADDED=1 (defined by layer_bwd.cu and layer_loss.cu before they include this file):
 // the reader-owned transposition layout without the XOR swizzle -- thread tid' owns E + 4 words at
 // tid' * (E + 4), register r at word r.  Conflict-free on both sides like the swizzle
 // (tools/sim_layout.cpp proves it for every transposition in use) and every address is a thread
-// base plus a compile-time constant (no LOP3 per access), at 12.5% more scratch.  Not measured yet
-// (DESIGN.md section 9); the product library is always built with WHVI_PADDED=0.
+// base plus a compile-time constant (no LOP3 per access), at 12.5% more scratch.  Measured ~4% faster
+// in the backward and no faster in the two-view forward (profiles/r02_ab_padbwd.txt), so the other
+// translation units keep the swizzled layout.
 #ifndef WHVI_PADDED
 #define WHVI_PADDED 0
 #endif
